@@ -5,6 +5,7 @@ table, SA ratio 8.
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU algorithm (oracle port)
+    python bench.py ... --dump-outputs DIR                    # also writes the headline counts for comparing builds
 
 One process per GPU (torchrun for N > 1); the index is replicated per GPU, every rank searches its
 own 10 M-read batch (weak scaling), no collective on the data path.  A "step" is one pass of the hot
@@ -38,6 +39,8 @@ os.environ.setdefault("AWRY_B200_LEAN_SA", "1")
 TEXT_SEED = 3          # BASELINE.md cfg2
 QUERY_SEED = 4
 ALG_BYTES_PER_BLOCK = 104   # SURVEY.md 8(d): 3 x 32 B planes + one 8-B milestone per rank-block access
+DUMP_ROWS = 1 << 21         # --dump-outputs: 2 x 16 MB of float64 at most
+DUMP_SEED = 5
 
 
 def parse_args():
@@ -65,7 +68,25 @@ def parse_args():
     ap.add_argument("--no-inprocess", action="store_true", help="N > 1: skip rank 0's one-call-over-N-replicas leg")
     ap.add_argument("--cfg4-len", type=int, default=2_000_000_000)
     ap.add_argument("--cfg5-len", type=int, default=1_000_000_000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the counts of the headline leg's last step (rank 0's batch) to "
+                         "DIR/counts.npy and the reads they belong to to DIR/count_rows.npy, both float64; batches above "
+                         f"{DUMP_ROWS} reads are sampled with a fixed seed")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "awry_b200":
+        ap.error("--dump-outputs writes the outputs of --impl awry_b200")
+    return a
+
+
+def dump_counts(out_dir, counts):
+    """--dump-outputs: the per-read counts a caller of the headline path receives, as float64 (exact below 2**53).
+    The same arguments give the same reads, so two builds can be compared file for file."""
+    n = len(counts)
+    rows = np.arange(n)
+    if n > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+    np.save(os.path.join(out_dir, "counts.npy"), counts[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "count_rows.npy"), rows.astype(np.float64))
 
 
 def dist_env():
@@ -602,6 +623,8 @@ def main():
     if a.impl == "reference":
         return run_reference(a)
     rank, local_rank, world = dist_env()
+    if a.dump_outputs and rank == 0:
+        os.makedirs(a.dump_outputs, exist_ok=True)     # fail before the set-up, not after the timed steps
     import torch
     import torch.distributed as dist
     if not torch.cuda.is_available():
@@ -666,6 +689,8 @@ def main():
     prof = f.profile_get()
     f.profile_enable(False)
     ix.device_check(stream)
+    if a.dump_outputs and rank == 0:
+        dump_counts(a.dump_outputs, d_cnt.cpu().numpy().view(np.uint64))
     t_ms = torch.tensor([ms_total], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
