@@ -1123,6 +1123,244 @@ void locate_into_impl(const awry_index* ix, const QuerySource& qs, uint64_t nq, 
   free(tmp);
 }
 
+// ------------------------------------------------------------------ Hamming search (awry_*_hamming)
+
+// stream-ordered device allocations of one call or slice, released in stream order when it goes out of scope
+struct StreamScratch {
+  cudaStream_t st;
+  std::vector<void*> ptrs;
+  explicit StreamScratch(cudaStream_t s) : st(s) {}
+  ~StreamScratch() {
+    for (void* p : ptrs) cudaFreeAsync(p, st);
+  }
+  template <class T>
+  T* get(uint64_t n) {
+    void* p = nullptr;
+    const cudaError_t e = cudaMallocAsync(&p, size_t(n) * sizeof(T) + 16, st);
+    if (e == cudaErrorMemoryAllocation) {
+      cudaGetLastError();
+      fail(AWRY_ERR_NOMEM, "out of device memory for %llu bytes of Hamming-search scratch",
+           (unsigned long long)(n * sizeof(T)));
+    }
+    CU(e);
+    ptrs.push_back(p);
+    return static_cast<T*>(p);
+  }
+};
+
+// candidates verified per slice (AWRY_B200_HAMMING_SLICE, read per call): bounds the scratch of the verification
+static uint64_t hamming_slice() {
+  if (const char* e = getenv("AWRY_B200_HAMMING_SLICE"))
+    return std::min<uint64_t>(1ull << 30, std::max<uint64_t>(16, strtoull(e, nullptr, 10)));
+  return 1ull << 26;
+}
+
+void hamming_check_index(const awry_index* ix) {
+  if (ix->alphabet != AWRY_NUCLEOTIDE) fail(AWRY_ERR_UNSUPPORTED, "Hamming search exists for the nucleotide alphabet only");
+  for (auto& rp : ix->reps)
+    if (rp->view.wide || !rp->view.rtext || !rp->view.full_sa)
+      fail(AWRY_ERR_UNSUPPORTED,
+           "Hamming search needs the unsampled suffix array and the text on every device (not built for this index: "
+           "AWRY_B200_FULL_SA / AWRY_B200_TEXT, device memory, or 64-bit row pointers)");
+}
+
+// the hits of the locate call on one replica, in query order
+struct HammingSink {
+  std::vector<uint64_t> off;  // per query: offset of its first hit in `hits`
+  std::vector<awry_hit> hits;
+  std::vector<uint8_t> dist;
+};
+
+// One batch of reads on one replica, all on stream `st`: pieces -> exact search of the pieces -> candidates ->
+// verification against the text, in slices of at most hamming_slice() candidates.  Offsets are absolute and lie
+// in [b_lo, b_hi] (d_qbytes is biased accordingly).  Count: d_counts (nq * (k + 1)) is zeroed and filled.  Locate:
+// the hits are appended to `sink` (slices cut at read boundaries, the hits of a read sorted by text position).
+// `check_base` >= 0: a refused read fails the call (reported as read check_base + q) before anything is verified;
+// < 0 (the device-resident call): it stays latched in *d_flag for awry_device_check.
+void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+                 uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
+                 HammingSink* sink) {
+  const uint64_t P = k + 1, np = nq * P, nbytes = b_hi - b_lo;
+  if (np >= (1ull << 31)) fail(AWRY_ERR_INVALID_ARG, "batch too large for one Hamming search (%llu reads): split it", (unsigned long long)nq);
+  StreamScratch sc(st);
+  // 1. pieces, packed; the whole reads packed too (their prepass validates the offsets and latches what it refuses)
+  uint64_t* d_poff = sc.get<uint64_t>(np + 1);
+  unsigned long long* d_pflag = sc.get<unsigned long long>(1);  // (piece indices: what it latches is reported per read)
+  CU(cudaMemsetAsync(d_pflag, 0xff, 8, st));
+  CU(launch_hamming_pieces(d_qoff, nq, k, b_lo, b_hi, d_poff, d_flag, st));
+  const uint64_t pw_n = packed_words(0, np, nbytes), rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
+  uint64_t* const d_pw = sc.get<uint64_t>(pw_n) - w_lo;
+  uint64_t* const d_rw = sc.get<uint64_t>(rw_n) - w_lo;
+  {
+    ProfScope p(2, r.device, st);
+    CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_poff, np, d_pw, b_lo, b_hi, d_pflag, st));
+    CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
+  }
+  // 2. exact search of the pieces (the wave kernel stores a piece finished in the text as its position), CSR
+  // offsets of their occurrences = the candidates
+  uint2* d_sp = sc.get<uint2>(np);
+  {
+    ProfScope p(0, r.device, st);
+    SearchVariant v = current_variant();
+    v.avg_len = uint32_t(std::min<uint64_t>(nbytes / np, 1u << 30));
+    v.b_lo = b_lo;
+    v.b_hi = b_hi;
+    v.locate_positions = locate_positions_ok(r.view, v);
+    CU(launch_search(r.view, d_pw, d_poff, np, OUT_SP_CNT_U32, d_sp, sc.get<uint32_t>(defer_words(np)), v, r.sm_count, st));
+  }
+  uint64_t* d_hoff = sc.get<uint64_t>(np + 1);
+  size_t temp = 0;
+  CU(scan_hit_offsets(r.view, d_sp, np, d_hoff, nullptr, temp, st));
+  CU(scan_hit_offsets(r.view, d_sp, np, d_hoff, sc.get<uint8_t>(temp), temp, st));
+  // the candidate total (and, for locate, every read's candidate range) sizes the slices: one synchronisation
+  uint64_t total = 0;
+  unsigned long long flag = ~0ull;
+  std::vector<uint64_t> qcand;
+  uint64_t* d_qcand = nullptr;
+  if (sink) {
+    d_qcand = sc.get<uint64_t>(nq + 1);
+    CU(launch_hamming_query_bounds(d_hoff, k, nq, d_qcand, st));
+    qcand.resize(nq + 1);
+    CU(cudaMemcpyAsync(qcand.data(), d_qcand, (nq + 1) * 8, cudaMemcpyDeviceToHost, st));
+    g_prof.d2h += (nq + 1) * 8;
+  }
+  CU(cudaMemcpyAsync(&total, d_hoff + np, 8, cudaMemcpyDeviceToHost, st));
+  if (check_base >= 0) CU(cudaMemcpyAsync(&flag, d_flag, 8, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (flag != ~0ull && (flag & 1) == BAD_QUERY)
+    fail(AWRY_ERR_INVALID_QUERY,
+         "query %llu is empty, contains a sentinel ('$'/'#') or is not longer than max_mismatches = %u (every window "
+         "would match)", (unsigned long long)(uint64_t(check_base) + (flag >> 1)), k);
+  if (flag != ~0ull) fail_bad_query(flag, uint64_t(check_base));
+
+  HammingSlice a{};
+  a.qwords = d_rw;
+  a.qw_lo = w_lo;
+  a.qw_n = rw_n;
+  a.qoff = d_qoff;
+  a.b_lo = b_lo;
+  a.b_hi = b_hi;
+  a.sp_cnt = d_sp;
+  a.hoff = d_hoff;
+  a.npieces = np;
+  const uint64_t S = hamming_slice();
+  if (!sink) {  // 3. count: slices cut anywhere
+    CU(cudaMemsetAsync(d_counts, 0, nq * P * 8, st));
+    for (uint64_t c0 = 0; c0 < total; c0 += S) {
+      StreamScratch ss(st);
+      a.c0 = c0;
+      a.n = std::min(S, total - c0);
+      uint32_t* d_map = ss.get<uint32_t>(a.n);
+      CU(launch_hamming_map(d_hoff, np, c0, a.n, d_map, nullptr, temp, st));
+      CU(launch_hamming_map(d_hoff, np, c0, a.n, d_map, ss.get<uint8_t>(temp), temp, st));
+      a.map = d_map;
+      a.counts = d_counts;
+      ProfScope p(1, r.device, st);
+      CU(launch_hamming_verify(r.view, a, k, false, r.sm_count, st));
+    }
+    return;
+  }
+  // 3. locate: slices cut at read boundaries (a read with more candidates than a slice gets one of its own size)
+  sink->off.reserve(sink->off.size() + nq);
+  for (uint64_t q0 = 0; q0 < nq;) {
+    uint64_t q1 = q0 + 1;
+    while (q1 < nq && qcand[q1 + 1] - qcand[q0] <= S) q1++;
+    const uint64_t c0 = qcand[q0], n = qcand[q1] - c0, nr = q1 - q0;
+    if (n >= (1ull << 31))  // (a slice is sorted per read by one CUB call, whose offsets are int)
+      fail(AWRY_ERR_NOMEM, "query %llu has %llu candidate windows, more than one slice can sort (2^31)",
+           (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + q0), (unsigned long long)n);
+    const uint64_t base = sink->hits.size();
+    if (n == 0) {
+      sink->off.insert(sink->off.end(), nr, base);
+      q0 = q1;
+      continue;
+    }
+    StreamScratch ss(st);
+    a.c0 = c0;
+    a.n = n;
+    a.q0 = q0;
+    uint32_t* d_map = ss.get<uint32_t>(n);
+    CU(launch_hamming_map(d_hoff, np, c0, n, d_map, nullptr, temp, st));
+    CU(launch_hamming_map(d_hoff, np, c0, n, d_map, ss.get<uint8_t>(temp), temp, st));
+    a.map = d_map;
+    a.keys = ss.get<uint64_t>(n);
+    a.acc = ss.get<uint64_t>(nr + 1);
+    CU(cudaMemsetAsync(a.acc, 0, (nr + 1) * 8, st));
+    {
+      ProfScope p(1, r.device, st);
+      CU(launch_hamming_verify(r.view, a, k, true, r.sm_count, st));
+    }
+    uint64_t* d_sorted = ss.get<uint64_t>(n);
+    size_t t2 = 0;
+    CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, nullptr, t2, st));
+    CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, ss.get<uint8_t>(t2), t2, st));
+    uint64_t* d_qh = ss.get<uint64_t>(nr + 1);
+    size_t t3 = 0;
+    CU(scan_u64(a.acc, d_qh, nr + 1, nullptr, t3, st));
+    CU(scan_u64(a.acc, d_qh, nr + 1, ss.get<uint8_t>(t3), t3, st));
+    std::vector<uint64_t> qh(nr + 1);
+    CU(cudaMemcpyAsync(qh.data(), d_qh, (nr + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const uint64_t n_acc = qh[nr];
+    if (n_acc) {
+      uint64_t* d_pos = ss.get<uint64_t>(n_acc);
+      uint8_t* d_dist = ss.get<uint8_t>(n_acc);
+      uint64_t* d_hits = ss.get<uint64_t>(2 * n_acc);
+      CU(launch_hamming_compact(d_sorted, d_map, n, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
+      CU(launch_map_locations(r.view, d_pos, n_acc, d_hits, st));
+      sink->hits.resize(base + n_acc);
+      sink->dist.resize(base + n_acc);
+      CU(cudaMemcpyAsync(sink->hits.data() + base, d_hits, n_acc * 16, cudaMemcpyDeviceToHost, st));
+      CU(cudaMemcpyAsync(sink->dist.data() + base, d_dist, n_acc, cudaMemcpyDeviceToHost, st));
+      g_prof.d2h += n_acc * 17;
+      CU(cudaStreamSynchronize(st));
+    }
+    for (uint64_t i = 0; i < nr; i++) sink->off.push_back(base + qh[i]);
+    q0 = q1;
+  }
+}
+
+// reads [lo, hi) of host buffers on replica ri: chunks of reads uploaded and searched one after the other (the
+// host path does not overlap copies with compute yet)
+void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo,
+                        uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink) {
+  if (lo >= hi) return;
+  Replica& r = *ix->reps[ri];
+  DeviceGuard dg(r.device);
+  const uint64_t max_bytes = std::min(chunk_max_bytes(), locate_chunk_bytes());
+  if (qoff[hi] < qoff[lo]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone (queries %llu..%llu)",
+                                (unsigned long long)lo, (unsigned long long)hi);
+  auto chunks = make_chunks(qoff, lo, hi, locate_chunk_q(), max_bytes);
+  validate_chunks(chunks, max_bytes);
+  Workspace* ws = r.acquire();
+  try {
+    for (const Chunk& c : chunks) {
+      const uint64_t n = c.q1 - c.q0, nbytes = c.b1 - c.b0;
+      Workspace::grow_dev(ws->d_qbytes, ws->d_qbytes_cap, size_t(nbytes) + 16);
+      Workspace::grow_dev(ws->d_qoff, ws->d_qoff_cap, size_t(n) + 1);
+      if (nbytes) CU(cudaMemcpyAsync(ws->d_qbytes, qbytes + c.b0, nbytes, cudaMemcpyHostToDevice, ws->st));
+      CU(cudaMemcpyAsync(ws->d_qoff, qoff + c.q0, (n + 1) * 8, cudaMemcpyHostToDevice, ws->st));
+      g_prof.h2d += nbytes + (n + 1) * 8;
+      CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
+      if (sink) {
+        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr, sink);
+      } else {
+        StreamScratch sc(ws->st);
+        uint64_t* d_counts = sc.get<uint64_t>(n * (k + 1));
+        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts, nullptr);
+        CU(cudaMemcpyAsync(counts + c.q0 * (k + 1), d_counts, n * (k + 1) * 8, cudaMemcpyDeviceToHost, ws->st));
+        g_prof.d2h += n * (k + 1) * 8;
+      }
+      CU(cudaStreamSynchronize(ws->st));
+    }
+  } catch (...) {
+    cudaStreamSynchronize(ws->st);
+    r.release(ws);
+    throw;
+  }
+  r.release(ws);
+}
+
 }  // namespace host
 }  // namespace awry
 
@@ -1285,6 +1523,81 @@ int awry_locate_device(const awry_index* ix, int replica, const uint8_t* d_qbyte
       throw;
     }
     r.release(ws);
+  });
+}
+
+int awry_count_batch_hamming(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                             uint32_t max_mismatches, uint64_t* counts) {
+  return guarded([&] {
+    need(ix);
+    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+    if (nq == 0) return;
+    if (!qbytes || !qoff || !counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    hamming_check_index(ix);
+    for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
+      hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, max_mismatches, counts, nullptr);
+    });
+  });
+}
+
+int awry_locate_batch_hamming(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                              uint32_t max_mismatches, uint64_t* hit_off, awry_hit* hits, uint8_t* hit_mismatches,
+                              uint64_t capacity, uint64_t* n_hits) {
+  return guarded([&] {
+    need(ix);
+    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+    if (!hit_off || !n_hits || (!hits && capacity)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    *n_hits = 0;
+    hit_off[0] = 0;
+    if (nq == 0) return;
+    if (!qbytes || !qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    hamming_check_index(ix);
+    const size_t nr = ix->reps.size();
+    std::vector<HammingSink> sinks(nr);
+    std::vector<std::pair<uint64_t, uint64_t>> ranges(nr, {0, 0});
+    for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
+      ranges[ri] = {lo, hi};
+      hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, max_mismatches, nullptr, &sinks[ri]);
+    });
+    // the replicas' CSRs, concatenated in range order; hits past `capacity` are dropped (the total still counts them)
+    uint64_t total = 0;
+    for (size_t ri = 0; ri < nr; ri++) {
+      const auto [lo, hi] = ranges[ri];
+      const HammingSink& s = sinks[ri];
+      for (uint64_t i = 0; i < hi - lo; i++) hit_off[lo + i] = total + s.off[i];
+      const uint64_t n = s.hits.size(), fit = capacity > total ? std::min(n, capacity - total) : 0;
+      if (fit) {
+        memcpy(hits + total, s.hits.data(), fit * sizeof(awry_hit));
+        if (hit_mismatches) memcpy(hit_mismatches + total, s.dist.data(), fit);
+      }
+      total += n;
+    }
+    hit_off[nq] = total;
+    *n_hits = total;
+    if (total > capacity)
+      fail(AWRY_ERR_CAPACITY, "hit buffer holds %llu entries, %llu needed", (unsigned long long)capacity,
+           (unsigned long long)total);
+  });
+}
+
+int awry_count_device_hamming(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                              uint64_t nq, uint32_t max_mismatches, uint64_t* d_counts, void* cuda_stream) {
+  return guarded([&] {
+    need(ix);
+    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+    if (nq == 0) return;
+    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    hamming_check_index(ix);
+    Replica& r = *ix->reps[size_t(replica)];
+    DeviceGuard dg(r.device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    uint64_t ends[2] = {0, 0};
+    CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
+    hamming_run(r, d_qbytes, d_qoff, nq, ends[0], ends[1], max_mismatches, r.d_async_flag, -1, st, d_counts, nullptr);
   });
 }
 

@@ -154,6 +154,42 @@ cudaError_t sort_hit_segments(uint64_t* d_locs_in, uint64_t* d_locs_out, uint64_
 cudaError_t launch_map_locations(const IndexView& ix, const uint64_t* d_locs, uint64_t n_hits,
                                  uint64_t* d_hits_pairs, cudaStream_t s);
 
+// ---- kernels_hamming.cu: Hamming search (<= k substitutions) by k + 1 exactly searched pieces per read
+// piece offsets (k+1) nq + 1 of a batch; a query with L <= k is latched in *d_first_bad as BAD_QUERY
+cudaError_t launch_hamming_pieces(const uint64_t* d_qoff, uint64_t nq, uint32_t k, uint64_t b_lo, uint64_t b_hi,
+                                  uint64_t* d_poff, unsigned long long* d_first_bad, cudaStream_t s);
+// d_qcand[i] = d_hoff[(k+1) i] for i = 0 .. nq (candidate range of each query)
+cudaError_t launch_hamming_query_bounds(const uint64_t* d_hoff, uint32_t k, uint64_t nq, uint64_t* d_qcand, cudaStream_t s);
+// piece of every candidate of the slice [c0, c0 + n) (cub convention: d_temp == nullptr sizes the scratch)
+cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_t c0, uint64_t n, uint32_t* d_map,
+                               void* d_temp, size_t& temp_bytes, cudaStream_t s);
+// one slice of candidates for the verification kernel
+struct HammingSlice {
+  const uint64_t* qwords;       // packed reads, biased as for launch_search: read q at word 4 (q + (qoff[q] >> 6))
+  uint64_t qw_lo, qw_n;         // the words that exist: [qw_lo, qw_lo + qw_n) (checked build)
+  const uint64_t* qoff;         // the reads' offsets (nq + 1), absolute within [b_lo, b_hi]
+  uint64_t b_lo, b_hi;
+  const uint2* sp_cnt;          // exact search result of every piece (OUT_SP_CNT_U32)
+  const uint64_t* hoff;         // candidate offsets of every piece (npieces + 1)
+  uint64_t npieces;
+  const uint32_t* map;          // piece of candidate c0 + i
+  uint64_t c0, n;
+  uint64_t* counts;             // count: (k+1) per read, zeroed by the caller
+  uint64_t* keys;               // locate: (s << 2 | d) or ~0 per candidate of the slice
+  uint64_t* acc;                // locate: accepted candidates per read of the slice, zeroed by the caller
+  uint64_t q0;                  // locate: first read of the slice
+};
+cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, bool locate, int sm_count,
+                                  cudaStream_t s);
+// locate: the n < 2^31 keys of a slice sorted per read (segment i = d_qcand[i] - c0 .. d_qcand[i+1] - c0)
+cudaError_t sort_hamming_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg,
+                              const uint64_t* d_qcand, uint64_t c0, void* d_temp, size_t& temp_bytes, cudaStream_t s);
+cudaError_t scan_u64(const uint64_t* d_in, uint64_t* d_out, uint64_t n, void* d_temp, size_t& temp_bytes, cudaStream_t s);
+// accepted sorted keys -> text positions and distances at offset d_qh[q - q0] + rank in the read's segment
+cudaError_t launch_hamming_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
+                                   const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
+                                   uint8_t* d_dist, cudaStream_t s);
+
 cudaError_t launch_single_update(const IndexView& ix, uint64_t sp, uint64_t ep, uint32_t dsym,
                                  uint64_t* d_out2, cudaStream_t s);
 cudaError_t launch_single_backstep(const IndexView& ix, uint64_t row, uint64_t* d_out, cudaStream_t s);

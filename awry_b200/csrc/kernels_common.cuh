@@ -167,6 +167,32 @@ __device__ __forceinline__ uint32_t text_sector_mismatch(const u32x8& t, const u
   return bad;
 }
 
+// Hamming search (kernels_hamming.cu): the same comparison, COUNTING mismatched symbols per piece of the read
+// instead of testing for any.  `rq` = the read's packed words in global memory (search order, 8 symbols per u32;
+// reads of any length, through L1/L2), rb0 = reversed-text index of its search-order symbol 0, cut[0 .. P] =
+// ascending search-order piece bounds (piece t = symbols [cut[t], cut[t+1]), cut[0] = 0, cut[P] = read length).
+// A word's mismatches are the nibbles of q ^ t with any bit set: popc((x | x>>1 | x>>2 | x>>3) & 0x11111111).
+// Adds the mismatches of this 64-symbol sector to mm[t].
+template <int P>
+__device__ __forceinline__ void text_sector_mismatches(const u32x8& t, const uint32_t* rq, uint32_t sec, uint32_t rb0,
+                                                       const int (&cut)[P + 1], uint32_t (&mm)[P]) {
+  const int j0 = int(sec * 64u - rb0);
+  const int a = j0 >> 3;  // floor
+  const uint32_t sh = 4u * uint32_t(j0 & 7);
+  // (words in front of the read hold no symbol that takes part -- masked out -- so word 0 stands in for them)
+  uint32_t q_lo = __ldg(rq + (a < 0 ? 0 : a));
+#pragma unroll
+  for (int w = 0; w < 8; w++) {
+    const uint32_t q_hi = __ldg(rq + (a + w + 1 < 0 ? 0 : a + w + 1));
+    const uint32_t x = __funnelshift_r(q_lo, q_hi, sh) ^ t.v[w];  // read symbols j0 + 8 w .. + 7 against the text
+    const uint32_t diff = (x | (x >> 1) | (x >> 2) | (x >> 3)) & 0x11111111u;
+    const int jw = j0 + 8 * w;
+#pragma unroll
+    for (int p = 0; p < P; p++) mm[p] += __popc(diff & low_mask(4 * (cut[p + 1] - jw)) & ~low_mask(4 * (cut[p] - jw)));
+    q_lo = q_hi;
+  }
+}
+
 // protein: 8 bits per symbol, so a 32-byte sector holds 32 symbols, 4 per word, and the ring 128
 __device__ __forceinline__ uint32_t text_sector_mismatch8(const u32x8& t, const uint64_t* ring, uint32_t sec, uint32_t rb0,
                                                           uint32_t done, uint32_t len) {

@@ -127,7 +127,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_device_check", "awry_profile_enable", "awry_profile_reset", "awry_profile_get",
            "awry_bench_random_gather", "awry_set_search_variant", "awry_set_locate_variant", "awry_set_count_variant", "awry_set_host_pack",
            "awry_host_pack_dna", "awry_last_error", "awry_version", "awry_count_batch_packed2",
-           "awry_locate_batch_packed2", "awry_set_host_threads", "awry_host_threads"]
+           "awry_locate_batch_packed2", "awry_set_host_threads", "awry_host_threads", "awry_count_batch_hamming",
+           "awry_locate_batch_hamming", "awry_count_device_hamming"]
 
 
 def native():
@@ -193,6 +194,9 @@ def native():
     L.awry_count_batch_packed2.argtypes = [vp, vp, vp, u64, vp, u64, vp]
     L.awry_locate_batch_packed2.argtypes = [vp, vp, vp, u64, vp, u64, C.c_uint32, vp, vp, u64, C.POINTER(u64)]
     L.awry_set_host_threads.argtypes = [i32]
+    L.awry_count_batch_hamming.argtypes = [vp, vp, vp, u64, C.c_uint32, vp]
+    L.awry_locate_batch_hamming.argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, vp, u64, C.POINTER(u64)]
+    L.awry_count_device_hamming.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, vp]
     _LIB = L
     return L
 
@@ -442,6 +446,47 @@ class FmIndex:
             err.needed = n.value
             raise err
         return n.value
+
+    # ---- Hamming search: windows within max_mismatches <= 3 substitutions (include/awry_b200.h) --
+    def count_hamming_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_mismatches: int) -> np.ndarray:
+        """-> uint64[nq, max_mismatches + 1]: [q, d] = windows of the text at Hamming distance exactly d"""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        counts = np.zeros((nq, int(max_mismatches) + 1), dtype=np.uint64)
+        _check(native().awry_count_batch_hamming(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq, int(max_mismatches),
+                                                 counts.ctypes.data))
+        return counts
+
+    def locate_hamming_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_mismatches: int, capacity: int = None):
+        """-> (hit_off uint64[nq+1], hits uint64[n_hits, 2] = (seq_idx, local_pos) of the window start, mismatches
+        uint8[n_hits]); per query ascending by text position.  A first guess of `capacity` hits (default: one per
+        query) that proves too small is retried once with the total the library reports."""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        hit_off = np.zeros(nq + 1, dtype=np.uint64)
+        cap = max(1, nq if capacity is None else int(capacity))
+        n = C.c_uint64()
+        for _ in range(2):
+            hits = np.zeros((cap, 2), dtype=np.uint64)
+            mm = np.zeros(cap, dtype=np.uint8)
+            rc = native().awry_locate_batch_hamming(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq, int(max_mismatches),
+                                                    hit_off.ctypes.data, hits.ctypes.data, mm.ctypes.data, cap, C.byref(n))
+            if rc != -8:
+                break
+            cap = max(1, n.value)
+        if rc != 0:
+            err = AwryError(rc, native().awry_last_error().decode(errors="replace"))
+            err.needed = n.value
+            raise err
+        return hit_off, hits[: n.value], mm[: n.value]
+
+    def count_hamming_device(self, d_qbytes: int, d_qoff: int, nq: int, max_mismatches: int, d_counts: int,
+                             stream: int = 0, replica: int = 0):
+        """count_hamming_packed on device pointers (d_counts: nq * (max_mismatches + 1) u64); see device_check"""
+        _check(native().awry_count_device_hamming(self._h, replica, d_qbytes, d_qoff, nq, int(max_mismatches), d_counts,
+                                                  stream))
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

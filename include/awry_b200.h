@@ -223,6 +223,45 @@ int awry_locate_batch_packed2(const awry_index *index, const uint8_t *crumbs, co
                               uint64_t nq, const uint64_t *exceptions, uint64_t n_exc, uint32_t flags,
                               uint64_t *hit_off, awry_hit *hits, uint64_t capacity, uint64_t *n_hits);
 
+/* ------------------------------------------------------------------ Hamming search (<= k substitutions, no indels)
+ * The reference answers one question, where a query occurs EXACTLY (get_search_range_for_string, fm_index.rs:402-438,
+ * one update_range_with_symbol step per symbol, :559-582).  These calls extend it to windows of the text within
+ * Hamming distance k (Bowtie's `-v k`), nucleotide only.
+ *   text      the text the index holds: records joined by 'N', n = bwt_len - 1 symbols, no '$' (fm_index.rs:148-153).
+ *             A window is text[s .. s+L) for 0 <= s <= n - L; windows may cross record delimiters, where the 'N' is
+ *             an ordinary symbol, as for exact search.
+ *   distance  the number of positions whose symbols differ, query bytes mapped as for exact search (either case,
+ *             U = T, any other byte = N): a query N matches a text N and mismatches A / C / G / T.
+ *   count     counts[q * (k+1) + d] = the number of windows at distance exactly d, d = 0 .. k (caller-owned,
+ *             nq * (k+1) entries).  For k = 0 this equals awry_count_batch.
+ *   locate    every window at distance <= k, once each, per query in ascending text position, i.e. ascending
+ *             (seq_idx, local_pos) of the window start.  hit_mismatches (NULL or `capacity` entries) receives each
+ *             hit's distance.  capacity / AWRY_ERR_CAPACITY as in awry_locate_batch_into: hit_off (nq+1) and
+ *             *n_hits are complete even when `hits` is not.
+ *   errors    k > AWRY_HAMMING_MAX -> AWRY_ERR_INVALID_ARG; an empty query or one with '$' / '#', and a query of
+ *             length L <= k (every window would match) -> AWRY_ERR_INVALID_QUERY; a protein index, or one without
+ *             the unsampled suffix array and the text on the device (AWRY_B200_FULL_SA=0, AWRY_B200_TEXT=0, not
+ *             enough device memory, 64-bit row pointers) -> AWRY_ERR_UNSUPPORTED.
+ * Scheme (pigeonhole): the query is cut into k+1 pieces, piece j = bytes [a_j, a_{j+1}), a_j = floor(j L / (k+1));
+ * each piece is searched exactly, an occurrence of piece j at text position p names the window s = p - a_j, and the
+ * window is verified against the text on the device.  It is kept iff its distance is <= k and j is the smallest piece
+ * it matches exactly, so no window is reported twice.  Cost: about one exact search per piece plus one verification
+ * per candidate, and the candidates are about the sum over pieces of n / 4^(piece length): short queries at high k
+ * (12 bp at k = 3: 3-bp pieces) are legal but expensive. */
+enum { AWRY_HAMMING_MAX = 3 };
+int awry_count_batch_hamming(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                             uint32_t max_mismatches, uint64_t *counts /* nq * (max_mismatches + 1) */);
+int awry_locate_batch_hamming(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                              uint32_t max_mismatches, uint64_t *hit_off /* nq + 1 */, awry_hit *hits,
+                              uint8_t *hit_mismatches /* NULL or capacity entries */, uint64_t capacity,
+                              uint64_t *n_hits);
+/* awry_count_batch_hamming on device-resident queries (see awry_count_device below): pointers on replica `replica`'s
+ * device, work enqueued on `cuda_stream`.  It synchronises that stream once, after the pieces are searched (the
+ * candidate total sizes the verification), and returns without waiting for the verification.  An empty / sentinel /
+ * L <= k query is latched and reported by awry_device_check; its counts are 0. */
+int awry_count_device_hamming(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                              uint64_t nq, uint32_t max_mismatches, uint64_t *d_counts, void *cuda_stream);
+
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to
  * parallel_count / parallel_locate (fm_index.rs:455-487); these entry points take the FASTQ ('@') or

@@ -150,6 +150,45 @@ class FmIndex {
     awry_hits_free(hits);
     return out;
   }
+  // Hamming search (no counterpart in the reference): windows within max_mismatches <= AWRY_HAMMING_MAX substitutions.
+  // counts[q][d] = windows of query q at distance exactly d
+  std::vector<std::vector<uint64_t>> parallel_count_hamming(const std::vector<std::string_view>& queries,
+                                                            uint32_t max_mismatches) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::vector<uint64_t> flat(queries.size() * (size_t(max_mismatches) + 1));
+    check(awry_count_batch_hamming(h_, bytes.data(), off.data(), queries.size(), max_mismatches, flat.data()));
+    std::vector<std::vector<uint64_t>> out(queries.size());
+    for (size_t q = 0; q < queries.size(); q++)
+      out[q].assign(flat.begin() + q * (max_mismatches + 1), flat.begin() + (q + 1) * (max_mismatches + 1));
+    return out;
+  }
+  // per query: (window start, distance), ascending by position
+  std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> parallel_locate_hamming(
+      const std::vector<std::string_view>& queries, uint32_t max_mismatches) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::vector<uint64_t> hit_off(queries.size() + 1);
+    std::vector<awry_hit> hits(queries.size() + 1);
+    std::vector<uint8_t> dist(hits.size());
+    uint64_t n = 0;
+    int rc = awry_locate_batch_hamming(h_, bytes.data(), off.data(), queries.size(), max_mismatches, hit_off.data(),
+                                       hits.data(), dist.data(), hits.size(), &n);
+    if (rc == AWRY_ERR_CAPACITY) {  // the total is known now: once more with room for every hit
+      hits.resize(n);
+      dist.resize(n);
+      rc = awry_locate_batch_hamming(h_, bytes.data(), off.data(), queries.size(), max_mismatches, hit_off.data(),
+                                     hits.data(), dist.data(), hits.size(), &n);
+    }
+    check(rc);
+    std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> out(queries.size());
+    for (size_t q = 0; q < queries.size(); q++)
+      for (uint64_t i = hit_off[q]; i < hit_off[q + 1]; i++)
+        out[q].push_back({{hits[i].seq_idx, hits[i].local_pos}, uint32_t(dist[i])});
+    return out;
+  }
   awry_index* handle() const { return h_; }
 
  private:
