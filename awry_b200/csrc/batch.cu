@@ -239,6 +239,14 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
   Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nq));
   const uint64_t* src_o = qs.qoff + c.q0;
   uint64_t* const d_words = ws->d_qwords - 4 * (c.b0 >> ush);
+  SearchVariant v = current_variant();
+  v.avg_len = uint32_t(std::min<uint64_t>(nbytes / std::max<uint64_t>(1, nq), 1u << 30));
+  v.b_lo = c.b0;
+  v.b_hi = c.b1;
+  // locate: when pass 2 will be the gather from the unsampled array, queries finished in the text are stored as
+  // their text position (decided here, once, and remembered in the workspace for locate_chunk_walk)
+  v.locate_positions = mode == OUT_SP_CNT_U32 && locate_positions_ok(r.view, v);
+  bool in_wave = false;  // ASCII queries that the wave kernel packs itself (launch_search_ascii)
   ws->link_probe_bytes = 0;
   uint64_t uni_len = 0;
   const bool uniform = offsets_are_uniform(src_o, nq, uni_len);
@@ -349,7 +357,8 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
       g_prof.h2d += nbytes;
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
       // offsets stay absolute: the kernels subtract the chunk's byte base
-      {
+      in_wave = search_packs_ascii(r.view, mode, v);
+      if (!in_wave) {
         ProfScope p(2, r.device, ws->st);
         CU(launch_pack(ix->alphabet, ws->d_qbytes - c.b0, ws->d_qoff, nq, d_words, c.b0, c.b1, ws->d_flag, ws->st));
       }
@@ -358,13 +367,6 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
   gpu_mark(ws->st, "packed on device", (long long)c.q0);
   {
     ProfScope p(0, r.device, ws->st);
-    SearchVariant v = current_variant();
-    v.avg_len = uint32_t(std::min<uint64_t>(nbytes / std::max<uint64_t>(1, nq), 1u << 30));
-    v.b_lo = c.b0;
-    v.b_hi = c.b1;
-    // locate: when pass 2 will be the gather from the unsampled array, queries finished in the text are stored as
-    // their text position (decided here, once, and remembered in the workspace for locate_chunk_walk)
-    v.locate_positions = mode == OUT_SP_CNT_U32 && locate_positions_ok(r.view, v);
     ws->sp_cnt_positions = v.locate_positions;
     ws->gpu_probe_bytes = 0;
     const bool time_kernel = qs.pinned && !qs.crumbs && nbytes >= (8u << 20);  // PackBalance: what the GPU consumes
@@ -375,8 +377,12 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
       }
       CU(cudaEventRecord(ws->ev_s0, ws->st));
     }
-    CU(launch_search(r.view, d_words, ws->d_qoff, nq, mode, d_out_override ? d_out_override : ws->d_out, ws->d_defer, v,
-                     r.sm_count, ws->st));
+    void* const d_out = d_out_override ? d_out_override : ws->d_out;
+    if (in_wave)
+      CU(launch_search_ascii(r.view, ws->d_qbytes - c.b0, ws->d_qoff, nq, d_words, ws->d_flag, mode, d_out, ws->d_defer, v,
+                             r.sm_count, ws->st));
+    else
+      CU(launch_search(r.view, d_words, ws->d_qoff, nq, mode, d_out, ws->d_defer, v, r.sm_count, ws->st));
     if (time_kernel) {
       CU(cudaEventRecord(ws->ev_s1, ws->st));
       ws->gpu_probe_bytes = nbytes;
@@ -1457,17 +1463,23 @@ int awry_count_device(const awry_index* ix, int replica, const uint8_t* d_qbytes
     uint64_t* d_qwords = nullptr;  // packed queries, then the deferred-query list
     CU(cudaMallocAsync(reinterpret_cast<void**>(&d_qwords), words * 8 + defer_words(nq) * 4, st));
     uint32_t* d_defer = reinterpret_cast<uint32_t*>(d_qwords + words);
-    {
+    uint64_t* const d_words = d_qwords - 4 * (ends[0] >> sh);
+    SearchVariant v = current_variant();
+    v.avg_len = uint32_t(std::min<uint64_t>((ends[1] - ends[0]) / nq, 1u << 30));
+    v.b_lo = ends[0];
+    v.b_hi = ends[1];
+    const bool in_wave = search_packs_ascii(r.view, OUT_COUNT_U64, v);
+    if (!in_wave) {
       ProfScope p(2, r.device, st);
-      CU(launch_pack(ix->alphabet, d_qbytes, d_qoff, nq, d_qwords - 4 * (ends[0] >> sh), ends[0], ends[1], r.d_async_flag, st));
+      CU(launch_pack(ix->alphabet, d_qbytes, d_qoff, nq, d_words, ends[0], ends[1], r.d_async_flag, st));
     }
     {
       ProfScope p(0, r.device, st);
-      SearchVariant v = current_variant();
-      v.avg_len = uint32_t(std::min<uint64_t>((ends[1] - ends[0]) / nq, 1u << 30));
-      v.b_lo = ends[0];
-      v.b_hi = ends[1];
-      CU(launch_search(r.view, d_qwords - 4 * (ends[0] >> sh), d_qoff, nq, OUT_COUNT_U64, d_counts, d_defer, v, r.sm_count, st));
+      if (in_wave)
+        CU(launch_search_ascii(r.view, d_qbytes, d_qoff, nq, d_words, r.d_async_flag, OUT_COUNT_U64, d_counts, d_defer, v,
+                               r.sm_count, st));
+      else
+        CU(launch_search(r.view, d_words, d_qoff, nq, OUT_COUNT_U64, d_counts, d_defer, v, r.sm_count, st));
     }
     CU(cudaFreeAsync(d_qwords, st));
   });
@@ -1498,19 +1510,25 @@ int awry_locate_device(const awry_index* ix, int replica, const uint8_t* d_qbyte
       Workspace::grow_dev(ws->d_qwords, ws->d_qwords_cap, size_t(words));
       Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nq) * sp_cnt_bytes(r.view));
       Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nq));
-      {
+      uint64_t* const d_words = ws->d_qwords - 4 * (ends[0] >> sh);
+      SearchVariant v = current_variant();
+      v.avg_len = uint32_t(std::min<uint64_t>((ends[1] - ends[0]) / nq, 1u << 30));
+      v.b_lo = ends[0];
+      v.b_hi = ends[1];
+      v.locate_positions = locate_positions_ok(r.view, v);
+      ws->sp_cnt_positions = v.locate_positions;
+      const bool in_wave = search_packs_ascii(r.view, OUT_SP_CNT_U32, v);
+      if (!in_wave) {
         ProfScope p(2, r.device, st);
-        CU(launch_pack(ix->alphabet, d_qbytes, d_qoff, nq, ws->d_qwords - 4 * (ends[0] >> sh), ends[0], ends[1], r.d_async_flag, st));
+        CU(launch_pack(ix->alphabet, d_qbytes, d_qoff, nq, d_words, ends[0], ends[1], r.d_async_flag, st));
       }
       {
         ProfScope p(0, r.device, st);
-        SearchVariant v = current_variant();
-        v.avg_len = uint32_t(std::min<uint64_t>((ends[1] - ends[0]) / nq, 1u << 30));
-        v.b_lo = ends[0];
-        v.b_hi = ends[1];
-        v.locate_positions = locate_positions_ok(r.view, v);
-        ws->sp_cnt_positions = v.locate_positions;
-        CU(launch_search(r.view, ws->d_qwords - 4 * (ends[0] >> sh), d_qoff, nq, OUT_SP_CNT_U32, ws->d_out, ws->d_defer, v, r.sm_count, st));
+        if (in_wave)
+          CU(launch_search_ascii(r.view, d_qbytes, d_qoff, nq, d_words, r.d_async_flag, OUT_SP_CNT_U32, ws->d_out,
+                                 ws->d_defer, v, r.sm_count, st));
+        else
+          CU(launch_search(r.view, d_words, d_qoff, nq, OUT_SP_CNT_U32, ws->d_out, ws->d_defer, v, r.sm_count, st));
       }
       uint64_t n = 0;
       uint64_t* h = locate_chunk_device(ix, r, ws, nq, flags, d_hit_off, &n, st);

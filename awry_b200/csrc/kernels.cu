@@ -584,6 +584,20 @@ __device__ __forceinline__ uint64_t pack_word_bytes(const uint8_t* __restrict__ 
   return word;
 }
 
+// 4 ASCII bases (the first in the low byte) -> their 4 codes as nibbles in search order (the last base in the low
+// nibble), SIMD-in-register: ((c & 0xDF) >> 1) & 3 maps A,C,T,G to 0,1,2,3 and x ^ (x >> 1) swaps the last two.
+// `diff` gets a non-zero byte for every byte that is not one of ACGT/acgt (whose nibble is then meaningless).
+__device__ __forceinline__ uint32_t ascii4_to_nibbles(uint32_t w4, uint32_t& diff) {
+  const uint32_t rev = __byte_perm(w4, 0, 0x0123);  // search order: last byte first
+  const uint32_t up = rev & 0xDFDFDFDFu;
+  const uint32_t x4 = (up >> 1) & 0x03030303u;
+  const uint32_t c4 = x4 ^ ((x4 >> 1) & 0x01010101u);
+  const uint32_t sel = c4 | (c4 >> 4);
+  const uint32_t nib = (sel & 0xffu) | ((sel >> 8) & 0xff00u);  // 4 nibbles = 4 codes
+  diff = up ^ __byte_perm(0x54474341u, 0, nib);                 // "ACGT"[code] per byte
+  return nib;
+}
+
 template <int ALPHA, int PL = 8>
 __global__ void __launch_bounds__(256)
     pack_kernel(const uint8_t* __restrict__ qbytes, const uint64_t* __restrict__ qoff, uint64_t nq,
@@ -621,8 +635,7 @@ __global__ void __launch_bounds__(256)
       bool done = false;
       if (ALPHA == 0 && len >= 16) {
         // 16 ASCII bases -> 16 nibbles without per-byte loads: 4-5 aligned 32-bit loads, funnel
-        // shift to the byte offset, then SIMD-in-register: ((c & 0xDF) >> 1) & 3 maps A,C,T,G to
-        // 0,1,2,3 and x ^ (x >> 1) swaps the last two.  The query's final, partial word reuses the
+        // shift to the byte offset, then ascii4_to_nibbles.  The query's final, partial word reuses the
         // first 16 bytes of the query and shifts the surplus symbols out.  Any byte that is not
         // one of ACGT/acgt sends the word down the table path.
         const uint32_t have = len - first;               // symbols left from `first` on
@@ -638,15 +651,9 @@ __global__ void __launch_bounds__(256)
         bool clean = true;
 #pragma unroll
         for (int j = 0; j < 4; j++) {
-          uint32_t w4 = __funnelshift_r(u[j], u[j + 1], 8 * sh);  // bytes 4j .. 4j+3
-          uint32_t rev = __byte_perm(w4, 0, 0x0123);              // search order: last byte first
-          uint32_t up = rev & 0xDFDFDFDFu;
-          uint32_t x4 = (up >> 1) & 0x03030303u;
-          uint32_t c4 = x4 ^ ((x4 >> 1) & 0x01010101u);
-          uint32_t sel = c4 | (c4 >> 4);
-          uint32_t nib = (sel & 0xffu) | ((sel >> 8) & 0xff00u);  // 4 nibbles = 4 codes
-          clean &= up == __byte_perm(0x54474341u, 0, nib);        // "ACGT"[code] per byte
-          nibs[j] = nib;
+          uint32_t diff;
+          nibs[j] = ascii4_to_nibbles(__funnelshift_r(u[j], u[j + 1], 8 * sh), diff);  // bytes 4j .. 4j+3
+          clean &= diff == 0;
         }
         if (clean) {
           word = (uint64_t(nibs[1] | (nibs[0] << 16)) << 32) | uint64_t(nibs[3] | (nibs[2] << 16));
@@ -1337,16 +1344,95 @@ __global__ void __launch_bounds__(TPB, MINB)
 // WAVE_MAX_STEPS steps with the interval still wider than one row (repeats), or more than 256 symbols -> the
 // `rest` list, searched afterwards by search_dna_pair_kernel<VFY, LIST>; an ambiguity symbol -> the scalar kernel.
 // Both block reads of an interval that straddles two blocks are issued before either is used.
+// ASCII: the kernel reads the caller's query bytes (qbytes, indexed by the absolute offsets) instead of the words of
+// pack_kernel and is its own prepass: it latches what pack_kernel latches into *first_bad, stages each read into the
+// ring straight from its bytes (stage_ascii_ring), and writes the packed words of every query it hands on to `qw_out`
+// (biased like `qwords`, which it does not read), so that the list kernels find them where they always do.
 constexpr int WAVE_MAX_STEPS = 6;
 
-template <int MODE, int TPB, int MINB>
+// Query bytes [b, e) (addresses, at most 256 of them) -> the group's ring: every nibble of the read as pack_kernel
+// writes it (nibbles past the read's length are left as they come: the search never reads them).  The read's 32-byte
+// sectors are counted from its END: sector k holds bytes [end32 - 32 (k + 1), end32 - 32 k), end32 = e rounded up to
+// 32, and converts to the 32 nibbles [32 k, 32 k + 32) of a sector-aligned stream in search order whose nibble j + pad
+// is ring nibble j (pad = end32 - e).  Lane `sub` converts sectors sub, sub + 4, sub + 8 (aligned LDG.256) and writes
+// the four 32-bit ring halves that start in its sector; the last of them needs the first half of sector k + 1, which
+// the next lane holds (lane 3: lane 0 in the round before -- rounds run from the last sector down).  Returns non-zero
+// when a byte of the sectors is not one of ACGT/acgt -- bytes of the neighbouring reads included (see the caller).
+__device__ __forceinline__ uint32_t stage_ascii_ring(uintptr_t b, uintptr_t e, bool run, uint32_t sub, uint32_t gbase,
+                                                     uint64_t* ring) {
+  constexpr uint32_t FULL = 0xffffffffu;
+  const uint32_t nsec = run ? uint32_t(((e - 1) >> 5) - (b >> 5)) + 1 : 0u;
+  const uintptr_t end32 = (e + 31) & ~uintptr_t(31);
+  const uint32_t pad = uint32_t(end32 - e), ph = pad >> 3, pl4 = 4 * (pad & 7);
+  uint32_t* const r32 = reinterpret_cast<uint32_t*>(ring);
+  uint32_t dirty = 0, carry = 0;
+  const int rounds = int(__reduce_max_sync(FULL, (nsec + 3) >> 2));
+#pragma unroll 1
+  for (int i = rounds - 1; i >= 0; i--) {
+    const uint32_t k = sub + 4u * uint32_t(i);
+    uint32_t h[5] = {0u, 0u, 0u, 0u, 0u};
+    if (k < nsec) {
+      const u32x8 t = ldg256(reinterpret_cast<const void*>(end32 - 32 * uintptr_t(k + 1)));
+      uint32_t nib[8];
+#pragma unroll
+      for (int j = 0; j < 8; j++) {
+        uint32_t diff;
+        nib[j] = ascii4_to_nibbles(t.v[j], diff);
+        dirty |= diff;
+      }
+      h[0] = nib[7] | (nib[6] << 16);
+      h[1] = nib[5] | (nib[4] << 16);
+      h[2] = nib[3] | (nib[2] << 16);
+      h[3] = nib[1] | (nib[0] << 16);
+    }
+    const uint32_t x = __shfl_sync(FULL, h[0], gbase + ((sub + 1) & 3));
+    h[4] = sub == 3 ? carry : x;
+    carry = x;
+    if (k < nsec) {
+#pragma unroll
+      for (int j = 0; j < 4; j++) {
+        const int m = int(4 * k) - int(ph) + j;
+        if (m >= 0 && m < 32) r32[m] = __funnelshift_r(h[j], h[j + 1], pl4);
+      }
+    }
+  }
+  return dirty;
+}
+
+// whether bytes [src, src + len) hold anything but ACGT/acgt (the group's 4 lanes take every 4th byte)
+__device__ __forceinline__ uint32_t read_is_dirty(const uint8_t* src, uint32_t len, uint32_t sub) {
+  uint32_t dirty = 0;
+  for (uint32_t i = sub; i < len; i += 4) {
+    uint32_t diff;
+    ascii4_to_nibbles(0x41414100u | src[i], diff);  // the byte and three 'A'
+    dirty |= diff;
+  }
+  return dirty;
+}
+
+// a query the ASCII wave kernel hands on without a ring: its words by pack_kernel's table path, which also latches a
+// sentinel (the group's 4 lanes take words sub, sub + 4, ...)
+__device__ __forceinline__ void pack_query_lut(const uint8_t* src, uint32_t len, uint32_t nwords, uint64_t* dst,
+                                               uint32_t sub, const uint8_t* lut, uint64_t q, unsigned long long* first_bad) {
+  bool bad = false;
+  for (uint32_t wi = sub; wi < nwords; wi += 4) dst[wi] = pack_word_bytes<0>(src, len, wi << 4, lut, bad);
+  if (bad) atomicMin(first_bad, bad_query_code(q, BAD_QUERY));
+}
+
+template <int MODE, int TPB, int MINB, bool ASCII = false>
 __global__ void __launch_bounds__(TPB, MINB)
     search_dna_wave_kernel(IndexView ix, const uint64_t* __restrict__ qwords, const uint64_t* __restrict__ qoff,
                            uint64_t nq, void* __restrict__ out, uint32_t* __restrict__ defer, uint32_t ticket_sz,
-                           ByteRange br) {
+                           ByteRange br, const uint8_t* __restrict__ qbytes, uint64_t* qw_out,
+                           unsigned long long* first_bad) {
   constexpr uint32_t FULL = 0xffffffffu;
   enum : uint32_t { W_NONE = 0, W_RUN = 1, W_EMPTY = 2 };  // no query (or handed on) / in progress / refused by the prepass
   __shared__ uint64_t s_q[TPB / 4][16];
+  __shared__ uint8_t s_lut[ASCII ? 256 : 1];
+  if (ASCII) {
+    s_lut[threadIdx.x] = c_ascii_to_dsym[0][threadIdx.x];
+    __syncthreads();
+  }
   const uint32_t lane = threadIdx.x & 31, sub = lane & 3, gbase = lane - sub, gmask = 0xfu << gbase, grp = lane >> 2;
   uint64_t* const ring = s_q[threadIdx.x >> 2];
   const uint32_t nq32 = uint32_t(nq);
@@ -1373,17 +1459,28 @@ __global__ void __launch_bounds__(TPB, MINB)
     if (st == W_RUN) ov = __ldg(qoff + q + (sub & 1));  // lanes 0/1 fetch both ends with one request
     const uint64_t o0 = __shfl_sync(FULL, ov, gbase), o1 = __shfl_sync(FULL, ov, gbase + 1);
     const uint32_t len = st == W_RUN ? checked_len(o0, o1, br) : 0u;
-    if (st == W_RUN && len == 0) st = W_EMPTY;
+    if (st == W_RUN && len == 0) {
+      st = W_EMPTY;
+      if (ASCII && sub == 0)  // as pack_kernel: offsets outside [b_lo, b_hi] first, else the query is empty
+        atomicMin(first_bad, bad_query_code(q, o1 == o0 && o0 >= br.lo && o1 <= br.hi ? BAD_QUERY : BAD_OFFSETS));
+    }
     const uint32_t nwords = (len + 15) >> 4;
+    const uint32_t ubase = 4 * (q + uint32_t(o0 >> 6));
     if (st == W_RUN && nwords > 16) {  // longer than the ring: the refilling kernel slides it
+      if (ASCII) pack_query_lut(qbytes + o0, len, nwords, qw_out + ubase, sub, s_lut, q, first_bad);
       if (sub == 0) rest[2 + atomicAdd(rest, 1u)] = q;
       st = W_NONE;
     }
-    // ---- packed words -> ring; ambiguity symbols (code >= 4) are looked for here, once
+    // ---- query -> ring; ambiguity symbols (code >= 4; ASCII: any byte but ACGT/acgt) are looked for here, once
     uint32_t amb = 0;
     __syncwarp();  // the previous wave's ring reads are done
-    if (st == W_RUN && 4 * sub < nwords) {
-      const uint32_t ubase = 4 * (q + uint32_t(o0 >> 6));
+    if (ASCII) {
+      amb = stage_ascii_ring(uintptr_t(qbytes + o0), uintptr_t(qbytes + o1), st == W_RUN, sub, gbase, ring);
+      // the first and last sector also hold bytes of the neighbouring reads: a group that saw a byte outside ACGT/acgt
+      // looks again at its read's bytes alone (rare: a batch of clean reads never comes here)
+      const uint32_t dirty_groups = __ballot_sync(FULL, amb != 0);
+      if (dirty_groups) amb = st == W_RUN && (dirty_groups & gmask) ? read_is_dirty(qbytes + o0, len, sub) : 0u;
+    } else if (st == W_RUN && 4 * sub < nwords) {
       AWRY_CHK_QWORDS(ubase + 4 * sub, br, nq, 6);
       const u32x8 t = ldg256(qwords + ubase + 4 * sub);
 #pragma unroll
@@ -1395,6 +1492,7 @@ __global__ void __launch_bounds__(TPB, MINB)
     const uint32_t amb_groups = __ballot_sync(FULL, amb != 0);
     __syncwarp();
     if (st == W_RUN && (amb_groups & gmask) != 0) {  // the scalar kernel takes the whole query
+      if (ASCII) pack_query_lut(qbytes + o0, len, nwords, qw_out + ubase, sub, s_lut, q, first_bad);
       if (sub == 0) defer[1 + atomicAdd(defer, 1u)] = q;
       st = W_NONE;
     }
@@ -1424,6 +1522,16 @@ __global__ void __launch_bounds__(TPB, MINB)
       if (!__any_sync(FULL, active)) break;
       if (it == WAVE_MAX_STEPS) {  // still wide: a repeat -- handed on, searched from its start by the refilling kernel
         if (active) {
+          if (ASCII) {  // its words are the ring, with the nibbles past its length set to 0
+#pragma unroll
+            for (uint32_t j = 4 * sub; j < 4 * sub + 4; j++) {
+              if (j < nwords) {
+                AWRY_CHK_QWORDS(ubase + j, br, nq, 6);
+                const uint32_t tail = len - 16 * j;
+                qw_out[ubase + j] = tail >= 16 ? ring[j] : ring[j] & ((1ull << (4 * tail)) - 1);
+              }
+            }
+          }
           if (sub == 0) rest[2 + atomicAdd(rest, 1u)] = q;
           st = W_NONE;
         }
@@ -1866,16 +1974,23 @@ static cudaError_t launch_search_pair_b(const IndexView& ix, const uint64_t* d_q
 
 // the wave kernel, then the refilling kernel over the queries it handed on, then the scalar kernel over the
 // queries with ambiguity symbols (both lists are empty for a batch of clean sequencer reads)
-template <int MODE>
+// ASCII flavour (launch_search_ascii): where the kernel reads the query bytes, writes the words it hands on, latches
+struct AsciiQueries {
+  const uint8_t* qbytes = nullptr;
+  uint64_t* qwords = nullptr;
+  unsigned long long* first_bad = nullptr;
+};
+
+template <int MODE, bool ASCII = false>
 static cudaError_t launch_search_wave(const IndexView& ix, const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq,
                                       void* d_out, uint32_t* d_defer, int sm_count, cudaStream_t s, uint32_t avg_len,
-                                      ByteRange br) {
+                                      ByteRange br, const AsciiQueries& a = AsciiQueries()) {
   // 6 x 256 threads/SM (40 registers, 8-16 bytes of spill) beat 5 x 256 (47 registers, none): 1.70 against 1.80 ms
   // per 10 M x 150-bp reads with a k = 13 seed table
   constexpr int TPB = 256, MINB = 6;
   cudaError_t e = cudaMemsetAsync(d_defer + nq + 2, 0, 8, s);  // count of the rest list, its ticket counter
   if (e != cudaSuccess) return e;
-  auto kern = search_dna_wave_kernel<MODE, TPB, MINB>;
+  auto kern = search_dna_wave_kernel<MODE, TPB, MINB, ASCII>;
   auto kern_rest = search_dna_pair_kernel<MODE, TPB, 4, true, true>;  // (64 registers: the list-driven flavour spills at 48)
   int per_sm = 0, per_sm_rest = 0;
   if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, TPB, 0)) != cudaSuccess) return e;
@@ -1890,7 +2005,8 @@ static cudaError_t launch_search_wave(const IndexView& ix, const uint64_t* d_qwo
   // a ticket = 4 waves of 8 queries per warp; small batches get one wave per ticket so that every warp draws some
   uint32_t ticket_sz = nq >= uint64_t(grid) * (TPB / 32) * 128 ? 32u : 8u;
   if (ticket_env) ticket_sz = ticket_env;
-  e = launch_with_table_window(kern, grid, TPB, s, ix, ix, d_qwords, d_qoff, nq, d_out, d_defer, ticket_sz, br);
+  e = launch_with_table_window(kern, grid, TPB, s, ix, ix, d_qwords, d_qoff, nq, d_out, d_defer, ticket_sz, br, a.qbytes,
+                               a.qwords, a.first_bad);
   COUNT_LAUNCH();
   if (e != cudaSuccess) return e;
   uint32_t per_group = avg_len == 0 ? 2u : std::min(8u, std::max(1u, 200u / avg_len));
@@ -1933,28 +2049,46 @@ static cudaError_t launch_search_pairx_b(const IndexView& ix, const uint64_t* d_
   return cudaGetLastError();
 }
 
+static int slots_default() {
+  static const int d = [] {
+    if (const char* e = getenv("AWRY_B200_SLOTS")) return std::max(0, std::min(4, atoi(e)));
+    return 0;
+  }();
+  return d;
+}
+
+// With the text on the device one-row intervals are finished by comparing with it (see the kernels): count mode,
+// and locate pass 1 for a gather pass 2 (the hit stored as its text position).
+static bool finishes_in_text(const IndexView& ix, SearchOut mode, const SearchVariant& v) {
+  return v.finish_in_text && ix.rtext != nullptr && ix.full_sa != nullptr &&
+         (mode == OUT_COUNT_U64 || (mode == OUT_SP_CNT_U32 && v.locate_positions));
+}
+
+// Whether launch_search runs the nucleotide wave kernel: the default there (launch_search_mode -> launch_search_pair);
+// the refilling kernel with the same step (awry_set_search_variant(80), or a residency) and the state-machine one
+// (81-84, count only) stay selectable.
+static bool runs_wave_kernel(const IndexView& ix, SearchOut mode, const SearchVariant& v) {
+  return !ix.wide && ix.alphabet == 0 && ix.pair_blocks != nullptr && (v.lanes == 0 || v.lanes == 8) &&
+         finishes_in_text(ix, mode, v) && v.slots < 0 && slots_default() == 0 && v.blocks_per_sm == 0;
+}
+
+static cudaError_t reset_defer(uint64_t nq, uint32_t* d_defer, cudaStream_t s) {
+  if (nq >= (1ull << 32) - (1u << 24)) return cudaErrorInvalidValue;  // 32-bit ticket counter
+  cudaError_t e = cudaMemsetAsync(d_defer, 0, 4, s);                  // deferred-query count
+  if (e != cudaSuccess) return e;
+  return cudaMemsetAsync(d_defer + nq + 1, 0, 4, s);                  // ticket counter
+}
+
 template <int MODE>
 static cudaError_t launch_search_pair(const IndexView& ix, const uint64_t* d_qwords, const uint64_t* d_qoff,
                                       uint64_t nq, void* d_out, uint32_t* d_defer, const SearchVariant& v,
                                       int sm_count, cudaStream_t s) {
-  if (nq >= (1ull << 32) - (1u << 24)) return cudaErrorInvalidValue;  // 32-bit ticket counter
-  cudaError_t e = cudaMemsetAsync(d_defer, 0, 4, s);                  // deferred-query count
-  if (e != cudaSuccess) return e;
-  e = cudaMemsetAsync(d_defer + nq + 1, 0, 4, s);                     // ticket counter
+  cudaError_t e = reset_defer(nq, d_defer, s);
   if (e != cudaSuccess) return e;
   const ByteRange br{v.b_lo, v.b_hi};
-  static const int slots_default = [] {
-    if (const char* e = getenv("AWRY_B200_SLOTS")) return std::max(0, std::min(4, atoi(e)));
-    return 0;
-  }();
-  const int slots = v.slots >= 0 ? v.slots : slots_default;
-  // With the text on the device one-row intervals are finished by comparing with it (see the kernels): count mode,
-  // and locate pass 1 for a gather pass 2 (the hit stored as its text position).  Default: the wave kernel; the
-  // refilling kernel with the same step (awry_set_search_variant(80), or a residency) and the state-machine one
-  // (81-84, count only) stay selectable.
-  const bool in_text = v.finish_in_text && ix.rtext != nullptr && ix.full_sa != nullptr &&
-                       (MODE == OUT_COUNT_U64 || (MODE == OUT_SP_CNT_U32 && v.locate_positions));
-  if (in_text && v.slots < 0 && slots_default == 0 && v.blocks_per_sm == 0) {
+  const int slots = v.slots >= 0 ? v.slots : slots_default();
+  const bool in_text = finishes_in_text(ix, SearchOut(MODE), v);
+  if (runs_wave_kernel(ix, SearchOut(MODE), v)) {
     if (MODE == OUT_COUNT_U64) return launch_search_wave<OUT_COUNT_U64>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br);
     if (MODE == OUT_SP_CNT_U32) return launch_search_wave<OUT_SP_CNT_U32>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br);
   }
@@ -2413,6 +2547,28 @@ static cudaError_t launch_search_mode(const IndexView& ix, const uint64_t* d_qwo
     search_scalar_kernel<1, MODE, false><<<grid, 256, 0, s>>>(ix, d_qwords, d_qoff, nq, d_out, nullptr, ByteRange{v.b_lo, v.b_hi});
   COUNT_LAUNCH();
   return cudaGetLastError();
+}
+
+bool search_packs_ascii(const IndexView& ix, SearchOut mode, const SearchVariant& v) {
+  const char* e = getenv("AWRY_B200_ASCII_WAVE");  // read per call: "0" keeps launch_pack + launch_search (A/B runs, tests)
+  return !(e && e[0] == '0') && runs_wave_kernel(ix, mode, v);
+}
+
+cudaError_t launch_search_ascii(const IndexView& ix, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                                uint64_t* d_qwords, unsigned long long* d_first_bad, SearchOut mode, void* d_out,
+                                uint32_t* d_defer, const SearchVariant& v, int sm_count, cudaStream_t s) {
+  if (nq == 0) return cudaSuccess;
+  if (!runs_wave_kernel(ix, mode, v)) return cudaErrorInvalidValue;
+  cudaError_t e = reset_defer(nq, d_defer, s);
+  if (e != cudaSuccess) return e;
+  const ByteRange br{v.b_lo, v.b_hi};
+  AsciiQueries a;
+  a.qbytes = d_qbytes;
+  a.qwords = d_qwords;
+  a.first_bad = d_first_bad;
+  if (mode == OUT_COUNT_U64)
+    return launch_search_wave<OUT_COUNT_U64, true>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br, a);
+  return launch_search_wave<OUT_SP_CNT_U32, true>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br, a);
 }
 
 cudaError_t launch_search(const IndexView& ix, const uint64_t* d_qwords, const uint64_t* d_qoff,

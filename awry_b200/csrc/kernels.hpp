@@ -130,6 +130,15 @@ inline size_t defer_words(uint64_t nq) { return 2 * size_t(nq) + 8; }
 cudaError_t launch_search(const IndexView& ix, const uint64_t* d_qwords, const uint64_t* d_qoff,
                           uint64_t nq, SearchOut mode, void* d_out, uint32_t* d_defer,
                           const SearchVariant& v, int sm_count, cudaStream_t s);
+// ASCII queries searched by the wave kernel straight from their bytes: it packs them itself (the ring of every read it
+// searches, and in d_qwords the words of the queries it hands on to the list kernels) and latches in *d_first_bad what
+// launch_pack would.  search_packs_ascii: whether launch_search would run the wave kernel for this batch (and
+// AWRY_B200_ASCII_WAVE, read per call, is not "0"); only then may launch_search_ascii be called -- otherwise the
+// queries go through launch_pack + launch_search.
+bool search_packs_ascii(const IndexView& ix, SearchOut mode, const SearchVariant& v);
+cudaError_t launch_search_ascii(const IndexView& ix, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                                uint64_t* d_qwords, unsigned long long* d_first_bad, SearchOut mode, void* d_out,
+                                uint32_t* d_defer, const SearchVariant& v, int sm_count, cudaStream_t s);
 
 // locate: CSR offsets from pass 1, LF-walk pass 2
 // d_sp_cnt: the search kernels' OUT_SP_CNT result -- uint2 (sp, count) per query, ulonglong2 for a wide index
