@@ -182,6 +182,9 @@ struct QuerySource {
   uint64_t n_exc = 0;
   const uint64_t* qoff = nullptr;
   bool pinned = false;  // bytes / crumbs and offsets are page-locked: the copy engine reads them in place
+  bool strands = false;  // nucleotide, both strands: query q is searched as the virtual queries 2q and 2q + 1 (its
+                         // reverse complement), whose results and CSR entries the outputs hold
+  uint64_t per_query() const { return strands ? 2 : 1; }  // virtual queries (result slots) per query
 };
 
 // The chunker binary-searches the offsets and sizes every buffer from a chunk's byte range, so the ends of
@@ -230,13 +233,18 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
                     const Chunk& c, SearchOut mode, bool may_pack = true, bool probe_link = false, bool copy_flag = true,
                     void* d_out_override = nullptr) {
   const uint64_t nq = c.q1 - c.q0, nbytes = c.b1 - c.b0;
+  const uint64_t nv = nq * qs.per_query();  // queries searched
   const size_t out_elem = mode == OUT_COUNT_U64 ? 8 : mode == OUT_RANGE_U64 ? 16 : sp_cnt_bytes(r.view);
   const int ush = packed_unit_shift(ix->alphabet);
   Workspace::grow_dev(ws->d_qbytes, ws->d_qbytes_cap, size_t(nbytes) + 16);
   Workspace::grow_dev(ws->d_qoff, ws->d_qoff_cap, size_t(nq) + 1);
   Workspace::grow_dev(ws->d_qwords, ws->d_qwords_cap, size_t(packed_words(ix->alphabet, nq, nbytes)));
-  Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nq) * out_elem);
-  Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nq));
+  Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nv) * out_elem);
+  Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nv));
+  if (qs.strands) {
+    Workspace::grow_dev(ws->d_voff, ws->d_voff_cap, size_t(nv) + 1);
+    Workspace::grow_dev(ws->d_vwords, ws->d_vwords_cap, size_t(packed_words(0, nv, 2 * nbytes)));
+  }
   const uint64_t* src_o = qs.qoff + c.q0;
   uint64_t* const d_words = ws->d_qwords - 4 * (c.b0 >> ush);
   SearchVariant v = current_variant();
@@ -357,12 +365,25 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
       g_prof.h2d += nbytes;
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
       // offsets stay absolute: the kernels subtract the chunk's byte base
-      in_wave = search_packs_ascii(r.view, mode, v);
+      in_wave = qs.strands ? search_strands_ascii(r.view, mode, v) : search_packs_ascii(r.view, mode, v);
       if (!in_wave) {
         ProfScope p(2, r.device, ws->st);
         CU(launch_pack(ix->alphabet, ws->d_qbytes - c.b0, ws->d_qoff, nq, d_words, c.b0, c.b1, ws->d_flag, ws->st));
       }
     }
+  }
+  // both strands: the virtual queries (kernels.hpp); the strand wave kernel stages them from the bytes itself
+  const uint64_t* d_soff = ws->d_qoff;
+  const uint64_t* d_swords = d_words;
+  SearchVariant sv = v;
+  if (qs.strands) {
+    uint64_t* const d_vwords = ws->d_vwords - 4 * ((2 * c.b0) >> 6);
+    CU(launch_strand_offsets(ws->d_qoff, nq, c.b0, c.b1, ws->d_voff, ws->st));
+    if (!in_wave) CU(launch_strand_words(d_words, ws->d_qoff, nq, c.b0, c.b1, ws->d_voff, d_vwords, ws->st));
+    d_soff = ws->d_voff;
+    d_swords = d_vwords;
+    sv.b_lo = 2 * c.b0;
+    sv.b_hi = 2 * c.b1;
   }
   gpu_mark(ws->st, "packed on device", (long long)c.q0);
   {
@@ -379,10 +400,10 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
     }
     void* const d_out = d_out_override ? d_out_override : ws->d_out;
     if (in_wave)
-      CU(launch_search_ascii(r.view, ws->d_qbytes - c.b0, ws->d_qoff, nq, d_words, ws->d_flag, mode, d_out, ws->d_defer, v,
-                             r.sm_count, ws->st));
+      CU(launch_search_ascii(r.view, ws->d_qbytes - c.b0, d_soff, nv, const_cast<uint64_t*>(d_swords), ws->d_flag, mode,
+                             d_out, ws->d_defer, sv, r.sm_count, ws->st, qs.strands));
     else
-      CU(launch_search(r.view, d_words, ws->d_qoff, nq, mode, d_out, ws->d_defer, v, r.sm_count, ws->st));
+      CU(launch_search(r.view, d_swords, d_soff, nv, mode, d_out, ws->d_defer, sv, r.sm_count, ws->st));
     if (time_kernel) {
       CU(cudaEventRecord(ws->ev_s1, ws->st));
       ws->gpu_probe_bytes = nbytes;
@@ -415,7 +436,7 @@ void search_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, u
   Replica& r = *ix->reps[ri];
   PackBalance& bal = ix->balance_of(ri);
   DeviceGuard dg(r.device);
-  const size_t out_elem = mode == OUT_COUNT_U64 ? 8 : 16;
+  const size_t out_elem = (mode == OUT_COUNT_U64 ? 8 : 16) * qs.per_query();  // per query
   const uint64_t* qoff = qs.qoff;
   const bool src_pinned = qs.pinned;
   const bool dst_pinned = is_pinned(out);
@@ -638,7 +659,8 @@ static uint64_t locate_chunk_bytes() {
 void locate_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, uint64_t q_lo, uint64_t q_hi,
                        uint32_t flags, LocatePart& part) {
   const bool ext = part.ext_cap != 0 || part.ext_off != nullptr;
-  if (!part.ext_off) part.hit_off.assign(q_hi - q_lo + 1, 0);
+  const uint64_t m = qs.per_query();  // CSR entries per query
+  if (!part.ext_off) part.hit_off.assign(m * (q_hi - q_lo) + 1, 0);
   uint64_t* off_base = part.ext_off ? part.ext_off : part.hit_off.data();
   if (q_lo >= q_hi) return;
   Replica& r = *ix->reps[ri];
@@ -663,8 +685,8 @@ void locate_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, u
     if (s.phase != 2) return;
     const Chunk& c = chunks[size_t(s.chunk)];
     CU(cudaEventSynchronize(s.ws->done));
-    uint64_t* dst_off = off_base + (c.q0 - q_lo);
-    const uint64_t nq = c.q1 - c.q0, base = s.base;
+    uint64_t* dst_off = off_base + m * (c.q0 - q_lo);
+    const uint64_t nq = m * (c.q1 - c.q0), base = s.base;
     if (base)
       for (uint64_t i = 0; i < nq; i++) dst_off[i] += base;
     s.phase = 0;
@@ -676,7 +698,7 @@ void locate_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, u
     stage_c(s);
     Workspace* ws = s.ws;
     const Chunk& c = chunks[size_t(i)];
-    const uint64_t nq = c.q1 - c.q0;
+    const uint64_t nq = m * (c.q1 - c.q0);
     mark("A begin", i);
     gpu_mark(ws->st, "chunk begins", i);
     enqueue_search(ix, r, bal, ws, qs, c, OUT_SP_CNT_U32, true, false, false);
@@ -696,7 +718,7 @@ void locate_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, u
     Slot& s = slot[i % DEPTH];
     Workspace* ws = s.ws;
     const Chunk& c = chunks[size_t(i)];
-    const uint64_t nq = c.q1 - c.q0;
+    const uint64_t nq = m * (c.q1 - c.q0);
     mark("B wait", i);
     CU(cudaEventSynchronize(ws->done));
     mark("B total known", i);
@@ -704,7 +726,7 @@ void locate_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, u
     check_flag(ws, c);
     s.base = part.n_hits;
     gpu_mark(ws->st, "pass 2 begins", i);
-    CU(cudaMemcpyAsync(off_base + (c.q0 - q_lo), ws->d_hit_off, nq * 8, cudaMemcpyDeviceToHost, ws->st));
+    CU(cudaMemcpyAsync(off_base + m * (c.q0 - q_lo), ws->d_hit_off, nq * 8, cudaMemcpyDeviceToHost, ws->st));
     gpu_mark(ws->st, "offsets copied", i);
     g_prof.d2h += nq * 8;
     const bool fits = !ext || part.n_hits + n_hits <= part.ext_cap;
@@ -737,7 +759,7 @@ void locate_on_replica(const awry_index* ix, size_t ri, const QuerySource& qs, u
       stage_b(i);
     }
     for (auto& s : slot) stage_c(s);
-    off_base[q_hi - q_lo] = part.n_hits;
+    off_base[m * (q_hi - q_lo)] = part.n_hits;
     mark("done", int(chunks.size()));
     g_gpu_trace = nullptr;
     gpu_trace.dump();
@@ -786,6 +808,7 @@ uint64_t locate_direct_on_replica(const awry_index* ix, size_t ri, const QuerySo
     first_raw = true;
   }
   const bool off_pinned = is_pinned(hit_off);
+  const uint64_t m = qs.per_query();  // CSR entries per query
   constexpr int DEPTH = 3;
   Workspace* ws[DEPTH] = {nullptr, nullptr, nullptr};
   int pending[DEPTH] = {-1, -1, -1};
@@ -794,7 +817,7 @@ uint64_t locate_direct_on_replica(const awry_index* ix, size_t ri, const QuerySo
     const Chunk& c = chunks[size_t(pending[s])];
     CU(cudaEventSynchronize(ws[s]->done));
     check_flag(ws[s], c);
-    if (!off_pinned) memcpy(hit_off + c.q0, ws[s]->h_out, (c.q1 - c.q0) * 8);
+    if (!off_pinned) memcpy(hit_off + m * c.q0, ws[s]->h_out, m * (c.q1 - c.q0) * 8);
     pending[s] = -1;
   };
   GpuTrace gpu_trace;
@@ -812,7 +835,7 @@ uint64_t locate_direct_on_replica(const awry_index* ix, size_t ri, const QuerySo
       finish(s);
       Workspace* w = ws[s];
       const Chunk& c = chunks[i];
-      const uint64_t n = c.q1 - c.q0;
+      const uint64_t n = m * (c.q1 - c.q0);
       gpu_mark(w->st, "chunk begins", (long long)i);
       enqueue_search(ix, r, bal, w, qs, c, OUT_SP_CNT_U32, !(first_raw && i == 0), false, false);
       Workspace::grow_dev(w->d_hit_off, w->d_hit_off_cap, size_t(n) + 1);
@@ -825,7 +848,7 @@ uint64_t locate_direct_on_replica(const awry_index* ix, size_t ri, const QuerySo
                               hits_dev, capacity, w->d_off_out, r.sm_count, prev_adv, w->ev_adv, w->st));
       prev_adv = w->ev_adv;
       gpu_mark(w->st, "hits written", (long long)i);
-      uint64_t* dst = hit_off + c.q0;
+      uint64_t* dst = hit_off + m * c.q0;
       if (!off_pinned) {
         Workspace::grow_host(w->h_out, w->h_out_cap, size_t(n) * 8);
         dst = reinterpret_cast<uint64_t*>(w->h_out);
@@ -841,7 +864,7 @@ uint64_t locate_direct_on_replica(const awry_index* ix, size_t ri, const QuerySo
     for (int s = 0; s < DEPTH; s++) finish((last + 1 + s) % DEPTH);  // oldest first; the last chunk carries the total
     total = *ws[last]->h_total;
     g_prof.d2h += std::min(total, capacity) * sizeof(awry_hit);
-    hit_off[nq] = total;
+    hit_off[m * nq] = total;
     g_gpu_trace = nullptr;
     gpu_trace.dump();
   } catch (...) {
@@ -939,15 +962,16 @@ void locate_owned_impl(const awry_index* ix, const QuerySource& qs, uint64_t nq,
     }
   }
   uint64_t base = 0;
+  const uint64_t m = qs.per_query();
   for (size_t ri = 0; ri < nr; ri++) {
     auto [lo, hi] = ranges[ri];
     if (hi > lo)
-      for (uint64_t i = 0; i <= hi - lo; i++) hit_off[lo + i] = base + parts[ri].hit_off[i];
+      for (uint64_t i = 0; i <= m * (hi - lo); i++) hit_off[m * lo + i] = base + parts[ri].hit_off[i];
     if (nr > 1 && parts[ri].n_hits) memcpy(all + base, parts[ri].hits, parts[ri].n_hits * sizeof(awry_hit));
     base += parts[ri].n_hits;
     if (nr > 1) free(parts[ri].hits);
   }
-  hit_off[nq] = total;
+  hit_off[m * nq] = total;
   *hits = all;
   *n_hits = total;
 }
@@ -970,7 +994,8 @@ void locate_multi_phase1(const awry_index* ix, size_t ri, const QuerySource& qs,
   Replica& r = *ix->reps[ri];
   PackBalance& bal = ix->balance_of(ri);
   DeviceGuard dg(r.device);
-  const uint64_t n = st.hi - st.lo;
+  const uint64_t m = qs.per_query();
+  const uint64_t n = m * (st.hi - st.lo);  // CSR entries
   const uint64_t max_bytes = std::min(chunk_max_bytes(), locate_chunk_bytes());
   auto chunks = make_chunks(qs.qoff, st.lo, st.hi, locate_chunk_q(), max_bytes);
   validate_chunks(chunks, max_bytes);
@@ -996,7 +1021,7 @@ void locate_multi_phase1(const awry_index* ix, size_t ri, const QuerySource& qs,
       finish(s);
       const Chunk& c = chunks[i];
       enqueue_search(ix, r, bal, ws[s], qs, c, OUT_SP_CNT_U32, true, false, true,
-                     top->d_out + size_t(c.q0 - st.lo) * pair_bytes);
+                     top->d_out + size_t(m * (c.q0 - st.lo)) * pair_bytes);
       CU(cudaEventRecord(ws[s]->done, ws[s]->st));
       pending[s] = int(i);
     }
@@ -1021,19 +1046,19 @@ void locate_multi_phase1(const awry_index* ix, size_t ri, const QuerySource& qs,
 }
 
 void locate_multi_phase2(const awry_index* ix, size_t ri, ReplicaLocateState& st, uint64_t* hit_off, void* hits_dev,
-                         uint64_t capacity) {
+                         uint64_t capacity, uint64_t m) {
   if (st.lo >= st.hi || !st.ws) return;
   Replica& r = *ix->reps[ri];
   DeviceGuard dg(r.device);
   Workspace* top = st.ws;
-  const uint64_t n = st.hi - st.lo;
+  const uint64_t n = m * (st.hi - st.lo);  // CSR entries
   const bool off_pinned = is_pinned(hit_off);
   try {
     unsigned long long base = st.base;
     CU(cudaMemcpyAsync(top->d_base + 1, &base, 8, cudaMemcpyHostToDevice, top->st));  // (pageable source: copied at the call)
     CU(launch_gather_direct(r.view, reinterpret_cast<const uint2*>(top->d_out), top->d_hit_off, n, top->d_base + 1, top->d_base,
                             hits_dev, capacity, top->d_off_out, r.sm_count, nullptr, nullptr, top->st));
-    uint64_t* dst = hit_off + st.lo;
+    uint64_t* dst = hit_off + m * st.lo;
     if (!off_pinned) {
       Workspace::grow_host(top->h_out, top->h_out_cap, size_t(n) * 8);
       dst = reinterpret_cast<uint64_t*>(top->h_out);
@@ -1041,7 +1066,7 @@ void locate_multi_phase2(const awry_index* ix, size_t ri, ReplicaLocateState& st
     CU(cudaMemcpyAsync(dst, top->d_off_out, n * 8, cudaMemcpyDeviceToHost, top->st));
     g_prof.d2h += n * 8 + std::min(st.total, capacity > st.base ? capacity - st.base : 0) * sizeof(awry_hit);
     CU(cudaStreamSynchronize(top->st));
-    if (!off_pinned) parallel_memcpy(hit_off + st.lo, top->h_out, n * 8);
+    if (!off_pinned) parallel_memcpy(hit_off + m * st.lo, top->h_out, n * 8);
   } catch (...) {
     cudaStreamSynchronize(top->st);
     r.release(top);
@@ -1105,9 +1130,9 @@ void locate_into_impl(const awry_index* ix, const QuerySource& qs, uint64_t nq, 
           total += x.total;
         }
         for_each_replica_range(ix, qs.qoff, nq, [&](size_t ri, uint64_t, uint64_t) {
-          locate_multi_phase2(ix, ri, st[ri], hit_off, hits_dev, capacity);
+          locate_multi_phase2(ix, ri, st[ri], hit_off, hits_dev, capacity, qs.per_query());
         });
-        hit_off[nq] = total;
+        hit_off[qs.per_query() * nq] = total;
         *n_hits = total;
       } catch (...) {
         release_all();
@@ -1367,6 +1392,54 @@ void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, 
   r.release(ws);
 }
 
+// ------------------------------------------------------------------ both strands (awry_*_strands)
+
+void strands_check_index(const awry_index* ix) {
+  if (ix->alphabet != AWRY_NUCLEOTIDE) fail(AWRY_ERR_UNSUPPORTED, "both-strand search exists for the nucleotide alphabet only");
+}
+
+// Device-resident batch of nq reads on both strands: the 2 nq virtual queries (kernels.hpp) searched into d_out, all on
+// stream `st`, scratch released in stream order with `sc`.  The strand wave kernel reads the bytes itself; otherwise
+// pack_kernel packs the reads and launch_strand_words derives the virtual words.  What the prepass refuses is latched
+// in r.d_async_flag.  Returns whether pass 1 stored one-hit queries as text positions (locate_positions).
+bool strands_search_device(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t e0, uint64_t e1,
+                           SearchOut mode, void* d_out, uint32_t* d_defer, StreamScratch& sc, cudaStream_t st) {
+  const uint64_t nv = 2 * nq;
+  uint64_t* const d_voff = sc.get<uint64_t>(nv + 1);
+  uint64_t* const d_vwords = sc.get<uint64_t>(packed_words(0, nv, 2 * (e1 - e0))) - 4 * ((2 * e0) >> 6);
+  SearchVariant v = current_variant();
+  v.avg_len = uint32_t(std::min<uint64_t>((e1 - e0) / nq, 1u << 30));
+  v.b_lo = 2 * e0;
+  v.b_hi = 2 * e1;
+  v.locate_positions = mode == OUT_SP_CNT_U32 && locate_positions_ok(r.view, v);
+  CU(launch_strand_offsets(d_qoff, nq, e0, e1, d_voff, st));
+  ProfScope p(0, r.device, st);
+  if (search_strands_ascii(r.view, mode, v)) {
+    CU(launch_search_ascii(r.view, d_qbytes, d_voff, nv, d_vwords, r.d_async_flag, mode, d_out, d_defer, v, r.sm_count, st,
+                           true));
+  } else {
+    uint64_t* const d_words = sc.get<uint64_t>(packed_words(0, nq, e1 - e0)) - 4 * (e0 >> 6);
+    CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_words, e0, e1, r.d_async_flag, st));
+    CU(launch_strand_words(d_words, d_qoff, nq, e0, e1, d_voff, d_vwords, st));
+    CU(launch_search(r.view, d_vwords, d_voff, nv, mode, d_out, d_defer, v, r.sm_count, st));
+  }
+  return v.locate_positions;
+}
+
+// the first and last offset of a device-resident batch (one 16-byte read-back), checked
+void device_batch_ends(const uint64_t* d_qoff, uint64_t nq, cudaStream_t st, uint64_t ends[2]) {
+  CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
+  if (ends[1] >= (1ull << 62)) fail(AWRY_ERR_INVALID_ARG, "query offsets beyond 2^62");
+}
+
+void strands_check_device_batch(uint64_t nq) {
+  if (2 * nq >= (1ull << 32) - (1u << 24))  // (the search kernels' 32-bit ticket counter)
+    fail(AWRY_ERR_INVALID_ARG, "batch too large for one both-strand search (%llu reads): split it", (unsigned long long)nq);
+}
+
 }  // namespace host
 }  // namespace awry
 
@@ -1616,6 +1689,97 @@ int awry_count_device_hamming(const awry_index* ix, int replica, const uint8_t* 
     CU(cudaStreamSynchronize(st));
     if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
     hamming_run(r, d_qbytes, d_qoff, nq, ends[0], ends[1], max_mismatches, r.d_async_flag, -1, st, d_counts, nullptr);
+  });
+}
+
+int awry_count_batch_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                             uint64_t* counts) {
+  return guarded([&] {
+    need(ix);
+    strands_check_index(ix);
+    if (nq == 0) return;
+    if (!qbytes || !qoff || !counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    QuerySource qs = ascii_source(qbytes, qoff);
+    qs.strands = true;
+    count_impl(ix, qs, nq, OUT_COUNT_U64, counts);
+  });
+}
+
+int awry_locate_batch_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                              uint32_t flags, uint64_t* hit_off, awry_hit* hits, uint64_t capacity, uint64_t* n_hits) {
+  return guarded([&] {
+    need(ix);
+    if (!hit_off || !n_hits || (!hits && capacity)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    *n_hits = 0;
+    hit_off[0] = 0;
+    strands_check_index(ix);
+    if (nq == 0) return;
+    if (!qbytes || !qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    QuerySource qs = ascii_source(qbytes, qoff);
+    qs.strands = true;
+    locate_into_impl(ix, qs, nq, flags, hit_off, hits, capacity, n_hits);
+  });
+}
+
+int awry_count_device_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                              uint64_t nq, uint64_t* d_counts, void* cuda_stream) {
+  return guarded([&] {
+    need(ix);
+    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+    strands_check_index(ix);
+    if (nq == 0) return;
+    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    strands_check_device_batch(nq);
+    Replica& r = *ix->reps[size_t(replica)];
+    DeviceGuard dg(r.device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    uint64_t ends[2] = {0, 0};
+    device_batch_ends(d_qoff, nq, st, ends);
+    StreamScratch sc(st);
+    strands_search_device(r, d_qbytes, d_qoff, nq, ends[0], ends[1], OUT_COUNT_U64, d_counts,
+                          sc.get<uint32_t>(defer_words(2 * nq)), sc, st);
+  });
+}
+
+int awry_locate_device_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                               uint64_t nq, uint32_t flags, uint64_t* d_hit_off, awry_hit** d_hits, uint64_t* n_hits,
+                               void* cuda_stream) {
+  return guarded([&] {
+    need(ix);
+    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+    if (!d_hit_off || !d_hits || !n_hits) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    *d_hits = nullptr;
+    *n_hits = 0;
+    strands_check_index(ix);
+    if (nq == 0) return;
+    if (!d_qbytes || !d_qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    strands_check_device_batch(nq);
+    Replica& r = *ix->reps[size_t(replica)];
+    DeviceGuard dg(r.device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    uint64_t ends[2] = {0, 0};
+    device_batch_ends(d_qoff, nq, st, ends);
+    Workspace* ws = r.acquire();
+    try {
+      const uint64_t nv = 2 * nq;
+      Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nv) * sp_cnt_bytes(r.view));
+      Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nv));
+      {
+        StreamScratch sc(st);
+        ws->sp_cnt_positions =
+            strands_search_device(r, d_qbytes, d_qoff, nq, ends[0], ends[1], OUT_SP_CNT_U32, ws->d_out, ws->d_defer, sc, st);
+      }
+      uint64_t n = 0;
+      uint64_t* h = locate_chunk_device(ix, r, ws, nv, flags, d_hit_off, &n, st);
+      CU(cudaStreamSynchronize(st));
+      *d_hits = reinterpret_cast<awry_hit*>(h);
+      *n_hits = n;
+    } catch (...) {
+      cudaStreamSynchronize(st);
+      r.release(ws);
+      throw;
+    }
+    r.release(ws);
   });
 }
 

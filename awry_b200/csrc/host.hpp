@@ -198,6 +198,10 @@ struct Workspace {
   cudaEvent_t ev_adv = nullptr;  // recorded after the chunk's advance_hit_base_kernel
   uint64_t* d_off_out = nullptr;  // rebased CSR offsets of the chunk, on their way to the caller
   size_t d_off_out_cap = 0;
+  uint64_t* d_voff = nullptr;  // both strands: the chunk's virtual offsets and words (kernels.hpp)
+  size_t d_voff_cap = 0;
+  uint64_t* d_vwords = nullptr;
+  size_t d_vwords_cap = 0;
   // reads-file front-end scratch, kept across calls (pinned allocations cost ~0.4 ms per MiB)
   struct ReadsScratch {
     uint64_t chunk = 0, carry = 0;
@@ -283,6 +287,8 @@ struct Workspace {
     cudaFree(d_flag);
     cudaFree(d_base);
     cudaFree(d_off_out);
+    cudaFree(d_voff);
+    cudaFree(d_vwords);
     if (ev_adv) cudaEventDestroy(ev_adv);
     rs.release();
     if (ev_a) cudaEventDestroy(ev_a);

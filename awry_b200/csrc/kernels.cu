@@ -565,7 +565,9 @@ cudaError_t build_pair_index(const IndexView& ix, uint4* d_pair_blocks, uint32_t
 // PL lanes per query; lane t packs words t, t+PL, ...  Flags the first empty / sentinel query.
 // The ASCII table is copied to shared memory first: per-lane indices differ, and divergent
 // constant-bank reads would serialise.
-template <int ALPHA>
+// RC (nucleotide): the words of the query's reverse complement instead -- search-order symbol si is the complement
+// of text byte si (codes below 4 XOR 3; N and the sentinel stay).
+template <int ALPHA, bool RC = false>
 __device__ __forceinline__ uint64_t pack_word_bytes(const uint8_t* __restrict__ src, uint32_t len, uint32_t first,
                                                     const uint8_t* lut, bool& bad) {
   constexpr int BITS = ALPHA == 0 ? 4 : 8;
@@ -576,26 +578,30 @@ __device__ __forceinline__ uint64_t pack_word_bytes(const uint8_t* __restrict__ 
   for (int t = 0; t < SPW; t++) {
     uint32_t si = first + t;
     if (si < len) {
-      uint32_t d = lut[src[len - 1 - si]];
+      uint32_t d = lut[src[RC ? si : len - 1 - si]];
       bad |= d == SENT;
+      if (RC && d < 4) d ^= 3u;
       word |= uint64_t(d) << (BITS * t);
     }
   }
   return word;
 }
 
-// 4 ASCII bases (the first in the low byte) -> their 4 codes as nibbles in search order (the last base in the low
+// 4 ASCII bases (the first in the low byte) -> their 4 codes as nibbles in the same order (the first base in the low
 // nibble), SIMD-in-register: ((c & 0xDF) >> 1) & 3 maps A,C,T,G to 0,1,2,3 and x ^ (x >> 1) swaps the last two.
 // `diff` gets a non-zero byte for every byte that is not one of ACGT/acgt (whose nibble is then meaningless).
-__device__ __forceinline__ uint32_t ascii4_to_nibbles(uint32_t w4, uint32_t& diff) {
-  const uint32_t rev = __byte_perm(w4, 0, 0x0123);  // search order: last byte first
-  const uint32_t up = rev & 0xDFDFDFDFu;
+__device__ __forceinline__ uint32_t ascii4_codes(uint32_t w4, uint32_t& diff) {
+  const uint32_t up = w4 & 0xDFDFDFDFu;
   const uint32_t x4 = (up >> 1) & 0x03030303u;
   const uint32_t c4 = x4 ^ ((x4 >> 1) & 0x01010101u);
   const uint32_t sel = c4 | (c4 >> 4);
   const uint32_t nib = (sel & 0xffu) | ((sel >> 8) & 0xff00u);  // 4 nibbles = 4 codes
   diff = up ^ __byte_perm(0x54474341u, 0, nib);                 // "ACGT"[code] per byte
   return nib;
+}
+// ... in search order (the last base in the low nibble)
+__device__ __forceinline__ uint32_t ascii4_to_nibbles(uint32_t w4, uint32_t& diff) {
+  return ascii4_codes(__byte_perm(w4, 0, 0x0123), diff);
 }
 
 template <int ALPHA, int PL = 8>
@@ -790,6 +796,80 @@ __global__ void fill_offsets_kernel(uint64_t* __restrict__ qoff, uint64_t first,
 }
 cudaError_t launch_fill_offsets(uint64_t* d_qoff, uint64_t first, uint64_t len, uint64_t n, cudaStream_t s) {
   fill_offsets_kernel<<<unsigned((n + 256) / 256), 256, 0, s>>>(d_qoff, first, len, n);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
+// ---- both strands: virtual offsets and words (kernels.hpp) ----
+__global__ void strand_offsets_kernel(const uint64_t* __restrict__ qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+                                      uint64_t* __restrict__ voff) {
+  const uint64_t q = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x;
+  if (q > nq) return;
+  const uint64_t o0 = qoff[q];
+  voff[2 * q] = 2 * o0;
+  if (q == nq) return;
+  const uint64_t o1 = qoff[q + 1];
+  const bool ok = o0 >= b_lo && o1 <= b_hi && o1 >= o0 && o1 - o0 < (1ull << 32);  // checked_len's rule
+  voff[2 * q + 1] = ok ? o0 + o1 : ~0ull;
+}
+
+cudaError_t launch_strand_offsets(const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi, uint64_t* d_voff,
+                                  cudaStream_t s) {
+  strand_offsets_kernel<<<unsigned((nq + 256) / 256), 256, 0, s>>>(d_qoff, nq, b_lo, b_hi, d_voff);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
+// 16 nibbles -> the same 16 in reverse order
+__device__ __forceinline__ uint64_t reverse_nibbles(uint64_t x) {
+  x = ((x >> 4) & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);
+  const uint32_t lo = uint32_t(x), hi = uint32_t(x >> 32);
+  return (uint64_t(__byte_perm(lo, 0, 0x0123)) << 32) | __byte_perm(hi, 0, 0x0123);
+}
+
+// 4 lanes per read; lane `sub` writes words sub, sub + 4, ... of both virtual queries.  Reverse-complement word w holds
+// search-order symbols 16 w .. 16 w + 15 = the complements of the read's symbols L - 1 - 16 w down to L - 16 w - 16,
+// which span at most two of the read's words.
+__global__ void __launch_bounds__(256)
+    strand_words_kernel(const uint64_t* __restrict__ qwords, const uint64_t* __restrict__ qoff, uint64_t nq,
+                        ByteRange br, const uint64_t* __restrict__ voff, uint64_t* __restrict__ vwords) {
+  const uint32_t sub = threadIdx.x & 3;
+  const uint64_t ngroups = (gridDim.x * uint64_t(blockDim.x)) >> 2;
+  for (uint64_t q = (blockIdx.x * uint64_t(blockDim.x) + threadIdx.x) >> 2; q < nq; q += ngroups) {
+    const uint64_t o0 = qoff[q], o1 = qoff[q + 1];
+    const uint32_t len = checked_len(o0, o1, br);
+    if (len == 0) continue;  // refused by the prepass (its words do not exist) or empty
+    const uint32_t nwords = (len + 15) >> 4;
+    const uint64_t* const src = qwords + 4 * (q + (o0 >> 6));
+    uint64_t* const fwd = vwords + 4 * (2 * q + (voff[2 * q] >> 6));
+    uint64_t* const rev = vwords + 4 * (2 * q + 1 + (voff[2 * q + 1] >> 6));
+    for (uint32_t w = sub; w < nwords; w += 4) {
+      fwd[w] = src[w];
+      // read symbols [a, a + 16) with a = L - 16 w - 16 (those below 0 do not exist)
+      const int a = int(len) - 16 * int(w) - 16;
+      uint64_t x;
+      if (a >= 0) {
+        const uint32_t wi = uint32_t(a) >> 4, sh = 4 * (uint32_t(a) & 15);
+        const uint64_t lo = src[wi], hi = sh && 16 * (wi + 1) < len ? src[wi + 1] : 0ull;
+        x = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
+      } else {
+        x = src[0] << (4 * uint32_t(-a));
+      }
+      x = reverse_nibbles(x);
+      const uint64_t lt4 = ~(x >> 2) & 0x1111111111111111ull;  // codes below 4 (bit 2 clear)
+      x ^= lt4 | (lt4 << 1);
+      const uint32_t have = len - 16 * w;                       // symbols of this word (the rest stay 0)
+      if (have < 16) x &= (1ull << (4 * have)) - 1;
+      rev[w] = x;
+    }
+  }
+}
+
+cudaError_t launch_strand_words(const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+                                const uint64_t* d_voff, uint64_t* d_vwords, cudaStream_t s) {
+  if (nq == 0) return cudaSuccess;
+  const unsigned grid = unsigned(std::min<uint64_t>((nq * 4 + 255) / 256, 148 * 64));
+  strand_words_kernel<<<grid, 256, 0, s>>>(d_qwords, d_qoff, nq, ByteRange{b_lo, b_hi}, d_voff, d_vwords);
   COUNT_LAUNCH();
   return cudaGetLastError();
 }
@@ -1399,6 +1479,52 @@ __device__ __forceinline__ uint32_t stage_ascii_ring(uintptr_t b, uintptr_t e, b
   return dirty;
 }
 
+// The same for the strand flavour, whose lanes with `rc` set stage the ring of the read's reverse complement: its
+// search order is the read's text order with every code complemented.  Their sectors are counted from the read's START
+// (sector k holds bytes [b32 + 32 k, b32 + 32 k + 32), b32 = b rounded down to 32, pad = b - b32) and convert without
+// the byte reversal, XOR 3 per code; the ring halves and the hand-over between lanes are the same, so both strands of a
+// read load the same sectors.  (A function of its own: the single-strand kernels keep their code as it was.)
+__device__ __forceinline__ uint32_t stage_strand_ring(uintptr_t b, uintptr_t e, bool run, uint32_t sub, uint32_t gbase,
+                                                      uint64_t* ring, bool r) {
+  constexpr uint32_t FULL = 0xffffffffu;
+  const uint32_t nsec = run ? uint32_t(((e - 1) >> 5) - (b >> 5)) + 1 : 0u;
+  const uintptr_t end32 = (e + 31) & ~uintptr_t(31), b32 = b & ~uintptr_t(31);
+  const uint32_t pad = r ? uint32_t(b - b32) : uint32_t(end32 - e), ph = pad >> 3, pl4 = 4 * (pad & 7);
+  uint32_t* const r32 = reinterpret_cast<uint32_t*>(ring);
+  uint32_t dirty = 0, carry = 0;
+  const int rounds = int(__reduce_max_sync(FULL, (nsec + 3) >> 2));
+#pragma unroll 1
+  for (int i = rounds - 1; i >= 0; i--) {
+    const uint32_t k = sub + 4u * uint32_t(i);
+    uint32_t h[5] = {0u, 0u, 0u, 0u, 0u};
+    if (k < nsec) {
+      const uintptr_t at = r ? b32 + 32 * uintptr_t(k) : end32 - 32 * uintptr_t(k + 1);
+      const u32x8 t = ldg256(reinterpret_cast<const void*>(at));
+      uint32_t nib[8];
+#pragma unroll
+      for (int j = 0; j < 8; j++) {
+        uint32_t diff;
+        nib[j] = ascii4_codes(__byte_perm(t.v[j], 0, r ? 0x3210u : 0x0123u), diff) ^ (r ? 0x3333u : 0u);
+        dirty |= diff;
+      }
+#pragma unroll
+      for (int j = 0; j < 4; j++)
+        h[j] = r ? nib[2 * j] | (nib[2 * j + 1] << 16) : nib[7 - 2 * j] | (nib[6 - 2 * j] << 16);
+    }
+    const uint32_t x = __shfl_sync(FULL, h[0], gbase + ((sub + 1) & 3));
+    h[4] = sub == 3 ? carry : x;
+    carry = x;
+    if (k < nsec) {
+#pragma unroll
+      for (int j = 0; j < 4; j++) {
+        const int m = int(4 * k) - int(ph) + j;
+        if (m >= 0 && m < 32) r32[m] = __funnelshift_r(h[j], h[j + 1], pl4);
+      }
+    }
+  }
+  return dirty;
+}
+
 // whether bytes [src, src + len) hold anything but ACGT/acgt (the group's 4 lanes take every 4th byte)
 __device__ __forceinline__ uint32_t read_is_dirty(const uint8_t* src, uint32_t len, uint32_t sub) {
   uint32_t dirty = 0;
@@ -1411,20 +1537,30 @@ __device__ __forceinline__ uint32_t read_is_dirty(const uint8_t* src, uint32_t l
 }
 
 // a query the ASCII wave kernel hands on without a ring: its words by pack_kernel's table path, which also latches a
-// sentinel (the group's 4 lanes take words sub, sub + 4, ...)
+// sentinel (the group's 4 lanes take words sub, sub + 4, ...); rc: the words of its reverse complement
+template <bool STRAND = false>
 __device__ __forceinline__ void pack_query_lut(const uint8_t* src, uint32_t len, uint32_t nwords, uint64_t* dst,
-                                               uint32_t sub, const uint8_t* lut, uint64_t q, unsigned long long* first_bad) {
+                                               uint32_t sub, const uint8_t* lut, uint64_t q, unsigned long long* first_bad,
+                                               bool rc = false) {
   bool bad = false;
-  for (uint32_t wi = sub; wi < nwords; wi += 4) dst[wi] = pack_word_bytes<0>(src, len, wi << 4, lut, bad);
+  for (uint32_t wi = sub; wi < nwords; wi += 4)
+    dst[wi] = STRAND && rc ? pack_word_bytes<0, true>(src, len, wi << 4, lut, bad) : pack_word_bytes<0>(src, len, wi << 4, lut, bad);
   if (bad) atomicMin(first_bad, bad_query_code(q, BAD_QUERY));
 }
 
-template <int MODE, int TPB, int MINB, bool ASCII = false>
-__global__ void __launch_bounds__(TPB, MINB)
-    search_dna_wave_kernel(IndexView ix, const uint64_t* __restrict__ qwords, const uint64_t* __restrict__ qoff,
-                           uint64_t nq, void* __restrict__ out, uint32_t* __restrict__ defer, uint32_t ticket_sz,
-                           ByteRange br, const uint8_t* __restrict__ qbytes, uint64_t* qw_out,
-                           unsigned long long* first_bad) {
+// STRAND (ASCII flavour for both strands, launch_search_ascii with strands): the kernel hands out the batch's VIRTUAL
+// queries v = 2q (read q) and v = 2q + 1 (its reverse complement); `qoff` and `br` are the virtual offsets of
+// launch_strand_offsets and their byte range, from which the read's own ends are recovered (qoff[2q] / 2,
+// qoff[2q + 2] / 2; a refused read has qoff[2q + 1] = ~0).  The two strands of a read sit in neighbouring lane groups
+// of a warp (tickets and waves start at even v) and stage their rings from the same sectors; results, lists and
+// handed-on words are per virtual query, what the kernel latches names the read.
+template <int MODE, int TPB, bool ASCII, bool STRAND>
+__device__ __forceinline__ void search_dna_wave(const IndexView& ix, const uint64_t* __restrict__ qwords,
+                                                const uint64_t* __restrict__ qoff, uint64_t nq, void* __restrict__ out,
+                                                uint32_t* __restrict__ defer, uint32_t ticket_sz, const ByteRange& br,
+                                                const uint8_t* __restrict__ qbytes, uint64_t* qw_out,
+                                                unsigned long long* first_bad) {
+  static_assert(ASCII || !STRAND, "the strand flavour reads the caller's bytes");
   constexpr uint32_t FULL = 0xffffffffu;
   enum : uint32_t { W_NONE = 0, W_RUN = 1, W_EMPTY = 2 };  // no query (or handed on) / in progress / refused by the prepass
   __shared__ uint64_t s_q[TPB / 4][16];
@@ -1456,18 +1592,29 @@ __global__ void __launch_bounds__(TPB, MINB)
 
     // ---- offsets
     uint64_t ov = 0;
-    if (st == W_RUN) ov = __ldg(qoff + q + (sub & 1));  // lanes 0/1 fetch both ends with one request
-    const uint64_t o0 = __shfl_sync(FULL, ov, gbase), o1 = __shfl_sync(FULL, ov, gbase + 1);
-    const uint32_t len = st == W_RUN ? checked_len(o0, o1, br) : 0u;
+    if (STRAND) {  // lanes 0/1/2: qoff[2r], qoff[2r + 1], qoff[2r + 2] of read r = q / 2
+      if (st == W_RUN && sub < 3) ov = __ldg(qoff + (q & ~1u) + sub);
+    } else if (st == W_RUN) {
+      ov = __ldg(qoff + q + (sub & 1));  // lanes 0/1 fetch both ends with one request
+    }
+    const uint64_t x0 = __shfl_sync(FULL, ov, gbase), x1 = __shfl_sync(FULL, ov, gbase + 1);
+    const uint64_t x2 = STRAND ? __shfl_sync(FULL, ov, gbase + 2) : 0ull;
+    const bool rc = STRAND && (q & 1u), refused = STRAND && x1 == ~0ull;
+    const uint64_t o0 = STRAND ? x0 >> 1 : x0, o1 = STRAND ? x2 >> 1 : x1;  // the read's bytes
+    const uint64_t vo0 = rc ? x1 : x0;                                      // the query's own offset (its word slot)
+    const uint32_t rq = STRAND ? q >> 1 : q;                                // the read (what is latched)
+    const ByteRange rbr = STRAND ? ByteRange{br.lo >> 1, br.hi >> 1} : br;
+    const uint32_t len = st == W_RUN && !refused ? checked_len(o0, o1, rbr) : 0u;
     if (st == W_RUN && len == 0) {
       st = W_EMPTY;
       if (ASCII && sub == 0)  // as pack_kernel: offsets outside [b_lo, b_hi] first, else the query is empty
-        atomicMin(first_bad, bad_query_code(q, o1 == o0 && o0 >= br.lo && o1 <= br.hi ? BAD_QUERY : BAD_OFFSETS));
+        atomicMin(first_bad,
+                  bad_query_code(rq, !refused && o1 == o0 && o0 >= rbr.lo && o1 <= rbr.hi ? BAD_QUERY : BAD_OFFSETS));
     }
     const uint32_t nwords = (len + 15) >> 4;
-    const uint32_t ubase = 4 * (q + uint32_t(o0 >> 6));
+    const uint32_t ubase = 4 * (q + uint32_t(vo0 >> 6));
     if (st == W_RUN && nwords > 16) {  // longer than the ring: the refilling kernel slides it
-      if (ASCII) pack_query_lut(qbytes + o0, len, nwords, qw_out + ubase, sub, s_lut, q, first_bad);
+      if (ASCII) pack_query_lut<STRAND>(qbytes + o0, len, nwords, qw_out + ubase, sub, s_lut, rq, first_bad, rc);
       if (sub == 0) rest[2 + atomicAdd(rest, 1u)] = q;
       st = W_NONE;
     }
@@ -1475,7 +1622,10 @@ __global__ void __launch_bounds__(TPB, MINB)
     uint32_t amb = 0;
     __syncwarp();  // the previous wave's ring reads are done
     if (ASCII) {
-      amb = stage_ascii_ring(uintptr_t(qbytes + o0), uintptr_t(qbytes + o1), st == W_RUN, sub, gbase, ring);
+      if (STRAND)
+        amb = stage_strand_ring(uintptr_t(qbytes + o0), uintptr_t(qbytes + o1), st == W_RUN, sub, gbase, ring, rc);
+      else
+        amb = stage_ascii_ring(uintptr_t(qbytes + o0), uintptr_t(qbytes + o1), st == W_RUN, sub, gbase, ring);
       // the first and last sector also hold bytes of the neighbouring reads: a group that saw a byte outside ACGT/acgt
       // looks again at its read's bytes alone (rare: a batch of clean reads never comes here)
       const uint32_t dirty_groups = __ballot_sync(FULL, amb != 0);
@@ -1492,7 +1642,7 @@ __global__ void __launch_bounds__(TPB, MINB)
     const uint32_t amb_groups = __ballot_sync(FULL, amb != 0);
     __syncwarp();
     if (st == W_RUN && (amb_groups & gmask) != 0) {  // the scalar kernel takes the whole query
-      if (ASCII) pack_query_lut(qbytes + o0, len, nwords, qw_out + ubase, sub, s_lut, q, first_bad);
+      if (ASCII) pack_query_lut<STRAND>(qbytes + o0, len, nwords, qw_out + ubase, sub, s_lut, rq, first_bad, rc);
       if (sub == 0) defer[1 + atomicAdd(defer, 1u)] = q;
       st = W_NONE;
     }
@@ -1615,6 +1765,24 @@ __global__ void __launch_bounds__(TPB, MINB)
       }
     }
   }
+}
+
+template <int MODE, int TPB, int MINB, bool ASCII = false>
+__global__ void __launch_bounds__(TPB, MINB)
+    search_dna_wave_kernel(IndexView ix, const uint64_t* __restrict__ qwords, const uint64_t* __restrict__ qoff,
+                           uint64_t nq, void* __restrict__ out, uint32_t* __restrict__ defer, uint32_t ticket_sz,
+                           ByteRange br, const uint8_t* __restrict__ qbytes, uint64_t* qw_out,
+                           unsigned long long* first_bad) {
+  search_dna_wave<MODE, TPB, ASCII, false>(ix, qwords, qoff, nq, out, defer, ticket_sz, br, qbytes, qw_out, first_bad);
+}
+
+template <int MODE, int TPB, int MINB>
+__global__ void __launch_bounds__(TPB, MINB)
+    search_dna_strand_wave_kernel(IndexView ix, const uint64_t* __restrict__ qwords, const uint64_t* __restrict__ qoff,
+                                  uint64_t nq, void* __restrict__ out, uint32_t* __restrict__ defer, uint32_t ticket_sz,
+                                  ByteRange br, const uint8_t* __restrict__ qbytes, uint64_t* qw_out,
+                                  unsigned long long* first_bad) {
+  search_dna_wave<MODE, TPB, true, true>(ix, qwords, qoff, nq, out, defer, ticket_sz, br, qbytes, qw_out, first_bad);
 }
 
 // ---- nucleotide pair kernel, NS queries per lane group, every load of a query's life in the same slot of
@@ -1981,7 +2149,7 @@ struct AsciiQueries {
   unsigned long long* first_bad = nullptr;
 };
 
-template <int MODE, bool ASCII = false>
+template <int MODE, bool ASCII = false, bool STRAND = false>
 static cudaError_t launch_search_wave(const IndexView& ix, const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq,
                                       void* d_out, uint32_t* d_defer, int sm_count, cudaStream_t s, uint32_t avg_len,
                                       ByteRange br, const AsciiQueries& a = AsciiQueries()) {
@@ -1990,7 +2158,7 @@ static cudaError_t launch_search_wave(const IndexView& ix, const uint64_t* d_qwo
   constexpr int TPB = 256, MINB = 6;
   cudaError_t e = cudaMemsetAsync(d_defer + nq + 2, 0, 8, s);  // count of the rest list, its ticket counter
   if (e != cudaSuccess) return e;
-  auto kern = search_dna_wave_kernel<MODE, TPB, MINB, ASCII>;
+  auto kern = STRAND ? search_dna_strand_wave_kernel<MODE, TPB, MINB> : search_dna_wave_kernel<MODE, TPB, MINB, ASCII>;
   auto kern_rest = search_dna_pair_kernel<MODE, TPB, 4, true, true>;  // (64 registers: the list-driven flavour spills at 48)
   int per_sm = 0, per_sm_rest = 0;
   if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, TPB, 0)) != cudaSuccess) return e;
@@ -2003,6 +2171,7 @@ static cudaError_t launch_search_wave(const IndexView& ix, const uint64_t* d_qwo
     return 0u;
   }();
   // a ticket = 4 waves of 8 queries per warp; small batches get one wave per ticket so that every warp draws some
+  // (tickets are multiples of 8: the strand flavour relies on waves that start at an even query)
   uint32_t ticket_sz = nq >= uint64_t(grid) * (TPB / 32) * 128 ? 32u : 8u;
   if (ticket_env) ticket_sz = ticket_env;
   e = launch_with_table_window(kern, grid, TPB, s, ix, ix, d_qwords, d_qoff, nq, d_out, d_defer, ticket_sz, br, a.qbytes,
@@ -2554,11 +2723,16 @@ bool search_packs_ascii(const IndexView& ix, SearchOut mode, const SearchVariant
   return !(e && e[0] == '0') && runs_wave_kernel(ix, mode, v);
 }
 
+bool search_strands_ascii(const IndexView& ix, SearchOut mode, const SearchVariant& v) {
+  const char* e = getenv("AWRY_B200_STRAND_WAVE");  // read per call: "0" keeps the generic route (A/B runs, tests)
+  return !(e && e[0] == '0') && search_packs_ascii(ix, mode, v);
+}
+
 cudaError_t launch_search_ascii(const IndexView& ix, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
                                 uint64_t* d_qwords, unsigned long long* d_first_bad, SearchOut mode, void* d_out,
-                                uint32_t* d_defer, const SearchVariant& v, int sm_count, cudaStream_t s) {
+                                uint32_t* d_defer, const SearchVariant& v, int sm_count, cudaStream_t s, bool strands) {
   if (nq == 0) return cudaSuccess;
-  if (!runs_wave_kernel(ix, mode, v)) return cudaErrorInvalidValue;
+  if (!runs_wave_kernel(ix, mode, v) || (strands && (nq & 1))) return cudaErrorInvalidValue;
   cudaError_t e = reset_defer(nq, d_defer, s);
   if (e != cudaSuccess) return e;
   const ByteRange br{v.b_lo, v.b_hi};
@@ -2566,6 +2740,11 @@ cudaError_t launch_search_ascii(const IndexView& ix, const uint8_t* d_qbytes, co
   a.qbytes = d_qbytes;
   a.qwords = d_qwords;
   a.first_bad = d_first_bad;
+  if (strands) {
+    if (mode == OUT_COUNT_U64)
+      return launch_search_wave<OUT_COUNT_U64, true, true>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br, a);
+    return launch_search_wave<OUT_SP_CNT_U32, true, true>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br, a);
+  }
   if (mode == OUT_COUNT_U64)
     return launch_search_wave<OUT_COUNT_U64, true>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br, a);
   return launch_search_wave<OUT_SP_CNT_U32, true>(ix, d_qwords, d_qoff, nq, d_out, d_defer, sm_count, s, v.avg_len, br, a);

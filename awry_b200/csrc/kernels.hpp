@@ -138,7 +138,25 @@ cudaError_t launch_search(const IndexView& ix, const uint64_t* d_qwords, const u
 bool search_packs_ascii(const IndexView& ix, SearchOut mode, const SearchVariant& v);
 cudaError_t launch_search_ascii(const IndexView& ix, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
                                 uint64_t* d_qwords, unsigned long long* d_first_bad, SearchOut mode, void* d_out,
-                                uint32_t* d_defer, const SearchVariant& v, int sm_count, cudaStream_t s);
+                                uint32_t* d_defer, const SearchVariant& v, int sm_count, cudaStream_t s,
+                                bool strands = false);
+
+// ---- both strands (awry_*_strands): read q of a batch stands for the VIRTUAL queries 2q (the read) and 2q + 1 (its
+// reverse complement), which every search and locate kernel runs like any other queries.
+// d_voff[2q] = 2 qoff[q], d_voff[2q + 1] = qoff[q] + qoff[q + 1] (2 nq + 1 entries, within [2 b_lo, 2 b_hi]): both
+// virtual queries have the read's length and their own word slot.  A read whose offsets leave [b_lo, b_hi] gets
+// d_voff[2q + 1] = ~0, which refuses both of its virtual queries (and no other).
+cudaError_t launch_strand_offsets(const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi, uint64_t* d_voff,
+                                  cudaStream_t s);
+// the words of the virtual queries from those of the reads (any prepass: launch_pack, launch_pack2): v = 2q a copy,
+// v = 2q + 1 the reverse complement (nibble order reversed, codes below 4 XOR 3).  d_qwords is biased for the reads'
+// range [b_lo, b_hi], d_vwords for the virtual one; a read the prepass refused (or an empty one) is skipped.
+cudaError_t launch_strand_words(const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+                                const uint64_t* d_voff, uint64_t* d_vwords, cudaStream_t s);
+// whether the strand flavour of the ASCII wave kernel may search the virtual queries straight from the reads' bytes
+// (launch_search_ascii with strands = true, d_qoff = the virtual offsets, v.b_lo / b_hi their range): where
+// search_packs_ascii holds and AWRY_B200_STRAND_WAVE, read per call, is not "0"
+bool search_strands_ascii(const IndexView& ix, SearchOut mode, const SearchVariant& v);
 
 // locate: CSR offsets from pass 1, LF-walk pass 2
 // d_sp_cnt: the search kernels' OUT_SP_CNT result -- uint2 (sp, count) per query, ulonglong2 for a wide index

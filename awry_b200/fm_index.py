@@ -128,7 +128,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_bench_random_gather", "awry_set_search_variant", "awry_set_locate_variant", "awry_set_count_variant", "awry_set_host_pack",
            "awry_host_pack_dna", "awry_last_error", "awry_version", "awry_count_batch_packed2",
            "awry_locate_batch_packed2", "awry_set_host_threads", "awry_host_threads", "awry_count_batch_hamming",
-           "awry_locate_batch_hamming", "awry_count_device_hamming"]
+           "awry_locate_batch_hamming", "awry_count_device_hamming", "awry_count_batch_strands",
+           "awry_locate_batch_strands", "awry_count_device_strands", "awry_locate_device_strands"]
 
 
 def native():
@@ -197,6 +198,10 @@ def native():
     L.awry_count_batch_hamming.argtypes = [vp, vp, vp, u64, C.c_uint32, vp]
     L.awry_locate_batch_hamming.argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, vp, u64, C.POINTER(u64)]
     L.awry_count_device_hamming.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, vp]
+    L.awry_count_batch_strands.argtypes = [vp, vp, vp, u64, vp]
+    L.awry_locate_batch_strands.argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, u64, C.POINTER(u64)]
+    L.awry_count_device_strands.argtypes = [vp, i32, vp, vp, u64, vp, vp]
+    L.awry_locate_device_strands.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, C.POINTER(vp), C.POINTER(u64), vp]
     _LIB = L
     return L
 
@@ -487,6 +492,56 @@ class FmIndex:
         """count_hamming_packed on device pointers (d_counts: nq * (max_mismatches + 1) u64); see device_check"""
         _check(native().awry_count_device_hamming(self._h, replica, d_qbytes, d_qoff, nq, int(max_mismatches), d_counts,
                                                   stream))
+
+    # ---- both strands: every query and its reverse complement (include/awry_b200.h) ----------
+    def count_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray) -> np.ndarray:
+        """-> uint64[nq, 2]: [q, 0] = count of q, [q, 1] = count of its reverse complement"""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        counts = np.empty((nq, 2), dtype=np.uint64)
+        _check(native().awry_count_batch_strands(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq, counts.ctypes.data))
+        return counts
+
+    def locate_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray, sorted_hits: bool = False,
+                              capacity: int = None):
+        """-> (hit_off uint64[2 nq + 1], hits uint64[n_hits, 2] = (seq_idx, local_pos)): query q's forward hits are
+        hits[hit_off[2q]:hit_off[2q+1]], its reverse-strand hits hits[hit_off[2q+1]:hit_off[2q+2]].  A first guess of
+        `capacity` hits (default: two per query) that proves too small is retried once with the reported total."""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        hit_off = np.zeros(2 * nq + 1, dtype=np.uint64)
+        cap = max(1, 2 * nq if capacity is None else int(capacity))
+        n = C.c_uint64()
+        for _ in range(2):
+            hits = np.zeros((cap, 2), dtype=np.uint64)
+            rc = native().awry_locate_batch_strands(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq,
+                                                    LOCATE_SORTED if sorted_hits else LOCATE_BWT_ORDER,
+                                                    hit_off.ctypes.data, hits.ctypes.data, cap, C.byref(n))
+            if rc != -8:
+                break
+            cap = max(1, n.value)
+        if rc != 0:
+            err = AwryError(rc, native().awry_last_error().decode(errors="replace"))
+            err.needed = n.value
+            raise err
+        return hit_off, hits[: n.value]
+
+    def count_strands_device(self, d_qbytes: int, d_qoff: int, nq: int, d_counts: int, stream: int = 0,
+                             replica: int = 0):
+        """count_strands_packed on device pointers (d_counts: 2 nq u64, [2q] forward, [2q+1] reverse); see device_check"""
+        _check(native().awry_count_device_strands(self._h, replica, d_qbytes, d_qoff, nq, d_counts, stream))
+
+    def locate_strands_device(self, d_qbytes: int, d_qoff: int, nq: int, d_hit_off: int, sorted_hits=False,
+                              stream: int = 0, replica: int = 0):
+        """locate_strands_packed on device pointers (d_hit_off: 2 nq + 1 u64) -> (device pointer to n_hits x
+        {u64 seq_idx, u64 local_pos}, n_hits); free with device_free"""
+        hits, n = C.c_void_p(), C.c_uint64()
+        _check(native().awry_locate_device_strands(self._h, replica, d_qbytes, d_qoff, nq,
+                                                   LOCATE_SORTED if sorted_hits else LOCATE_BWT_ORDER,
+                                                   d_hit_off, C.byref(hits), C.byref(n), stream))
+        return hits.value, n.value
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

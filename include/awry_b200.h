@@ -262,6 +262,38 @@ int awry_locate_batch_hamming(const awry_index *index, const uint8_t *qbytes, co
 int awry_count_device_hamming(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
                               uint64_t nq, uint32_t max_mismatches, uint64_t *d_counts, void *cuda_stream);
 
+/* ------------------------------------------------------------------ both strands (query and reverse complement)
+ * A read comes from either strand of the DNA; the index holds one.  These calls search every query together with its
+ * reverse complement, nucleotide only (a protein index -> AWRY_ERR_UNSUPPORTED).
+ *   rc(q)      the query's bytes mapped as for exact search (either case, U = T, any other byte except '$' / '#' =
+ *              N), complemented (A <-> T, C <-> G, N = N) and reversed.
+ *   virtual    query q of a batch stands for two searches: v = 2q (the query) and v = 2q + 1 (rc(q)).  Every result
+ *              for v = 2q + 1 is bit for bit what awry_count_batch / awry_locate_batch_into return for the ASCII
+ *              string rc(q) over ACGTN, BWT-row order under AWRY_LOCATE_BWT_ORDER included; v = 2q is q itself.
+ *   hits       a reverse-strand hit is the (seq_idx, local_pos) of the start of the window of the indexed text that
+ *              equals rc(q) (the usual leftmost coordinate); windows may cross record delimiters, as for exact
+ *              search.  A query equal to its reverse complement reports the same windows on both strands (nothing is
+ *              deduplicated).
+ *   counts     counts[2q] forward, counts[2q + 1] reverse complement (2 nq entries).
+ *   locate     hit_off is the CSR over the virtual queries (2 nq + 1 entries): query q's forward hits are
+ *              [hit_off[2q], hit_off[2q+1]), its reverse-strand hits [hit_off[2q+1], hit_off[2q+2]).  `flags` orders
+ *              the hits within each strand; capacity / AWRY_ERR_CAPACITY as in awry_locate_batch_into.
+ *   errors     an empty query or one with '$' / '#' -> AWRY_ERR_INVALID_QUERY, naming the caller's query index q;
+ *              non-monotone offsets -> AWRY_ERR_INVALID_ARG.  The device calls latch refused queries for
+ *              awry_device_check as awry_count_device does, and refuse (AWRY_ERR_INVALID_ARG) a batch whose 2 nq
+ *              virtual queries would not fit the kernels' 32-bit query counters (2 nq >= 2^32 - 2^24).
+ * Device hits (*d_hits) are released with awry_device_free. */
+int awry_count_batch_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                             uint64_t *counts /* 2*nq: [2q] forward, [2q+1] reverse complement */);
+int awry_locate_batch_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                              uint32_t flags, uint64_t *hit_off /* 2*nq + 1 */, awry_hit *hits, uint64_t capacity,
+                              uint64_t *n_hits);
+int awry_count_device_strands(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                              uint64_t nq, uint64_t *d_counts /* 2*nq */, void *cuda_stream);
+int awry_locate_device_strands(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                               uint64_t nq, uint32_t flags, uint64_t *d_hit_off /* 2*nq + 1 */, awry_hit **d_hits,
+                               uint64_t *n_hits, void *cuda_stream);
+
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to
  * parallel_count / parallel_locate (fm_index.rs:455-487); these entry points take the FASTQ ('@') or

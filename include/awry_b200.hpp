@@ -6,6 +6,7 @@
 // behaviour follow /root/reference/src/fm_index.rs: where the reference returns io::Error this
 // throws awry::Error; where it panics (empty query, sentinel in a query) this throws too.
 #pragma once
+#include <array>
 #include <cstdint>
 #include <stdexcept>
 #include <string>
@@ -187,6 +188,40 @@ class FmIndex {
     for (size_t q = 0; q < queries.size(); q++)
       for (uint64_t i = hit_off[q]; i < hit_off[q + 1]; i++)
         out[q].push_back({{hits[i].seq_idx, hits[i].local_pos}, uint32_t(dist[i])});
+    return out;
+  }
+  // Both strands (no counterpart in the reference): every query and its reverse complement.
+  // counts[q] = {forward count, reverse-complement count}
+  std::vector<std::array<uint64_t, 2>> parallel_count_strands(const std::vector<std::string_view>& queries) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::vector<std::array<uint64_t, 2>> out(queries.size());
+    check(awry_count_batch_strands(h_, bytes.data(), off.data(), queries.size(), out.empty() ? nullptr : out[0].data()));
+    return out;
+  }
+  // per query: {forward hits, reverse-strand hits (start of the window equal to the reverse complement)}, each in
+  // BWT-row order (or sorted ascending)
+  std::vector<std::array<std::vector<LocalizedSequencePosition>, 2>> parallel_locate_strands(
+      const std::vector<std::string_view>& queries, bool sorted = false) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    const uint32_t flags = sorted ? AWRY_LOCATE_SORTED : AWRY_LOCATE_BWT_ORDER;
+    std::vector<uint64_t> hit_off(2 * queries.size() + 1);
+    std::vector<awry_hit> hits(2 * queries.size() + 1);
+    uint64_t n = 0;
+    int rc = awry_locate_batch_strands(h_, bytes.data(), off.data(), queries.size(), flags, hit_off.data(), hits.data(),
+                                       hits.size(), &n);
+    if (rc == AWRY_ERR_CAPACITY) {  // the total is known now: once more with room for every hit
+      hits.resize(n);
+      rc = awry_locate_batch_strands(h_, bytes.data(), off.data(), queries.size(), flags, hit_off.data(), hits.data(),
+                                     hits.size(), &n);
+    }
+    check(rc);
+    std::vector<std::array<std::vector<LocalizedSequencePosition>, 2>> out(queries.size());
+    for (size_t v = 0; v < 2 * queries.size(); v++)
+      for (uint64_t i = hit_off[v]; i < hit_off[v + 1]; i++) out[v / 2][v % 2].push_back({hits[i].seq_idx, hits[i].local_pos});
     return out;
   }
   awry_index* handle() const { return h_; }
