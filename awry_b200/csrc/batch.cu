@@ -1197,7 +1197,7 @@ void hamming_check_index(const awry_index* ix) {
 
 // the hits of the locate call on one replica, in query order
 struct HammingSink {
-  std::vector<uint64_t> off;  // per query: offset of its first hit in `hits`
+  std::vector<uint64_t> off;  // per (virtual) query: offset of its first hit in `hits`
   std::vector<awry_hit> hits;
   std::vector<uint8_t> dist;
 };
@@ -1208,24 +1208,44 @@ struct HammingSink {
 // the hits are appended to `sink` (slices cut at read boundaries, the hits of a read sorted by text position).
 // `check_base` >= 0: a refused read fails the call (reported as read check_base + q) before anything is verified;
 // < 0 (the device-resident call): it stays latched in *d_flag for awry_device_check.
+// `strands`: the nq reads are searched as the 2 nq virtual queries of both strands (kernels.hpp), which take the
+// place of the reads from the piece offsets on: counts, CSR offsets and the hits are per virtual query.
 void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
                  uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
-                 HammingSink* sink) {
-  const uint64_t P = k + 1, np = nq * P, nbytes = b_hi - b_lo;
+                 HammingSink* sink, bool strands = false) {
+  const uint32_t shift = strands ? 1 : 0;  // virtual query -> read
+  const uint64_t P = k + 1, nbytes = b_hi - b_lo, nv = nq << shift, np = nv * P;
   if (np >= (1ull << 31)) fail(AWRY_ERR_INVALID_ARG, "batch too large for one Hamming search (%llu reads): split it", (unsigned long long)nq);
   StreamScratch sc(st);
-  // 1. pieces, packed; the whole reads packed too (their prepass validates the offsets and latches what it refuses)
+  // 1. pieces, packed; the whole reads packed too (their prepass validates the offsets and latches what it refuses).
+  // Single strand: the pieces are packed from the caller's bytes (DESIGN.md §1c: cutting them out of the read words
+  // measured slower at k = 1 and 3).  Both strands: the virtual queries' offsets and words come from the reads', and
+  // the pieces' words are cut out of the virtual words (a reverse-complement piece has no bytes to pack).
+  const uint64_t rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
+  const uint64_t v_lo = b_lo << shift, v_hi = b_hi << shift, vw_n = packed_words(0, nv, nbytes << shift), vw_lo = 4 * (v_lo >> 6);
+  const uint64_t* d_voff = d_qoff;
   uint64_t* d_poff = sc.get<uint64_t>(np + 1);
-  unsigned long long* d_pflag = sc.get<unsigned long long>(1);  // (piece indices: what it latches is reported per read)
-  CU(cudaMemsetAsync(d_pflag, 0xff, 8, st));
-  CU(launch_hamming_pieces(d_qoff, nq, k, b_lo, b_hi, d_poff, d_flag, st));
-  const uint64_t pw_n = packed_words(0, np, nbytes), rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
-  uint64_t* const d_pw = sc.get<uint64_t>(pw_n) - w_lo;
+  uint64_t* const d_pw = sc.get<uint64_t>(packed_words(0, np, nbytes << shift)) - vw_lo;
   uint64_t* const d_rw = sc.get<uint64_t>(rw_n) - w_lo;
+  uint64_t* d_vw = d_rw;
   {
     ProfScope p(2, r.device, st);
-    CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_poff, np, d_pw, b_lo, b_hi, d_pflag, st));
-    CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
+    if (!strands) {
+      unsigned long long* d_pflag = sc.get<unsigned long long>(1);  // (piece indices: what it latches is reported per read)
+      CU(cudaMemsetAsync(d_pflag, 0xff, 8, st));
+      CU(launch_hamming_pieces(d_qoff, nq, k, b_lo, b_hi, 0, d_poff, d_flag, st));
+      CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_poff, np, d_pw, b_lo, b_hi, d_pflag, st));
+      CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
+    } else {
+      uint64_t* const voff = sc.get<uint64_t>(nv + 1);
+      d_vw = sc.get<uint64_t>(vw_n) - vw_lo;
+      CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
+      CU(launch_strand_offsets(d_qoff, nq, b_lo, b_hi, voff, st));
+      CU(launch_strand_words(d_rw, d_qoff, nq, b_lo, b_hi, voff, d_vw, st));
+      d_voff = voff;
+      CU(launch_hamming_pieces(d_voff, nv, k, v_lo, v_hi, shift, d_poff, d_flag, st));
+      CU(launch_hamming_piece_words(d_vw, d_voff, nv, v_lo, v_hi, k, d_pw, st));
+    }
   }
   // 2. exact search of the pieces (the wave kernel stores a piece finished in the text as its position), CSR
   // offsets of their occurrences = the candidates
@@ -1233,9 +1253,9 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   {
     ProfScope p(0, r.device, st);
     SearchVariant v = current_variant();
-    v.avg_len = uint32_t(std::min<uint64_t>(nbytes / np, 1u << 30));
-    v.b_lo = b_lo;
-    v.b_hi = b_hi;
+    v.avg_len = uint32_t(std::min<uint64_t>((nbytes << shift) / np, 1u << 30));
+    v.b_lo = v_lo;
+    v.b_hi = v_hi;
     v.locate_positions = locate_positions_ok(r.view, v);
     CU(launch_search(r.view, d_pw, d_poff, np, OUT_SP_CNT_U32, d_sp, sc.get<uint32_t>(defer_words(np)), v, r.sm_count, st));
   }
@@ -1249,11 +1269,11 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   std::vector<uint64_t> qcand;
   uint64_t* d_qcand = nullptr;
   if (sink) {
-    d_qcand = sc.get<uint64_t>(nq + 1);
-    CU(launch_hamming_query_bounds(d_hoff, k, nq, d_qcand, st));
-    qcand.resize(nq + 1);
-    CU(cudaMemcpyAsync(qcand.data(), d_qcand, (nq + 1) * 8, cudaMemcpyDeviceToHost, st));
-    g_prof.d2h += (nq + 1) * 8;
+    d_qcand = sc.get<uint64_t>(nv + 1);
+    CU(launch_hamming_query_bounds(d_hoff, k, nv, d_qcand, st));
+    qcand.resize(nv + 1);
+    CU(cudaMemcpyAsync(qcand.data(), d_qcand, (nv + 1) * 8, cudaMemcpyDeviceToHost, st));
+    g_prof.d2h += (nv + 1) * 8;
   }
   CU(cudaMemcpyAsync(&total, d_hoff + np, 8, cudaMemcpyDeviceToHost, st));
   if (check_base >= 0) CU(cudaMemcpyAsync(&flag, d_flag, 8, cudaMemcpyDeviceToHost, st));
@@ -1265,18 +1285,18 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   if (flag != ~0ull) fail_bad_query(flag, uint64_t(check_base));
 
   HammingSlice a{};
-  a.qwords = d_rw;
-  a.qw_lo = w_lo;
-  a.qw_n = rw_n;
-  a.qoff = d_qoff;
-  a.b_lo = b_lo;
-  a.b_hi = b_hi;
+  a.qwords = d_vw;
+  a.qw_lo = strands ? vw_lo : w_lo;
+  a.qw_n = strands ? vw_n : rw_n;
+  a.qoff = d_voff;
+  a.b_lo = v_lo;
+  a.b_hi = v_hi;
   a.sp_cnt = d_sp;
   a.hoff = d_hoff;
   a.npieces = np;
   const uint64_t S = hamming_slice();
   if (!sink) {  // 3. count: slices cut anywhere
-    CU(cudaMemsetAsync(d_counts, 0, nq * P * 8, st));
+    CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
     for (uint64_t c0 = 0; c0 < total; c0 += S) {
       StreamScratch ss(st);
       a.c0 = c0;
@@ -1292,14 +1312,14 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     return;
   }
   // 3. locate: slices cut at read boundaries (a read with more candidates than a slice gets one of its own size)
-  sink->off.reserve(sink->off.size() + nq);
-  for (uint64_t q0 = 0; q0 < nq;) {
+  sink->off.reserve(sink->off.size() + nv);
+  for (uint64_t q0 = 0; q0 < nv;) {
     uint64_t q1 = q0 + 1;
-    while (q1 < nq && qcand[q1 + 1] - qcand[q0] <= S) q1++;
+    while (q1 < nv && qcand[q1 + 1] - qcand[q0] <= S) q1++;
     const uint64_t c0 = qcand[q0], n = qcand[q1] - c0, nr = q1 - q0;
     if (n >= (1ull << 31))  // (a slice is sorted per read by one CUB call, whose offsets are int)
       fail(AWRY_ERR_NOMEM, "query %llu has %llu candidate windows, more than one slice can sort (2^31)",
-           (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + q0), (unsigned long long)n);
+           (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + (q0 >> shift)), (unsigned long long)n);
     const uint64_t base = sink->hits.size();
     if (n == 0) {
       sink->off.insert(sink->off.end(), nr, base);
@@ -1352,9 +1372,9 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
 }
 
 // reads [lo, hi) of host buffers on replica ri: chunks of reads uploaded and searched one after the other (the
-// host path does not overlap copies with compute yet)
+// host path does not overlap copies with compute yet).  `strands`: a chunk of n reads fills 2 n result slots.
 void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo,
-                        uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink) {
+                        uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink, bool strands = false) {
   if (lo >= hi) return;
   Replica& r = *ix->reps[ri];
   DeviceGuard dg(r.device);
@@ -1374,13 +1394,16 @@ void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, 
       g_prof.h2d += nbytes + (n + 1) * 8;
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
       if (sink) {
-        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr, sink);
+        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr, sink,
+                    strands);
       } else {
         StreamScratch sc(ws->st);
-        uint64_t* d_counts = sc.get<uint64_t>(n * (k + 1));
-        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts, nullptr);
-        CU(cudaMemcpyAsync(counts + c.q0 * (k + 1), d_counts, n * (k + 1) * 8, cudaMemcpyDeviceToHost, ws->st));
-        g_prof.d2h += n * (k + 1) * 8;
+        const uint64_t slots = (strands ? 2 : 1) * (k + 1);  // counts per read
+        uint64_t* d_counts = sc.get<uint64_t>(n * slots);
+        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts, nullptr,
+                    strands);
+        CU(cudaMemcpyAsync(counts + c.q0 * slots, d_counts, n * slots * 8, cudaMemcpyDeviceToHost, ws->st));
+        g_prof.d2h += n * slots * 8;
       }
       CU(cudaStreamSynchronize(ws->st));
     }
@@ -1438,6 +1461,61 @@ void device_batch_ends(const uint64_t* d_qoff, uint64_t nq, cudaStream_t st, uin
 void strands_check_device_batch(uint64_t nq) {
   if (2 * nq >= (1ull << 32) - (1u << 24))  // (the search kernels' 32-bit ticket counter)
     fail(AWRY_ERR_INVALID_ARG, "batch too large for one both-strand search (%llu reads): split it", (unsigned long long)nq);
+}
+
+// awry_count_batch_hamming[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
+void hamming_count_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t k,
+                        uint64_t* counts, bool strands) {
+  need(ix);
+  if (k > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  if (nq == 0) return;
+  if (!qbytes || !qoff || !counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (strands) strands_check_index(ix);
+  hamming_check_index(ix);
+  for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
+    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, counts, nullptr, strands);
+  });
+}
+
+// awry_locate_batch_hamming[_strands]: hit_off is the CSR over the nq (or 2 nq virtual) queries
+void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t k,
+                         uint64_t* hit_off, awry_hit* hits, uint8_t* hit_mismatches, uint64_t capacity, uint64_t* n_hits,
+                         bool strands) {
+  need(ix);
+  if (k > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  if (!hit_off || !n_hits || (!hits && capacity)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  *n_hits = 0;
+  hit_off[0] = 0;
+  if (nq == 0) return;
+  if (!qbytes || !qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (strands) strands_check_index(ix);
+  hamming_check_index(ix);
+  const uint64_t per = strands ? 2 : 1;  // result slots per read
+  const size_t nr = ix->reps.size();
+  std::vector<HammingSink> sinks(nr);
+  std::vector<std::pair<uint64_t, uint64_t>> ranges(nr, {0, 0});
+  for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
+    ranges[ri] = {lo, hi};
+    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, nullptr, &sinks[ri], strands);
+  });
+  // the replicas' CSRs, concatenated in range order; hits past `capacity` are dropped (the total still counts them)
+  uint64_t total = 0;
+  for (size_t ri = 0; ri < nr; ri++) {
+    const auto [lo, hi] = ranges[ri];
+    const HammingSink& s = sinks[ri];
+    for (uint64_t i = 0; i < per * (hi - lo); i++) hit_off[per * lo + i] = total + s.off[i];
+    const uint64_t n = s.hits.size(), fit = capacity > total ? std::min(n, capacity - total) : 0;
+    if (fit) {
+      memcpy(hits + total, s.hits.data(), fit * sizeof(awry_hit));
+      if (hit_mismatches) memcpy(hit_mismatches + total, s.dist.data(), fit);
+    }
+    total += n;
+  }
+  hit_off[per * nq] = total;
+  *n_hits = total;
+  if (total > capacity)
+    fail(AWRY_ERR_CAPACITY, "hit buffer holds %llu entries, %llu needed", (unsigned long long)capacity,
+         (unsigned long long)total);
 }
 
 }  // namespace host
@@ -1619,55 +1697,14 @@ int awry_locate_device(const awry_index* ix, int replica, const uint8_t* d_qbyte
 
 int awry_count_batch_hamming(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
                              uint32_t max_mismatches, uint64_t* counts) {
-  return guarded([&] {
-    need(ix);
-    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
-    if (nq == 0) return;
-    if (!qbytes || !qoff || !counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    hamming_check_index(ix);
-    for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
-      hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, max_mismatches, counts, nullptr);
-    });
-  });
+  return guarded([&] { hamming_count_impl(ix, qbytes, qoff, nq, max_mismatches, counts, false); });
 }
 
 int awry_locate_batch_hamming(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
                               uint32_t max_mismatches, uint64_t* hit_off, awry_hit* hits, uint8_t* hit_mismatches,
                               uint64_t capacity, uint64_t* n_hits) {
   return guarded([&] {
-    need(ix);
-    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
-    if (!hit_off || !n_hits || (!hits && capacity)) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    *n_hits = 0;
-    hit_off[0] = 0;
-    if (nq == 0) return;
-    if (!qbytes || !qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    hamming_check_index(ix);
-    const size_t nr = ix->reps.size();
-    std::vector<HammingSink> sinks(nr);
-    std::vector<std::pair<uint64_t, uint64_t>> ranges(nr, {0, 0});
-    for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
-      ranges[ri] = {lo, hi};
-      hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, max_mismatches, nullptr, &sinks[ri]);
-    });
-    // the replicas' CSRs, concatenated in range order; hits past `capacity` are dropped (the total still counts them)
-    uint64_t total = 0;
-    for (size_t ri = 0; ri < nr; ri++) {
-      const auto [lo, hi] = ranges[ri];
-      const HammingSink& s = sinks[ri];
-      for (uint64_t i = 0; i < hi - lo; i++) hit_off[lo + i] = total + s.off[i];
-      const uint64_t n = s.hits.size(), fit = capacity > total ? std::min(n, capacity - total) : 0;
-      if (fit) {
-        memcpy(hits + total, s.hits.data(), fit * sizeof(awry_hit));
-        if (hit_mismatches) memcpy(hit_mismatches + total, s.dist.data(), fit);
-      }
-      total += n;
-    }
-    hit_off[nq] = total;
-    *n_hits = total;
-    if (total > capacity)
-      fail(AWRY_ERR_CAPACITY, "hit buffer holds %llu entries, %llu needed", (unsigned long long)capacity,
-           (unsigned long long)total);
+    hamming_locate_impl(ix, qbytes, qoff, nq, max_mismatches, hit_off, hits, hit_mismatches, capacity, n_hits, false);
   });
 }
 
@@ -1689,6 +1726,38 @@ int awry_count_device_hamming(const awry_index* ix, int replica, const uint8_t* 
     CU(cudaStreamSynchronize(st));
     if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
     hamming_run(r, d_qbytes, d_qoff, nq, ends[0], ends[1], max_mismatches, r.d_async_flag, -1, st, d_counts, nullptr);
+  });
+}
+
+int awry_count_batch_hamming_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                                     uint32_t max_mismatches, uint64_t* counts) {
+  return guarded([&] { hamming_count_impl(ix, qbytes, qoff, nq, max_mismatches, counts, true); });
+}
+
+int awry_locate_batch_hamming_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                                      uint32_t max_mismatches, uint64_t* hit_off, awry_hit* hits, uint8_t* hit_mismatches,
+                                      uint64_t capacity, uint64_t* n_hits) {
+  return guarded([&] {
+    hamming_locate_impl(ix, qbytes, qoff, nq, max_mismatches, hit_off, hits, hit_mismatches, capacity, n_hits, true);
+  });
+}
+
+int awry_count_device_hamming_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                      uint64_t nq, uint32_t max_mismatches, uint64_t* d_counts, void* cuda_stream) {
+  return guarded([&] {
+    need(ix);
+    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+    if (nq == 0) return;
+    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+    strands_check_index(ix);
+    hamming_check_index(ix);
+    Replica& r = *ix->reps[size_t(replica)];
+    DeviceGuard dg(r.device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    uint64_t ends[2] = {0, 0};
+    device_batch_ends(d_qoff, nq, st, ends);
+    hamming_run(r, d_qbytes, d_qoff, nq, ends[0], ends[1], max_mismatches, r.d_async_flag, -1, st, d_counts, nullptr, true);
   });
 }
 

@@ -182,9 +182,14 @@ cudaError_t launch_map_locations(const IndexView& ix, const uint64_t* d_locs, ui
                                  uint64_t* d_hits_pairs, cudaStream_t s);
 
 // ---- kernels_hamming.cu: Hamming search (<= k substitutions) by k + 1 exactly searched pieces per read
-// piece offsets (k+1) nq + 1 of a batch; a query with L <= k is latched in *d_first_bad as BAD_QUERY
+// piece offsets (k+1) nq + 1 of a batch; a query with L <= k is latched in *d_first_bad as BAD_QUERY of query q >> shift
 cudaError_t launch_hamming_pieces(const uint64_t* d_qoff, uint64_t nq, uint32_t k, uint64_t b_lo, uint64_t b_hi,
-                                  uint64_t* d_poff, unsigned long long* d_first_bad, cudaStream_t s);
+                                  uint32_t shift, uint64_t* d_poff, unsigned long long* d_first_bad, cudaStream_t s);
+// the words of the (k+1) nq pieces from the words of their queries (any prepass, or launch_strand_words), bit for bit
+// what launch_pack writes for the pieces' bytes.  d_qwords is biased for [b_lo, b_hi] as for launch_search, d_pwords
+// likewise with the piece offsets of launch_hamming_pieces; a query refused by its prepass (or empty) is skipped.
+cudaError_t launch_hamming_piece_words(const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo,
+                                       uint64_t b_hi, uint32_t k, uint64_t* d_pwords, cudaStream_t s);
 // d_qcand[i] = d_hoff[(k+1) i] for i = 0 .. nq (candidate range of each query)
 cudaError_t launch_hamming_query_bounds(const uint64_t* d_hoff, uint32_t k, uint64_t nq, uint64_t* d_qcand, cudaStream_t s);
 // piece of every candidate of the slice [c0, c0 + n) (cub convention: d_temp == nullptr sizes the scratch)

@@ -15,27 +15,70 @@
 namespace awry {
 
 // piece offsets of every query: poff[(k+1) q + j] = qoff[q] + a_j, poff[(k+1) nq] = qoff[nq].  A query with L <= k
-// has empty pieces (and every window would match): it is latched like an empty query.  Offsets outside [b_lo,
+// has empty pieces (and every window would match): it is latched like an empty query, as the caller's query
+// q >> shift (shift 1: the queries are the virtual ones of both strands, kernels.hpp).  Offsets outside [b_lo,
 // b_hi] are left to the read's own prepass (launch_pack), which latches them with the query's index.
 __global__ void __launch_bounds__(256)
     hamming_pieces_kernel(const uint64_t* __restrict__ qoff, uint64_t nq, uint32_t k, uint64_t b_lo, uint64_t b_hi,
-                          uint64_t* __restrict__ poff, unsigned long long* first_bad) {
+                          uint32_t shift, uint64_t* __restrict__ poff, unsigned long long* first_bad) {
   const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
   for (uint64_t q = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; q < nq; q += stride) {
     const uint64_t o0 = qoff[q], o1 = qoff[q + 1];
     const bool valid = !(o0 < b_lo || o1 > b_hi || o1 < o0 || o1 - o0 >= (1ull << 32));
     const uint64_t len = valid ? o1 - o0 : 0;
-    if (valid && len <= k) atomicMin(first_bad, bad_query_code(q, BAD_QUERY));
+    if (valid && len <= k) atomicMin(first_bad, bad_query_code(q >> shift, BAD_QUERY));
     for (uint32_t j = 0; j <= k; j++) poff[(k + 1) * q + j] = o0 + j * len / (k + 1);
     if (q + 1 == nq) poff[(k + 1) * nq] = o1;
   }
 }
 
 cudaError_t launch_hamming_pieces(const uint64_t* d_qoff, uint64_t nq, uint32_t k, uint64_t b_lo, uint64_t b_hi,
-                                  uint64_t* d_poff, unsigned long long* d_first_bad, cudaStream_t s) {
+                                  uint32_t shift, uint64_t* d_poff, unsigned long long* d_first_bad, cudaStream_t s) {
   if (nq == 0) return cudaSuccess;
   const unsigned grid = unsigned(std::min<uint64_t>((nq + 255) / 256, 148 * 16));
-  hamming_pieces_kernel<<<grid, 256, 0, s>>>(d_qoff, nq, k, b_lo, b_hi, d_poff, d_first_bad);
+  hamming_pieces_kernel<<<grid, 256, 0, s>>>(d_qoff, nq, k, b_lo, b_hi, shift, d_poff, d_first_bad);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
+// the words of every piece from those of its query, 4 lanes per query (as strand_words_kernel).  Piece j = bytes
+// [a_j, a_{j+1}) is the search-order nibble range [L - a_{j+1}, L - a_j) of the query's stream, so its word w is
+// one funnel shift of the query's words wi, wi + 1 (wi = (L - a_{j+1} + 16 w) / 16).  What pack_kernel writes for the
+// piece's bytes comes out: the same codes (pack_kernel maps every byte the same way wherever the query is cut), the
+// nibbles past the piece's last symbol zero, and no word past its last.  A query the prepass refused (or an empty
+// one) has no words; its pieces are empty or refused themselves (hamming_pieces_kernel), so none is written.
+__global__ void __launch_bounds__(256)
+    hamming_piece_words_kernel(const uint64_t* __restrict__ qwords, const uint64_t* __restrict__ qoff, uint64_t nq,
+                               ByteRange br, uint32_t k, uint64_t* __restrict__ pwords) {
+  const uint32_t sub = threadIdx.x & 3, P = k + 1;
+  const uint64_t ngroups = (gridDim.x * uint64_t(blockDim.x)) >> 2;
+  for (uint64_t q = (blockIdx.x * uint64_t(blockDim.x) + threadIdx.x) >> 2; q < nq; q += ngroups) {
+    const uint64_t o0 = qoff[q];
+    const uint32_t len = checked_len(o0, qoff[q + 1], br);
+    if (len == 0) continue;
+    const uint64_t* const src = qwords + 4 * (q + (o0 >> 6));
+    uint32_t a0 = 0;  // a_j
+    for (uint32_t j = 0; j < P; j++) {
+      const uint32_t a1 = uint32_t(uint64_t(j + 1) * len / P), m = a1 - a0, s0 = len - a1;
+      uint64_t* const dst = pwords + 4 * (uint64_t(P) * q + j + ((o0 + a0) >> 6));
+      for (uint32_t w = sub; 16 * w < m; w += 4) {
+        const uint32_t si = s0 + 16 * w, wi = si >> 4, sh = 4 * (si & 15);
+        const uint64_t lo = src[wi], hi = sh && 16 * (wi + 1) < len ? src[wi + 1] : 0ull;
+        uint64_t x = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
+        const uint32_t have = m - 16 * w;  // symbols of this word (the rest stay 0)
+        if (have < 16) x &= (1ull << (4 * have)) - 1;
+        dst[w] = x;
+      }
+      a0 = a1;
+    }
+  }
+}
+
+cudaError_t launch_hamming_piece_words(const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo,
+                                       uint64_t b_hi, uint32_t k, uint64_t* d_pwords, cudaStream_t s) {
+  if (nq == 0) return cudaSuccess;
+  const unsigned grid = unsigned(std::min<uint64_t>((nq * 4 + 255) / 256, 148 * 64));
+  hamming_piece_words_kernel<<<grid, 256, 0, s>>>(d_qwords, d_qoff, nq, ByteRange{b_lo, b_hi}, k, d_pwords);
   COUNT_LAUNCH();
   return cudaGetLastError();
 }

@@ -129,7 +129,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_host_pack_dna", "awry_last_error", "awry_version", "awry_count_batch_packed2",
            "awry_locate_batch_packed2", "awry_set_host_threads", "awry_host_threads", "awry_count_batch_hamming",
            "awry_locate_batch_hamming", "awry_count_device_hamming", "awry_count_batch_strands",
-           "awry_locate_batch_strands", "awry_count_device_strands", "awry_locate_device_strands"]
+           "awry_locate_batch_strands", "awry_count_device_strands", "awry_locate_device_strands",
+           "awry_count_batch_hamming_strands", "awry_locate_batch_hamming_strands", "awry_count_device_hamming_strands"]
 
 
 def native():
@@ -202,6 +203,9 @@ def native():
     L.awry_locate_batch_strands.argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, u64, C.POINTER(u64)]
     L.awry_count_device_strands.argtypes = [vp, i32, vp, vp, u64, vp, vp]
     L.awry_locate_device_strands.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, C.POINTER(vp), C.POINTER(u64), vp]
+    L.awry_count_batch_hamming_strands.argtypes = [vp, vp, vp, u64, C.c_uint32, vp]
+    L.awry_locate_batch_hamming_strands.argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, vp, u64, C.POINTER(u64)]
+    L.awry_count_device_hamming_strands.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, vp]
     _LIB = L
     return L
 
@@ -542,6 +546,52 @@ class FmIndex:
                                                    LOCATE_SORTED if sorted_hits else LOCATE_BWT_ORDER,
                                                    d_hit_off, C.byref(hits), C.byref(n), stream))
         return hits.value, n.value
+
+    # ---- Hamming search on both strands (include/awry_b200.h) ----------------------------------
+    def count_hamming_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_mismatches: int) -> np.ndarray:
+        """-> uint64[nq, 2, max_mismatches + 1]: [q, s, d] = windows at Hamming distance exactly d from q (s = 0) or
+        from its reverse complement (s = 1)"""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        counts = np.zeros((nq, 2, int(max_mismatches) + 1), dtype=np.uint64)
+        _check(native().awry_count_batch_hamming_strands(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq,
+                                                         int(max_mismatches), counts.ctypes.data))
+        return counts
+
+    def locate_hamming_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_mismatches: int,
+                                      capacity: int = None):
+        """-> (hit_off uint64[2 nq + 1], hits uint64[n_hits, 2], mismatches uint8[n_hits]): query q's forward hits are
+        hits[hit_off[2q]:hit_off[2q+1]], its reverse-strand hits hits[hit_off[2q+1]:hit_off[2q+2]], each ascending by
+        text position.  A first guess of `capacity` hits (default: two per query) that proves too small is retried
+        once with the total the library reports."""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        hit_off = np.zeros(2 * nq + 1, dtype=np.uint64)
+        cap = max(1, 2 * nq if capacity is None else int(capacity))
+        n = C.c_uint64()
+        for _ in range(2):
+            hits = np.zeros((cap, 2), dtype=np.uint64)
+            mm = np.zeros(cap, dtype=np.uint8)
+            rc = native().awry_locate_batch_hamming_strands(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq,
+                                                            int(max_mismatches), hit_off.ctypes.data, hits.ctypes.data,
+                                                            mm.ctypes.data, cap, C.byref(n))
+            if rc != -8:
+                break
+            cap = max(1, n.value)
+        if rc != 0:
+            err = AwryError(rc, native().awry_last_error().decode(errors="replace"))
+            err.needed = n.value
+            raise err
+        return hit_off, hits[: n.value], mm[: n.value]
+
+    def count_hamming_strands_device(self, d_qbytes: int, d_qoff: int, nq: int, max_mismatches: int, d_counts: int,
+                                     stream: int = 0, replica: int = 0):
+        """count_hamming_strands_packed on device pointers (d_counts: 2 nq (max_mismatches + 1) u64, [(2q + s)(k+1) +
+        d]); see device_check"""
+        _check(native().awry_count_device_hamming_strands(self._h, replica, d_qbytes, d_qoff, nq, int(max_mismatches),
+                                                          d_counts, stream))
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

@@ -294,6 +294,30 @@ int awry_locate_device_strands(const awry_index *index, int replica, const uint8
                                uint64_t nq, uint32_t flags, uint64_t *d_hit_off /* 2*nq + 1 */, awry_hit **d_hits,
                                uint64_t *n_hits, void *cuda_stream);
 
+/* ------------------------------------------------------------------ Hamming search on both strands
+ * The two blocks above together: every query and its reverse complement, each with up to k substitutions.
+ *   virtual    query q stands for v = 2q (q) and v = 2q + 1 (rc(q), as in the both-strands block).  Every result for
+ *              v = 2q + 1 is bit for bit what awry_count_batch_hamming / awry_locate_batch_hamming return for the
+ *              ASCII string rc(q): counts per distance, the hits in ascending text position and each hit's distance;
+ *              v = 2q is q itself.  A query equal to its reverse complement reports the same windows on both strands.
+ *   counts     counts[(2q + s) * (k+1) + d], s = 0 forward, s = 1 reverse complement (2 nq (k+1) entries).
+ *   locate     hit_off is the CSR over the virtual queries (2 nq + 1 entries); capacity / AWRY_ERR_CAPACITY, and
+ *              hit_mismatches, as in awry_locate_batch_hamming.
+ *   errors     those of both blocks: k > AWRY_HAMMING_MAX -> AWRY_ERR_INVALID_ARG; an empty query, one with '$' / '#'
+ *              or one of length L <= k -> AWRY_ERR_INVALID_QUERY, naming the caller's query index q; a protein index
+ *              or one without the unsampled suffix array and the text -> AWRY_ERR_UNSUPPORTED.
+ * The device call behaves as awry_count_device_hamming (one synchronisation, refused queries latched for
+ * awry_device_check with counts 0) and refuses (AWRY_ERR_INVALID_ARG) a batch with 2 nq (k+1) >= 2^31 pieces. */
+int awry_count_batch_hamming_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                                     uint32_t max_mismatches, uint64_t *counts /* 2*nq * (max_mismatches + 1) */);
+int awry_locate_batch_hamming_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                                      uint32_t max_mismatches, uint64_t *hit_off /* 2*nq + 1 */, awry_hit *hits,
+                                      uint8_t *hit_mismatches /* NULL or capacity entries */, uint64_t capacity,
+                                      uint64_t *n_hits);
+int awry_count_device_hamming_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
+                                      const uint64_t *d_qoff, uint64_t nq, uint32_t max_mismatches,
+                                      uint64_t *d_counts /* 2*nq * (max_mismatches + 1) */, void *cuda_stream);
+
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to
  * parallel_count / parallel_locate (fm_index.rs:455-487); these entry points take the FASTQ ('@') or

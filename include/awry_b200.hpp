@@ -224,6 +224,45 @@ class FmIndex {
       for (uint64_t i = hit_off[v]; i < hit_off[v + 1]; i++) out[v / 2][v % 2].push_back({hits[i].seq_idx, hits[i].local_pos});
     return out;
   }
+  // Hamming search on both strands: counts[q][s][d] = windows at distance exactly d from query q (s = 0) or from its
+  // reverse complement (s = 1)
+  std::vector<std::array<std::vector<uint64_t>, 2>> parallel_count_hamming_strands(
+      const std::vector<std::string_view>& queries, uint32_t max_mismatches) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    const size_t P = size_t(max_mismatches) + 1;
+    std::vector<uint64_t> flat(2 * queries.size() * P);
+    check(awry_count_batch_hamming_strands(h_, bytes.data(), off.data(), queries.size(), max_mismatches, flat.data()));
+    std::vector<std::array<std::vector<uint64_t>, 2>> out(queries.size());
+    for (size_t v = 0; v < 2 * queries.size(); v++) out[v / 2][v % 2].assign(flat.begin() + v * P, flat.begin() + (v + 1) * P);
+    return out;
+  }
+  // per query: {forward hits, reverse-strand hits}, each (window start, distance) ascending by position
+  std::vector<std::array<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>, 2>> parallel_locate_hamming_strands(
+      const std::vector<std::string_view>& queries, uint32_t max_mismatches) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::vector<uint64_t> hit_off(2 * queries.size() + 1);
+    std::vector<awry_hit> hits(2 * queries.size() + 1);
+    std::vector<uint8_t> dist(hits.size());
+    uint64_t n = 0;
+    int rc = awry_locate_batch_hamming_strands(h_, bytes.data(), off.data(), queries.size(), max_mismatches,
+                                               hit_off.data(), hits.data(), dist.data(), hits.size(), &n);
+    if (rc == AWRY_ERR_CAPACITY) {  // the total is known now: once more with room for every hit
+      hits.resize(n);
+      dist.resize(n);
+      rc = awry_locate_batch_hamming_strands(h_, bytes.data(), off.data(), queries.size(), max_mismatches,
+                                             hit_off.data(), hits.data(), dist.data(), hits.size(), &n);
+    }
+    check(rc);
+    std::vector<std::array<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>, 2>> out(queries.size());
+    for (size_t v = 0; v < 2 * queries.size(); v++)
+      for (uint64_t i = hit_off[v]; i < hit_off[v + 1]; i++)
+        out[v / 2][v % 2].push_back({{hits[i].seq_idx, hits[i].local_pos}, uint32_t(dist[i])});
+    return out;
+  }
   awry_index* handle() const { return h_; }
 
  private:
