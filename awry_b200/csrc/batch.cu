@@ -225,6 +225,84 @@ bool offsets_are_uniform(const uint64_t* off, uint64_t nq, uint64_t& len) {
   return ok.load();
 }
 
+// u64 words of a packed-query buffer for n queries whose offsets lie in [b_lo, b_hi]: query q starts at word
+// 4 * (q + (qoff[q] >> sh)) - 4 * (b_lo >> sh) (kernels.hpp)
+uint64_t query_words(int alphabet, uint64_t n, uint64_t b_lo, uint64_t b_hi) {
+  const int sh = packed_unit_shift(alphabet);
+  return 4 * (n + (b_hi >> sh) - (b_lo >> sh) + 2) + 32;
+}
+
+// What one search_reads call works in, all sized by the caller: `words` (query_words of the reads), for both strands
+// also `voff` (2 nq + 1) and `vwords` (query_words of the virtual queries on [2 b_lo, 2 b_hi]); `out` and `defer`
+// for the searched queries; `flag` latches what the prepass refuses.
+struct SearchBuffers {
+  uint64_t* words;
+  uint64_t* voff;
+  uint64_t* vwords;
+  void* out;
+  uint32_t* defer;
+  unsigned long long* flag;
+};
+
+// ws's buffers for search_reads of nq reads on [b_lo, b_hi], `out_elem` bytes of result per searched query, grown as
+// needed
+SearchBuffers workspace_buffers(Workspace* ws, int alphabet, uint64_t nq, uint64_t b_lo, uint64_t b_hi, bool strands,
+                                size_t out_elem, unsigned long long* flag) {
+  const uint64_t nv = strands ? 2 * nq : nq;
+  Workspace::grow_dev(ws->d_qwords, ws->d_qwords_cap, size_t(query_words(alphabet, nq, b_lo, b_hi)));
+  Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nv) * out_elem);
+  Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nv));
+  if (strands) {
+    Workspace::grow_dev(ws->d_voff, ws->d_voff_cap, size_t(nv) + 1);
+    Workspace::grow_dev(ws->d_vwords, ws->d_vwords_cap, size_t(query_words(AWRY_NUCLEOTIDE, nv, 2 * b_lo, 2 * b_hi)));
+  }
+  return SearchBuffers{ws->d_qwords, ws->d_voff, ws->d_vwords, ws->d_out, ws->d_defer, flag};
+}
+
+// Searches nq reads that are on the device, on one strand or both (the 2 nq virtual queries of kernels.hpp), into
+// b.out, on stream `st`.  Their offsets are absolute and lie in [b_lo, b_hi].  d_qbytes: their ASCII bytes, biased
+// accordingly -- the wave kernel packs them itself where it runs, launch_pack does otherwise; nullptr: b.words holds
+// their words already (launch_pack2).  The pack runs under profile slot 2 and the search under slot 0, the strand
+// kernels under neither; t0 / t1 (if set) are recorded around the search launch alone (PackBalance).  Returns
+// whether one-hit queries were stored as text positions (SearchVariant::locate_positions).
+bool search_reads(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+                  bool strands, SearchOut mode, const SearchBuffers& b, cudaStream_t st, cudaEvent_t t0 = nullptr,
+                  cudaEvent_t t1 = nullptr, long long trace_i = -1) {
+  const int alphabet = int(r.view.alphabet);
+  uint64_t* const words = b.words - 4 * (b_lo >> packed_unit_shift(alphabet));
+  SearchVariant v = current_variant();
+  v.avg_len = uint32_t(std::min<uint64_t>((b_hi - b_lo) / std::max<uint64_t>(1, nq), 1u << 30));
+  v.b_lo = b_lo;
+  v.b_hi = b_hi;
+  v.locate_positions = mode == OUT_SP_CNT_U32 && locate_positions_ok(r.view, v);
+  const bool in_wave = d_qbytes && (strands ? search_strands_ascii(r.view, mode, v) : search_packs_ascii(r.view, mode, v));
+  if (d_qbytes && !in_wave) {
+    ProfScope p(2, r.device, st);
+    CU(launch_pack(alphabet, d_qbytes, d_qoff, nq, words, b_lo, b_hi, b.flag, st));
+  }
+  const uint64_t* qoff = d_qoff;
+  uint64_t* qwords = words;
+  uint64_t n = nq;
+  if (strands) {  // the strand wave kernel stages the virtual queries from the bytes itself
+    qwords = b.vwords - 4 * ((2 * b_lo) >> 6);
+    CU(launch_strand_offsets(d_qoff, nq, b_lo, b_hi, b.voff, st));
+    if (!in_wave) CU(launch_strand_words(words, d_qoff, nq, b_lo, b_hi, b.voff, qwords, st));
+    qoff = b.voff;
+    n = 2 * nq;
+    v.b_lo = 2 * b_lo;
+    v.b_hi = 2 * b_hi;
+  }
+  gpu_mark(st, "packed on device", trace_i);
+  ProfScope p(0, r.device, st);
+  if (t0) CU(cudaEventRecord(t0, st));
+  if (in_wave)
+    CU(launch_search_ascii(r.view, d_qbytes, qoff, n, qwords, b.flag, mode, b.out, b.defer, v, r.sm_count, st, strands));
+  else
+    CU(launch_search(r.view, qwords, qoff, n, mode, b.out, b.defer, v, r.sm_count, st));
+  if (t1) CU(cudaEventRecord(t1, st));
+  return v.locate_positions;
+}
+
 // Uploads one chunk of queries and runs prepass + search on ws->st.  The search result lands
 // in ws->d_out in the requested mode.
 // `may_pack`: the caller's say on host packing for this chunk (PackBalance)
@@ -233,28 +311,13 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
                     const Chunk& c, SearchOut mode, bool may_pack = true, bool probe_link = false, bool copy_flag = true,
                     void* d_out_override = nullptr) {
   const uint64_t nq = c.q1 - c.q0, nbytes = c.b1 - c.b0;
-  const uint64_t nv = nq * qs.per_query();  // queries searched
   const size_t out_elem = mode == OUT_COUNT_U64 ? 8 : mode == OUT_RANGE_U64 ? 16 : sp_cnt_bytes(r.view);
-  const int ush = packed_unit_shift(ix->alphabet);
   Workspace::grow_dev(ws->d_qbytes, ws->d_qbytes_cap, size_t(nbytes) + 16);
   Workspace::grow_dev(ws->d_qoff, ws->d_qoff_cap, size_t(nq) + 1);
-  Workspace::grow_dev(ws->d_qwords, ws->d_qwords_cap, size_t(packed_words(ix->alphabet, nq, nbytes)));
-  Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nv) * out_elem);
-  Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nv));
-  if (qs.strands) {
-    Workspace::grow_dev(ws->d_voff, ws->d_voff_cap, size_t(nv) + 1);
-    Workspace::grow_dev(ws->d_vwords, ws->d_vwords_cap, size_t(packed_words(0, nv, 2 * nbytes)));
-  }
+  SearchBuffers b = workspace_buffers(ws, ix->alphabet, nq, c.b0, c.b1, qs.strands, out_elem, ws->d_flag);
+  if (d_out_override) b.out = d_out_override;
   const uint64_t* src_o = qs.qoff + c.q0;
-  uint64_t* const d_words = ws->d_qwords - 4 * (c.b0 >> ush);
-  SearchVariant v = current_variant();
-  v.avg_len = uint32_t(std::min<uint64_t>(nbytes / std::max<uint64_t>(1, nq), 1u << 30));
-  v.b_lo = c.b0;
-  v.b_hi = c.b1;
-  // locate: when pass 2 will be the gather from the unsampled array, queries finished in the text are stored as
-  // their text position (decided here, once, and remembered in the workspace for locate_chunk_walk)
-  v.locate_positions = mode == OUT_SP_CNT_U32 && locate_positions_ok(r.view, v);
-  bool in_wave = false;  // ASCII queries that the wave kernel packs itself (launch_search_ascii)
+  const uint8_t* d_ascii = nullptr;  // the chunk's ASCII bytes on the device (nullptr: launch_pack2 wrote its words)
   ws->link_probe_bytes = 0;
   uint64_t uni_len = 0;
   const bool uniform = offsets_are_uniform(src_o, nq, uni_len);
@@ -272,40 +335,41 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
     parallel_memcpy(ws->h_qoff, src_o, (nq + 1) * 8);
     src_o = ws->h_qoff;
   };
-  if (qs.crumbs) {
-    // pre-packed by the caller: bytes [b0/4, ceil(b1/4)) of the crumb array, exceptions of [b0, b1)
-    const uint64_t cb0 = c.b0 >> 2, cb1 = (c.b1 + 3) >> 2;
-    const size_t pbytes = size_t(cb1 - cb0);
-    const uint8_t* src_c = qs.crumbs + cb0;
-    const uint64_t* e_lo = std::lower_bound(qs.exc, qs.exc + qs.n_exc, c.b0 << 8);
-    const uint64_t* e_hi = std::lower_bound(e_lo, qs.exc + qs.n_exc, c.b1 << 8);
-    const size_t n_exc = size_t(e_hi - e_lo);
+  // 2-bit crumbs up, `base` the query byte the first one stands for, and launch_pack2 writes the words; the exceptions
+  // carry their position relative to `exc_base`.  Pageable crumbs and exceptions are staged through pinned memory.
+  auto upload_crumbs = [&](const uint8_t* src_c, bool pinned, size_t cbytes, uint64_t base, const uint64_t* src_e,
+                           size_t n_exc, uint64_t exc_base) {
     stage_offsets();
-    if (!qs.pinned) {
-      Workspace::grow_host(ws->h_qbytes, ws->h_qbytes_cap, pbytes + 64);
-      parallel_memcpy(ws->h_qbytes, src_c, pbytes);
+    if (!pinned) {
+      Workspace::grow_host(ws->h_qbytes, ws->h_qbytes_cap, cbytes + 64);
+      parallel_memcpy(ws->h_qbytes, src_c, cbytes);
       src_c = ws->h_qbytes;
     }
-    if (pbytes) CU(cudaMemcpyAsync(ws->d_qbytes, src_c, pbytes, cudaMemcpyHostToDevice, ws->st));
+    if (cbytes) CU(cudaMemcpyAsync(ws->d_qbytes, src_c, cbytes, cudaMemcpyHostToDevice, ws->st));
     upload_offsets();
     if (n_exc) {
       Workspace::grow_dev(ws->d_exc, ws->d_exc_cap, n_exc);
-      const uint64_t* src_e = e_lo;
-      if (!qs.pinned) {
+      if (!pinned) {
         Workspace::grow_host(ws->h_exc, ws->h_exc_cap, n_exc);
-        memcpy(ws->h_exc, e_lo, n_exc * 8);
+        memcpy(ws->h_exc, src_e, n_exc * 8);
         src_e = ws->h_exc;
       }
       CU(cudaMemcpyAsync(ws->d_exc, src_e, n_exc * 8, cudaMemcpyHostToDevice, ws->st));
     }
-    g_prof.h2d += pbytes + n_exc * 8;
+    g_prof.h2d += cbytes + n_exc * 8;
     gpu_mark(ws->st, "h2d done", (long long)c.q0);
     CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
-    {
-      ProfScope p(2, r.device, ws->st);
-      CU(launch_pack2(reinterpret_cast<const uint32_t*>(ws->d_qbytes), cb0 << 2, ws->d_qoff, nq, d_words, ws->d_exc, n_exc,
-                      0, c.b0, c.b1, ws->d_flag, ws->st));
-    }
+    ProfScope p(2, r.device, ws->st);
+    CU(launch_pack2(reinterpret_cast<const uint32_t*>(ws->d_qbytes), base, ws->d_qoff, nq,
+                    b.words - 4 * (c.b0 >> packed_unit_shift(ix->alphabet)), ws->d_exc, n_exc, exc_base, c.b0, c.b1, ws->d_flag,
+                    ws->st));
+  };
+  if (qs.crumbs) {
+    // pre-packed by the caller: bytes [b0/4, ceil(b1/4)) of the crumb array, exceptions of [b0, b1)
+    const uint64_t cb0 = c.b0 >> 2, cb1 = (c.b1 + 3) >> 2;
+    const uint64_t* e_lo = std::lower_bound(qs.exc, qs.exc + qs.n_exc, c.b0 << 8);
+    const uint64_t* e_hi = std::lower_bound(e_lo, qs.exc + qs.n_exc, c.b1 << 8);
+    upload_crumbs(qs.crumbs + cb0, qs.pinned, size_t(cb1 - cb0), cb0 << 2, e_lo, size_t(e_hi - e_lo), 0);
   } else {
     const uint8_t* src_b = qs.qbytes + c.b0;
     // Nucleotide chunks are packed to 2 bits per base by the host cores before the copy (a quarter of
@@ -321,26 +385,11 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
         bal.note_host(double(nbytes), std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(), sharers);
       trace_mark("  host pack done, bytes", (long long)nbytes);
     }
-    if (packed) {
+    if (packed) {  // the crumbs are in pinned memory already; the exceptions join them there
       const size_t n_exc = ws->exc_tmp.size();
-      const size_t pbytes = (size_t(nbytes) + 3) / 4;
-      stage_offsets();
-      CU(cudaMemcpyAsync(ws->d_qbytes, ws->h_qbytes, pbytes + 8, cudaMemcpyHostToDevice, ws->st));
-      upload_offsets();
-      if (n_exc) {
-        Workspace::grow_host(ws->h_exc, ws->h_exc_cap, n_exc);
-        Workspace::grow_dev(ws->d_exc, ws->d_exc_cap, n_exc);
-        memcpy(ws->h_exc, ws->exc_tmp.data(), n_exc * 8);
-        CU(cudaMemcpyAsync(ws->d_exc, ws->h_exc, n_exc * 8, cudaMemcpyHostToDevice, ws->st));
-      }
-      g_prof.h2d += pbytes + 8 + n_exc * 8;
-      gpu_mark(ws->st, "h2d done", (long long)c.q0);
-      CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
-      {
-        ProfScope p(2, r.device, ws->st);
-        CU(launch_pack2(reinterpret_cast<const uint32_t*>(ws->d_qbytes), c.b0, ws->d_qoff, nq, d_words, ws->d_exc, n_exc,
-                        c.b0, c.b0, c.b1, ws->d_flag, ws->st));
-      }
+      Workspace::grow_host(ws->h_exc, ws->h_exc_cap, n_exc);
+      if (n_exc) memcpy(ws->h_exc, ws->exc_tmp.data(), n_exc * 8);
+      upload_crumbs(ws->h_qbytes, true, (size_t(nbytes) + 3) / 4 + 8, c.b0, ws->h_exc, n_exc, c.b0);
     } else {
       if (!qs.pinned) {
         Workspace::grow_host(ws->h_qbytes, ws->h_qbytes_cap, size_t(nbytes) + 16);
@@ -364,51 +413,19 @@ void enqueue_search(const awry_index* ix, Replica& r, PackBalance& bal, Workspac
       upload_offsets();
       g_prof.h2d += nbytes;
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
-      // offsets stay absolute: the kernels subtract the chunk's byte base
-      in_wave = qs.strands ? search_strands_ascii(r.view, mode, v) : search_packs_ascii(r.view, mode, v);
-      if (!in_wave) {
-        ProfScope p(2, r.device, ws->st);
-        CU(launch_pack(ix->alphabet, ws->d_qbytes - c.b0, ws->d_qoff, nq, d_words, c.b0, c.b1, ws->d_flag, ws->st));
-      }
+      d_ascii = ws->d_qbytes - c.b0;  // offsets stay absolute: the kernels subtract the chunk's byte base
     }
   }
-  // both strands: the virtual queries (kernels.hpp); the strand wave kernel stages them from the bytes itself
-  const uint64_t* d_soff = ws->d_qoff;
-  const uint64_t* d_swords = d_words;
-  SearchVariant sv = v;
-  if (qs.strands) {
-    uint64_t* const d_vwords = ws->d_vwords - 4 * ((2 * c.b0) >> 6);
-    CU(launch_strand_offsets(ws->d_qoff, nq, c.b0, c.b1, ws->d_voff, ws->st));
-    if (!in_wave) CU(launch_strand_words(d_words, ws->d_qoff, nq, c.b0, c.b1, ws->d_voff, d_vwords, ws->st));
-    d_soff = ws->d_voff;
-    d_swords = d_vwords;
-    sv.b_lo = 2 * c.b0;
-    sv.b_hi = 2 * c.b1;
+  ws->gpu_probe_bytes = 0;
+  const bool time_kernel = qs.pinned && !qs.crumbs && nbytes >= (8u << 20);  // PackBalance: what the GPU consumes
+  if (time_kernel && !ws->ev_s0) {
+    CU(cudaEventCreate(&ws->ev_s0));
+    CU(cudaEventCreate(&ws->ev_s1));
   }
-  gpu_mark(ws->st, "packed on device", (long long)c.q0);
-  {
-    ProfScope p(0, r.device, ws->st);
-    ws->sp_cnt_positions = v.locate_positions;
-    ws->gpu_probe_bytes = 0;
-    const bool time_kernel = qs.pinned && !qs.crumbs && nbytes >= (8u << 20);  // PackBalance: what the GPU consumes
-    if (time_kernel) {
-      if (!ws->ev_s0) {
-        CU(cudaEventCreate(&ws->ev_s0));
-        CU(cudaEventCreate(&ws->ev_s1));
-      }
-      CU(cudaEventRecord(ws->ev_s0, ws->st));
-    }
-    void* const d_out = d_out_override ? d_out_override : ws->d_out;
-    if (in_wave)
-      CU(launch_search_ascii(r.view, ws->d_qbytes - c.b0, d_soff, nv, const_cast<uint64_t*>(d_swords), ws->d_flag, mode,
-                             d_out, ws->d_defer, sv, r.sm_count, ws->st, qs.strands));
-    else
-      CU(launch_search(r.view, d_swords, d_soff, nv, mode, d_out, ws->d_defer, sv, r.sm_count, ws->st));
-    if (time_kernel) {
-      CU(cudaEventRecord(ws->ev_s1, ws->st));
-      ws->gpu_probe_bytes = nbytes;
-    }
-  }
+  // (remembered for locate_chunk_walk: pass 2 must then be the gather from the unsampled array)
+  ws->sp_cnt_positions = search_reads(r, d_ascii, ws->d_qoff, nq, c.b0, c.b1, qs.strands, mode, b, ws->st,
+                                      time_kernel ? ws->ev_s0 : nullptr, time_kernel ? ws->ev_s1 : nullptr, (long long)c.q0);
+  if (time_kernel) ws->gpu_probe_bytes = nbytes;
   gpu_mark(ws->st, "searched", (long long)c.q0);
   // (the locate pipeline copies the flag together with the hit total, after the scan: one hand-over between
   // the compute and copy engines per chunk instead of two)
@@ -1421,43 +1438,6 @@ void strands_check_index(const awry_index* ix) {
   if (ix->alphabet != AWRY_NUCLEOTIDE) fail(AWRY_ERR_UNSUPPORTED, "both-strand search exists for the nucleotide alphabet only");
 }
 
-// Device-resident batch of nq reads on both strands: the 2 nq virtual queries (kernels.hpp) searched into d_out, all on
-// stream `st`, scratch released in stream order with `sc`.  The strand wave kernel reads the bytes itself; otherwise
-// pack_kernel packs the reads and launch_strand_words derives the virtual words.  What the prepass refuses is latched
-// in r.d_async_flag.  Returns whether pass 1 stored one-hit queries as text positions (locate_positions).
-bool strands_search_device(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t e0, uint64_t e1,
-                           SearchOut mode, void* d_out, uint32_t* d_defer, StreamScratch& sc, cudaStream_t st) {
-  const uint64_t nv = 2 * nq;
-  uint64_t* const d_voff = sc.get<uint64_t>(nv + 1);
-  uint64_t* const d_vwords = sc.get<uint64_t>(packed_words(0, nv, 2 * (e1 - e0))) - 4 * ((2 * e0) >> 6);
-  SearchVariant v = current_variant();
-  v.avg_len = uint32_t(std::min<uint64_t>((e1 - e0) / nq, 1u << 30));
-  v.b_lo = 2 * e0;
-  v.b_hi = 2 * e1;
-  v.locate_positions = mode == OUT_SP_CNT_U32 && locate_positions_ok(r.view, v);
-  CU(launch_strand_offsets(d_qoff, nq, e0, e1, d_voff, st));
-  ProfScope p(0, r.device, st);
-  if (search_strands_ascii(r.view, mode, v)) {
-    CU(launch_search_ascii(r.view, d_qbytes, d_voff, nv, d_vwords, r.d_async_flag, mode, d_out, d_defer, v, r.sm_count, st,
-                           true));
-  } else {
-    uint64_t* const d_words = sc.get<uint64_t>(packed_words(0, nq, e1 - e0)) - 4 * (e0 >> 6);
-    CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_words, e0, e1, r.d_async_flag, st));
-    CU(launch_strand_words(d_words, d_qoff, nq, e0, e1, d_voff, d_vwords, st));
-    CU(launch_search(r.view, d_vwords, d_voff, nv, mode, d_out, d_defer, v, r.sm_count, st));
-  }
-  return v.locate_positions;
-}
-
-// the first and last offset of a device-resident batch (one 16-byte read-back), checked
-void device_batch_ends(const uint64_t* d_qoff, uint64_t nq, cudaStream_t st, uint64_t ends[2]) {
-  CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
-  if (ends[1] >= (1ull << 62)) fail(AWRY_ERR_INVALID_ARG, "query offsets beyond 2^62");
-}
-
 void strands_check_device_batch(uint64_t nq) {
   if (2 * nq >= (1ull << 32) - (1u << 24))  // (the search kernels' 32-bit ticket counter)
     fail(AWRY_ERR_INVALID_ARG, "batch too large for one both-strand search (%llu reads): split it", (unsigned long long)nq);
@@ -1516,6 +1496,104 @@ void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint
   if (total > capacity)
     fail(AWRY_ERR_CAPACITY, "hit buffer holds %llu entries, %llu needed", (unsigned long long)capacity,
          (unsigned long long)total);
+}
+
+// ------------------------------------------------------------------ device-resident batches (awry_*_device*)
+// What the prepass refuses stays latched in r.d_async_flag for awry_device_check.
+
+// the first and last offset of a device-resident batch (one 16-byte read-back), checked; both strands also need the
+// virtual offsets 2 e to fit
+void device_batch_ends(const uint64_t* d_qoff, uint64_t nq, cudaStream_t st, uint64_t ends[2], bool strands) {
+  CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
+  if (strands && ends[1] >= (1ull << 62)) fail(AWRY_ERR_INVALID_ARG, "query offsets beyond 2^62");
+}
+
+// awry_count_device[_strands]: counts of the nq (or 2 nq virtual) queries
+void count_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                       uint64_t* d_counts, void* cuda_stream, bool strands) {
+  need(ix);
+  if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+  if (strands) strands_check_index(ix);
+  if (nq == 0) return;
+  if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (strands) strands_check_device_batch(nq);
+  Replica& r = *ix->reps[size_t(replica)];
+  DeviceGuard dg(r.device);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  uint64_t e[2] = {0, 0};
+  device_batch_ends(d_qoff, nq, st, e, strands);
+  const uint64_t nv = strands ? 2 * nq : nq;
+  const uint64_t w = query_words(ix->alphabet, nq, e[0], e[1]);
+  const uint64_t vw = strands ? query_words(AWRY_NUCLEOTIDE, nv, 2 * e[0], 2 * e[1]) : 0, vo = strands ? nv + 1 : 0;
+  uint64_t* buf = nullptr;  // one stream-ordered allocation: read words, [virtual words, virtual offsets,] defer list
+  CU(cudaMallocAsync(reinterpret_cast<void**>(&buf), (w + vw + vo) * 8 + defer_words(nv) * 4, st));
+  try {
+    search_reads(r, d_qbytes, d_qoff, nq, e[0], e[1], strands, OUT_COUNT_U64,
+                 SearchBuffers{buf, buf + w + vw, buf + w, d_counts, reinterpret_cast<uint32_t*>(buf + w + vw + vo),
+                               r.d_async_flag},
+                 st);
+  } catch (...) {
+    cudaFreeAsync(buf, st);
+    throw;
+  }
+  CU(cudaFreeAsync(buf, st));
+}
+
+// awry_locate_device[_strands]: the hits of the nq (or 2 nq virtual) queries, in a stream-ordered device buffer
+void locate_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                        uint32_t flags, uint64_t* d_hit_off, awry_hit** d_hits, uint64_t* n_hits, void* cuda_stream,
+                        bool strands) {
+  need(ix);
+  if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+  if (!d_hit_off || !d_hits || !n_hits) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  *d_hits = nullptr;
+  *n_hits = 0;
+  if (strands) strands_check_index(ix);
+  if (nq == 0) return;
+  if (!d_qbytes || !d_qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (strands) strands_check_device_batch(nq);
+  Replica& r = *ix->reps[size_t(replica)];
+  DeviceGuard dg(r.device);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  uint64_t e[2] = {0, 0};
+  device_batch_ends(d_qoff, nq, st, e, strands);
+  const uint64_t nv = strands ? 2 * nq : nq;
+  Workspace* ws = r.acquire();
+  try {
+    const SearchBuffers b = workspace_buffers(ws, ix->alphabet, nq, e[0], e[1], strands, sp_cnt_bytes(r.view), r.d_async_flag);
+    ws->sp_cnt_positions = search_reads(r, d_qbytes, d_qoff, nq, e[0], e[1], strands, OUT_SP_CNT_U32, b, st);
+    uint64_t n = 0;
+    uint64_t* h = locate_chunk_device(ix, r, ws, nv, flags, d_hit_off, &n, st);
+    CU(cudaStreamSynchronize(st));
+    *d_hits = reinterpret_cast<awry_hit*>(h);
+    *n_hits = n;
+  } catch (...) {
+    cudaStreamSynchronize(st);
+    r.release(ws);
+    throw;
+  }
+  r.release(ws);
+}
+
+// awry_count_device_hamming[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
+void hamming_count_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                               uint64_t nq, uint32_t k, uint64_t* d_counts, void* cuda_stream, bool strands) {
+  need(ix);
+  if (k > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+  if (nq == 0) return;
+  if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (strands) strands_check_index(ix);
+  hamming_check_index(ix);
+  Replica& r = *ix->reps[size_t(replica)];
+  DeviceGuard dg(r.device);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  uint64_t e[2] = {0, 0};
+  device_batch_ends(d_qoff, nq, st, e, strands);
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands);
 }
 
 }  // namespace host
@@ -1595,103 +1673,13 @@ int awry_locate_batch_packed2(const awry_index* ix, const uint8_t* crumbs, const
 
 int awry_count_device(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
                       uint64_t* d_counts, void* cuda_stream) {
-  return guarded([&] {
-    need(ix);
-    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
-    if (nq == 0) return;
-    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    Replica& r = *ix->reps[size_t(replica)];
-    DeviceGuard dg(r.device);
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    // total query bytes bound the packed size; read the last offset (one 8-byte D2H)
-    uint64_t ends[2] = {0, 0};
-    CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
-    const int sh = packed_unit_shift(ix->alphabet);
-    uint64_t words = 4 * (nq + ((ends[1] >> sh) - (ends[0] >> sh)) + 2) + 32;
-    uint64_t* d_qwords = nullptr;  // packed queries, then the deferred-query list
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&d_qwords), words * 8 + defer_words(nq) * 4, st));
-    uint32_t* d_defer = reinterpret_cast<uint32_t*>(d_qwords + words);
-    uint64_t* const d_words = d_qwords - 4 * (ends[0] >> sh);
-    SearchVariant v = current_variant();
-    v.avg_len = uint32_t(std::min<uint64_t>((ends[1] - ends[0]) / nq, 1u << 30));
-    v.b_lo = ends[0];
-    v.b_hi = ends[1];
-    const bool in_wave = search_packs_ascii(r.view, OUT_COUNT_U64, v);
-    if (!in_wave) {
-      ProfScope p(2, r.device, st);
-      CU(launch_pack(ix->alphabet, d_qbytes, d_qoff, nq, d_words, ends[0], ends[1], r.d_async_flag, st));
-    }
-    {
-      ProfScope p(0, r.device, st);
-      if (in_wave)
-        CU(launch_search_ascii(r.view, d_qbytes, d_qoff, nq, d_words, r.d_async_flag, OUT_COUNT_U64, d_counts, d_defer, v,
-                               r.sm_count, st));
-      else
-        CU(launch_search(r.view, d_words, d_qoff, nq, OUT_COUNT_U64, d_counts, d_defer, v, r.sm_count, st));
-    }
-    CU(cudaFreeAsync(d_qwords, st));
-  });
+  return guarded([&] { count_device_impl(ix, replica, d_qbytes, d_qoff, nq, d_counts, cuda_stream, false); });
 }
 
 int awry_locate_device(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
                        uint32_t flags, uint64_t* d_hit_off, awry_hit** d_hits, uint64_t* n_hits, void* cuda_stream) {
   return guarded([&] {
-    need(ix);
-    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
-    if (!d_hit_off || !d_hits || !n_hits) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    *d_hits = nullptr;
-    *n_hits = 0;
-    if (nq == 0) return;
-    if (!d_qbytes || !d_qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    Replica& r = *ix->reps[size_t(replica)];
-    DeviceGuard dg(r.device);
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    uint64_t ends[2] = {0, 0};
-    CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
-    const int sh = packed_unit_shift(ix->alphabet);
-    Workspace* ws = r.acquire();
-    try {
-      uint64_t words = 4 * (nq + ((ends[1] >> sh) - (ends[0] >> sh)) + 2) + 32;
-      Workspace::grow_dev(ws->d_qwords, ws->d_qwords_cap, size_t(words));
-      Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nq) * sp_cnt_bytes(r.view));
-      Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nq));
-      uint64_t* const d_words = ws->d_qwords - 4 * (ends[0] >> sh);
-      SearchVariant v = current_variant();
-      v.avg_len = uint32_t(std::min<uint64_t>((ends[1] - ends[0]) / nq, 1u << 30));
-      v.b_lo = ends[0];
-      v.b_hi = ends[1];
-      v.locate_positions = locate_positions_ok(r.view, v);
-      ws->sp_cnt_positions = v.locate_positions;
-      const bool in_wave = search_packs_ascii(r.view, OUT_SP_CNT_U32, v);
-      if (!in_wave) {
-        ProfScope p(2, r.device, st);
-        CU(launch_pack(ix->alphabet, d_qbytes, d_qoff, nq, d_words, ends[0], ends[1], r.d_async_flag, st));
-      }
-      {
-        ProfScope p(0, r.device, st);
-        if (in_wave)
-          CU(launch_search_ascii(r.view, d_qbytes, d_qoff, nq, d_words, r.d_async_flag, OUT_SP_CNT_U32, ws->d_out,
-                                 ws->d_defer, v, r.sm_count, st));
-        else
-          CU(launch_search(r.view, d_words, d_qoff, nq, OUT_SP_CNT_U32, ws->d_out, ws->d_defer, v, r.sm_count, st));
-      }
-      uint64_t n = 0;
-      uint64_t* h = locate_chunk_device(ix, r, ws, nq, flags, d_hit_off, &n, st);
-      CU(cudaStreamSynchronize(st));
-      *d_hits = reinterpret_cast<awry_hit*>(h);
-      *n_hits = n;
-    } catch (...) {
-      cudaStreamSynchronize(st);
-      r.release(ws);
-      throw;
-    }
-    r.release(ws);
+    locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, flags, d_hit_off, d_hits, n_hits, cuda_stream, false);
   });
 }
 
@@ -1711,21 +1699,7 @@ int awry_locate_batch_hamming(const awry_index* ix, const uint8_t* qbytes, const
 int awry_count_device_hamming(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
                               uint64_t nq, uint32_t max_mismatches, uint64_t* d_counts, void* cuda_stream) {
   return guarded([&] {
-    need(ix);
-    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
-    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
-    if (nq == 0) return;
-    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    hamming_check_index(ix);
-    Replica& r = *ix->reps[size_t(replica)];
-    DeviceGuard dg(r.device);
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    uint64_t ends[2] = {0, 0};
-    CU(cudaMemcpyAsync(&ends[0], d_qoff, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ends[1], d_qoff + nq, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (ends[1] < ends[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
-    hamming_run(r, d_qbytes, d_qoff, nq, ends[0], ends[1], max_mismatches, r.d_async_flag, -1, st, d_counts, nullptr);
+    hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_mismatches, d_counts, cuda_stream, false);
   });
 }
 
@@ -1745,19 +1719,7 @@ int awry_locate_batch_hamming_strands(const awry_index* ix, const uint8_t* qbyte
 int awry_count_device_hamming_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
                                       uint64_t nq, uint32_t max_mismatches, uint64_t* d_counts, void* cuda_stream) {
   return guarded([&] {
-    need(ix);
-    if (max_mismatches > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
-    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
-    if (nq == 0) return;
-    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    strands_check_index(ix);
-    hamming_check_index(ix);
-    Replica& r = *ix->reps[size_t(replica)];
-    DeviceGuard dg(r.device);
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    uint64_t ends[2] = {0, 0};
-    device_batch_ends(d_qoff, nq, st, ends);
-    hamming_run(r, d_qbytes, d_qoff, nq, ends[0], ends[1], max_mismatches, r.d_async_flag, -1, st, d_counts, nullptr, true);
+    hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_mismatches, d_counts, cuda_stream, true);
   });
 }
 
@@ -1792,63 +1754,14 @@ int awry_locate_batch_strands(const awry_index* ix, const uint8_t* qbytes, const
 
 int awry_count_device_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
                               uint64_t nq, uint64_t* d_counts, void* cuda_stream) {
-  return guarded([&] {
-    need(ix);
-    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
-    strands_check_index(ix);
-    if (nq == 0) return;
-    if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    strands_check_device_batch(nq);
-    Replica& r = *ix->reps[size_t(replica)];
-    DeviceGuard dg(r.device);
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    uint64_t ends[2] = {0, 0};
-    device_batch_ends(d_qoff, nq, st, ends);
-    StreamScratch sc(st);
-    strands_search_device(r, d_qbytes, d_qoff, nq, ends[0], ends[1], OUT_COUNT_U64, d_counts,
-                          sc.get<uint32_t>(defer_words(2 * nq)), sc, st);
-  });
+  return guarded([&] { count_device_impl(ix, replica, d_qbytes, d_qoff, nq, d_counts, cuda_stream, true); });
 }
 
 int awry_locate_device_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
                                uint64_t nq, uint32_t flags, uint64_t* d_hit_off, awry_hit** d_hits, uint64_t* n_hits,
                                void* cuda_stream) {
   return guarded([&] {
-    need(ix);
-    if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
-    if (!d_hit_off || !d_hits || !n_hits) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    *d_hits = nullptr;
-    *n_hits = 0;
-    strands_check_index(ix);
-    if (nq == 0) return;
-    if (!d_qbytes || !d_qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
-    strands_check_device_batch(nq);
-    Replica& r = *ix->reps[size_t(replica)];
-    DeviceGuard dg(r.device);
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    uint64_t ends[2] = {0, 0};
-    device_batch_ends(d_qoff, nq, st, ends);
-    Workspace* ws = r.acquire();
-    try {
-      const uint64_t nv = 2 * nq;
-      Workspace::grow_dev(ws->d_out, ws->d_out_cap, size_t(nv) * sp_cnt_bytes(r.view));
-      Workspace::grow_dev(ws->d_defer, ws->d_defer_cap, defer_words(nv));
-      {
-        StreamScratch sc(st);
-        ws->sp_cnt_positions =
-            strands_search_device(r, d_qbytes, d_qoff, nq, ends[0], ends[1], OUT_SP_CNT_U32, ws->d_out, ws->d_defer, sc, st);
-      }
-      uint64_t n = 0;
-      uint64_t* h = locate_chunk_device(ix, r, ws, nv, flags, d_hit_off, &n, st);
-      CU(cudaStreamSynchronize(st));
-      *d_hits = reinterpret_cast<awry_hit*>(h);
-      *n_hits = n;
-    } catch (...) {
-      cudaStreamSynchronize(st);
-      r.release(ws);
-      throw;
-    }
-    r.release(ws);
+    locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, flags, d_hit_off, d_hits, n_hits, cuda_stream, true);
   });
 }
 
