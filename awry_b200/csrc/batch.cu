@@ -1203,13 +1203,13 @@ static uint64_t hamming_slice() {
   return 1ull << 26;
 }
 
-void hamming_check_index(const awry_index* ix) {
-  if (ix->alphabet != AWRY_NUCLEOTIDE) fail(AWRY_ERR_UNSUPPORTED, "Hamming search exists for the nucleotide alphabet only");
+void hamming_check_index(const awry_index* ix, const char* what = "Hamming") {
+  if (ix->alphabet != AWRY_NUCLEOTIDE) fail(AWRY_ERR_UNSUPPORTED, "%s search exists for the nucleotide alphabet only", what);
   for (auto& rp : ix->reps)
     if (rp->view.wide || !rp->view.rtext || !rp->view.full_sa)
       fail(AWRY_ERR_UNSUPPORTED,
-           "Hamming search needs the unsampled suffix array and the text on every device (not built for this index: "
-           "AWRY_B200_FULL_SA / AWRY_B200_TEXT, device memory, or 64-bit row pointers)");
+           "%s search needs the unsampled suffix array and the text on every device (not built for this index: "
+           "AWRY_B200_FULL_SA / AWRY_B200_TEXT, device memory, or 64-bit row pointers)", what);
 }
 
 // the hits of the locate call on one replica, in query order
@@ -1227,12 +1227,20 @@ struct HammingSink {
 // < 0 (the device-resident call): it stays latched in *d_flag for awry_device_check.
 // `strands`: the nq reads are searched as the 2 nq virtual queries of both strands (kernels.hpp), which take the
 // place of the reads from the piece offsets on: counts, CSR offsets and the hits are per virtual query.
+// `metric`: substitutions (Hamming, one window per candidate) or edits (awry_*_edit: 2k + 1 starts per candidate,
+// kernels_edit.cu).  Stages 1 and 2 are the same for both; the metric picks the verification kernel and, for locate,
+// the key slots per candidate.  A slice holds at most hamming_slice() key slots.
+enum Metric { METRIC_HAMMING = 0, METRIC_EDIT = 1 };
+const char* metric_name(Metric metric) { return metric == METRIC_EDIT ? "edit-distance" : "Hamming"; }
 void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
                  uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
-                 HammingSink* sink, bool strands = false) {
+                 HammingSink* sink, bool strands = false, Metric metric = METRIC_HAMMING) {
+  const bool edit = metric == METRIC_EDIT;
+  const char* const what = metric_name(metric);
   const uint32_t shift = strands ? 1 : 0;  // virtual query -> read
   const uint64_t P = k + 1, nbytes = b_hi - b_lo, nv = nq << shift, np = nv * P;
-  if (np >= (1ull << 31)) fail(AWRY_ERR_INVALID_ARG, "batch too large for one Hamming search (%llu reads): split it", (unsigned long long)nq);
+  const uint64_t slots = edit ? 2 * k + 1 : 1;  // key slots per candidate
+  if (np >= (1ull << 31)) fail(AWRY_ERR_INVALID_ARG, "batch too large for one %s search (%llu reads): split it", what, (unsigned long long)nq);
   StreamScratch sc(st);
   // 1. pieces, packed; the whole reads packed too (their prepass validates the offsets and latches what it refuses).
   // Single strand: the pieces are packed from the caller's bytes (DESIGN.md §1c: cutting them out of the read words
@@ -1297,8 +1305,8 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   CU(cudaStreamSynchronize(st));
   if (flag != ~0ull && (flag & 1) == BAD_QUERY)
     fail(AWRY_ERR_INVALID_QUERY,
-         "query %llu is empty, contains a sentinel ('$'/'#') or is not longer than max_mismatches = %u (every window "
-         "would match)", (unsigned long long)(uint64_t(check_base) + (flag >> 1)), k);
+         "query %llu is empty, contains a sentinel ('$'/'#') or is not longer than %s = %u (every window "
+         "would match)", (unsigned long long)(uint64_t(check_base) + (flag >> 1)), edit ? "max_edits" : "max_mismatches", k);
   if (flag != ~0ull) fail_bad_query(flag, uint64_t(check_base));
 
   HammingSlice a{};
@@ -1311,7 +1319,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   a.sp_cnt = d_sp;
   a.hoff = d_hoff;
   a.npieces = np;
-  const uint64_t S = hamming_slice();
+  const uint64_t S = std::max<uint64_t>(1, hamming_slice() / slots);  // candidates per slice
   if (!sink) {  // 3. count: slices cut anywhere
     CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
     for (uint64_t c0 = 0; c0 < total; c0 += S) {
@@ -1324,7 +1332,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       a.map = d_map;
       a.counts = d_counts;
       ProfScope p(1, r.device, st);
-      CU(launch_hamming_verify(r.view, a, k, false, r.sm_count, st));
+      CU(edit ? launch_edit_verify(r.view, a, k, false, r.sm_count, st) : launch_hamming_verify(r.view, a, k, false, r.sm_count, st));
     }
     return;
   }
@@ -1334,9 +1342,9 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     uint64_t q1 = q0 + 1;
     while (q1 < nv && qcand[q1 + 1] - qcand[q0] <= S) q1++;
     const uint64_t c0 = qcand[q0], n = qcand[q1] - c0, nr = q1 - q0;
-    if (n >= (1ull << 31))  // (a slice is sorted per read by one CUB call, whose offsets are int)
+    if (n * slots >= (1ull << 31))  // (a slice is sorted per read by one CUB call, whose offsets are int)
       fail(AWRY_ERR_NOMEM, "query %llu has %llu candidate windows, more than one slice can sort (2^31)",
-           (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + (q0 >> shift)), (unsigned long long)n);
+           (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + (q0 >> shift)), (unsigned long long)(n * slots));
     const uint64_t base = sink->hits.size();
     if (n == 0) {
       sink->off.insert(sink->off.end(), nr, base);
@@ -1351,17 +1359,22 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     CU(launch_hamming_map(d_hoff, np, c0, n, d_map, nullptr, temp, st));
     CU(launch_hamming_map(d_hoff, np, c0, n, d_map, ss.get<uint8_t>(temp), temp, st));
     a.map = d_map;
-    a.keys = ss.get<uint64_t>(n);
+    a.keys = ss.get<uint64_t>(n * slots);
     a.acc = ss.get<uint64_t>(nr + 1);
     CU(cudaMemsetAsync(a.acc, 0, (nr + 1) * 8, st));
     {
       ProfScope p(1, r.device, st);
-      CU(launch_hamming_verify(r.view, a, k, true, r.sm_count, st));
+      CU(edit ? launch_edit_verify(r.view, a, k, true, r.sm_count, st) : launch_hamming_verify(r.view, a, k, true, r.sm_count, st));
     }
-    uint64_t* d_sorted = ss.get<uint64_t>(n);
+    uint64_t* d_sorted = ss.get<uint64_t>(n * slots);
     size_t t2 = 0;
-    CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, nullptr, t2, st));
-    CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, ss.get<uint8_t>(t2), t2, st));
+    if (edit) {
+      CU(sort_edit_keys(a.keys, d_sorted, n * slots, nr, d_qcand + q0, c0, uint32_t(slots), nullptr, t2, st));
+      CU(sort_edit_keys(a.keys, d_sorted, n * slots, nr, d_qcand + q0, c0, uint32_t(slots), ss.get<uint8_t>(t2), t2, st));
+    } else {
+      CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, nullptr, t2, st));
+      CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, ss.get<uint8_t>(t2), t2, st));
+    }
     uint64_t* d_qh = ss.get<uint64_t>(nr + 1);
     size_t t3 = 0;
     CU(scan_u64(a.acc, d_qh, nr + 1, nullptr, t3, st));
@@ -1374,7 +1387,10 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       uint64_t* d_pos = ss.get<uint64_t>(n_acc);
       uint8_t* d_dist = ss.get<uint8_t>(n_acc);
       uint64_t* d_hits = ss.get<uint64_t>(2 * n_acc);
-      CU(launch_hamming_compact(d_sorted, d_map, n, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
+      if (edit)
+        CU(launch_edit_compact(d_sorted, d_map, n * slots, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
+      else
+        CU(launch_hamming_compact(d_sorted, d_map, n, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
       CU(launch_map_locations(r.view, d_pos, n_acc, d_hits, st));
       sink->hits.resize(base + n_acc);
       sink->dist.resize(base + n_acc);
@@ -1391,7 +1407,8 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
 // reads [lo, hi) of host buffers on replica ri: chunks of reads uploaded and searched one after the other (the
 // host path does not overlap copies with compute yet).  `strands`: a chunk of n reads fills 2 n result slots.
 void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo,
-                        uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink, bool strands = false) {
+                        uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink, bool strands = false,
+                        Metric metric = METRIC_HAMMING) {
   if (lo >= hi) return;
   Replica& r = *ix->reps[ri];
   DeviceGuard dg(r.device);
@@ -1412,13 +1429,13 @@ void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, 
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
       if (sink) {
         hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr, sink,
-                    strands);
+                    strands, metric);
       } else {
         StreamScratch sc(ws->st);
         const uint64_t slots = (strands ? 2 : 1) * (k + 1);  // counts per read
         uint64_t* d_counts = sc.get<uint64_t>(n * slots);
         hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts, nullptr,
-                    strands);
+                    strands, metric);
         CU(cudaMemcpyAsync(counts + c.q0 * slots, d_counts, n * slots * 8, cudaMemcpyDeviceToHost, ws->st));
         g_prof.d2h += n * slots * 8;
       }
@@ -1443,40 +1460,49 @@ void strands_check_device_batch(uint64_t nq) {
     fail(AWRY_ERR_INVALID_ARG, "batch too large for one both-strand search (%llu reads): split it", (unsigned long long)nq);
 }
 
-// awry_count_batch_hamming[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
+// the bound on k of each metric (the same number, named after its argument)
+void check_max_k(uint32_t k, Metric metric) {
+  if (metric == METRIC_EDIT) {
+    if (k > AWRY_EDIT_MAX) fail(AWRY_ERR_INVALID_ARG, "max_edits must be 0 .. %d", AWRY_EDIT_MAX);
+  } else if (k > AWRY_HAMMING_MAX) {
+    fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  }
+}
+
+// awry_count_batch_{hamming,edit}[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
 void hamming_count_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t k,
-                        uint64_t* counts, bool strands) {
+                        uint64_t* counts, bool strands, Metric metric = METRIC_HAMMING) {
   need(ix);
-  if (k > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  check_max_k(k, metric);
   if (nq == 0) return;
   if (!qbytes || !qoff || !counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
   if (strands) strands_check_index(ix);
-  hamming_check_index(ix);
+  hamming_check_index(ix, metric_name(metric));
   for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
-    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, counts, nullptr, strands);
+    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, counts, nullptr, strands, metric);
   });
 }
 
-// awry_locate_batch_hamming[_strands]: hit_off is the CSR over the nq (or 2 nq virtual) queries
+// awry_locate_batch_{hamming,edit}[_strands]: hit_off is the CSR over the nq (or 2 nq virtual) queries
 void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t k,
                          uint64_t* hit_off, awry_hit* hits, uint8_t* hit_mismatches, uint64_t capacity, uint64_t* n_hits,
-                         bool strands) {
+                         bool strands, Metric metric = METRIC_HAMMING) {
   need(ix);
-  if (k > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  check_max_k(k, metric);
   if (!hit_off || !n_hits || (!hits && capacity)) fail(AWRY_ERR_INVALID_ARG, "null argument");
   *n_hits = 0;
   hit_off[0] = 0;
   if (nq == 0) return;
   if (!qbytes || !qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
   if (strands) strands_check_index(ix);
-  hamming_check_index(ix);
+  hamming_check_index(ix, metric_name(metric));
   const uint64_t per = strands ? 2 : 1;  // result slots per read
   const size_t nr = ix->reps.size();
   std::vector<HammingSink> sinks(nr);
   std::vector<std::pair<uint64_t, uint64_t>> ranges(nr, {0, 0});
   for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
     ranges[ri] = {lo, hi};
-    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, nullptr, &sinks[ri], strands);
+    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, nullptr, &sinks[ri], strands, metric);
   });
   // the replicas' CSRs, concatenated in range order; hits past `capacity` are dropped (the total still counts them)
   uint64_t total = 0;
@@ -1578,22 +1604,23 @@ void locate_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbyt
   r.release(ws);
 }
 
-// awry_count_device_hamming[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
+// awry_count_device_{hamming,edit}[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
 void hamming_count_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
-                               uint64_t nq, uint32_t k, uint64_t* d_counts, void* cuda_stream, bool strands) {
+                               uint64_t nq, uint32_t k, uint64_t* d_counts, void* cuda_stream, bool strands,
+                               Metric metric = METRIC_HAMMING) {
   need(ix);
-  if (k > AWRY_HAMMING_MAX) fail(AWRY_ERR_INVALID_ARG, "max_mismatches must be 0 .. %d", AWRY_HAMMING_MAX);
+  check_max_k(k, metric);
   if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
   if (nq == 0) return;
   if (!d_qbytes || !d_qoff || !d_counts) fail(AWRY_ERR_INVALID_ARG, "null argument");
   if (strands) strands_check_index(ix);
-  hamming_check_index(ix);
+  hamming_check_index(ix, metric_name(metric));
   Replica& r = *ix->reps[size_t(replica)];
   DeviceGuard dg(r.device);
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
   uint64_t e[2] = {0, 0};
   device_batch_ends(d_qoff, nq, st, e, strands);
-  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands);
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands, metric);
 }
 
 }  // namespace host
@@ -1720,6 +1747,46 @@ int awry_count_device_hamming_strands(const awry_index* ix, int replica, const u
                                       uint64_t nq, uint32_t max_mismatches, uint64_t* d_counts, void* cuda_stream) {
   return guarded([&] {
     hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_mismatches, d_counts, cuda_stream, true);
+  });
+}
+
+int awry_count_batch_edit(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                          uint32_t max_edits, uint64_t* counts) {
+  return guarded([&] { hamming_count_impl(ix, qbytes, qoff, nq, max_edits, counts, false, METRIC_EDIT); });
+}
+
+int awry_locate_batch_edit(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                           uint32_t max_edits, uint64_t* hit_off, awry_hit* hits, uint8_t* hit_edits, uint64_t capacity,
+                           uint64_t* n_hits) {
+  return guarded([&] {
+    hamming_locate_impl(ix, qbytes, qoff, nq, max_edits, hit_off, hits, hit_edits, capacity, n_hits, false, METRIC_EDIT);
+  });
+}
+
+int awry_count_device_edit(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                           uint64_t nq, uint32_t max_edits, uint64_t* d_counts, void* cuda_stream) {
+  return guarded([&] {
+    hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_counts, cuda_stream, false, METRIC_EDIT);
+  });
+}
+
+int awry_count_batch_edit_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                                  uint32_t max_edits, uint64_t* counts) {
+  return guarded([&] { hamming_count_impl(ix, qbytes, qoff, nq, max_edits, counts, true, METRIC_EDIT); });
+}
+
+int awry_locate_batch_edit_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                                   uint32_t max_edits, uint64_t* hit_off, awry_hit* hits, uint8_t* hit_edits,
+                                   uint64_t capacity, uint64_t* n_hits) {
+  return guarded([&] {
+    hamming_locate_impl(ix, qbytes, qoff, nq, max_edits, hit_off, hits, hit_edits, capacity, n_hits, true, METRIC_EDIT);
+  });
+}
+
+int awry_count_device_edit_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                   uint64_t nq, uint32_t max_edits, uint64_t* d_counts, void* cuda_stream) {
+  return guarded([&] {
+    hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_counts, cuda_stream, true, METRIC_EDIT);
   });
 }
 

@@ -222,6 +222,17 @@ cudaError_t launch_hamming_compact(const uint64_t* d_sorted, const uint32_t* d_m
                                    const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
                                    uint8_t* d_dist, cudaStream_t s);
 
+// ---- kernels_edit.cu: edit-distance search (<= k substitutions, insertions, deletions) on the Hamming candidates.
+// Every candidate names 2k + 1 starts, so locate keeps 2k + 1 key slots per candidate (slot k + δ: start s0 - δ).
+cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, bool locate, int sm_count,
+                               cudaStream_t s);
+// locate: the n < 2^31 key slots of a slice sorted per read (segment i = slots * (d_qcand[i] - c0) ..)
+cudaError_t sort_edit_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg, const uint64_t* d_qcand,
+                           uint64_t c0, uint32_t slots, void* d_temp, size_t& temp_bytes, cudaStream_t s);
+cudaError_t launch_edit_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
+                                const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
+                                uint8_t* d_dist, cudaStream_t s);
+
 cudaError_t launch_single_update(const IndexView& ix, uint64_t sp, uint64_t ep, uint32_t dsym,
                                  uint64_t* d_out2, cudaStream_t s);
 cudaError_t launch_single_backstep(const IndexView& ix, uint64_t row, uint64_t* d_out, cudaStream_t s);

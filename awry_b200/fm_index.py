@@ -130,7 +130,9 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_locate_batch_packed2", "awry_set_host_threads", "awry_host_threads", "awry_count_batch_hamming",
            "awry_locate_batch_hamming", "awry_count_device_hamming", "awry_count_batch_strands",
            "awry_locate_batch_strands", "awry_count_device_strands", "awry_locate_device_strands",
-           "awry_count_batch_hamming_strands", "awry_locate_batch_hamming_strands", "awry_count_device_hamming_strands"]
+           "awry_count_batch_hamming_strands", "awry_locate_batch_hamming_strands", "awry_count_device_hamming_strands",
+           "awry_count_batch_edit", "awry_locate_batch_edit", "awry_count_device_edit", "awry_count_batch_edit_strands",
+           "awry_locate_batch_edit_strands", "awry_count_device_edit_strands"]
 
 
 def native():
@@ -206,6 +208,11 @@ def native():
     L.awry_count_batch_hamming_strands.argtypes = [vp, vp, vp, u64, C.c_uint32, vp]
     L.awry_locate_batch_hamming_strands.argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, vp, u64, C.POINTER(u64)]
     L.awry_count_device_hamming_strands.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, vp]
+    for strands in ("", "_strands"):
+        getattr(L, "awry_count_batch_edit" + strands).argtypes = [vp, vp, vp, u64, C.c_uint32, vp]
+        getattr(L, "awry_locate_batch_edit" + strands).argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, vp, u64,
+                                                                   C.POINTER(u64)]
+        getattr(L, "awry_count_device_edit" + strands).argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, vp]
     _LIB = L
     return L
 
@@ -592,6 +599,69 @@ class FmIndex:
         d]); see device_check"""
         _check(native().awry_count_device_hamming_strands(self._h, replica, d_qbytes, d_qoff, nq, int(max_mismatches),
                                                           d_counts, stream))
+
+    # ---- edit-distance search: starts within max_edits <= 3 substitutions, insertions, deletions -------------
+    def _count_edit(self, fn, qbytes, qoff, max_edits, per):
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        counts = np.zeros((nq,) + per + (int(max_edits) + 1,), dtype=np.uint64)
+        _check(fn(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq, int(max_edits), counts.ctypes.data))
+        return counts
+
+    def _locate_edit(self, fn, qbytes, qoff, max_edits, per, capacity):
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        hit_off = np.zeros(per * nq + 1, dtype=np.uint64)
+        cap = max(1, per * nq if capacity is None else int(capacity))
+        n = C.c_uint64()
+        for _ in range(2):
+            hits = np.zeros((cap, 2), dtype=np.uint64)
+            ed = np.zeros(cap, dtype=np.uint8)
+            rc = fn(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq, int(max_edits), hit_off.ctypes.data,
+                    hits.ctypes.data, ed.ctypes.data, cap, C.byref(n))
+            if rc != -8:
+                break
+            cap = max(1, n.value)
+        if rc != 0:
+            err = AwryError(rc, native().awry_last_error().decode(errors="replace"))
+            err.needed = n.value
+            raise err
+        return hit_off, hits[: n.value], ed[: n.value]
+
+    def count_edit_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int) -> np.ndarray:
+        """-> uint64[nq, max_edits + 1]: [q, d] = text starts s whose edit distance d(s) to q is exactly d"""
+        return self._count_edit(native().awry_count_batch_edit, qbytes, qoff, max_edits, ())
+
+    def locate_edit_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int, capacity: int = None):
+        """-> (hit_off uint64[nq+1], hits uint64[n_hits, 2] = (seq_idx, local_pos) of the start, edits uint8[n_hits]);
+        per query ascending by text position.  Neighbouring starts of one locus are all reported.  A first guess of
+        `capacity` hits (default: one per query) that proves too small is retried once with the reported total."""
+        return self._locate_edit(native().awry_locate_batch_edit, qbytes, qoff, max_edits, 1, capacity)
+
+    def count_edit_device(self, d_qbytes: int, d_qoff: int, nq: int, max_edits: int, d_counts: int, stream: int = 0,
+                          replica: int = 0):
+        """count_edit_packed on device pointers (d_counts: nq * (max_edits + 1) u64); see device_check"""
+        _check(native().awry_count_device_edit(self._h, replica, d_qbytes, d_qoff, nq, int(max_edits), d_counts, stream))
+
+    def count_edit_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int) -> np.ndarray:
+        """-> uint64[nq, 2, max_edits + 1]: [q, s, d] = starts at edit distance exactly d from q (s = 0) or from its
+        reverse complement (s = 1)"""
+        return self._count_edit(native().awry_count_batch_edit_strands, qbytes, qoff, max_edits, (2,))
+
+    def locate_edit_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int, capacity: int = None):
+        """-> (hit_off uint64[2 nq + 1], hits uint64[n_hits, 2], edits uint8[n_hits]): query q's forward hits are
+        hits[hit_off[2q]:hit_off[2q+1]], its reverse-strand hits hits[hit_off[2q+1]:hit_off[2q+2]], each ascending by
+        text position (default capacity: two per query, retried once as locate_edit_packed)"""
+        return self._locate_edit(native().awry_locate_batch_edit_strands, qbytes, qoff, max_edits, 2, capacity)
+
+    def count_edit_strands_device(self, d_qbytes: int, d_qoff: int, nq: int, max_edits: int, d_counts: int,
+                                  stream: int = 0, replica: int = 0):
+        """count_edit_strands_packed on device pointers (d_counts: 2 nq (max_edits + 1) u64, [(2q + s)(k+1) + d]);
+        see device_check"""
+        _check(native().awry_count_device_edit_strands(self._h, replica, d_qbytes, d_qoff, nq, int(max_edits), d_counts,
+                                                       stream))
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

@@ -226,7 +226,7 @@ int awry_locate_batch_packed2(const awry_index *index, const uint8_t *crumbs, co
 /* ------------------------------------------------------------------ Hamming search (<= k substitutions, no indels)
  * The reference answers one question, where a query occurs EXACTLY (get_search_range_for_string, fm_index.rs:402-438,
  * one update_range_with_symbol step per symbol, :559-582).  These calls extend it to windows of the text within
- * Hamming distance k (Bowtie's `-v k`), nucleotide only.
+ * Hamming distance k (Bowtie's `-v k`), nucleotide only.  Insertions and deletions: the edit-distance block below.
  *   text      the text the index holds: records joined by 'N', n = bwt_len - 1 symbols, no '$' (fm_index.rs:148-153).
  *             A window is text[s .. s+L) for 0 <= s <= n - L; windows may cross record delimiters, where the 'N' is
  *             an ordinary symbol, as for exact search.
@@ -317,6 +317,53 @@ int awry_locate_batch_hamming_strands(const awry_index *index, const uint8_t *qb
 int awry_count_device_hamming_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
                                       const uint64_t *d_qoff, uint64_t nq, uint32_t max_mismatches,
                                       uint64_t *d_counts /* 2*nq * (max_mismatches + 1) */, void *cuda_stream);
+
+/* ------------------------------------------------------------------ edit-distance search (<= k substitutions,
+ * insertions and deletions).  The Hamming block above with indels: a read with a one-base insertion or deletion
+ * (homopolymer runs, a guide with a bulge) is found.  Nucleotide only.
+ *   text      as in the Hamming block: n = bwt_len - 1 symbols, records joined by 'N'; an alignment may cross record
+ *             delimiters.  Query bytes are mapped as for exact search, so a query N equals a text N.
+ *   distance  Levenshtein distance (substitution, insertion, deletion: 1 each).  For a start position s (0 <= s < n),
+ *             d(s) = min over l >= 0 with s + l <= n of ed(query, text[s .. s+l)).  An occurrence is a start s with
+ *             d(s) <= k, reported once, with d(s).
+ *   neighbouring starts  an occurrence is a START, not a locus: an exact occurrence at s also makes s - 1 .. s - k
+ *             and s + 1 .. s + k occurrences at distances 1 .. k (insert text symbols in front of the query, or delete
+ *             its leading symbols), and all of them are reported.  Nothing merges them into one locus.
+ *   count     counts[q * (k+1) + d] = the number of starts with d(s) = d (nq * (k+1) entries).  For k = 0 this equals
+ *             awry_count_batch; for every k the d = 0 column equals that of the Hamming calls.
+ *   locate    every start with d(s) <= k, once each, per query in ascending text position, as (seq_idx, local_pos) of
+ *             s.  hit_edits (NULL or `capacity` entries) receives d(s).  capacity / AWRY_ERR_CAPACITY and hit_off (nq+1)
+ *             as in awry_locate_batch_hamming.
+ *   errors    k > AWRY_EDIT_MAX -> AWRY_ERR_INVALID_ARG; an empty query, one with '$' / '#' or one of length L <= k ->
+ *             AWRY_ERR_INVALID_QUERY naming the caller's query; a protein index, or one without the unsampled suffix
+ *             array and the text on the device -> AWRY_ERR_UNSUPPORTED.  The device calls latch refused queries for
+ *             awry_device_check, and their counts are 0.
+ * Scheme: the pieces, their exact search and the candidates are those of the Hamming calls.  An exact occurrence of
+ * piece j at p names the starts [s0 - k, s0 + k], s0 = p - a_j, and each start's d(s) comes from one banded DP on the
+ * device (4k + 1 diagonals).  A start is reported by the smallest (piece, position) occurrence within k of it, so
+ * nothing is deduplicated globally.
+ * The _strands calls search both strands, as the Hamming-on-both-strands block: v = 2q is q, v = 2q + 1 is rc(q),
+ * counts[(2q + s) * (k+1) + d], hit_off over the 2 nq virtual queries; every v = 2q + 1 result is bit for bit that
+ * of the single-strand call on rc(q).  There is no device-resident locate.  The device calls behave as
+ * awry_count_device_hamming: one synchronisation, after the pieces are searched. */
+enum { AWRY_EDIT_MAX = 3 };
+int awry_count_batch_edit(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                          uint32_t max_edits, uint64_t *counts /* nq * (max_edits + 1) */);
+int awry_locate_batch_edit(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                           uint32_t max_edits, uint64_t *hit_off /* nq + 1 */, awry_hit *hits,
+                           uint8_t *hit_edits /* NULL or capacity entries */, uint64_t capacity, uint64_t *n_hits);
+int awry_count_device_edit(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                           uint64_t nq, uint32_t max_edits, uint64_t *d_counts /* nq * (max_edits + 1) */,
+                           void *cuda_stream);
+int awry_count_batch_edit_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                                  uint32_t max_edits, uint64_t *counts /* 2*nq * (max_edits + 1) */);
+int awry_locate_batch_edit_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                                   uint32_t max_edits, uint64_t *hit_off /* 2*nq + 1 */, awry_hit *hits,
+                                   uint8_t *hit_edits /* NULL or capacity entries */, uint64_t capacity,
+                                   uint64_t *n_hits);
+int awry_count_device_edit_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
+                                   const uint64_t *d_qoff, uint64_t nq, uint32_t max_edits,
+                                   uint64_t *d_counts /* 2*nq * (max_edits + 1) */, void *cuda_stream);
 
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to

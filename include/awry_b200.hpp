@@ -263,10 +263,79 @@ class FmIndex {
         out[v / 2][v % 2].push_back({{hits[i].seq_idx, hits[i].local_pos}, uint32_t(dist[i])});
     return out;
   }
+  // Edit-distance search (no counterpart in the reference): text starts within max_edits <= AWRY_EDIT_MAX
+  // substitutions, insertions and deletions.  counts[q][d] = starts of query q at distance exactly d
+  std::vector<std::vector<uint64_t>> parallel_count_edit(const std::vector<std::string_view>& queries,
+                                                         uint32_t max_edits) const {
+    const size_t P = size_t(max_edits) + 1;
+    const std::vector<uint64_t> flat = count_edit_flat(queries, max_edits, false);
+    std::vector<std::vector<uint64_t>> out(queries.size());
+    for (size_t q = 0; q < queries.size(); q++) out[q].assign(flat.begin() + q * P, flat.begin() + (q + 1) * P);
+    return out;
+  }
+  // per query: (start, distance), ascending by position; the neighbouring starts of one locus are all there
+  std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> parallel_locate_edit(
+      const std::vector<std::string_view>& queries, uint32_t max_edits) const {
+    return locate_edit_flat(queries, max_edits, false);
+  }
+  // both strands: counts[q][s][d] = starts at distance exactly d from query q (s = 0) or its reverse complement (s = 1)
+  std::vector<std::array<std::vector<uint64_t>, 2>> parallel_count_edit_strands(
+      const std::vector<std::string_view>& queries, uint32_t max_edits) const {
+    const size_t P = size_t(max_edits) + 1;
+    const std::vector<uint64_t> flat = count_edit_flat(queries, max_edits, true);
+    std::vector<std::array<std::vector<uint64_t>, 2>> out(queries.size());
+    for (size_t v = 0; v < 2 * queries.size(); v++) out[v / 2][v % 2].assign(flat.begin() + v * P, flat.begin() + (v + 1) * P);
+    return out;
+  }
+  // per query: {forward hits, reverse-strand hits}, each (start, distance) ascending by position
+  std::vector<std::array<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>, 2>> parallel_locate_edit_strands(
+      const std::vector<std::string_view>& queries, uint32_t max_edits) const {
+    const auto flat = locate_edit_flat(queries, max_edits, true);
+    std::vector<std::array<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>, 2>> out(queries.size());
+    for (size_t v = 0; v < flat.size(); v++) out[v / 2][v % 2] = flat[v];
+    return out;
+  }
   awry_index* handle() const { return h_; }
 
  private:
   explicit FmIndex(awry_index* h) : h_(h) { check(awry_index_info(h_, &info_)); }
+  // the edit calls' flat results: counts (nq or 2 nq) x (k+1), and the hits of each (virtual) query
+  std::vector<uint64_t> count_edit_flat(const std::vector<std::string_view>& queries, uint32_t max_edits,
+                                        bool strands) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::vector<uint64_t> flat((strands ? 2 : 1) * queries.size() * (size_t(max_edits) + 1));
+    check((strands ? awry_count_batch_edit_strands : awry_count_batch_edit)(h_, bytes.data(), off.data(), queries.size(),
+                                                                            max_edits, flat.data()));
+    return flat;
+  }
+  std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> locate_edit_flat(
+      const std::vector<std::string_view>& queries, uint32_t max_edits, bool strands) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    const size_t nv = (strands ? 2 : 1) * queries.size();
+    auto call = strands ? awry_locate_batch_edit_strands : awry_locate_batch_edit;
+    std::vector<uint64_t> hit_off(nv + 1);
+    std::vector<awry_hit> hits(nv + 1);
+    std::vector<uint8_t> dist(hits.size());
+    uint64_t n = 0;
+    int rc = call(h_, bytes.data(), off.data(), queries.size(), max_edits, hit_off.data(), hits.data(), dist.data(),
+                  hits.size(), &n);
+    if (rc == AWRY_ERR_CAPACITY) {  // the total is known now: once more with room for every hit
+      hits.resize(n);
+      dist.resize(n);
+      rc = call(h_, bytes.data(), off.data(), queries.size(), max_edits, hit_off.data(), hits.data(), dist.data(),
+                hits.size(), &n);
+    }
+    check(rc);
+    std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> out(nv);
+    for (size_t v = 0; v < nv; v++)
+      for (uint64_t i = hit_off[v]; i < hit_off[v + 1]; i++)
+        out[v].push_back({{hits[i].seq_idx, hits[i].local_pos}, uint32_t(dist[i])});
+    return out;
+  }
   static void check(int rc) {
     if (rc != AWRY_OK) throw Error(rc, awry_last_error());
   }

@@ -160,6 +160,21 @@ extern "C" {
     pub fn awry_count_device_hamming_strands(index: *const awry_index, replica: c_int, d_qbytes: *const u8,
                                              d_qoff: *const u64, nq: u64, max_mismatches: u32, d_counts: *mut u64,
                                              cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_count_batch_edit(index: *const awry_index, qbytes: *const u8, qoff: *const u64, nq: u64, max_edits: u32,
+                                 counts: *mut u64) -> c_int;
+    pub fn awry_locate_batch_edit(index: *const awry_index, qbytes: *const u8, qoff: *const u64, nq: u64, max_edits: u32,
+                                  hit_off: *mut u64, hits: *mut awry_hit, hit_edits: *mut u8, capacity: u64,
+                                  n_hits: *mut u64) -> c_int;
+    pub fn awry_count_device_edit(index: *const awry_index, replica: c_int, d_qbytes: *const u8, d_qoff: *const u64,
+                                  nq: u64, max_edits: u32, d_counts: *mut u64, cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_count_batch_edit_strands(index: *const awry_index, qbytes: *const u8, qoff: *const u64, nq: u64,
+                                         max_edits: u32, counts: *mut u64) -> c_int;
+    pub fn awry_locate_batch_edit_strands(index: *const awry_index, qbytes: *const u8, qoff: *const u64, nq: u64,
+                                          max_edits: u32, hit_off: *mut u64, hits: *mut awry_hit, hit_edits: *mut u8,
+                                          capacity: u64, n_hits: *mut u64) -> c_int;
+    pub fn awry_count_device_edit_strands(index: *const awry_index, replica: c_int, d_qbytes: *const u8,
+                                          d_qoff: *const u64, nq: u64, max_edits: u32, d_counts: *mut u64,
+                                          cuda_stream: *mut c_void) -> c_int;
     pub fn awry_set_host_threads(n: c_int) -> c_int;
     pub fn awry_host_threads() -> c_int;
     pub fn awry_profile_enable(on: c_int) -> c_int;
