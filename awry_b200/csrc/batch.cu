@@ -1219,10 +1219,20 @@ struct HammingSink {
   std::vector<uint8_t> dist;
 };
 
+// the outputs of the device-resident locate (awry_locate_device_{hamming,edit}[_strands])
+struct DeviceHits {
+  uint64_t* hit_off;  // device, nv + 1: the CSR over the (virtual) queries
+  awry_hit** hits;    // a device allocation of *n_hits hits (not set when there are none)
+  uint8_t** dist;     // likewise, each hit's distance; nullptr: not wanted
+  uint64_t* n_hits;
+};
+
 // One batch of reads on one replica, all on stream `st`: pieces -> exact search of the pieces -> candidates ->
 // verification against the text, in slices of at most hamming_slice() candidates.  Offsets are absolute and lie
 // in [b_lo, b_hi] (d_qbytes is biased accordingly).  Count: d_counts (nq * (k + 1)) is zeroed and filled.  Locate:
 // the hits are appended to `sink` (slices cut at read boundaries, the hits of a read sorted by text position).
+// Device-resident locate (`dev`): a count pass and a place pass over the same slices, then one segmented sort; the
+// hits stay on the device, and the call returns without waiting for the last kernels.
 // `check_base` >= 0: a refused read fails the call (reported as read check_base + q) before anything is verified;
 // < 0 (the device-resident call): it stays latched in *d_flag for awry_device_check.
 // `strands`: the nq reads are searched as the 2 nq virtual queries of both strands (kernels.hpp), which take the
@@ -1234,7 +1244,7 @@ enum Metric { METRIC_HAMMING = 0, METRIC_EDIT = 1 };
 const char* metric_name(Metric metric) { return metric == METRIC_EDIT ? "edit-distance" : "Hamming"; }
 void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
                  uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
-                 HammingSink* sink, bool strands = false, Metric metric = METRIC_HAMMING) {
+                 HammingSink* sink, bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr) {
   const bool edit = metric == METRIC_EDIT;
   const char* const what = metric_name(metric);
   const uint32_t shift = strands ? 1 : 0;  // virtual query -> read
@@ -1320,8 +1330,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   a.hoff = d_hoff;
   a.npieces = np;
   const uint64_t S = std::max<uint64_t>(1, hamming_slice() / slots);  // candidates per slice
-  if (!sink) {  // 3. count: slices cut anywhere
-    CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
+  auto verify_all = [&](VerifyMode mode) {  // every candidate, in slices cut anywhere
     for (uint64_t c0 = 0; c0 < total; c0 += S) {
       StreamScratch ss(st);
       a.c0 = c0;
@@ -1330,10 +1339,84 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       CU(launch_hamming_map(d_hoff, np, c0, a.n, d_map, nullptr, temp, st));
       CU(launch_hamming_map(d_hoff, np, c0, a.n, d_map, ss.get<uint8_t>(temp), temp, st));
       a.map = d_map;
-      a.counts = d_counts;
       ProfScope p(1, r.device, st);
-      CU(edit ? launch_edit_verify(r.view, a, k, false, r.sm_count, st) : launch_hamming_verify(r.view, a, k, false, r.sm_count, st));
+      CU(edit ? launch_edit_verify(r.view, a, k, mode, r.sm_count, st) : launch_hamming_verify(r.view, a, k, mode, r.sm_count, st));
     }
+  };
+  if (dev) {  // 3. device-resident locate (DESIGN.md §1e)
+    // count pass: the CSR over the queries, and the hit total that sizes the outputs (the second synchronisation)
+    a.counts = sc.get<uint64_t>(nv * P);
+    CU(cudaMemsetAsync(a.counts, 0, nv * P * 8, st));
+    verify_all(VERIFY_COUNT);
+    uint64_t* d_sums = sc.get<uint64_t>(nv + 1);
+    CU(launch_hamming_row_sums(a.counts, k, nv, d_sums, st));
+    CU(scan_u64(d_sums, dev->hit_off, nv + 1, nullptr, temp, st));
+    CU(scan_u64(d_sums, dev->hit_off, nv + 1, sc.get<uint8_t>(temp), temp, st));
+    uint64_t n = 0;
+    CU(cudaMemcpyAsync(&n, dev->hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (n == 0) return;
+    // CUB's segmented sort reads its offsets as int: more than 2^31 - 1 keys are sorted in parts cut at query
+    // boundaries, which needs the offsets on the host (the only case that reads them back)
+    std::vector<std::pair<uint64_t, uint64_t>> parts{{0, nv}};  // query ranges
+    std::vector<uint64_t> off;
+    if (n >= (1ull << 31)) {
+      off.resize(nv + 1);
+      CU(cudaMemcpyAsync(off.data(), dev->hit_off, (nv + 1) * 8, cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
+      parts.clear();
+      for (uint64_t q0 = 0; q0 < nv;) {
+        if (off[q0 + 1] - off[q0] >= (1ull << 31))
+          fail(AWRY_ERR_NOMEM, "query %llu has %llu hits, more than one sort can order (2^31)",
+               (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + (q0 >> shift)),
+               (unsigned long long)(off[q0 + 1] - off[q0]));
+        uint64_t q1 = q0 + 1;
+        while (q1 < nv && off[q1 + 1] - off[q0] < (1ull << 31)) q1++;
+        parts.push_back({q0, q1});
+        q0 = q1;
+      }
+    }
+    // the outputs (released in stream order unless the call succeeds), then the scratch the hit total sizes
+    StreamScratch out(st);
+    awry_hit* d_hits = nullptr;
+    uint8_t* d_dist = nullptr;
+    uint64_t *d_keys = nullptr, *d_sorted = nullptr;
+    try {
+      d_hits = out.get<awry_hit>(n);  // (16 spare bytes behind the last hit, as every hit buffer)
+      if (dev->dist) d_dist = out.get<uint8_t>(n);
+      d_keys = sc.get<uint64_t>(n);
+      d_sorted = sc.get<uint64_t>(n);
+    } catch (const ApiError& x) {
+      if (x.code != AWRY_ERR_NOMEM) throw;
+      fail(AWRY_ERR_NOMEM, "out of device memory for the %llu hits of this %s locate", (unsigned long long)n, what);
+    }
+    // place pass: the same slices and the same acceptance as the count pass; each key takes a slot of its query's range
+    a.keys = d_keys;
+    a.acc = sc.get<uint64_t>(nv);
+    a.q0 = 0;
+    a.hit_off = dev->hit_off;
+    CU(cudaMemsetAsync(a.acc, 0, nv * 8, st));
+    verify_all(VERIFY_PLACE);
+    // order: a query's positions are distinct, so the sorted keys do not depend on the order the atomics gave
+    for (const auto& [q0, q1] : parts) {
+      const uint64_t b = off.empty() ? 0 : off[q0], m = off.empty() ? n : off[q1] - off[q0];
+      StreamScratch ss(st);
+      size_t t2 = 0;
+      CU(sort_hamming_keys(d_keys + b, d_sorted + b, m, q1 - q0, dev->hit_off + q0, b, nullptr, t2, st));
+      CU(sort_hamming_keys(d_keys + b, d_sorted + b, m, q1 - q0, dev->hit_off + q0, b, ss.get<uint8_t>(t2), t2, st));
+    }
+    CU(launch_hamming_decode(d_sorted, n, d_dist, st));
+    CU(launch_map_locations(r.view, d_sorted, n, reinterpret_cast<uint64_t*>(d_hits), st));
+    out.ptrs.clear();  // the caller's now
+    *dev->hits = d_hits;
+    if (dev->dist) *dev->dist = d_dist;
+    *dev->n_hits = n;
+    return;
+  }
+  if (!sink) {  // 3. count
+    CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
+    a.counts = d_counts;
+    verify_all(VERIFY_COUNT);
     return;
   }
   // 3. locate: slices cut at read boundaries (a read with more candidates than a slice gets one of its own size)
@@ -1364,7 +1447,8 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     CU(cudaMemsetAsync(a.acc, 0, (nr + 1) * 8, st));
     {
       ProfScope p(1, r.device, st);
-      CU(edit ? launch_edit_verify(r.view, a, k, true, r.sm_count, st) : launch_hamming_verify(r.view, a, k, true, r.sm_count, st));
+      CU(edit ? launch_edit_verify(r.view, a, k, VERIFY_LOCATE, r.sm_count, st)
+              : launch_hamming_verify(r.view, a, k, VERIFY_LOCATE, r.sm_count, st));
     }
     uint64_t* d_sorted = ss.get<uint64_t>(n * slots);
     size_t t2 = 0;
@@ -1623,6 +1707,31 @@ void hamming_count_device_impl(const awry_index* ix, int replica, const uint8_t*
   hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands, metric);
 }
 
+// awry_locate_device_{hamming,edit}[_strands]: the hits of the nq (or 2 nq virtual) queries, in stream-ordered device
+// buffers; argument checks and errors as hamming_count_device_impl, outputs as locate_device_impl
+void hamming_locate_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                uint64_t nq, uint32_t k, uint64_t* d_hit_off, awry_hit** d_hits, uint8_t** d_dist,
+                                uint64_t* n_hits, void* cuda_stream, bool strands, Metric metric) {
+  need(ix);
+  check_max_k(k, metric);
+  if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+  if (!d_hit_off || !d_hits || !n_hits) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  *d_hits = nullptr;
+  if (d_dist) *d_dist = nullptr;
+  *n_hits = 0;
+  if (nq == 0) return;
+  if (!d_qbytes || !d_qoff) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (strands) strands_check_index(ix);
+  hamming_check_index(ix, metric_name(metric));
+  Replica& r = *ix->reps[size_t(replica)];
+  DeviceGuard dg(r.device);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  uint64_t e[2] = {0, 0};
+  device_batch_ends(d_qoff, nq, st, e, strands);
+  DeviceHits out{d_hit_off, d_hits, d_dist, n_hits};
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, nullptr, strands, metric, &out);
+}
+
 }  // namespace host
 }  // namespace awry
 
@@ -1787,6 +1896,42 @@ int awry_count_device_edit_strands(const awry_index* ix, int replica, const uint
                                    uint64_t nq, uint32_t max_edits, uint64_t* d_counts, void* cuda_stream) {
   return guarded([&] {
     hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_counts, cuda_stream, true, METRIC_EDIT);
+  });
+}
+
+int awry_locate_device_hamming(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                               uint64_t nq, uint32_t max_mismatches, uint64_t* d_hit_off, awry_hit** d_hits,
+                               uint8_t** d_hit_mismatches, uint64_t* n_hits, void* cuda_stream) {
+  return guarded([&] {
+    hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_mismatches, d_hit_off, d_hits, d_hit_mismatches,
+                               n_hits, cuda_stream, false, METRIC_HAMMING);
+  });
+}
+
+int awry_locate_device_hamming_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                       uint64_t nq, uint32_t max_mismatches, uint64_t* d_hit_off, awry_hit** d_hits,
+                                       uint8_t** d_hit_mismatches, uint64_t* n_hits, void* cuda_stream) {
+  return guarded([&] {
+    hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_mismatches, d_hit_off, d_hits, d_hit_mismatches,
+                               n_hits, cuda_stream, true, METRIC_HAMMING);
+  });
+}
+
+int awry_locate_device_edit(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                            uint64_t nq, uint32_t max_edits, uint64_t* d_hit_off, awry_hit** d_hits,
+                            uint8_t** d_hit_edits, uint64_t* n_hits, void* cuda_stream) {
+  return guarded([&] {
+    hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_hit_off, d_hits, d_hit_edits, n_hits,
+                               cuda_stream, false, METRIC_EDIT);
+  });
+}
+
+int awry_locate_device_edit_strands(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                    uint64_t nq, uint32_t max_edits, uint64_t* d_hit_off, awry_hit** d_hits,
+                                    uint8_t** d_hit_edits, uint64_t* n_hits, void* cuda_stream) {
+  return guarded([&] {
+    hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_hit_off, d_hits, d_hit_edits, n_hits,
+                               cuda_stream, true, METRIC_EDIT);
   });
 }
 

@@ -195,6 +195,10 @@ cudaError_t launch_hamming_query_bounds(const uint64_t* d_hoff, uint32_t k, uint
 // piece of every candidate of the slice [c0, c0 + n) (cub convention: d_temp == nullptr sizes the scratch)
 cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_t c0, uint64_t n, uint32_t* d_map,
                                void* d_temp, size_t& temp_bytes, cudaStream_t s);
+// what the verification kernels do with an accepted candidate: COUNT adds it to counts, LOCATE writes a key per
+// candidate of the slice (slices cut at read boundaries, sorted per slice), PLACE writes the key into its query's
+// range of a CSR computed by a COUNT pass over the same candidates (device-resident locate, DESIGN.md §1e)
+enum VerifyMode { VERIFY_COUNT = 0, VERIFY_LOCATE = 1, VERIFY_PLACE = 2 };
 // one slice of candidates for the verification kernel
 struct HammingSlice {
   const uint64_t* qwords;       // packed reads, biased as for launch_search: read q at word 4 (q + (qoff[q] >> 6))
@@ -206,17 +210,26 @@ struct HammingSlice {
   uint64_t npieces;
   const uint32_t* map;          // piece of candidate c0 + i
   uint64_t c0, n;
-  uint64_t* counts;             // count: (k+1) per read, zeroed by the caller
-  uint64_t* keys;               // locate: (s << 2 | d) or ~0 per candidate of the slice
-  uint64_t* acc;                // locate: accepted candidates per read of the slice, zeroed by the caller
-  uint64_t q0;                  // locate: first read of the slice
+  union {
+    uint64_t* counts;           // count: (k+1) per read, zeroed by the caller
+    const uint64_t* hit_off;    // place: read q's keys go to keys[hit_off[q] .. hit_off[q + 1])
+  };
+  uint64_t* keys;               // locate: (s << 2 | d) or ~0 per candidate of the slice; place: the keys of the batch
+  uint64_t* acc;                // locate: accepted candidates per read of the slice, zeroed by the caller;
+                                // place: keys placed so far per read of the batch (the cursor), zeroed by the caller
+  uint64_t q0;                  // locate: first read of the slice (place: 0)
 };
-cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, bool locate, int sm_count,
+cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                   cudaStream_t s);
 // locate: the n < 2^31 keys of a slice sorted per read (segment i = d_qcand[i] - c0 .. d_qcand[i+1] - c0)
 cudaError_t sort_hamming_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg,
                               const uint64_t* d_qcand, uint64_t c0, void* d_temp, size_t& temp_bytes, cudaStream_t s);
 cudaError_t scan_u64(const uint64_t* d_in, uint64_t* d_out, uint64_t n, void* d_temp, size_t& temp_bytes, cudaStream_t s);
+// device-resident locate: d_sums[q] = the sum of read q's k + 1 counts, q < nq, and d_sums[nq] = 0 (its exclusive scan
+// is the CSR over the reads)
+cudaError_t launch_hamming_row_sums(const uint64_t* d_counts, uint32_t k, uint64_t nq, uint64_t* d_sums, cudaStream_t s);
+// sorted keys (s << 2 | d) -> the text positions s in place, and the distances d to d_dist unless it is null
+cudaError_t launch_hamming_decode(uint64_t* d_keys, uint64_t n, uint8_t* d_dist, cudaStream_t s);
 // accepted sorted keys -> text positions and distances at offset d_qh[q - q0] + rank in the read's segment
 cudaError_t launch_hamming_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
                                    const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
@@ -224,7 +237,7 @@ cudaError_t launch_hamming_compact(const uint64_t* d_sorted, const uint32_t* d_m
 
 // ---- kernels_edit.cu: edit-distance search (<= k substitutions, insertions, deletions) on the Hamming candidates.
 // Every candidate names 2k + 1 starts, so locate keeps 2k + 1 key slots per candidate (slot k + δ: start s0 - δ).
-cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, bool locate, int sm_count,
+cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                cudaStream_t s);
 // locate: the n < 2^31 key slots of a slice sorted per read (segment i = slots * (d_qcand[i] - c0) ..)
 cudaError_t sort_edit_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg, const uint64_t* d_qcand,

@@ -55,8 +55,9 @@ __device__ __forceinline__ bool piece_at(const IndexView& ix, const uint32_t* rq
 // Start s (d(s) <= k) is reported by its OWNER only: the smallest (j', p') over exact occurrences of piece j' at
 // p' with |p' - a_j' - s| <= k -- such an occurrence exists and is a candidate whose range contains s, so every
 // start comes out once.  Count: counts[q (k+1) + d] += 1.  Locate: keys[(2k+1) i + k + δ] = (s << 2) | d, or ~0,
-// and acc[q - q0] += the candidate's accepted starts.
-template <int K, bool LOCATE>
+// and acc[q - q0] += the candidate's accepted starts.  Place: the candidate takes popc(acc) consecutive slots
+// keys[hit_off[q] + acc[q] ..] (acc[q] += popc) and writes its accepted starts' keys there.
+template <int K, int MODE>
 __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingSlice a) {
   constexpr int P = K + 1, W = 4 * K + 1, B = 2 * K;  // pieces, band width, diagonal offset of δ = 0
   constexpr uint64_t ONES = 0x1111111111111111ull >> (4 * (16 - W));  // one bit per band nibble
@@ -156,12 +157,21 @@ __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingS
         acc &= ~smaller;
       }
     }
-    if (LOCATE) {
+    if (MODE == VERIFY_LOCATE) {
       uint64_t* const keys = a.keys + uint64_t(2 * K + 1) * i;
 #pragma unroll
       for (int t = 0; t <= 2 * K; t++)
         keys[t] = (acc >> t) & 1u ? (uint64_t(s0 - (t - K)) << 2) | dist[t] : ~0ull;
       if (acc) atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + (q - a.q0), (unsigned long long)__popc(acc));
+    } else if (MODE == VERIFY_PLACE) {
+      if (acc) {
+        uint64_t at = a.hit_off[q] + atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + q,
+                                               (unsigned long long)__popc(acc));
+        AWRY_CHK(at + __popc(acc) <= a.hit_off[q + 1]);
+#pragma unroll
+        for (int t = 0; t <= 2 * K; t++)
+          if ((acc >> t) & 1u) a.keys[at++] = (uint64_t(s0 - (t - K)) << 2) | dist[t];
+      }
     } else if (acc) {
 #pragma unroll
       for (int t = 0; t <= 2 * K; t++)
@@ -171,23 +181,26 @@ __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingS
 }
 
 template <int K>
-static void launch_edit_verify_k(const IndexView& ix, const HammingSlice& a, bool locate, unsigned grid, cudaStream_t s) {
-  if (locate)
-    edit_verify_kernel<K, true><<<grid, 256, 0, s>>>(ix, a);
+static void launch_edit_verify_k(const IndexView& ix, const HammingSlice& a, VerifyMode mode, unsigned grid,
+                                 cudaStream_t s) {
+  if (mode == VERIFY_LOCATE)
+    edit_verify_kernel<K, VERIFY_LOCATE><<<grid, 256, 0, s>>>(ix, a);
+  else if (mode == VERIFY_PLACE)
+    edit_verify_kernel<K, VERIFY_PLACE><<<grid, 256, 0, s>>>(ix, a);
   else
-    edit_verify_kernel<K, false><<<grid, 256, 0, s>>>(ix, a);
+    edit_verify_kernel<K, VERIFY_COUNT><<<grid, 256, 0, s>>>(ix, a);
 }
 
-cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, bool locate, int sm_count,
+cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                cudaStream_t s) {
   if (a.n == 0) return cudaSuccess;
   if (k > 3 || ix.rtext == nullptr || ix.full_sa == nullptr) return cudaErrorInvalidValue;
   const unsigned grid = unsigned(std::max<uint64_t>(1, std::min<uint64_t>(uint64_t(sm_count) * 8, (a.n + 255) / 256)));
   switch (k) {
-    case 0: launch_edit_verify_k<0>(ix, a, locate, grid, s); break;
-    case 1: launch_edit_verify_k<1>(ix, a, locate, grid, s); break;
-    case 2: launch_edit_verify_k<2>(ix, a, locate, grid, s); break;
-    default: launch_edit_verify_k<3>(ix, a, locate, grid, s); break;
+    case 0: launch_edit_verify_k<0>(ix, a, mode, grid, s); break;
+    case 1: launch_edit_verify_k<1>(ix, a, mode, grid, s); break;
+    case 2: launch_edit_verify_k<2>(ix, a, mode, grid, s); break;
+    default: launch_edit_verify_k<3>(ix, a, mode, grid, s); break;
   }
   COUNT_LAUNCH();
   return cudaGetLastError();

@@ -137,8 +137,9 @@ cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_
 // The window of search-order symbol j is rtext[rb0 + j] with rb0 = bwt_len - s - L (rtext[i] = text[bwt_len - 1 - i],
 // layout.cuh): read and text are two forward streams.  A candidate is accepted iff its distance d <= k and its piece
 // j is the smallest one without a mismatch.  Count: counts[q (k+1) + d] += 1.  Locate: keys[i] = (s << 2) | d, or ~0
-// (rejected), and acc[q - q0] += 1.
-template <int K, bool LOCATE>
+// (rejected), and acc[q - q0] += 1.  Place: (s << 2) | d goes to keys[hit_off[q] + acc[q]++] (one slot of the range
+// the count pass gave q; the order within it is settled by the sort that follows).
+template <int K, int MODE>
 __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, HammingSlice a) {
   constexpr uint32_t FULL = 0xffffffffu;
   constexpr int P = K + 1;
@@ -211,9 +212,15 @@ __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, Hammi
     const uint32_t before = ((1u << P) - 1u) & ~((1u << (P - j)) - 1u);
     const bool accept = live && tot <= uint32_t(K) && (hit_pieces & before) == before;
     if (sub == 0 && i < a.n) {
-      if (LOCATE) {
+      if (MODE == VERIFY_LOCATE) {
         a.keys[i] = accept ? (s << 2) | tot : ~0ull;
         if (accept) atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + (q - a.q0), 1ull);
+      } else if (MODE == VERIFY_PLACE) {
+        if (accept) {
+          const uint64_t at = a.hit_off[q] + atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + q, 1ull);
+          AWRY_CHK(at < a.hit_off[q + 1]);
+          a.keys[at] = (s << 2) | tot;
+        }
       } else if (accept) {
         atomicAdd(reinterpret_cast<unsigned long long*>(a.counts) + (uint64_t(q) * P + tot), 1ull);
       }
@@ -222,23 +229,25 @@ __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, Hammi
 }
 
 template <int K>
-static void launch_verify_k(const IndexView& ix, const HammingSlice& a, bool locate, unsigned grid, cudaStream_t s) {
-  if (locate)
-    hamming_verify_kernel<K, true><<<grid, 256, 0, s>>>(ix, a);
+static void launch_verify_k(const IndexView& ix, const HammingSlice& a, VerifyMode mode, unsigned grid, cudaStream_t s) {
+  if (mode == VERIFY_LOCATE)
+    hamming_verify_kernel<K, VERIFY_LOCATE><<<grid, 256, 0, s>>>(ix, a);
+  else if (mode == VERIFY_PLACE)
+    hamming_verify_kernel<K, VERIFY_PLACE><<<grid, 256, 0, s>>>(ix, a);
   else
-    hamming_verify_kernel<K, false><<<grid, 256, 0, s>>>(ix, a);
+    hamming_verify_kernel<K, VERIFY_COUNT><<<grid, 256, 0, s>>>(ix, a);
 }
 
-cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, bool locate, int sm_count,
+cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                   cudaStream_t s) {
   if (a.n == 0) return cudaSuccess;
   if (k > 3 || ix.rtext == nullptr || ix.full_sa == nullptr) return cudaErrorInvalidValue;
   const unsigned grid = unsigned(std::max<uint64_t>(1, std::min<uint64_t>(uint64_t(sm_count) * 8, (a.n + 63) / 64)));
   switch (k) {
-    case 0: launch_verify_k<0>(ix, a, locate, grid, s); break;
-    case 1: launch_verify_k<1>(ix, a, locate, grid, s); break;
-    case 2: launch_verify_k<2>(ix, a, locate, grid, s); break;
-    default: launch_verify_k<3>(ix, a, locate, grid, s); break;
+    case 0: launch_verify_k<0>(ix, a, mode, grid, s); break;
+    case 1: launch_verify_k<1>(ix, a, mode, grid, s); break;
+    case 2: launch_verify_k<2>(ix, a, mode, grid, s); break;
+    default: launch_verify_k<3>(ix, a, mode, grid, s); break;
   }
   COUNT_LAUNCH();
   return cudaGetLastError();
@@ -268,6 +277,41 @@ cudaError_t scan_u64(const uint64_t* d_in, uint64_t* d_out, uint64_t n, void* d_
   cudaError_t e = cub::DeviceScan::ExclusiveSum(d_temp, temp_bytes, d_in, d_out, (long long)n, s);
   if (d_temp != nullptr) COUNT_LAUNCH();
   return e;
+}
+
+__global__ void hamming_row_sums_kernel(const uint64_t* __restrict__ counts, uint32_t P, uint64_t nq,
+                                        uint64_t* __restrict__ sums) {
+  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
+  for (uint64_t q = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; q <= nq; q += stride) {
+    uint64_t t = 0;
+    if (q < nq)
+      for (uint32_t d = 0; d < P; d++) t += counts[q * P + d];
+    sums[q] = t;
+  }
+}
+
+cudaError_t launch_hamming_row_sums(const uint64_t* d_counts, uint32_t k, uint64_t nq, uint64_t* d_sums, cudaStream_t s) {
+  const unsigned grid = unsigned(std::min<uint64_t>((nq + 256) / 256, 148 * 16));
+  hamming_row_sums_kernel<<<grid, 256, 0, s>>>(d_counts, k + 1, nq, d_sums);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
+__global__ void hamming_decode_kernel(uint64_t* __restrict__ keys, uint64_t n, uint8_t* __restrict__ dist) {
+  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
+  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
+    const uint64_t key = keys[i];
+    keys[i] = key >> 2;
+    if (dist) dist[i] = uint8_t(key & 3);
+  }
+}
+
+cudaError_t launch_hamming_decode(uint64_t* d_keys, uint64_t n, uint8_t* d_dist, cudaStream_t s) {
+  if (n == 0) return cudaSuccess;
+  const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
+  hamming_decode_kernel<<<grid, 256, 0, s>>>(d_keys, n, d_dist);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
 }
 
 // sorted keys -> text positions and distances at the query's CSR slot: the accepted keys lead their segment

@@ -132,7 +132,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_locate_batch_strands", "awry_count_device_strands", "awry_locate_device_strands",
            "awry_count_batch_hamming_strands", "awry_locate_batch_hamming_strands", "awry_count_device_hamming_strands",
            "awry_count_batch_edit", "awry_locate_batch_edit", "awry_count_device_edit", "awry_count_batch_edit_strands",
-           "awry_locate_batch_edit_strands", "awry_count_device_edit_strands"]
+           "awry_locate_batch_edit_strands", "awry_count_device_edit_strands", "awry_locate_device_hamming",
+           "awry_locate_device_hamming_strands", "awry_locate_device_edit", "awry_locate_device_edit_strands"]
 
 
 def native():
@@ -213,6 +214,10 @@ def native():
         getattr(L, "awry_locate_batch_edit" + strands).argtypes = [vp, vp, vp, u64, C.c_uint32, vp, vp, vp, u64,
                                                                    C.POINTER(u64)]
         getattr(L, "awry_count_device_edit" + strands).argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp, vp]
+        for metric in ("hamming", "edit"):
+            getattr(L, "awry_locate_device_" + metric + strands).argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp,
+                                                                             C.POINTER(vp), C.POINTER(vp),
+                                                                             C.POINTER(u64), vp]
     _LIB = L
     return L
 
@@ -504,6 +509,20 @@ class FmIndex:
         _check(native().awry_count_device_hamming(self._h, replica, d_qbytes, d_qoff, nq, int(max_mismatches), d_counts,
                                                   stream))
 
+    def _locate_approx_device(self, fn, d_qbytes, d_qoff, nq, k, d_hit_off, distances, stream, replica):
+        hits, dist, n = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        _check(fn(self._h, replica, d_qbytes, d_qoff, nq, int(k), d_hit_off, C.byref(hits),
+                  C.byref(dist) if distances else None, C.byref(n), stream))
+        return hits.value, dist.value, n.value
+
+    def locate_hamming_device(self, d_qbytes: int, d_qoff: int, nq: int, max_mismatches: int, d_hit_off: int,
+                              distances: bool = True, stream: int = 0, replica: int = 0):
+        """locate_hamming_packed on device pointers (d_hit_off: nq + 1 u64) -> (device pointer to n_hits x {u64
+        seq_idx, u64 local_pos}, device pointer to n_hits u8 mismatches (None without `distances`), n_hits); both
+        pointers are None when there are no hits.  Free each with device_free; see device_check"""
+        return self._locate_approx_device(native().awry_locate_device_hamming, d_qbytes, d_qoff, nq, max_mismatches,
+                                          d_hit_off, distances, stream, replica)
+
     # ---- both strands: every query and its reverse complement (include/awry_b200.h) ----------
     def count_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray) -> np.ndarray:
         """-> uint64[nq, 2]: [q, 0] = count of q, [q, 1] = count of its reverse complement"""
@@ -600,6 +619,13 @@ class FmIndex:
         _check(native().awry_count_device_hamming_strands(self._h, replica, d_qbytes, d_qoff, nq, int(max_mismatches),
                                                           d_counts, stream))
 
+    def locate_hamming_strands_device(self, d_qbytes: int, d_qoff: int, nq: int, max_mismatches: int, d_hit_off: int,
+                                      distances: bool = True, stream: int = 0, replica: int = 0):
+        """locate_hamming_strands_packed on device pointers (d_hit_off: 2 nq + 1 u64) -> (hits pointer, mismatches
+        pointer or None, n_hits), as locate_hamming_device; free each with device_free"""
+        return self._locate_approx_device(native().awry_locate_device_hamming_strands, d_qbytes, d_qoff, nq,
+                                          max_mismatches, d_hit_off, distances, stream, replica)
+
     # ---- edit-distance search: starts within max_edits <= 3 substitutions, insertions, deletions -------------
     def _count_edit(self, fn, qbytes, qoff, max_edits, per):
         qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
@@ -645,6 +671,14 @@ class FmIndex:
         """count_edit_packed on device pointers (d_counts: nq * (max_edits + 1) u64); see device_check"""
         _check(native().awry_count_device_edit(self._h, replica, d_qbytes, d_qoff, nq, int(max_edits), d_counts, stream))
 
+    def locate_edit_device(self, d_qbytes: int, d_qoff: int, nq: int, max_edits: int, d_hit_off: int,
+                           distances: bool = True, stream: int = 0, replica: int = 0):
+        """locate_edit_packed on device pointers (d_hit_off: nq + 1 u64) -> (device pointer to n_hits x {u64 seq_idx,
+        u64 local_pos}, device pointer to n_hits u8 edits (None without `distances`), n_hits); both pointers are None
+        when there are no hits.  Free each with device_free; see device_check"""
+        return self._locate_approx_device(native().awry_locate_device_edit, d_qbytes, d_qoff, nq, max_edits, d_hit_off,
+                                          distances, stream, replica)
+
     def count_edit_strands_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int) -> np.ndarray:
         """-> uint64[nq, 2, max_edits + 1]: [q, s, d] = starts at edit distance exactly d from q (s = 0) or from its
         reverse complement (s = 1)"""
@@ -662,6 +696,13 @@ class FmIndex:
         see device_check"""
         _check(native().awry_count_device_edit_strands(self._h, replica, d_qbytes, d_qoff, nq, int(max_edits), d_counts,
                                                        stream))
+
+    def locate_edit_strands_device(self, d_qbytes: int, d_qoff: int, nq: int, max_edits: int, d_hit_off: int,
+                                   distances: bool = True, stream: int = 0, replica: int = 0):
+        """locate_edit_strands_packed on device pointers (d_hit_off: 2 nq + 1 u64) -> (hits pointer, edits pointer or
+        None, n_hits), as locate_edit_device; free each with device_free"""
+        return self._locate_approx_device(native().awry_locate_device_edit_strands, d_qbytes, d_qoff, nq, max_edits,
+                                          d_hit_off, distances, stream, replica)
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

@@ -262,6 +262,28 @@ int awry_locate_batch_hamming(const awry_index *index, const uint8_t *qbytes, co
  * L <= k query is latched and reported by awry_device_check; its counts are 0. */
 int awry_count_device_hamming(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
                               uint64_t nq, uint32_t max_mismatches, uint64_t *d_counts, void *cuda_stream);
+/* awry_locate_batch_hamming on device-resident queries (see awry_locate_device below).  No per-read data goes to the
+ * host.
+ *   results   bit for bit those of awry_locate_batch_hamming on the same reads: d_hit_off (nq + 1, device), the hits
+ *             of each query in ascending text position as (seq_idx, local_pos), and each hit's distance.
+ *   output    *d_hits and *d_hit_mismatches are device allocations from the library's stream-ordered pool, released
+ *             with awry_device_free.  d_hit_mismatches == NULL: no distances are produced.  No hits: *n_hits = 0 and
+ *             both pointers NULL.  nq = 0 behaves as awry_locate_device.
+ *   sync      besides the read-back of the batch's first and last offset, the call synchronises `cuda_stream` twice:
+ *             after the pieces are searched (the candidate total, as awry_count_device_hamming) and after a count pass
+ *             over the candidates (the hit total sizes the output).  It returns without waiting for the last kernels;
+ *             the results are valid in stream order.
+ *   refused   an empty / sentinel / L <= k query, or one whose offsets leave the batch, is latched for
+ *             awry_device_check as by awry_count_device_hamming, and gets the hit range that call's counts give it.
+ *   errors    those of awry_count_device_hamming (k, replica, null pointers, 2 nq (k+1) >= 2^31 pieces ->
+ *             AWRY_ERR_INVALID_ARG; the index -> AWRY_ERR_UNSUPPORTED); the hits do not fit the device, or one query
+ *             has 2^31 hits or more -> AWRY_ERR_NOMEM, naming the hit total.
+ * Scheme (DESIGN.md §1e): a count pass verifies every candidate and sizes each query's range, a place pass verifies them
+ * again and writes each accepted window into its query's range, and a segmented sort puts each range in text order. */
+int awry_locate_device_hamming(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                               uint64_t nq, uint32_t max_mismatches, uint64_t *d_hit_off /* nq + 1 */,
+                               awry_hit **d_hits, uint8_t **d_hit_mismatches /* NULL: not wanted */, uint64_t *n_hits,
+                               void *cuda_stream);
 
 /* ------------------------------------------------------------------ both strands (query and reverse complement)
  * A read comes from either strand of the DNA; the index holds one.  These calls search every query together with its
@@ -307,8 +329,10 @@ int awry_locate_device_strands(const awry_index *index, int replica, const uint8
  *   errors     those of both blocks: k > AWRY_HAMMING_MAX -> AWRY_ERR_INVALID_ARG; an empty query, one with '$' / '#'
  *              or one of length L <= k -> AWRY_ERR_INVALID_QUERY, naming the caller's query index q; a protein index
  *              or one without the unsampled suffix array and the text -> AWRY_ERR_UNSUPPORTED.
- * The device call behaves as awry_count_device_hamming (one synchronisation, refused queries latched for
- * awry_device_check with counts 0) and refuses (AWRY_ERR_INVALID_ARG) a batch with 2 nq (k+1) >= 2^31 pieces. */
+ * The device count behaves as awry_count_device_hamming (one synchronisation, refused queries latched for
+ * awry_device_check with counts 0) and refuses (AWRY_ERR_INVALID_ARG) a batch with 2 nq (k+1) >= 2^31 pieces.  The
+ * device locate behaves as awry_locate_device_hamming over the 2 nq virtual queries (d_hit_off: 2 nq + 1 entries);
+ * its results are bit for bit those of awry_locate_batch_hamming_strands. */
 int awry_count_batch_hamming_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
                                      uint32_t max_mismatches, uint64_t *counts /* 2*nq * (max_mismatches + 1) */);
 int awry_locate_batch_hamming_strands(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
@@ -318,6 +342,11 @@ int awry_locate_batch_hamming_strands(const awry_index *index, const uint8_t *qb
 int awry_count_device_hamming_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
                                       const uint64_t *d_qoff, uint64_t nq, uint32_t max_mismatches,
                                       uint64_t *d_counts /* 2*nq * (max_mismatches + 1) */, void *cuda_stream);
+int awry_locate_device_hamming_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
+                                       const uint64_t *d_qoff, uint64_t nq, uint32_t max_mismatches,
+                                       uint64_t *d_hit_off /* 2*nq + 1 */, awry_hit **d_hits,
+                                       uint8_t **d_hit_mismatches /* NULL: not wanted */, uint64_t *n_hits,
+                                       void *cuda_stream);
 
 /* ------------------------------------------------------------------ edit-distance search (<= k substitutions,
  * insertions and deletions).  The Hamming block above with indels: a read with a one-base insertion or deletion
@@ -345,8 +374,9 @@ int awry_count_device_hamming_strands(const awry_index *index, int replica, cons
  * nothing is deduplicated globally.
  * The _strands calls search both strands, as the Hamming-on-both-strands block: v = 2q is q, v = 2q + 1 is rc(q),
  * counts[(2q + s) * (k+1) + d], hit_off over the 2 nq virtual queries; every v = 2q + 1 result is bit for bit that
- * of the single-strand call on rc(q).  There is no device-resident locate.  The device calls behave as
- * awry_count_device_hamming: one synchronisation, after the pieces are searched. */
+ * of the single-strand call on rc(q).  The device counts behave as awry_count_device_hamming: one synchronisation,
+ * after the pieces are searched.  The device locates behave as awry_locate_device_hamming (d_hit_edits receives d(s));
+ * their results are bit for bit those of awry_locate_batch_edit and awry_locate_batch_edit_strands. */
 enum { AWRY_EDIT_MAX = 3 };
 int awry_count_batch_edit(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
                           uint32_t max_edits, uint64_t *counts /* nq * (max_edits + 1) */);
@@ -365,6 +395,13 @@ int awry_locate_batch_edit_strands(const awry_index *index, const uint8_t *qbyte
 int awry_count_device_edit_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
                                    const uint64_t *d_qoff, uint64_t nq, uint32_t max_edits,
                                    uint64_t *d_counts /* 2*nq * (max_edits + 1) */, void *cuda_stream);
+int awry_locate_device_edit(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                            uint64_t nq, uint32_t max_edits, uint64_t *d_hit_off /* nq + 1 */, awry_hit **d_hits,
+                            uint8_t **d_hit_edits /* NULL: not wanted */, uint64_t *n_hits, void *cuda_stream);
+int awry_locate_device_edit_strands(const awry_index *index, int replica, const uint8_t *d_qbytes,
+                                    const uint64_t *d_qoff, uint64_t nq, uint32_t max_edits,
+                                    uint64_t *d_hit_off /* 2*nq + 1 */, awry_hit **d_hits,
+                                    uint8_t **d_hit_edits /* NULL: not wanted */, uint64_t *n_hits, void *cuda_stream);
 
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to

@@ -175,6 +175,21 @@ extern "C" {
     pub fn awry_count_device_edit_strands(index: *const awry_index, replica: c_int, d_qbytes: *const u8,
                                           d_qoff: *const u64, nq: u64, max_edits: u32, d_counts: *mut u64,
                                           cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_locate_device_hamming(index: *const awry_index, replica: c_int, d_qbytes: *const u8, d_qoff: *const u64,
+                                      nq: u64, max_mismatches: u32, d_hit_off: *mut u64, d_hits: *mut *mut awry_hit,
+                                      d_hit_mismatches: *mut *mut u8, n_hits: *mut u64, cuda_stream: *mut c_void)
+                                      -> c_int;
+    pub fn awry_locate_device_hamming_strands(index: *const awry_index, replica: c_int, d_qbytes: *const u8,
+                                              d_qoff: *const u64, nq: u64, max_mismatches: u32, d_hit_off: *mut u64,
+                                              d_hits: *mut *mut awry_hit, d_hit_mismatches: *mut *mut u8,
+                                              n_hits: *mut u64, cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_locate_device_edit(index: *const awry_index, replica: c_int, d_qbytes: *const u8, d_qoff: *const u64,
+                                   nq: u64, max_edits: u32, d_hit_off: *mut u64, d_hits: *mut *mut awry_hit,
+                                   d_hit_edits: *mut *mut u8, n_hits: *mut u64, cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_locate_device_edit_strands(index: *const awry_index, replica: c_int, d_qbytes: *const u8,
+                                           d_qoff: *const u64, nq: u64, max_edits: u32, d_hit_off: *mut u64,
+                                           d_hits: *mut *mut awry_hit, d_hit_edits: *mut *mut u8, n_hits: *mut u64,
+                                           cuda_stream: *mut c_void) -> c_int;
     pub fn awry_set_host_threads(n: c_int) -> c_int;
     pub fn awry_host_threads() -> c_int;
     pub fn awry_profile_enable(on: c_int) -> c_int;
