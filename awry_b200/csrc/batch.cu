@@ -1732,6 +1732,195 @@ void hamming_locate_device_impl(const awry_index* ix, int replica, const uint8_t
   hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, nullptr, strands, metric, &out);
 }
 
+// ------------------------------------------------------------------ alignment of located hits (awry_align_*)
+
+// One batch of reads on one replica, on stream `st`: the prepass of hamming_run (the reads packed; both strands: the
+// virtual offsets and words), each search query's length (0: refused), then the hits in slices of at most
+// hamming_slice(): the query of every hit from the hit offsets (hamming_map's scatter and max-scan), and one
+// alignment per hit.  d_hit_off (nv + 1) holds absolute hit indices; hit hit0 + i is d_hits[i] and gets d_out[i].
+// `check_base` >= 0: a refused read fails the call, reported as read check_base + q; < 0: it stays latched in *d_flag.
+void align_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+               Metric metric, bool strands, uint32_t k, unsigned long long* d_flag, long long check_base,
+               const uint64_t* d_hit_off, uint64_t hit0, const awry_hit* d_hits, uint64_t n_hits, awry_alignment* d_out,
+               cudaStream_t st) {
+  const uint32_t shift = strands ? 1 : 0;
+  const uint64_t nv = nq << shift, nbytes = b_hi - b_lo;
+  StreamScratch sc(st);
+  const uint64_t rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
+  const uint64_t v_lo = b_lo << shift, v_hi = b_hi << shift, vw_n = packed_words(0, nv, nbytes << shift), vw_lo = 4 * (v_lo >> 6);
+  uint64_t* const d_rw = sc.get<uint64_t>(rw_n) - w_lo;
+  const uint64_t *d_vw = d_rw, *d_voff = d_qoff;
+  CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
+  if (strands) {
+    uint64_t* const voff = sc.get<uint64_t>(nv + 1);
+    uint64_t* const vw = sc.get<uint64_t>(vw_n) - vw_lo;
+    CU(launch_strand_offsets(d_qoff, nq, b_lo, b_hi, voff, st));
+    CU(launch_strand_words(d_rw, d_qoff, nq, b_lo, b_hi, voff, vw, st));
+    d_voff = voff;
+    d_vw = vw;
+  }
+  uint32_t* const d_qlen = sc.get<uint32_t>(nv);
+  AlignSlice a{};
+  a.qwords = d_vw;
+  a.qw_lo = strands ? vw_lo : w_lo;
+  a.qw_n = strands ? vw_n : rw_n;
+  a.qoff = d_voff;
+  a.qlen = d_qlen;
+  a.nq = nv;
+  a.hit_end = d_hit_off + nv;
+  a.hit_total = hit0 + n_hits;
+  CU(launch_align_reads(d_vw, d_voff, nv, v_lo, v_hi, a.qw_lo, a.qw_n, k, shift, d_qlen, d_flag, st));
+  if (check_base >= 0) {
+    unsigned long long flag = ~0ull;
+    CU(cudaMemcpyAsync(&flag, d_flag, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (flag != ~0ull && (flag & 1) == BAD_QUERY)
+      fail(AWRY_ERR_INVALID_QUERY, "query %llu is empty, contains a sentinel ('$'/'#') or is not longer than k = %u",
+           (unsigned long long)(uint64_t(check_base) + (flag >> 1)), k);
+    if (flag != ~0ull) fail_bad_query(flag, uint64_t(check_base));
+  }
+  const uint64_t S = hamming_slice();
+  for (uint64_t c0 = 0; c0 < n_hits; c0 += S) {
+    StreamScratch ss(st);
+    a.n = std::min(S, n_hits - c0);
+    uint32_t* const d_map = ss.get<uint32_t>(a.n);
+    size_t temp = 0;
+    CU(launch_hamming_map(d_hit_off, nv, hit0 + c0, a.n, d_map, nullptr, temp, st));
+    CU(launch_hamming_map(d_hit_off, nv, hit0 + c0, a.n, d_map, ss.get<uint8_t>(temp), temp, st));
+    a.map = d_map;
+    a.hits = reinterpret_cast<const uint64_t*>(d_hits + c0);
+    a.out = reinterpret_cast<uint32_t*>(d_out + c0);
+    ProfScope p(1, r.device, st);
+    CU(launch_align_hits(r.view, a, k, metric == METRIC_EDIT, r.sm_count, st));
+  }
+}
+
+// the checks both align calls make before touching the index
+void align_check_args(uint32_t metric, uint32_t strands, uint32_t k) {
+  if (metric > AWRY_METRIC_EDIT) fail(AWRY_ERR_INVALID_ARG, "metric must be AWRY_METRIC_HAMMING (0) or AWRY_METRIC_EDIT (1)");
+  if (strands > 1) fail(AWRY_ERR_INVALID_ARG, "strands must be 0 or 1");
+  check_max_k(k, Metric(metric));
+}
+
+void align_check_index(const awry_index* ix, uint64_t nv) {
+  need(ix);
+  hamming_check_index(ix, "alignment");
+  if (nv >= (1ull << 32) - 1) fail(AWRY_ERR_INVALID_ARG, "batch too large for one alignment call: split it");
+}
+
+// awry_align_batch: reads [lo, hi) of host buffers on replica ri, in chunks of reads; each chunk uploads its reads, its
+// part of hit_off and its hits, and copies its alignments back
+void align_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo, uint64_t hi,
+                      Metric metric, bool strands, uint32_t k, const uint64_t* hit_off, const awry_hit* hits,
+                      awry_alignment* out) {
+  if (lo >= hi) return;
+  Replica& r = *ix->reps[ri];
+  DeviceGuard dg(r.device);
+  const uint64_t max_bytes = std::min(chunk_max_bytes(), locate_chunk_bytes()), per = strands ? 2 : 1;
+  auto chunks = make_chunks(qoff, lo, hi, locate_chunk_q(), max_bytes);
+  validate_chunks(chunks, max_bytes);
+  Workspace* ws = r.acquire();
+  try {
+    for (const Chunk& c : chunks) {
+      const uint64_t n = c.q1 - c.q0, nbytes = c.b1 - c.b0, v0 = per * c.q0, nv = per * n;
+      const uint64_t h0 = hit_off[v0], nh = hit_off[v0 + nv] - h0;
+      StreamScratch sc(ws->st);
+      Workspace::grow_dev(ws->d_qbytes, ws->d_qbytes_cap, size_t(nbytes) + 16);
+      Workspace::grow_dev(ws->d_qoff, ws->d_qoff_cap, size_t(n) + 1);
+      uint64_t* const d_hoff = sc.get<uint64_t>(nv + 1);
+      awry_hit* const d_hits = sc.get<awry_hit>(nh);
+      awry_alignment* const d_out = sc.get<awry_alignment>(nh);
+      if (nbytes) CU(cudaMemcpyAsync(ws->d_qbytes, qbytes + c.b0, nbytes, cudaMemcpyHostToDevice, ws->st));
+      CU(cudaMemcpyAsync(ws->d_qoff, qoff + c.q0, (n + 1) * 8, cudaMemcpyHostToDevice, ws->st));
+      CU(cudaMemcpyAsync(d_hoff, hit_off + v0, (nv + 1) * 8, cudaMemcpyHostToDevice, ws->st));
+      if (nh) CU(cudaMemcpyAsync(d_hits, hits + h0, nh * sizeof(awry_hit), cudaMemcpyHostToDevice, ws->st));
+      g_prof.h2d += nbytes + (n + 1) * 8 + (nv + 1) * 8 + nh * sizeof(awry_hit);
+      CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
+      align_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, metric, strands, k, ws->d_flag, (long long)c.q0,
+                d_hoff, h0, d_hits, nh, d_out, ws->st);
+      if (nh) CU(cudaMemcpyAsync(out + h0, d_out, nh * sizeof(awry_alignment), cudaMemcpyDeviceToHost, ws->st));
+      g_prof.d2h += nh * sizeof(awry_alignment);
+      CU(cudaStreamSynchronize(ws->st));
+    }
+  } catch (...) {
+    cudaStreamSynchronize(ws->st);
+    r.release(ws);
+    throw;
+  }
+  r.release(ws);
+}
+
+void align_batch_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t metric,
+                      uint32_t strands, uint32_t k, const uint64_t* hit_off, const awry_hit* hits, awry_alignment* out) {
+  align_check_args(metric, strands, k);
+  if (!hit_off) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  const uint64_t nv = nq << strands;
+  if (hit_off[0] != 0) fail(AWRY_ERR_INVALID_ARG, "hit_off[0] must be 0");
+  for (uint64_t v = 0; v < nv; v++)
+    if (hit_off[v + 1] < hit_off[v]) fail(AWRY_ERR_INVALID_ARG, "hit offsets are not monotone at query %llu", (unsigned long long)(v >> strands));
+  if (nq && (!qbytes || !qoff)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (hit_off[nv] && (!hits || !out)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  align_check_index(ix, nv);
+  if (nq == 0) return;
+  if (qoff[nq] < qoff[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
+  for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
+    align_on_replica(ix, ri, qbytes, qoff, lo, hi, Metric(metric), strands != 0, k, hit_off, hits, out);
+  });
+}
+
+void align_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                       uint32_t metric, uint32_t strands, uint32_t k, const uint64_t* d_hit_off, const awry_hit* d_hits,
+                       uint64_t n_hits, awry_alignment* d_out, void* cuda_stream) {
+  align_check_args(metric, strands, k);
+  if (!d_hit_off || (nq && (!d_qbytes || !d_qoff)) || (n_hits && (!d_hits || !d_out)))
+    fail(AWRY_ERR_INVALID_ARG, "null argument");
+  align_check_index(ix, nq << strands);
+  if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+  if (nq == 0) return;
+  if (strands) strands_check_device_batch(nq);
+  Replica& r = *ix->reps[size_t(replica)];
+  DeviceGuard dg(r.device);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  uint64_t e[2] = {0, 0};
+  device_batch_ends(d_qoff, nq, st, e, strands != 0);
+  align_run(r, d_qbytes, d_qoff, nq, e[0], e[1], Metric(metric), strands != 0, k, r.d_async_flag, -1, d_hit_off, 0, d_hits,
+            n_hits, d_out, st);
+}
+
+// awry_alignment_cigar: run-length encoded op letters; '=' runs fill the query between the ops
+void alignment_cigar_impl(const awry_alignment* a, uint32_t query_len, char* buf, size_t cap, size_t* needed) {
+  if (!a || (!buf && cap)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (a->n_ops != a->distance || a->n_ops > AWRY_EDIT_MAX)
+    fail(AWRY_ERR_INVALID_ARG, "not an alignment (distance %u, %u ops)", unsigned(a->distance), unsigned(a->n_ops));
+  std::string s;
+  char last = 0;
+  uint64_t run = 0, at = 0;  // query symbols used
+  auto put = [&](char c, uint64_t n) {  // (adjacent ops of one kind merge: "2X")
+    if (n == 0) return;
+    if (c != last) {
+      if (run) s += std::to_string(run) + last;
+      last = c;
+      run = 0;
+    }
+    run += n;
+  };
+  for (unsigned t = 0; t < a->n_ops; t++) {
+    const awry_edit_op& o = a->ops[t];
+    const bool uses_q = o.op == 'X' || o.op == 'I';
+    if ((!uses_q && o.op != 'D') || o.qpos < at || o.qpos + (uses_q ? 1u : 0u) > query_len)
+      fail(AWRY_ERR_INVALID_ARG, "op %u ('%c' at query position %u) is out of order or outside the query", t,
+           o.op >= 32 && o.op < 127 ? char(o.op) : '?', o.qpos);
+    put('=', o.qpos - at);
+    put(char(o.op), 1);
+    at = o.qpos + (uses_q ? 1 : 0);
+  }
+  put('=', query_len - at);
+  if (run) s += std::to_string(run) + last;
+  if (needed) *needed = s.size() + 1;
+  if (s.size() + 1 > cap) fail(AWRY_ERR_CAPACITY, "the CIGAR needs %zu bytes, the buffer holds %zu", s.size() + 1, cap);
+  memcpy(buf, s.c_str(), s.size() + 1);
+}
+
 }  // namespace host
 }  // namespace awry
 
@@ -1933,6 +2122,23 @@ int awry_locate_device_edit_strands(const awry_index* ix, int replica, const uin
     hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_hit_off, d_hits, d_hit_edits, n_hits,
                                cuda_stream, true, METRIC_EDIT);
   });
+}
+
+int awry_align_batch(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t metric,
+                     uint32_t strands, uint32_t k, const uint64_t* hit_off, const awry_hit* hits, awry_alignment* out) {
+  return guarded([&] { align_batch_impl(ix, qbytes, qoff, nq, metric, strands, k, hit_off, hits, out); });
+}
+
+int awry_align_device(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                      uint32_t metric, uint32_t strands, uint32_t k, const uint64_t* d_hit_off, const awry_hit* d_hits,
+                      uint64_t n_hits, awry_alignment* d_out, void* cuda_stream) {
+  return guarded([&] {
+    align_device_impl(ix, replica, d_qbytes, d_qoff, nq, metric, strands, k, d_hit_off, d_hits, n_hits, d_out, cuda_stream);
+  });
+}
+
+int awry_alignment_cigar(const awry_alignment* a, uint32_t query_len, char* buf, size_t cap, size_t* needed) {
+  return guarded([&] { alignment_cigar_impl(a, query_len, buf, cap, needed); });
 }
 
 int awry_count_batch_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,

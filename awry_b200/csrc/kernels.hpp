@@ -246,6 +246,29 @@ cudaError_t launch_edit_compact(const uint64_t* d_sorted, const uint32_t* d_map,
                                 const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
                                 uint8_t* d_dist, cudaStream_t s);
 
+// ---- kernels_align.cu: the alignment of located Hamming and edit-distance hits (awry_align_*, DESIGN.md §1f)
+// d_qlen[v] = the length L of search query v (read or virtual query, packed in d_qwords as for launch_search), or 0 when
+// the prepass refused it, it is empty, holds '$' / '#' or has L <= k; the last is latched in *d_first_bad as BAD_QUERY
+// of read v >> shift (the prepass latches the others)
+cudaError_t launch_align_reads(const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
+                               uint64_t qw_lo, uint64_t qw_n, uint32_t k, uint32_t shift, uint32_t* d_qlen,
+                               unsigned long long* d_first_bad, cudaStream_t s);
+// one slice of hits for the alignment kernel
+struct AlignSlice {
+  const uint64_t* qwords;  // packed search queries, biased as for launch_search
+  uint64_t qw_lo, qw_n;    // the words that exist: [qw_lo, qw_lo + qw_n) (checked build)
+  const uint64_t* qoff;    // their offsets (nq + 1)
+  const uint32_t* qlen;    // launch_align_reads
+  uint64_t nq;
+  const uint32_t* map;     // query of every hit of the slice (launch_hamming_map over the hit offsets)
+  const uint64_t* hits;    // (seq_idx, local_pos) of every hit of the slice
+  uint32_t* out;           // one awry_alignment (11 u32) per hit of the slice
+  uint64_t n;
+  const uint64_t* hit_end; // checked build: *hit_end == hit_total (the hit offsets end where the hits do)
+  uint64_t hit_total;
+};
+cudaError_t launch_align_hits(const IndexView& ix, const AlignSlice& a, uint32_t k, bool edit, int sm_count, cudaStream_t s);
+
 cudaError_t launch_single_update(const IndexView& ix, uint64_t sp, uint64_t ep, uint32_t dsym,
                                  uint64_t* d_out2, cudaStream_t s);
 cudaError_t launch_single_backstep(const IndexView& ix, uint64_t row, uint64_t* d_out, cudaStream_t s);

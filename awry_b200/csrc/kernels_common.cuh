@@ -193,6 +193,39 @@ __device__ __forceinline__ void text_sector_mismatches(const u32x8& t, const uin
   }
 }
 
+// ---- word readers of the edit-distance verification (kernels_edit.cu) and the alignment (kernels_align.cu)
+// 8 symbols of the reversed text from nibble index x on (symbol t in nibble t); indices outside [0, bwt_len) read as
+// 0xF, a code no read symbol has (as '$' at index 0, it is a text symbol nothing matches)
+__device__ __forceinline__ uint32_t rtext8(const IndexView& ix, int64_t x) {
+  const int64_t w = x >> 3;  // floor
+  const uint32_t sh = 4u * uint32_t(x & 7);
+  const uint64_t nw = ix.n_rtext / 4;
+  const uint32_t* const rt = reinterpret_cast<const uint32_t*>(ix.rtext);
+  const uint32_t lo = (w >= 0 && uint64_t(w) < nw) ? __ldg(rt + w) : 0xffffffffu;
+  const uint32_t hi = (w + 1 >= 0 && uint64_t(w + 1) < nw) ? __ldg(rt + w + 1) : 0xffffffffu;
+  uint32_t v = sh ? __funnelshift_r(lo, hi, sh) : lo;
+  if (x < 0 || x + 8 > int64_t(ix.bwt_len)) {
+#pragma unroll
+    for (int t = 0; t < 8; t++)
+      if (x + t < 0 || x + t >= int64_t(ix.bwt_len)) v |= 0xfu << (4 * t);
+  }
+  return v;
+}
+
+// 8 symbols of a packed read (search order, 8 per u32) from symbol y on; the buffer is padded behind every read
+__device__ __forceinline__ uint32_t read8(const uint32_t* rq, uint32_t y) {
+  const uint32_t w = y >> 3, sh = 4u * (y & 7);
+  const uint32_t lo = __ldg(rq + w);
+  return sh ? __funnelshift_r(lo, __ldg(rq + w + 1), sh) : lo;
+}
+
+// the descending reader: the 8 search-order symbols y, y - 1, .. y - 7 of a packed read with symbol y - t in nibble
+// 7 - t (those below symbol 0 are garbage).  Search order runs backwards through the read, so these are 8 read
+// symbols in their ORIGINAL order from the top nibble down; rtext8(ix, x - 7) is the same for the text from x on.
+__device__ __forceinline__ uint32_t desc8(const uint32_t* rq, uint32_t y) {
+  return y >= 7 ? read8(rq, y - 7) : read8(rq, 0) << (4 * (7 - y));
+}
+
 // protein: 8 bits per symbol, so a 32-byte sector holds 32 symbols, 4 per word, and the ring 128
 __device__ __forceinline__ uint32_t text_sector_mismatch8(const u32x8& t, const uint64_t* ring, uint32_t sec, uint32_t rb0,
                                                           uint32_t done, uint32_t len) {

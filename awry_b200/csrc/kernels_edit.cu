@@ -12,31 +12,6 @@
 
 namespace awry {
 
-// 8 symbols of the reversed text from nibble index x on (symbol t in nibble t); indices outside [0, bwt_len) read as
-// 0xF, a code no read symbol has (as '$' at index 0, it is a text symbol nothing matches)
-__device__ __forceinline__ uint32_t rtext8(const IndexView& ix, int64_t x) {
-  const int64_t w = x >> 3;  // floor
-  const uint32_t sh = 4u * uint32_t(x & 7);
-  const uint64_t nw = ix.n_rtext / 4;
-  const uint32_t* const rt = reinterpret_cast<const uint32_t*>(ix.rtext);
-  const uint32_t lo = (w >= 0 && uint64_t(w) < nw) ? __ldg(rt + w) : 0xffffffffu;
-  const uint32_t hi = (w + 1 >= 0 && uint64_t(w + 1) < nw) ? __ldg(rt + w + 1) : 0xffffffffu;
-  uint32_t v = sh ? __funnelshift_r(lo, hi, sh) : lo;
-  if (x < 0 || x + 8 > int64_t(ix.bwt_len)) {
-#pragma unroll
-    for (int t = 0; t < 8; t++)
-      if (x + t < 0 || x + t >= int64_t(ix.bwt_len)) v |= 0xfu << (4 * t);
-  }
-  return v;
-}
-
-// 8 symbols of a packed read (search order, 8 per u32) from symbol y on; the buffer is padded behind every read
-__device__ __forceinline__ uint32_t read8(const uint32_t* rq, uint32_t y) {
-  const uint32_t w = y >> 3, sh = 4u * (y & 7);
-  const uint32_t lo = __ldg(rq + w);
-  return sh ? __funnelshift_r(lo, __ldg(rq + w + 1), sh) : lo;
-}
-
 // whether search-order symbols [y, y + m) of the read equal reversed-text symbols [x, x + m)
 __device__ __forceinline__ bool piece_at(const IndexView& ix, const uint32_t* rq, uint32_t y, int64_t x, uint32_t m) {
   for (uint32_t u = 0; u < m; u += 8) {

@@ -133,7 +133,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_count_batch_hamming_strands", "awry_locate_batch_hamming_strands", "awry_count_device_hamming_strands",
            "awry_count_batch_edit", "awry_locate_batch_edit", "awry_count_device_edit", "awry_count_batch_edit_strands",
            "awry_locate_batch_edit_strands", "awry_count_device_edit_strands", "awry_locate_device_hamming",
-           "awry_locate_device_hamming_strands", "awry_locate_device_edit", "awry_locate_device_edit_strands"]
+           "awry_locate_device_hamming_strands", "awry_locate_device_edit", "awry_locate_device_edit_strands",
+           "awry_align_batch", "awry_align_device", "awry_alignment_cigar"]
 
 
 def native():
@@ -218,6 +219,9 @@ def native():
             getattr(L, "awry_locate_device_" + metric + strands).argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp,
                                                                              C.POINTER(vp), C.POINTER(vp),
                                                                              C.POINTER(u64), vp]
+    L.awry_align_batch.argtypes = [vp, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, vp]
+    L.awry_align_device.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, u64, vp, vp]
+    L.awry_alignment_cigar.argtypes = [vp, C.c_uint32, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
     _LIB = L
     return L
 
@@ -239,6 +243,26 @@ def pack_queries(queries: Iterable) -> Tuple[np.ndarray, np.ndarray]:
 
 
 LOCATE_BWT_ORDER, LOCATE_SORTED = 0, 1
+METRIC_HAMMING, METRIC_EDIT = 0, 1
+_METRICS = {"hamming": METRIC_HAMMING, "edit": METRIC_EDIT, METRIC_HAMMING: METRIC_HAMMING, METRIC_EDIT: METRIC_EDIT}
+
+# awry_alignment / awry_edit_op (include/awry_b200.h): 44 bytes, ops[t] = (qpos, tpos, op, query_sym, text_sym, pad)
+EDIT_OP_DTYPE = np.dtype([("qpos", "<u4"), ("tpos", "<u4"), ("op", "u1"), ("query_sym", "u1"), ("text_sym", "u1"),
+                          ("pad", "u1")])
+ALIGNMENT_DTYPE = np.dtype([("text_len", "<u4"), ("distance", "u1"), ("n_ops", "u1"), ("pad", "u1", (2,)),
+                            ("ops", EDIT_OP_DTYPE, (3,))])
+assert ALIGNMENT_DTYPE.itemsize == 44
+
+
+def cigar(alignment, query_len: int) -> str:
+    """awry_alignment_cigar: the extended CIGAR (=, X, I, D) of one alignment (a record of ALIGNMENT_DTYPE) of a query of
+    length query_len; no device needed"""
+    rec = np.ascontiguousarray(np.asarray(alignment, dtype=ALIGNMENT_DTYPE).reshape(1))
+    need = C.c_size_t()
+    native().awry_alignment_cigar(rec.ctypes.data, int(query_len), None, 0, C.byref(need))
+    buf = C.create_string_buffer(max(1, need.value))
+    _check(native().awry_alignment_cigar(rec.ctypes.data, int(query_len), buf, len(buf), C.byref(need)))
+    return buf.value.decode()
 
 
 class FmIndex:
@@ -703,6 +727,29 @@ class FmIndex:
         None, n_hits), as locate_edit_device; free each with device_free"""
         return self._locate_approx_device(native().awry_locate_device_edit_strands, d_qbytes, d_qoff, nq, max_edits,
                                           d_hit_off, distances, stream, replica)
+
+    # ---- alignment of located Hamming / edit-distance hits (include/awry_b200.h) -------------
+    def align_hits_packed(self, qbytes: np.ndarray, qoff: np.ndarray, metric, max_dist: int, hit_off: np.ndarray,
+                          hits: np.ndarray, strands: bool = False) -> np.ndarray:
+        """-> ALIGNMENT_DTYPE[n_hits]: each hit of a locate_{hamming,edit}[_strands]_packed call (its hit_off and hits,
+        with that call's reads, metric "hamming" / "edit" and k) aligned: text_len, distance, the ops (a CIGAR: see
+        cigar()).  Reverse-strand hits are aligned as rc(q)."""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        hit_off = np.ascontiguousarray(hit_off, dtype=np.uint64)
+        hits = np.ascontiguousarray(hits, dtype=np.uint64).reshape(-1, 2)
+        out = np.zeros(max(1, len(hits)), dtype=ALIGNMENT_DTYPE)
+        _check(native().awry_align_batch(self._h, qbytes.ctypes.data, qoff.ctypes.data, len(qoff) - 1, _METRICS[metric],
+                                         int(bool(strands)), int(max_dist), hit_off.ctypes.data, hits.ctypes.data,
+                                         out.ctypes.data))
+        return out[:len(hits)]
+
+    def align_hits_device(self, d_qbytes: int, d_qoff: int, nq: int, metric, max_dist: int, d_hit_off: int, d_hits: int,
+                          n_hits: int, d_out: int, strands: bool = False, stream: int = 0, replica: int = 0):
+        """align_hits_packed on device pointers: the reads and the hits of a locate_*_device call, d_out = n_hits x 44
+        bytes (ALIGNMENT_DTYPE) on the device.  Returns without waiting; see device_check"""
+        _check(native().awry_align_device(self._h, replica, d_qbytes, d_qoff, nq, _METRICS[metric], int(bool(strands)),
+                                          int(max_dist), d_hit_off, d_hits, n_hits, d_out, stream))
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

@@ -403,6 +403,71 @@ int awry_locate_device_edit_strands(const awry_index *index, int replica, const 
                                     uint64_t *d_hit_off /* 2*nq + 1 */, awry_hit **d_hits,
                                     uint8_t **d_hit_edits /* NULL: not wanted */, uint64_t *n_hits, void *cuda_stream);
 
+/* ------------------------------------------------------------------ alignment of Hamming and edit-distance hits
+ * The locate calls above say where a query matches and at what distance; these calls say what matched: the end of
+ * each hit's alignment and its edit operations (a CIGAR), nucleotide only.  Text, query bytes, n and the virtual
+ * queries of both-strand search are as in the blocks above.
+ *   Q         the searched string: query q (single strand, or v = 2q), rc(q) for v = 2q + 1; L = its length.
+ *   s         the hit's global start, seq_starts[seq_idx] + local_pos; T = the text.
+ *   Hamming   window T[s .. s+L) inside the text with <= k mismatches: text_len = L, distance = the mismatches, one
+ *             'X' op per mismatching position, ascending.
+ *   edit      d(s) as in the edit-distance block (start fixed, end free, only T[s .. n) used).  If d(s) <= k the
+ *             alignment is the lexicographically smallest op string (order '=' < 'X' < 'I' < 'D') among all
+ *             alignments of Q against some T[s .. s+l) of cost d(s); text_len = l.  Equivalently: walk from cell (0, 0),
+ *             take a match whenever the symbols are equal, otherwise the first of X, I, D after which cost d(s) is
+ *             still reachable, and stop once all L query symbols are used (never a trailing D).  At s + j = n only I
+ *             is possible.
+ *   none      otherwise, and for a hit of a refused query, a hit with seq_idx >= n_sequences or s >= n: "no alignment
+ *             within k": distance = k + 1, n_ops = 0, text_len = 0.
+ *   ops       SAM conventions: I = a query symbol against nothing, D = a text symbol against nothing.  A reverse-strand
+ *             hit is reported in rc(q) coordinates, as SAM stores a reverse-strand record, so the ops read in
+ *             reference order.  Unused ops and every pad byte are 0.
+ *   promise   for every hit a locate call returns, with that call's query, metric, strands and k: distance = the
+ *             call's distance of the hit, n_ops = distance, and applying the ops to Q gives exactly T[s .. s+text_len).
+ *   inputs    hit_off / hits exactly as the locate calls produce them (awry_locate_{batch,device}_{hamming,edit}
+ *             [_strands]): hit_off has nv + 1 entries, nv = nq << strands, and hit_off[0] = 0; hits may be in any order
+ *             within their query's range and each is aligned on its own.  out[h] belongs to hits[h].
+ *   errors    k > 3, an unknown metric, strands > 1, a null pointer, hit_off not starting at 0 or not monotone (host
+ *             call) -> AWRY_ERR_INVALID_ARG; a protein index or one without the text on the device (as the approximate
+ *             calls) -> AWRY_ERR_UNSUPPORTED; the host call: an empty query, one with '$' / '#' or with L <= k ->
+ *             AWRY_ERR_INVALID_QUERY naming q.  The device call latches such queries for awry_device_check and their
+ *             hits get "no alignment".
+ *   device    awry_align_device reads back the batch's first and last query offset (one synchronisation) and returns
+ *             without waiting; it trusts d_hit_off[nv] == n_hits (the bounds-checked build asserts it).  All pointers
+ *             are on replica `replica`'s device.
+ * Scheme (DESIGN.md §1f): one thread per hit reads the packed query against the text on the device: Hamming compares 8
+ * symbols per step, edit distance runs an iterative-deepening search over budgets 0 .. k that extends matches 8
+ * symbols at a time and tries X, I, D at a mismatch. */
+enum { AWRY_METRIC_HAMMING = 0, AWRY_METRIC_EDIT = 1 };
+typedef struct awry_edit_op {
+  uint32_t qpos;     /* index into Q of the op's query symbol (I, X), or of the symbol it precedes (D) */
+  uint32_t tpos;     /* offset into the window: text[s + tpos] (X, D), or the text offset it precedes (I) */
+  uint8_t op;        /* 'X', 'I', 'D' */
+  uint8_t query_sym; /* 'A', 'C', 'G', 'T', 'N' of Q (0 for D) */
+  uint8_t text_sym;  /* 'A', 'C', 'G', 'T', 'N' of the text (0 for I) */
+  uint8_t pad;
+} awry_edit_op;
+typedef struct awry_alignment {
+  uint32_t text_len; /* l: the window is text[s .. s+l) */
+  uint8_t distance;  /* k + 1: no alignment within k */
+  uint8_t n_ops;     /* == distance when aligned */
+  uint8_t pad[2];
+  awry_edit_op ops[AWRY_EDIT_MAX]; /* the first n_ops are valid, ascending by qpos */
+} awry_alignment;
+typedef char awry_edit_op_is_12_bytes[sizeof(awry_edit_op) == 12 ? 1 : -1];
+typedef char awry_alignment_is_44_bytes[sizeof(awry_alignment) == 44 ? 1 : -1];
+int awry_align_batch(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq, uint32_t metric,
+                     uint32_t strands /* 0 or 1 */, uint32_t k, const uint64_t *hit_off /* nv + 1, nv = nq << strands */,
+                     const awry_hit *hits, awry_alignment *out /* hit_off[nv] entries */);
+int awry_align_device(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff, uint64_t nq,
+                      uint32_t metric, uint32_t strands, uint32_t k, const uint64_t *d_hit_off, const awry_hit *d_hits,
+                      uint64_t n_hits, awry_alignment *d_out, void *cuda_stream);
+/* Host only, no device: the extended CIGAR (op letters =, X, I, D; e.g. "47=1X102=") of one alignment of a query of
+ * length L = query_len.  Writes at most cap bytes including the NUL; *needed (may be NULL) = full length + 1.
+ * AWRY_ERR_CAPACITY if it did not fit (buf then holds nothing useful); AWRY_ERR_INVALID_ARG for a "no alignment"
+ * record, n_ops > 3, or ops that are out of order or do not fit L. */
+int awry_alignment_cigar(const awry_alignment *a, uint32_t query_len, char *buf, size_t cap, size_t *needed);
+
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to
  * parallel_count / parallel_locate (fm_index.rs:455-487); these entry points take the FASTQ ('@') or

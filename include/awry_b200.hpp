@@ -295,6 +295,30 @@ class FmIndex {
     for (size_t v = 0; v < flat.size(); v++) out[v / 2][v % 2] = flat[v];
     return out;
   }
+  // Alignment of located hits (no counterpart in the reference): hit_off / hits as a locate_{hamming,edit}[_strands]
+  // call with the same queries, metric (AWRY_METRIC_HAMMING / AWRY_METRIC_EDIT) and k returned them; one alignment per
+  // hit (text_len, distance, the ops: see cigar)
+  std::vector<awry_alignment> align_hits(const std::vector<std::string_view>& queries, uint32_t metric, uint32_t k,
+                                         const std::vector<uint64_t>& hit_off, const std::vector<awry_hit>& hits,
+                                         bool strands = false) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::vector<awry_alignment> out(hits.size());
+    check(awry_align_batch(h_, bytes.data(), off.data(), queries.size(), metric, strands ? 1 : 0, k, hit_off.data(),
+                           hits.data(), out.data()));
+    return out;
+  }
+  // the extended CIGAR (=, X, I, D) of one alignment of a query of length query_len, e.g. "47=1X102="
+  static std::string cigar(const awry_alignment& a, uint32_t query_len) {
+    size_t need = 0;
+    const int rc = awry_alignment_cigar(&a, query_len, nullptr, 0, &need);
+    if (rc != AWRY_ERR_CAPACITY) check(rc);
+    std::string s(need, '\0');
+    check(awry_alignment_cigar(&a, query_len, &s[0], s.size(), &need));
+    s.resize(need - 1);
+    return s;
+  }
   awry_index* handle() const { return h_; }
 
  private:

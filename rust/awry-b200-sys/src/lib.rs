@@ -21,6 +21,32 @@ pub struct awry_hit {
     pub local_pos: u64,
 }
 
+pub const AWRY_METRIC_HAMMING: u32 = 0;
+pub const AWRY_METRIC_EDIT: u32 = 1;
+
+/// one edit operation of an alignment (include/awry_b200.h: awry_edit_op, 12 bytes)
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default, PartialEq, Eq)]
+pub struct awry_edit_op {
+    pub qpos: u32,
+    pub tpos: u32,
+    pub op: u8,
+    pub query_sym: u8,
+    pub text_sym: u8,
+    pub pad: u8,
+}
+
+/// the alignment of one located hit (include/awry_b200.h: awry_alignment, 44 bytes)
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default, PartialEq, Eq)]
+pub struct awry_alignment {
+    pub text_len: u32,
+    pub distance: u8,
+    pub n_ops: u8,
+    pub pad: [u8; 2],
+    pub ops: [awry_edit_op; 3],
+}
+
 #[repr(C)]
 #[derive(Clone, Copy)]
 pub struct awry_info {
@@ -190,6 +216,14 @@ extern "C" {
                                            d_qoff: *const u64, nq: u64, max_edits: u32, d_hit_off: *mut u64,
                                            d_hits: *mut *mut awry_hit, d_hit_edits: *mut *mut u8, n_hits: *mut u64,
                                            cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_align_batch(index: *const awry_index, qbytes: *const u8, qoff: *const u64, nq: u64, metric: u32,
+                            strands: u32, k: u32, hit_off: *const u64, hits: *const awry_hit,
+                            out: *mut awry_alignment) -> c_int;
+    pub fn awry_align_device(index: *const awry_index, replica: c_int, d_qbytes: *const u8, d_qoff: *const u64, nq: u64,
+                             metric: u32, strands: u32, k: u32, d_hit_off: *const u64, d_hits: *const awry_hit,
+                             n_hits: u64, d_out: *mut awry_alignment, cuda_stream: *mut c_void) -> c_int;
+    pub fn awry_alignment_cigar(a: *const awry_alignment, query_len: u32, buf: *mut c_char, cap: usize,
+                                needed: *mut usize) -> c_int;
     pub fn awry_set_host_threads(n: c_int) -> c_int;
     pub fn awry_host_threads() -> c_int;
     pub fn awry_profile_enable(on: c_int) -> c_int;
