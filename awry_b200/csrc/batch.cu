@@ -1227,6 +1227,25 @@ struct DeviceHits {
   uint64_t* n_hits;
 };
 
+// The loci of n edit-distance hits sorted per query (DESIGN.md §1g), no synchronisation.  d_off (nq + 1, from 0) is the
+// hits' CSR; a hit is the key (s << 2 | d) at d_pos when d_dist is null, else d_pos / d_dist.  Count (d_counts, nq (k+1),
+// zeroed): every locus adds 1 at [q (k+1) + d].  Otherwise d_P (n + 1) becomes the exclusive scan of the keep flags and
+// d_off the CSR of the loci; launch_edit_loci_compact then moves them.
+void edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, uint64_t* d_off, uint64_t nq, uint64_t n, uint32_t k,
+               uint64_t* d_P, uint64_t* d_counts, cudaStream_t st) {
+  StreamScratch ss(st);
+  size_t temp = 0;
+  uint32_t* const d_map = ss.get<uint32_t>(n);
+  CU(launch_hamming_map(d_off, nq, 0, n, d_map, nullptr, temp, st));
+  CU(launch_hamming_map(d_off, nq, 0, n, d_map, ss.get<uint8_t>(temp), temp, st));
+  CU(launch_edit_loci(d_pos, d_dist, d_off, d_map, n, k, d_P, d_counts, st));
+  if (d_counts) return;
+  size_t t2 = 0;
+  CU(scan_u64(d_P, d_P, n + 1, nullptr, t2, st));
+  CU(scan_u64(d_P, d_P, n + 1, ss.get<uint8_t>(t2), t2, st));
+  CU(launch_edit_loci_offsets(d_P, d_off, nq, st));
+}
+
 // One batch of reads on one replica, all on stream `st`: pieces -> exact search of the pieces -> candidates ->
 // verification against the text, in slices of at most hamming_slice() candidates.  Offsets are absolute and lie
 // in [b_lo, b_hi] (d_qbytes is biased accordingly).  Count: d_counts (nq * (k + 1)) is zeroed and filled.  Locate:
@@ -1240,11 +1259,15 @@ struct DeviceHits {
 // `metric`: substitutions (Hamming, one window per candidate) or edits (awry_*_edit: 2k + 1 starts per candidate,
 // kernels_edit.cu).  Stages 1 and 2 are the same for both; the metric picks the verification kernel and, for locate,
 // the key slots per candidate.  A slice holds at most hamming_slice() key slots.
+// `loci` (edit only, awry_*_edit_loci, DESIGN.md §1g): only the loci of each query's sorted hits are kept.  Locate
+// filters each slice's hits before they are mapped and copied; count and the device locate take the device-resident
+// flow (a count without `dev` into a CSR of its own) and filter the sorted keys.
 enum Metric { METRIC_HAMMING = 0, METRIC_EDIT = 1 };
 const char* metric_name(Metric metric) { return metric == METRIC_EDIT ? "edit-distance" : "Hamming"; }
 void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
                  uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
-                 HammingSink* sink, bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr) {
+                 HammingSink* sink, bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr,
+                 bool loci = false) {
   const bool edit = metric == METRIC_EDIT;
   const char* const what = metric_name(metric);
   const uint32_t shift = strands ? 1 : 0;  // virtual query -> read
@@ -1343,17 +1366,19 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       CU(edit ? launch_edit_verify(r.view, a, k, mode, r.sm_count, st) : launch_hamming_verify(r.view, a, k, mode, r.sm_count, st));
     }
   };
-  if (dev) {  // 3. device-resident locate (DESIGN.md §1e)
+  if (dev || (loci && !sink)) {  // 3. device-resident locate (DESIGN.md §1e), and the loci count (§1g)
+    uint64_t* const hit_off = dev ? dev->hit_off : sc.get<uint64_t>(nv + 1);
+    if (!dev) CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
     // count pass: the CSR over the queries, and the hit total that sizes the outputs (the second synchronisation)
     a.counts = sc.get<uint64_t>(nv * P);
     CU(cudaMemsetAsync(a.counts, 0, nv * P * 8, st));
     verify_all(VERIFY_COUNT);
     uint64_t* d_sums = sc.get<uint64_t>(nv + 1);
     CU(launch_hamming_row_sums(a.counts, k, nv, d_sums, st));
-    CU(scan_u64(d_sums, dev->hit_off, nv + 1, nullptr, temp, st));
-    CU(scan_u64(d_sums, dev->hit_off, nv + 1, sc.get<uint8_t>(temp), temp, st));
+    CU(scan_u64(d_sums, hit_off, nv + 1, nullptr, temp, st));
+    CU(scan_u64(d_sums, hit_off, nv + 1, sc.get<uint8_t>(temp), temp, st));
     uint64_t n = 0;
-    CU(cudaMemcpyAsync(&n, dev->hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&n, hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (n == 0) return;
     // CUB's segmented sort reads its offsets as int: more than 2^31 - 1 keys are sorted in parts cut at query
@@ -1362,7 +1387,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     std::vector<uint64_t> off;
     if (n >= (1ull << 31)) {
       off.resize(nv + 1);
-      CU(cudaMemcpyAsync(off.data(), dev->hit_off, (nv + 1) * 8, cudaMemcpyDeviceToHost, st));
+      CU(cudaMemcpyAsync(off.data(), hit_off, (nv + 1) * 8, cudaMemcpyDeviceToHost, st));
       CU(cudaStreamSynchronize(st));
       parts.clear();
       for (uint64_t q0 = 0; q0 < nv;) {
@@ -1376,15 +1401,19 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
         q0 = q1;
       }
     }
-    // the outputs (released in stream order unless the call succeeds), then the scratch the hit total sizes
+    // the outputs (released in stream order unless the call succeeds), then the scratch the hit total sizes; the
+    // loci's outputs are sized by the locus total, after the filter
     StreamScratch out(st);
     awry_hit* d_hits = nullptr;
     uint8_t* d_dist = nullptr;
     uint64_t *d_keys = nullptr, *d_sorted = nullptr;
+    auto outputs = [&](uint64_t m) {
+      d_hits = out.get<awry_hit>(m);  // (16 spare bytes behind the last hit, as every hit buffer)
+      if (dev->dist) d_dist = out.get<uint8_t>(m);
+    };
     try {
-      d_hits = out.get<awry_hit>(n);  // (16 spare bytes behind the last hit, as every hit buffer)
-      if (dev->dist) d_dist = out.get<uint8_t>(n);
-      d_keys = sc.get<uint64_t>(n);
+      if (!loci) outputs(n);
+      d_keys = sc.get<uint64_t>(loci ? n + 1 : n);
       d_sorted = sc.get<uint64_t>(n);
     } catch (const ApiError& x) {
       if (x.code != AWRY_ERR_NOMEM) throw;
@@ -1394,7 +1423,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     a.keys = d_keys;
     a.acc = sc.get<uint64_t>(nv);
     a.q0 = 0;
-    a.hit_off = dev->hit_off;
+    a.hit_off = hit_off;
     CU(cudaMemsetAsync(a.acc, 0, nv * 8, st));
     verify_all(VERIFY_PLACE);
     // order: a query's positions are distinct, so the sorted keys do not depend on the order the atomics gave
@@ -1402,8 +1431,29 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       const uint64_t b = off.empty() ? 0 : off[q0], m = off.empty() ? n : off[q1] - off[q0];
       StreamScratch ss(st);
       size_t t2 = 0;
-      CU(sort_hamming_keys(d_keys + b, d_sorted + b, m, q1 - q0, dev->hit_off + q0, b, nullptr, t2, st));
-      CU(sort_hamming_keys(d_keys + b, d_sorted + b, m, q1 - q0, dev->hit_off + q0, b, ss.get<uint8_t>(t2), t2, st));
+      CU(sort_hamming_keys(d_keys + b, d_sorted + b, m, q1 - q0, hit_off + q0, b, nullptr, t2, st));
+      CU(sort_hamming_keys(d_keys + b, d_sorted + b, m, q1 - q0, hit_off + q0, b, ss.get<uint8_t>(t2), t2, st));
+    }
+    if (loci) {
+      // the filter over the whole batch at once (its scans take 64-bit sizes); d_keys, free after the sort, takes
+      // the scan of the keep flags.  The locus total sizes the outputs: the third synchronisation.
+      edit_loci(d_sorted, nullptr, hit_off, nv, n, k, d_keys, dev ? nullptr : d_counts, st);
+      if (!dev) return;
+      uint64_t m = 0;
+      CU(cudaMemcpyAsync(&m, hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
+      if (m == 0) return;
+      uint64_t* d_loci = nullptr;
+      try {
+        outputs(m);
+        d_loci = sc.get<uint64_t>(m);
+      } catch (const ApiError& x) {
+        if (x.code != AWRY_ERR_NOMEM) throw;
+        fail(AWRY_ERR_NOMEM, "out of device memory for the %llu loci of this %s locate", (unsigned long long)m, what);
+      }
+      CU(launch_edit_loci_compact(d_keys, n, d_sorted, nullptr, d_loci, nullptr, st));
+      d_sorted = d_loci;
+      n = m;
     }
     CU(launch_hamming_decode(d_sorted, n, d_dist, st));
     CU(launch_map_locations(r.view, d_sorted, n, reinterpret_cast<uint64_t*>(d_hits), st));
@@ -1466,15 +1516,31 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     std::vector<uint64_t> qh(nr + 1);
     CU(cudaMemcpyAsync(qh.data(), d_qh, (nr + 1) * 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    const uint64_t n_acc = qh[nr];
+    uint64_t n_acc = qh[nr];
+    uint64_t* d_pos = nullptr;
+    uint8_t* d_dist = nullptr;
     if (n_acc) {
-      uint64_t* d_pos = ss.get<uint64_t>(n_acc);
-      uint8_t* d_dist = ss.get<uint8_t>(n_acc);
-      uint64_t* d_hits = ss.get<uint64_t>(2 * n_acc);
+      d_pos = ss.get<uint64_t>(n_acc);
+      d_dist = ss.get<uint8_t>(n_acc);
       if (edit)
         CU(launch_edit_compact(d_sorted, d_map, n * slots, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
       else
         CU(launch_hamming_compact(d_sorted, d_map, n, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
+      if (loci) {  // a read's hits are all in this slice: only the loci go on (d_qh becomes their CSR)
+        uint64_t* const d_P = ss.get<uint64_t>(n_acc + 1);
+        edit_loci(d_pos, d_dist, d_qh, nr, n_acc, k, d_P, nullptr, st);
+        CU(cudaMemcpyAsync(qh.data(), d_qh, (nr + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        uint64_t* const pos = ss.get<uint64_t>(qh[nr]);
+        uint8_t* const dist = ss.get<uint8_t>(qh[nr]);
+        CU(launch_edit_loci_compact(d_P, n_acc, d_pos, d_dist, pos, dist, st));
+        d_pos = pos;
+        d_dist = dist;
+        n_acc = qh[nr];
+      }
+    }
+    if (n_acc) {
+      uint64_t* d_hits = ss.get<uint64_t>(2 * n_acc);
       CU(launch_map_locations(r.view, d_pos, n_acc, d_hits, st));
       sink->hits.resize(base + n_acc);
       sink->dist.resize(base + n_acc);
@@ -1492,7 +1558,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
 // host path does not overlap copies with compute yet).  `strands`: a chunk of n reads fills 2 n result slots.
 void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo,
                         uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink, bool strands = false,
-                        Metric metric = METRIC_HAMMING) {
+                        Metric metric = METRIC_HAMMING, bool loci = false) {
   if (lo >= hi) return;
   Replica& r = *ix->reps[ri];
   DeviceGuard dg(r.device);
@@ -1513,13 +1579,13 @@ void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, 
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
       if (sink) {
         hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr, sink,
-                    strands, metric);
+                    strands, metric, nullptr, loci);
       } else {
         StreamScratch sc(ws->st);
         const uint64_t slots = (strands ? 2 : 1) * (k + 1);  // counts per read
         uint64_t* d_counts = sc.get<uint64_t>(n * slots);
         hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts, nullptr,
-                    strands, metric);
+                    strands, metric, nullptr, loci);
         CU(cudaMemcpyAsync(counts + c.q0 * slots, d_counts, n * slots * 8, cudaMemcpyDeviceToHost, ws->st));
         g_prof.d2h += n * slots * 8;
       }
@@ -1555,7 +1621,7 @@ void check_max_k(uint32_t k, Metric metric) {
 
 // awry_count_batch_{hamming,edit}[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
 void hamming_count_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t k,
-                        uint64_t* counts, bool strands, Metric metric = METRIC_HAMMING) {
+                        uint64_t* counts, bool strands, Metric metric = METRIC_HAMMING, bool loci = false) {
   need(ix);
   check_max_k(k, metric);
   if (nq == 0) return;
@@ -1563,14 +1629,14 @@ void hamming_count_impl(const awry_index* ix, const uint8_t* qbytes, const uint6
   if (strands) strands_check_index(ix);
   hamming_check_index(ix, metric_name(metric));
   for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
-    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, counts, nullptr, strands, metric);
+    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, counts, nullptr, strands, metric, loci);
   });
 }
 
 // awry_locate_batch_{hamming,edit}[_strands]: hit_off is the CSR over the nq (or 2 nq virtual) queries
 void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t k,
                          uint64_t* hit_off, awry_hit* hits, uint8_t* hit_mismatches, uint64_t capacity, uint64_t* n_hits,
-                         bool strands, Metric metric = METRIC_HAMMING) {
+                         bool strands, Metric metric = METRIC_HAMMING, bool loci = false) {
   need(ix);
   check_max_k(k, metric);
   if (!hit_off || !n_hits || (!hits && capacity)) fail(AWRY_ERR_INVALID_ARG, "null argument");
@@ -1586,7 +1652,7 @@ void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint
   std::vector<std::pair<uint64_t, uint64_t>> ranges(nr, {0, 0});
   for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
     ranges[ri] = {lo, hi};
-    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, nullptr, &sinks[ri], strands, metric);
+    hamming_on_replica(ix, ri, qbytes, qoff, lo, hi, k, nullptr, &sinks[ri], strands, metric, loci);
   });
   // the replicas' CSRs, concatenated in range order; hits past `capacity` are dropped (the total still counts them)
   uint64_t total = 0;
@@ -1691,7 +1757,7 @@ void locate_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbyt
 // awry_count_device_{hamming,edit}[_strands]: counts (nq or 2 nq virtual queries) x (k+1)
 void hamming_count_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
                                uint64_t nq, uint32_t k, uint64_t* d_counts, void* cuda_stream, bool strands,
-                               Metric metric = METRIC_HAMMING) {
+                               Metric metric = METRIC_HAMMING, bool loci = false) {
   need(ix);
   check_max_k(k, metric);
   if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
@@ -1704,14 +1770,15 @@ void hamming_count_device_impl(const awry_index* ix, int replica, const uint8_t*
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
   uint64_t e[2] = {0, 0};
   device_batch_ends(d_qoff, nq, st, e, strands);
-  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands, metric);
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands, metric, nullptr,
+              loci);
 }
 
 // awry_locate_device_{hamming,edit}[_strands]: the hits of the nq (or 2 nq virtual) queries, in stream-ordered device
 // buffers; argument checks and errors as hamming_count_device_impl, outputs as locate_device_impl
 void hamming_locate_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
                                 uint64_t nq, uint32_t k, uint64_t* d_hit_off, awry_hit** d_hits, uint8_t** d_dist,
-                                uint64_t* n_hits, void* cuda_stream, bool strands, Metric metric) {
+                                uint64_t* n_hits, void* cuda_stream, bool strands, Metric metric, bool loci = false) {
   need(ix);
   check_max_k(k, metric);
   if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
@@ -1729,7 +1796,7 @@ void hamming_locate_device_impl(const awry_index* ix, int replica, const uint8_t
   uint64_t e[2] = {0, 0};
   device_batch_ends(d_qoff, nq, st, e, strands);
   DeviceHits out{d_hit_off, d_hits, d_dist, n_hits};
-  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, nullptr, strands, metric, &out);
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, nullptr, strands, metric, &out, loci);
 }
 
 // ------------------------------------------------------------------ alignment of located hits (awry_align_*)
@@ -2121,6 +2188,47 @@ int awry_locate_device_edit_strands(const awry_index* ix, int replica, const uin
   return guarded([&] {
     hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_hit_off, d_hits, d_hit_edits, n_hits,
                                cuda_stream, true, METRIC_EDIT);
+  });
+}
+
+static void loci_check_strands(uint32_t strands) {
+  if (strands > 1) fail(AWRY_ERR_INVALID_ARG, "strands must be 0 or 1");
+}
+
+int awry_count_batch_edit_loci(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                               uint32_t strands, uint32_t max_edits, uint64_t* counts) {
+  return guarded([&] {
+    loci_check_strands(strands);
+    hamming_count_impl(ix, qbytes, qoff, nq, max_edits, counts, strands != 0, METRIC_EDIT, true);
+  });
+}
+
+int awry_locate_batch_edit_loci(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,
+                                uint32_t strands, uint32_t max_edits, uint64_t* hit_off, awry_hit* hits,
+                                uint8_t* hit_edits, uint64_t capacity, uint64_t* n_hits) {
+  return guarded([&] {
+    loci_check_strands(strands);
+    hamming_locate_impl(ix, qbytes, qoff, nq, max_edits, hit_off, hits, hit_edits, capacity, n_hits, strands != 0,
+                        METRIC_EDIT, true);
+  });
+}
+
+int awry_count_device_edit_loci(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                uint64_t nq, uint32_t strands, uint32_t max_edits, uint64_t* d_counts, void* cuda_stream) {
+  return guarded([&] {
+    loci_check_strands(strands);
+    hamming_count_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_counts, cuda_stream, strands != 0,
+                              METRIC_EDIT, true);
+  });
+}
+
+int awry_locate_device_edit_loci(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff,
+                                 uint64_t nq, uint32_t strands, uint32_t max_edits, uint64_t* d_hit_off,
+                                 awry_hit** d_hits, uint8_t** d_hit_edits, uint64_t* n_hits, void* cuda_stream) {
+  return guarded([&] {
+    loci_check_strands(strands);
+    hamming_locate_device_impl(ix, replica, d_qbytes, d_qoff, nq, max_edits, d_hit_off, d_hits, d_hit_edits, n_hits,
+                               cuda_stream, strands != 0, METRIC_EDIT, true);
   });
 }
 

@@ -245,6 +245,17 @@ cudaError_t sort_edit_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t 
 cudaError_t launch_edit_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
                                 const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
                                 uint8_t* d_dist, cudaStream_t s);
+// loci of n edit-distance hits sorted per query (DESIGN.md §1g); d_off: their CSR (nq + 1, from 0), d_map: the query of
+// every hit (launch_hamming_map over d_off).  A hit is the key (s << 2 | d) at d_pos when d_dist is null, else d_pos /
+// d_dist.  d_counts (nq (k+1), zeroed) not null: each locus adds 1 to d_counts[q (k+1) + d]; otherwise d_keep (n + 1)
+// gets 1 per locus, 0 per other hit and at n.
+cudaError_t launch_edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, const uint64_t* d_off, const uint32_t* d_map,
+                             uint64_t n, uint32_t k, uint64_t* d_keep, uint64_t* d_counts, cudaStream_t s);
+// d_off[q] = d_P[d_off[q]], q = 0 .. nq: the loci's CSR from the exclusive scan d_P of the keep flags
+cudaError_t launch_edit_loci_offsets(const uint64_t* d_P, uint64_t* d_off, uint64_t nq, cudaStream_t s);
+// the loci (d_P[i + 1] > d_P[i]) of the n hits d_pos [/ d_dist] to slot d_P[i] of d_pos_out [/ d_dist_out]
+cudaError_t launch_edit_loci_compact(const uint64_t* d_P, uint64_t n, const uint64_t* d_pos, const uint8_t* d_dist,
+                                     uint64_t* d_pos_out, uint8_t* d_dist_out, cudaStream_t s);
 
 // ---- kernels_align.cu: the alignment of located Hamming and edit-distance hits (awry_align_*, DESIGN.md §1f)
 // d_qlen[v] = the length L of search query v (read or virtual query, packed in d_qwords as for launch_search), or 0 when

@@ -225,4 +225,93 @@ cudaError_t launch_edit_compact(const uint64_t* d_sorted, const uint32_t* d_map,
   return cudaGetLastError();
 }
 
+// ---- loci (awry_*_edit_loci, DESIGN.md §1g): one thread per hit of hits sorted per query (ascending, distinct starts).
+// Hit i of query q = map[i] (range off[q] .. off[q + 1]) is a locus unless (a) a hit within k of it has a smaller
+// distance, or (b) its distance is >= 1 and the start just before it is a hit at the same distance.  Positions are
+// distinct, so the hits within k of i are among its k neighbours on each side.  Hit i: key pos[i] = (s << 2) | d when
+// dist is null, else s = pos[i], d = dist[i].  Count: counts[q (k+1) + d] += 1 per locus.  Otherwise keep[i] = 1 for a
+// locus, else 0, and keep[n] = 0.
+__device__ __forceinline__ void loci_hit(const uint64_t* pos, const uint8_t* dist, uint64_t i, uint64_t& s, uint32_t& d) {
+  const uint64_t x = pos[i];
+  s = dist ? x : x >> 2;
+  d = dist ? dist[i] : uint32_t(x & 3);
+}
+
+__global__ void edit_loci_kernel(const uint64_t* __restrict__ pos, const uint8_t* __restrict__ dist,
+                                 const uint64_t* __restrict__ off, const uint32_t* __restrict__ map, uint64_t n,
+                                 uint32_t k, uint64_t* __restrict__ keep, uint64_t* __restrict__ counts) {
+  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
+  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
+    const uint32_t q = map[i];
+    const uint64_t lo = off[q], hi = off[q + 1];
+    AWRY_CHK(lo <= i && i < hi);
+    uint64_t s, t;
+    uint32_t d, e;
+    loci_hit(pos, dist, i, s, d);
+    bool locus = true;
+    for (uint32_t j = 1; j <= k && i - lo >= j && locus; j++) {
+      loci_hit(pos, dist, i - j, t, e);
+      AWRY_CHK(t < s);
+      if (s - t > k) break;
+      locus = e > d || (e == d && (d == 0 || t + 1 != s));
+    }
+    for (uint32_t j = 1; j <= k && i + j < hi && locus; j++) {
+      loci_hit(pos, dist, i + j, t, e);
+      AWRY_CHK(t > s);
+      if (t - s > k) break;
+      locus = e >= d;
+    }
+    if (counts) {
+      if (locus) atomicAdd(reinterpret_cast<unsigned long long*>(counts) + (uint64_t(q) * (k + 1) + d), 1ull);
+    } else {
+      keep[i] = locus;
+      if (i == 0) keep[n] = 0;
+    }
+  }
+}
+
+cudaError_t launch_edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, const uint64_t* d_off, const uint32_t* d_map,
+                             uint64_t n, uint32_t k, uint64_t* d_keep, uint64_t* d_counts, cudaStream_t s) {
+  if (n == 0) return cudaSuccess;
+  const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
+  edit_loci_kernel<<<grid, 256, 0, s>>>(d_pos, d_dist, d_off, d_map, n, k, d_keep, d_counts);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
+// the CSR of the loci: off[q] = P[off[q]], q = 0 .. nq, P the exclusive scan of the keep flags (in place)
+__global__ void edit_loci_offsets_kernel(const uint64_t* __restrict__ P, uint64_t* __restrict__ off, uint64_t nq) {
+  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
+  for (uint64_t q = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; q <= nq; q += stride) off[q] = P[off[q]];
+}
+
+cudaError_t launch_edit_loci_offsets(const uint64_t* d_P, uint64_t* d_off, uint64_t nq, cudaStream_t s) {
+  const unsigned grid = unsigned(std::min<uint64_t>((nq + 256) / 256, 148 * 16));
+  edit_loci_offsets_kernel<<<grid, 256, 0, s>>>(d_P, d_off, nq);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
+// hit i is a locus iff P[i + 1] > P[i]; it goes to slot P[i] of pos_out (and dist_out when dist is not null)
+__global__ void edit_loci_compact_kernel(const uint64_t* __restrict__ P, uint64_t n, const uint64_t* __restrict__ pos,
+                                         const uint8_t* __restrict__ dist, uint64_t* __restrict__ pos_out,
+                                         uint8_t* __restrict__ dist_out) {
+  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
+  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
+    const uint64_t o = P[i];
+    if (P[i + 1] == o) continue;
+    pos_out[o] = pos[i];
+    if (dist) dist_out[o] = dist[i];
+  }
+}
+
+cudaError_t launch_edit_loci_compact(const uint64_t* d_P, uint64_t n, const uint64_t* d_pos, const uint8_t* d_dist,
+                                     uint64_t* d_pos_out, uint8_t* d_dist_out, cudaStream_t s) {
+  if (n == 0) return cudaSuccess;
+  const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
+  edit_loci_compact_kernel<<<grid, 256, 0, s>>>(d_P, n, d_pos, d_dist, d_pos_out, d_dist_out);
+  COUNT_LAUNCH();
+  return cudaGetLastError();
+}
+
 }  // namespace awry

@@ -134,7 +134,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_count_batch_edit", "awry_locate_batch_edit", "awry_count_device_edit", "awry_count_batch_edit_strands",
            "awry_locate_batch_edit_strands", "awry_count_device_edit_strands", "awry_locate_device_hamming",
            "awry_locate_device_hamming_strands", "awry_locate_device_edit", "awry_locate_device_edit_strands",
-           "awry_align_batch", "awry_align_device", "awry_alignment_cigar"]
+           "awry_align_batch", "awry_align_device", "awry_alignment_cigar", "awry_count_batch_edit_loci",
+           "awry_locate_batch_edit_loci", "awry_count_device_edit_loci", "awry_locate_device_edit_loci"]
 
 
 def native():
@@ -219,6 +220,11 @@ def native():
             getattr(L, "awry_locate_device_" + metric + strands).argtypes = [vp, i32, vp, vp, u64, C.c_uint32, vp,
                                                                              C.POINTER(vp), C.POINTER(vp),
                                                                              C.POINTER(u64), vp]
+    L.awry_count_batch_edit_loci.argtypes = [vp, vp, vp, u64, C.c_uint32, C.c_uint32, vp]
+    L.awry_locate_batch_edit_loci.argtypes = [vp, vp, vp, u64, C.c_uint32, C.c_uint32, vp, vp, vp, u64, C.POINTER(u64)]
+    L.awry_count_device_edit_loci.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, C.c_uint32, vp, vp]
+    L.awry_locate_device_edit_loci.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, C.c_uint32, vp, C.POINTER(vp),
+                                               C.POINTER(vp), C.POINTER(u64), vp]
     L.awry_align_batch.argtypes = [vp, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, vp]
     L.awry_align_device.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, u64, vp, vp]
     L.awry_alignment_cigar.argtypes = [vp, C.c_uint32, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
@@ -727,6 +733,39 @@ class FmIndex:
         None, n_hits), as locate_edit_device; free each with device_free"""
         return self._locate_approx_device(native().awry_locate_device_edit_strands, d_qbytes, d_qoff, nq, max_edits,
                                           d_hit_off, distances, stream, replica)
+
+    # ---- edit-distance loci: one hit per occurrence, not every neighbouring start (include/awry_b200.h) ----------
+    def count_edit_loci_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int,
+                               strands: bool = False) -> np.ndarray:
+        """-> uint64[nq, max_edits + 1] (strands: [nq, 2, max_edits + 1]): [q, (s,) d] = loci of q (s = 0) or of its
+        reverse complement (s = 1) at edit distance exactly d"""
+        fn = native().awry_count_batch_edit_loci
+        return self._count_edit(lambda h, qb, qo, nq, k, c: fn(h, qb, qo, nq, int(bool(strands)), k, c), qbytes, qoff,
+                                max_edits, (2,) if strands else ())
+
+    def locate_edit_loci_packed(self, qbytes: np.ndarray, qoff: np.ndarray, max_edits: int, strands: bool = False,
+                                capacity: int = None):
+        """-> (hit_off, hits, edits) as locate_edit_packed (strands: as locate_edit_strands_packed), holding only the
+        loci: the hits no hit within max_edits beats and that do not continue a run of adjacent equal-distance starts"""
+        fn = native().awry_locate_batch_edit_loci
+        return self._locate_edit(lambda h, qb, qo, nq, k, *rest: fn(h, qb, qo, nq, int(bool(strands)), k, *rest), qbytes,
+                                 qoff, max_edits, 2 if strands else 1, capacity)
+
+    def count_edit_loci_device(self, d_qbytes: int, d_qoff: int, nq: int, max_edits: int, d_counts: int,
+                               strands: bool = False, stream: int = 0, replica: int = 0):
+        """count_edit_loci_packed on device pointers (d_counts: (nq << strands) (max_edits + 1) u64); costs about a
+        device locate (two synchronisations); see device_check"""
+        _check(native().awry_count_device_edit_loci(self._h, replica, d_qbytes, d_qoff, nq, int(bool(strands)),
+                                                    int(max_edits), d_counts, stream))
+
+    def locate_edit_loci_device(self, d_qbytes: int, d_qoff: int, nq: int, max_edits: int, d_hit_off: int,
+                                strands: bool = False, distances: bool = True, stream: int = 0, replica: int = 0):
+        """locate_edit_loci_packed on device pointers (d_hit_off: (nq << strands) + 1 u64) -> (hits pointer, edits
+        pointer or None, n_hits), as locate_edit_device; free each with device_free"""
+        fn = native().awry_locate_device_edit_loci
+        return self._locate_approx_device(
+            lambda h, rep, qb, qo, nq, k, *rest: fn(h, rep, qb, qo, nq, int(bool(strands)), k, *rest), d_qbytes, d_qoff,
+            nq, max_edits, d_hit_off, distances, stream, replica)
 
     # ---- alignment of located Hamming / edit-distance hits (include/awry_b200.h) -------------
     def align_hits_packed(self, qbytes: np.ndarray, qoff: np.ndarray, metric, max_dist: int, hit_off: np.ndarray,

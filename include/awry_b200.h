@@ -359,6 +359,7 @@ int awry_locate_device_hamming_strands(const awry_index *index, int replica, con
  *   neighbouring starts  an occurrence is a START, not a locus: an exact occurrence at s also makes s - 1 .. s - k
  *             and s + 1 .. s + k occurrences at distances 1 .. k (insert text symbols in front of the query, or delete
  *             its leading symbols), and all of them are reported.  Nothing merges them into one locus.
+ *             awry_*_edit_loci (the next block) report each locus once.
  *   count     counts[q * (k+1) + d] = the number of starts with d(s) = d (nq * (k+1) entries).  For k = 0 this equals
  *             awry_count_batch; for every k the d = 0 column equals that of the Hamming calls.
  *   locate    every start with d(s) <= k, once each, per query in ascending text position, as (seq_idx, local_pos) of
@@ -403,6 +404,55 @@ int awry_locate_device_edit_strands(const awry_index *index, int replica, const 
                                     uint64_t *d_hit_off /* 2*nq + 1 */, awry_hit **d_hits,
                                     uint8_t **d_hit_edits /* NULL: not wanted */, uint64_t *n_hits, void *cuda_stream);
 
+/* ------------------------------------------------------------------ edit-distance search by locus
+ * The edit-distance block above reports starts: one occurrence comes back as up to 2k + 1 neighbouring starts.  These
+ * calls report each locus once, so a read maps to one hit per place and per-distance counts count sites.
+ *   virtual   v = q (strands = 0), or v = 2q (q) and v = 2q + 1 (rc(q)) (strands = 1), as in the blocks above.
+ *   H         exactly the starts awry_locate_batch_edit[_strands] returns for v at that k, each with its distance d(s);
+ *             s is the global start seq_starts[seq_idx] + local_pos.
+ *   locus     a start s in H such that both hold:
+ *             (a) no s' in H with 0 < |s' - s| <= k has d(s') < d(s) (a start within k of a strictly better one is a
+ *                 shifted copy of it);
+ *             (b) if d(s) >= 1, s - 1 is not in H with d(s - 1) = d(s) (a run of adjacent starts at one nonzero
+ *                 distance is one locus, reported at its leftmost start).  Exact occurrences (d = 0) are never merged:
+ *                 adjacent exact occurrences in a homopolymer all stay, as in exact search.
+ *   so        k = 0: the loci are the hits of awry_locate_batch[_strands] with AWRY_LOCATE_SORTED.  The d = 0 loci are the
+ *             exact occurrences (that column of the counts equals awry_count_batch[_strands]).  The loci are a subset
+ *             of H with the same distances, in the same order.  The leftmost hit at a query's smallest distance is a
+ *             locus, so the best distance per query is unchanged.  Different virtual queries never interact (forward
+ *             and reverse-complement loci are decided separately).  Two occurrences more than k apart are both kept;
+ *             so are two of equal distance within k unless they are adjacent (b).  A plateau's locus is its leftmost
+ *             start: one optimal start, not necessarily the one a scoring aligner would prefer.
+ *   count     counts[v * (k+1) + d] = the number of loci of v at distance d ((nq << strands) * (k+1) entries).
+ *   locate    the loci of each v in ascending text position, as (seq_idx, local_pos), hit_off over the nq << strands
+ *             virtual queries; hit_edits (NULL or `capacity` entries) receives d(s); capacity / AWRY_ERR_CAPACITY as
+ *             in awry_locate_batch_edit.  awry_align_* aligns the loci as any edit-distance hit.
+ *   errors    strands > 1 -> AWRY_ERR_INVALID_ARG; otherwise exactly those of the matching edit calls (k > 3, null
+ *             pointers, a bad replica -> AWRY_ERR_INVALID_ARG; a refused query -> AWRY_ERR_INVALID_QUERY naming it in the
+ *             host calls, latched for awry_device_check by the device calls; an unsupported index ->
+ *             AWRY_ERR_UNSUPPORTED).  A refused query's device result is the filter applied to the range the device
+ *             edit locate gives it.
+ *   device    bit for bit the host calls' results.  The device locate synchronises three times (the candidate total,
+ *             the hit total, the locus total that sizes the outputs); its outputs come from the stream-ordered pool and
+ *             are released with awry_device_free.  The device count runs the place pass and the sort of the device
+ *             locate and synchronises twice: it costs about a device locate, not a count.  Where starts will do,
+ *             awry_count_device_edit is the cheaper call.
+ * Scheme (DESIGN.md §1g): the hits of each query are sorted by text position; one thread per hit reads at most k
+ * neighbours on each side, and the loci are compacted by a scan of the keep flags. */
+int awry_count_batch_edit_loci(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                               uint32_t strands /* 0 or 1 */, uint32_t max_edits,
+                               uint64_t *counts /* (nq << strands) * (max_edits + 1) */);
+int awry_locate_batch_edit_loci(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq,
+                                uint32_t strands, uint32_t max_edits, uint64_t *hit_off /* (nq << strands) + 1 */,
+                                awry_hit *hits, uint8_t *hit_edits /* NULL or capacity */, uint64_t capacity,
+                                uint64_t *n_hits);
+int awry_count_device_edit_loci(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                                uint64_t nq, uint32_t strands, uint32_t max_edits, uint64_t *d_counts, void *cuda_stream);
+int awry_locate_device_edit_loci(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff,
+                                 uint64_t nq, uint32_t strands, uint32_t max_edits, uint64_t *d_hit_off,
+                                 awry_hit **d_hits, uint8_t **d_hit_edits /* NULL: not wanted */, uint64_t *n_hits,
+                                 void *cuda_stream);
+
 /* ------------------------------------------------------------------ alignment of Hamming and edit-distance hits
  * The locate calls above say where a query matches and at what distance; these calls say what matched: the end of
  * each hit's alignment and its edit operations (a CIGAR), nucleotide only.  Text, query bytes, n and the virtual
@@ -422,10 +472,10 @@ int awry_locate_device_edit_strands(const awry_index *index, int replica, const 
  *   ops       SAM conventions: I = a query symbol against nothing, D = a text symbol against nothing.  A reverse-strand
  *             hit is reported in rc(q) coordinates, as SAM stores a reverse-strand record, so the ops read in
  *             reference order.  Unused ops and every pad byte are 0.
- *   promise   for every hit a locate call returns, with that call's query, metric, strands and k: distance = the
+ *   promise   for every hit a locate call returns, with that call's query, metric, strands and k (edit for the loci): distance = the
  *             call's distance of the hit, n_ops = distance, and applying the ops to Q gives exactly T[s .. s+text_len).
  *   inputs    hit_off / hits exactly as the locate calls produce them (awry_locate_{batch,device}_{hamming,edit}
- *             [_strands]): hit_off has nv + 1 entries, nv = nq << strands, and hit_off[0] = 0; hits may be in any order
+ *             [_strands], awry_locate_{batch,device}_edit_loci): hit_off has nv + 1 entries, nv = nq << strands, and hit_off[0] = 0; hits may be in any order
  *             within their query's range and each is aligned on its own.  out[h] belongs to hits[h].
  *   errors    k > 3, an unknown metric, strands > 1, a null pointer, hit_off not starting at 0 or not monotone (host
  *             call) -> AWRY_ERR_INVALID_ARG; a protein index or one without the text on the device (as the approximate

@@ -295,6 +295,35 @@ class FmIndex {
     for (size_t v = 0; v < flat.size(); v++) out[v / 2][v % 2] = flat[v];
     return out;
   }
+  // Edit-distance loci (no counterpart in the reference): as the four calls above, but each occurrence once, at its
+  // locus (include/awry_b200.h), not at every neighbouring start
+  std::vector<std::vector<uint64_t>> parallel_count_edit_loci(const std::vector<std::string_view>& queries,
+                                                              uint32_t max_edits) const {
+    const size_t P = size_t(max_edits) + 1;
+    const std::vector<uint64_t> flat = count_edit_flat(queries, max_edits, false, true);
+    std::vector<std::vector<uint64_t>> out(queries.size());
+    for (size_t q = 0; q < queries.size(); q++) out[q].assign(flat.begin() + q * P, flat.begin() + (q + 1) * P);
+    return out;
+  }
+  std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> parallel_locate_edit_loci(
+      const std::vector<std::string_view>& queries, uint32_t max_edits) const {
+    return locate_edit_flat(queries, max_edits, false, true);
+  }
+  std::vector<std::array<std::vector<uint64_t>, 2>> parallel_count_edit_loci_strands(
+      const std::vector<std::string_view>& queries, uint32_t max_edits) const {
+    const size_t P = size_t(max_edits) + 1;
+    const std::vector<uint64_t> flat = count_edit_flat(queries, max_edits, true, true);
+    std::vector<std::array<std::vector<uint64_t>, 2>> out(queries.size());
+    for (size_t v = 0; v < 2 * queries.size(); v++) out[v / 2][v % 2].assign(flat.begin() + v * P, flat.begin() + (v + 1) * P);
+    return out;
+  }
+  std::vector<std::array<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>, 2>> parallel_locate_edit_loci_strands(
+      const std::vector<std::string_view>& queries, uint32_t max_edits) const {
+    const auto flat = locate_edit_flat(queries, max_edits, true, true);
+    std::vector<std::array<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>, 2>> out(queries.size());
+    for (size_t v = 0; v < flat.size(); v++) out[v / 2][v % 2] = flat[v];
+    return out;
+  }
   // Alignment of located hits (no counterpart in the reference): hit_off / hits as a locate_{hamming,edit}[_strands]
   // call with the same queries, metric (AWRY_METRIC_HAMMING / AWRY_METRIC_EDIT) and k returned them; one alignment per
   // hit (text_len, distance, the ops: see cigar)
@@ -323,24 +352,34 @@ class FmIndex {
 
  private:
   explicit FmIndex(awry_index* h) : h_(h) { check(awry_index_info(h_, &info_)); }
-  // the edit calls' flat results: counts (nq or 2 nq) x (k+1), and the hits of each (virtual) query
+  // the edit calls' flat results: counts (nq or 2 nq) x (k+1), and the hits of each (virtual) query; `loci`: the
+  // awry_*_edit_loci calls
   std::vector<uint64_t> count_edit_flat(const std::vector<std::string_view>& queries, uint32_t max_edits,
-                                        bool strands) const {
+                                        bool strands, bool loci = false) const {
     std::vector<uint8_t> bytes;
     std::vector<uint64_t> off;
     pack(queries, bytes, off);
     std::vector<uint64_t> flat((strands ? 2 : 1) * queries.size() * (size_t(max_edits) + 1));
-    check((strands ? awry_count_batch_edit_strands : awry_count_batch_edit)(h_, bytes.data(), off.data(), queries.size(),
-                                                                            max_edits, flat.data()));
+    if (loci)
+      check(awry_count_batch_edit_loci(h_, bytes.data(), off.data(), queries.size(), strands ? 1 : 0, max_edits,
+                                       flat.data()));
+    else
+      check((strands ? awry_count_batch_edit_strands : awry_count_batch_edit)(h_, bytes.data(), off.data(),
+                                                                              queries.size(), max_edits, flat.data()));
     return flat;
   }
   std::vector<std::vector<std::pair<LocalizedSequencePosition, uint32_t>>> locate_edit_flat(
-      const std::vector<std::string_view>& queries, uint32_t max_edits, bool strands) const {
+      const std::vector<std::string_view>& queries, uint32_t max_edits, bool strands, bool loci = false) const {
     std::vector<uint8_t> bytes;
     std::vector<uint64_t> off;
     pack(queries, bytes, off);
     const size_t nv = (strands ? 2 : 1) * queries.size();
-    auto call = strands ? awry_locate_batch_edit_strands : awry_locate_batch_edit;
+    auto edit = strands ? awry_locate_batch_edit_strands : awry_locate_batch_edit;
+    auto call = [&](const awry_index* h, const uint8_t* b, const uint64_t* o, uint64_t nq, uint32_t k, uint64_t* ho,
+                    awry_hit* hs, uint8_t* d, uint64_t cap, uint64_t* n) {
+      return loci ? awry_locate_batch_edit_loci(h, b, o, nq, strands ? 1 : 0, k, ho, hs, d, cap, n)
+                  : edit(h, b, o, nq, k, ho, hs, d, cap, n);
+    };
     std::vector<uint64_t> hit_off(nv + 1);
     std::vector<awry_hit> hits(nv + 1);
     std::vector<uint8_t> dist(hits.size());
