@@ -1212,14 +1212,15 @@ void hamming_check_index(const awry_index* ix, const char* what = "Hamming") {
            "AWRY_B200_FULL_SA / AWRY_B200_TEXT, device memory, or 64-bit row pointers)", what);
 }
 
-// the hits of the locate call on one replica, in query order
-struct HammingSink {
+// the hits of the host-buffer locate on one replica, in query order
+struct HostHits {
+  bool want_dist;             // the caller asked for each hit's distance
   std::vector<uint64_t> off;  // per (virtual) query: offset of its first hit in `hits`
   std::vector<awry_hit> hits;
   std::vector<uint8_t> dist;
 };
 
-// the outputs of the device-resident locate (awry_locate_device_{hamming,edit}[_strands])
+// the outputs of the locate flow of hamming_run (the device-resident calls, and each chunk of the host-buffer ones)
 struct DeviceHits {
   uint64_t* hit_off;  // device, nv + 1: the CSR over the (virtual) queries
   awry_hit** hits;    // a device allocation of *n_hits hits (not set when there are none)
@@ -1228,17 +1229,17 @@ struct DeviceHits {
 };
 
 // The loci of n edit-distance hits sorted per query (DESIGN.md §1g), no synchronisation.  d_off (nq + 1, from 0) is the
-// hits' CSR; a hit is the key (s << 2 | d) at d_pos when d_dist is null, else d_pos / d_dist.  Count (d_counts, nq (k+1),
-// zeroed): every locus adds 1 at [q (k+1) + d].  Otherwise d_P (n + 1) becomes the exclusive scan of the keep flags and
-// d_off the CSR of the loci; launch_edit_loci_compact then moves them.
-void edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, uint64_t* d_off, uint64_t nq, uint64_t n, uint32_t k,
-               uint64_t* d_P, uint64_t* d_counts, cudaStream_t st) {
+// hits' CSR and d_keys their keys (s << 2 | d).  Count (d_counts, nq (k+1), zeroed): every locus adds 1 at
+// [q (k+1) + d].  Otherwise d_P (n + 1) becomes the exclusive scan of the keep flags and d_off the CSR of the loci;
+// launch_edit_loci_compact then moves them.
+void edit_loci(const uint64_t* d_keys, uint64_t* d_off, uint64_t nq, uint64_t n, uint32_t k, uint64_t* d_P,
+               uint64_t* d_counts, cudaStream_t st) {
   StreamScratch ss(st);
   size_t temp = 0;
   uint32_t* const d_map = ss.get<uint32_t>(n);
   CU(launch_hamming_map(d_off, nq, 0, n, d_map, nullptr, temp, st));
   CU(launch_hamming_map(d_off, nq, 0, n, d_map, ss.get<uint8_t>(temp), temp, st));
-  CU(launch_edit_loci(d_pos, d_dist, d_off, d_map, n, k, d_P, d_counts, st));
+  CU(launch_edit_loci(d_keys, d_off, d_map, n, k, d_P, d_counts, st));
   if (d_counts) return;
   size_t t2 = 0;
   CU(scan_u64(d_P, d_P, n + 1, nullptr, t2, st));
@@ -1246,63 +1247,73 @@ void edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, uint64_t* d_off, ui
   CU(launch_edit_loci_offsets(d_P, d_off, nq, st));
 }
 
+// The search queries of a batch of reads (offsets absolute within [b_lo, b_hi], d_qbytes biased accordingly), in
+// scratch of `sc`: the reads packed, their prepass validating the offsets and latching what it refuses in *d_flag;
+// both strands: the 2 nq virtual queries' offsets and words (kernels.hpp) made from them.
+struct SearchQueries {
+  const uint64_t* words;  // biased as for launch_search; the words [w_lo, w_lo + w_n) exist
+  uint64_t w_lo, w_n;
+  const uint64_t* off;    // nq (or 2 nq) + 1, absolute within [lo, hi]
+  uint64_t lo, hi;
+};
+SearchQueries pack_search_queries(StreamScratch& sc, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                                  uint64_t b_lo, uint64_t b_hi, bool strands, unsigned long long* d_flag, cudaStream_t st) {
+  const uint64_t nbytes = b_hi - b_lo, rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
+  uint64_t* const rw = sc.get<uint64_t>(rw_n) - w_lo;
+  CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, rw, b_lo, b_hi, d_flag, st));
+  if (!strands) return {rw, w_lo, rw_n, d_qoff, b_lo, b_hi};
+  const uint64_t nv = 2 * nq, vw_n = packed_words(0, nv, 2 * nbytes), vw_lo = 4 * ((2 * b_lo) >> 6);
+  uint64_t* const voff = sc.get<uint64_t>(nv + 1);
+  uint64_t* const vw = sc.get<uint64_t>(vw_n) - vw_lo;
+  CU(launch_strand_offsets(d_qoff, nq, b_lo, b_hi, voff, st));
+  CU(launch_strand_words(rw, d_qoff, nq, b_lo, b_hi, voff, vw, st));
+  return {vw, vw_lo, vw_n, voff, 2 * b_lo, 2 * b_hi};
+}
+
 // One batch of reads on one replica, all on stream `st`: pieces -> exact search of the pieces -> candidates ->
-// verification against the text, in slices of at most hamming_slice() candidates.  Offsets are absolute and lie
-// in [b_lo, b_hi] (d_qbytes is biased accordingly).  Count: d_counts (nq * (k + 1)) is zeroed and filled.  Locate:
-// the hits are appended to `sink` (slices cut at read boundaries, the hits of a read sorted by text position).
-// Device-resident locate (`dev`): a count pass and a place pass over the same slices, then one segmented sort; the
-// hits stay on the device, and the call returns without waiting for the last kernels.
+// verification against the text, in slices of at most hamming_slice() key slots.  Offsets are absolute and lie in
+// [b_lo, b_hi] (d_qbytes is biased accordingly).  Count: d_counts (nq * (k + 1)) is zeroed and filled.  Locate
+// (`dev`, DESIGN.md §1e): a count pass and a place pass over the same slices, then one segmented sort; the hits stay
+// on the device, and the call returns without waiting for the last kernels.
 // `check_base` >= 0: a refused read fails the call (reported as read check_base + q) before anything is verified;
-// < 0 (the device-resident call): it stays latched in *d_flag for awry_device_check.
+// < 0 (the device-resident calls): it stays latched in *d_flag for awry_device_check.
 // `strands`: the nq reads are searched as the 2 nq virtual queries of both strands (kernels.hpp), which take the
 // place of the reads from the piece offsets on: counts, CSR offsets and the hits are per virtual query.
 // `metric`: substitutions (Hamming, one window per candidate) or edits (awry_*_edit: 2k + 1 starts per candidate,
-// kernels_edit.cu).  Stages 1 and 2 are the same for both; the metric picks the verification kernel and, for locate,
-// the key slots per candidate.  A slice holds at most hamming_slice() key slots.
-// `loci` (edit only, awry_*_edit_loci, DESIGN.md §1g): only the loci of each query's sorted hits are kept.  Locate
-// filters each slice's hits before they are mapped and copied; count and the device locate take the device-resident
-// flow (a count without `dev` into a CSR of its own) and filter the sorted keys.
+// kernels_edit.cu).  Stages 1 and 2 are the same for both; the metric picks the verification kernel and the key
+// slots per candidate, 1 or 2k + 1, that a slice counts.
+// `loci` (edit only, awry_*_edit_loci, DESIGN.md §1g): only the loci of each query's sorted hits are kept.  Both
+// count and locate take the locate's flow (a count into a CSR of its own) and filter the sorted keys.
 enum Metric { METRIC_HAMMING = 0, METRIC_EDIT = 1 };
 const char* metric_name(Metric metric) { return metric == METRIC_EDIT ? "edit-distance" : "Hamming"; }
 void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
                  uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
-                 HammingSink* sink, bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr,
-                 bool loci = false) {
+                 bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr, bool loci = false) {
   const bool edit = metric == METRIC_EDIT;
   const char* const what = metric_name(metric);
   const uint32_t shift = strands ? 1 : 0;  // virtual query -> read
-  const uint64_t P = k + 1, nbytes = b_hi - b_lo, nv = nq << shift, np = nv * P;
+  const uint64_t P = k + 1, nv = nq << shift, np = nv * P;
   const uint64_t slots = edit ? 2 * k + 1 : 1;  // key slots per candidate
   if (np >= (1ull << 31)) fail(AWRY_ERR_INVALID_ARG, "batch too large for one %s search (%llu reads): split it", what, (unsigned long long)nq);
   StreamScratch sc(st);
-  // 1. pieces, packed; the whole reads packed too (their prepass validates the offsets and latches what it refuses).
-  // Single strand: the pieces are packed from the caller's bytes (DESIGN.md §1c: cutting them out of the read words
-  // measured slower at k = 1 and 3).  Both strands: the virtual queries' offsets and words come from the reads', and
-  // the pieces' words are cut out of the virtual words (a reverse-complement piece has no bytes to pack).
-  const uint64_t rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
-  const uint64_t v_lo = b_lo << shift, v_hi = b_hi << shift, vw_n = packed_words(0, nv, nbytes << shift), vw_lo = 4 * (v_lo >> 6);
-  const uint64_t* d_voff = d_qoff;
-  uint64_t* d_poff = sc.get<uint64_t>(np + 1);
-  uint64_t* const d_pw = sc.get<uint64_t>(packed_words(0, np, nbytes << shift)) - vw_lo;
-  uint64_t* const d_rw = sc.get<uint64_t>(rw_n) - w_lo;
-  uint64_t* d_vw = d_rw;
+  // 1. the reads packed (pack_search_queries), then the pieces and their words.  Single strand: the pieces are packed
+  // from the caller's bytes (DESIGN.md §1c: cutting them out of the read words measured slower at k = 1 and 3).  Both
+  // strands: they are cut out of the virtual words (a reverse-complement piece has no bytes to pack).  Every refusal
+  // is latched by an atomicMin, so the order of the prepasses does not change which read is reported.
+  uint64_t* const d_poff = sc.get<uint64_t>(np + 1);
+  SearchQueries sq;
+  uint64_t* d_pw;
   {
     ProfScope p(2, r.device, st);
+    sq = pack_search_queries(sc, d_qbytes, d_qoff, nq, b_lo, b_hi, strands, d_flag, st);
+    d_pw = sc.get<uint64_t>(packed_words(0, np, sq.hi - sq.lo)) - 4 * (sq.lo >> 6);
+    CU(launch_hamming_pieces(sq.off, nv, k, sq.lo, sq.hi, shift, d_poff, d_flag, st));
     if (!strands) {
       unsigned long long* d_pflag = sc.get<unsigned long long>(1);  // (piece indices: what it latches is reported per read)
       CU(cudaMemsetAsync(d_pflag, 0xff, 8, st));
-      CU(launch_hamming_pieces(d_qoff, nq, k, b_lo, b_hi, 0, d_poff, d_flag, st));
       CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_poff, np, d_pw, b_lo, b_hi, d_pflag, st));
-      CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
     } else {
-      uint64_t* const voff = sc.get<uint64_t>(nv + 1);
-      d_vw = sc.get<uint64_t>(vw_n) - vw_lo;
-      CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
-      CU(launch_strand_offsets(d_qoff, nq, b_lo, b_hi, voff, st));
-      CU(launch_strand_words(d_rw, d_qoff, nq, b_lo, b_hi, voff, d_vw, st));
-      d_voff = voff;
-      CU(launch_hamming_pieces(d_voff, nv, k, v_lo, v_hi, shift, d_poff, d_flag, st));
-      CU(launch_hamming_piece_words(d_vw, d_voff, nv, v_lo, v_hi, k, d_pw, st));
+      CU(launch_hamming_piece_words(sq.words, sq.off, nv, sq.lo, sq.hi, k, d_pw, st));
     }
   }
   // 2. exact search of the pieces (the wave kernel stores a piece finished in the text as its position), CSR
@@ -1311,9 +1322,9 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   {
     ProfScope p(0, r.device, st);
     SearchVariant v = current_variant();
-    v.avg_len = uint32_t(std::min<uint64_t>((nbytes << shift) / np, 1u << 30));
-    v.b_lo = v_lo;
-    v.b_hi = v_hi;
+    v.avg_len = uint32_t(std::min<uint64_t>((sq.hi - sq.lo) / np, 1u << 30));
+    v.b_lo = sq.lo;
+    v.b_hi = sq.hi;
     v.locate_positions = locate_positions_ok(r.view, v);
     CU(launch_search(r.view, d_pw, d_poff, np, OUT_SP_CNT_U32, d_sp, sc.get<uint32_t>(defer_words(np)), v, r.sm_count, st));
   }
@@ -1321,18 +1332,9 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   size_t temp = 0;
   CU(scan_hit_offsets(r.view, d_sp, np, d_hoff, nullptr, temp, st));
   CU(scan_hit_offsets(r.view, d_sp, np, d_hoff, sc.get<uint8_t>(temp), temp, st));
-  // the candidate total (and, for locate, every read's candidate range) sizes the slices: one synchronisation
+  // the candidate total sizes the slices: one synchronisation
   uint64_t total = 0;
   unsigned long long flag = ~0ull;
-  std::vector<uint64_t> qcand;
-  uint64_t* d_qcand = nullptr;
-  if (sink) {
-    d_qcand = sc.get<uint64_t>(nv + 1);
-    CU(launch_hamming_query_bounds(d_hoff, k, nv, d_qcand, st));
-    qcand.resize(nv + 1);
-    CU(cudaMemcpyAsync(qcand.data(), d_qcand, (nv + 1) * 8, cudaMemcpyDeviceToHost, st));
-    g_prof.d2h += (nv + 1) * 8;
-  }
   CU(cudaMemcpyAsync(&total, d_hoff + np, 8, cudaMemcpyDeviceToHost, st));
   if (check_base >= 0) CU(cudaMemcpyAsync(&flag, d_flag, 8, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
@@ -1343,12 +1345,12 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   if (flag != ~0ull) fail_bad_query(flag, uint64_t(check_base));
 
   HammingSlice a{};
-  a.qwords = d_vw;
-  a.qw_lo = strands ? vw_lo : w_lo;
-  a.qw_n = strands ? vw_n : rw_n;
-  a.qoff = d_voff;
-  a.b_lo = v_lo;
-  a.b_hi = v_hi;
+  a.qwords = sq.words;
+  a.qw_lo = sq.w_lo;
+  a.qw_n = sq.w_n;
+  a.qoff = sq.off;
+  a.b_lo = sq.lo;
+  a.b_hi = sq.hi;
   a.sp_cnt = d_sp;
   a.hoff = d_hoff;
   a.npieces = np;
@@ -1366,7 +1368,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       CU(edit ? launch_edit_verify(r.view, a, k, mode, r.sm_count, st) : launch_hamming_verify(r.view, a, k, mode, r.sm_count, st));
     }
   };
-  if (dev || (loci && !sink)) {  // 3. device-resident locate (DESIGN.md §1e), and the loci count (§1g)
+  if (dev || loci) {  // 3. locate (DESIGN.md §1e), and the loci count (§1g)
     uint64_t* const hit_off = dev ? dev->hit_off : sc.get<uint64_t>(nv + 1);
     if (!dev) CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
     // count pass: the CSR over the queries, and the hit total that sizes the outputs (the second synchronisation)
@@ -1422,7 +1424,6 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     // place pass: the same slices and the same acceptance as the count pass; each key takes a slot of its query's range
     a.keys = d_keys;
     a.acc = sc.get<uint64_t>(nv);
-    a.q0 = 0;
     a.hit_off = hit_off;
     CU(cudaMemsetAsync(a.acc, 0, nv * 8, st));
     verify_all(VERIFY_PLACE);
@@ -1437,7 +1438,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     if (loci) {
       // the filter over the whole batch at once (its scans take 64-bit sizes); d_keys, free after the sort, takes
       // the scan of the keep flags.  The locus total sizes the outputs: the third synchronisation.
-      edit_loci(d_sorted, nullptr, hit_off, nv, n, k, d_keys, dev ? nullptr : d_counts, st);
+      edit_loci(d_sorted, hit_off, nv, n, k, d_keys, dev ? nullptr : d_counts, st);
       if (!dev) return;
       uint64_t m = 0;
       CU(cudaMemcpyAsync(&m, hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
@@ -1451,7 +1452,7 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
         if (x.code != AWRY_ERR_NOMEM) throw;
         fail(AWRY_ERR_NOMEM, "out of device memory for the %llu loci of this %s locate", (unsigned long long)m, what);
       }
-      CU(launch_edit_loci_compact(d_keys, n, d_sorted, nullptr, d_loci, nullptr, st));
+      CU(launch_edit_loci_compact(d_keys, n, d_sorted, d_loci, st));
       d_sorted = d_loci;
       n = m;
     }
@@ -1463,101 +1464,17 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     *dev->n_hits = n;
     return;
   }
-  if (!sink) {  // 3. count
-    CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
-    a.counts = d_counts;
-    verify_all(VERIFY_COUNT);
-    return;
-  }
-  // 3. locate: slices cut at read boundaries (a read with more candidates than a slice gets one of its own size)
-  sink->off.reserve(sink->off.size() + nv);
-  for (uint64_t q0 = 0; q0 < nv;) {
-    uint64_t q1 = q0 + 1;
-    while (q1 < nv && qcand[q1 + 1] - qcand[q0] <= S) q1++;
-    const uint64_t c0 = qcand[q0], n = qcand[q1] - c0, nr = q1 - q0;
-    if (n * slots >= (1ull << 31))  // (a slice is sorted per read by one CUB call, whose offsets are int)
-      fail(AWRY_ERR_NOMEM, "query %llu has %llu candidate windows, more than one slice can sort (2^31)",
-           (unsigned long long)(uint64_t(check_base < 0 ? 0 : check_base) + (q0 >> shift)), (unsigned long long)(n * slots));
-    const uint64_t base = sink->hits.size();
-    if (n == 0) {
-      sink->off.insert(sink->off.end(), nr, base);
-      q0 = q1;
-      continue;
-    }
-    StreamScratch ss(st);
-    a.c0 = c0;
-    a.n = n;
-    a.q0 = q0;
-    uint32_t* d_map = ss.get<uint32_t>(n);
-    CU(launch_hamming_map(d_hoff, np, c0, n, d_map, nullptr, temp, st));
-    CU(launch_hamming_map(d_hoff, np, c0, n, d_map, ss.get<uint8_t>(temp), temp, st));
-    a.map = d_map;
-    a.keys = ss.get<uint64_t>(n * slots);
-    a.acc = ss.get<uint64_t>(nr + 1);
-    CU(cudaMemsetAsync(a.acc, 0, (nr + 1) * 8, st));
-    {
-      ProfScope p(1, r.device, st);
-      CU(edit ? launch_edit_verify(r.view, a, k, VERIFY_LOCATE, r.sm_count, st)
-              : launch_hamming_verify(r.view, a, k, VERIFY_LOCATE, r.sm_count, st));
-    }
-    uint64_t* d_sorted = ss.get<uint64_t>(n * slots);
-    size_t t2 = 0;
-    if (edit) {
-      CU(sort_edit_keys(a.keys, d_sorted, n * slots, nr, d_qcand + q0, c0, uint32_t(slots), nullptr, t2, st));
-      CU(sort_edit_keys(a.keys, d_sorted, n * slots, nr, d_qcand + q0, c0, uint32_t(slots), ss.get<uint8_t>(t2), t2, st));
-    } else {
-      CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, nullptr, t2, st));
-      CU(sort_hamming_keys(a.keys, d_sorted, n, nr, d_qcand + q0, c0, ss.get<uint8_t>(t2), t2, st));
-    }
-    uint64_t* d_qh = ss.get<uint64_t>(nr + 1);
-    size_t t3 = 0;
-    CU(scan_u64(a.acc, d_qh, nr + 1, nullptr, t3, st));
-    CU(scan_u64(a.acc, d_qh, nr + 1, ss.get<uint8_t>(t3), t3, st));
-    std::vector<uint64_t> qh(nr + 1);
-    CU(cudaMemcpyAsync(qh.data(), d_qh, (nr + 1) * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    uint64_t n_acc = qh[nr];
-    uint64_t* d_pos = nullptr;
-    uint8_t* d_dist = nullptr;
-    if (n_acc) {
-      d_pos = ss.get<uint64_t>(n_acc);
-      d_dist = ss.get<uint8_t>(n_acc);
-      if (edit)
-        CU(launch_edit_compact(d_sorted, d_map, n * slots, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
-      else
-        CU(launch_hamming_compact(d_sorted, d_map, n, k, d_qcand, c0, q0, d_qh, d_pos, d_dist, st));
-      if (loci) {  // a read's hits are all in this slice: only the loci go on (d_qh becomes their CSR)
-        uint64_t* const d_P = ss.get<uint64_t>(n_acc + 1);
-        edit_loci(d_pos, d_dist, d_qh, nr, n_acc, k, d_P, nullptr, st);
-        CU(cudaMemcpyAsync(qh.data(), d_qh, (nr + 1) * 8, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        uint64_t* const pos = ss.get<uint64_t>(qh[nr]);
-        uint8_t* const dist = ss.get<uint8_t>(qh[nr]);
-        CU(launch_edit_loci_compact(d_P, n_acc, d_pos, d_dist, pos, dist, st));
-        d_pos = pos;
-        d_dist = dist;
-        n_acc = qh[nr];
-      }
-    }
-    if (n_acc) {
-      uint64_t* d_hits = ss.get<uint64_t>(2 * n_acc);
-      CU(launch_map_locations(r.view, d_pos, n_acc, d_hits, st));
-      sink->hits.resize(base + n_acc);
-      sink->dist.resize(base + n_acc);
-      CU(cudaMemcpyAsync(sink->hits.data() + base, d_hits, n_acc * 16, cudaMemcpyDeviceToHost, st));
-      CU(cudaMemcpyAsync(sink->dist.data() + base, d_dist, n_acc, cudaMemcpyDeviceToHost, st));
-      g_prof.d2h += n_acc * 17;
-      CU(cudaStreamSynchronize(st));
-    }
-    for (uint64_t i = 0; i < nr; i++) sink->off.push_back(base + qh[i]);
-    q0 = q1;
-  }
+  // 3. count
+  CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
+  a.counts = d_counts;
+  verify_all(VERIFY_COUNT);
 }
 
 // reads [lo, hi) of host buffers on replica ri: chunks of reads uploaded and searched one after the other (the
 // host path does not overlap copies with compute yet).  `strands`: a chunk of n reads fills 2 n result slots.
+// Locate (`out`): each chunk's hits are located on the device (hamming_run's locate flow), then appended to `out`.
 void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo,
-                        uint64_t hi, uint32_t k, uint64_t* counts, HammingSink* sink, bool strands = false,
+                        uint64_t hi, uint32_t k, uint64_t* counts, HostHits* out, bool strands = false,
                         Metric metric = METRIC_HAMMING, bool loci = false) {
   if (lo >= hi) return;
   Replica& r = *ix->reps[ri];
@@ -1577,19 +1494,36 @@ void hamming_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, 
       CU(cudaMemcpyAsync(ws->d_qoff, qoff + c.q0, (n + 1) * 8, cudaMemcpyHostToDevice, ws->st));
       g_prof.h2d += nbytes + (n + 1) * 8;
       CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
-      if (sink) {
-        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr, sink,
-                    strands, metric, nullptr, loci);
+      const uint64_t nv = strands ? 2 * n : n, o = out ? out->off.size() : 0, base = out ? out->hits.size() : 0;
+      if (out) {
+        StreamScratch sc(ws->st);
+        awry_hit* d_hits = nullptr;  // (hamming_run leaves them unset when there are no hits)
+        uint8_t* d_dist = nullptr;
+        uint64_t nh = 0;
+        DeviceHits dh{sc.get<uint64_t>(nv + 1), &d_hits, out->want_dist ? &d_dist : nullptr, &nh};
+        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr,
+                    strands, metric, &dh, loci);
+        if (d_hits) sc.ptrs.push_back(d_hits);  // released in stream order, after the copies below
+        if (d_dist) sc.ptrs.push_back(d_dist);
+        out->off.resize(o + nv);
+        out->hits.resize(base + nh);
+        if (d_dist) out->dist.resize(base + nh);
+        CU(cudaMemcpyAsync(out->off.data() + o, dh.hit_off, nv * 8, cudaMemcpyDeviceToHost, ws->st));
+        if (nh) CU(cudaMemcpyAsync(out->hits.data() + base, d_hits, nh * sizeof(awry_hit), cudaMemcpyDeviceToHost, ws->st));
+        if (d_dist) CU(cudaMemcpyAsync(out->dist.data() + base, d_dist, nh, cudaMemcpyDeviceToHost, ws->st));
+        g_prof.d2h += nv * 8 + nh * (sizeof(awry_hit) + (d_dist ? 1 : 0));
       } else {
         StreamScratch sc(ws->st);
         const uint64_t slots = (strands ? 2 : 1) * (k + 1);  // counts per read
         uint64_t* d_counts = sc.get<uint64_t>(n * slots);
-        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts, nullptr,
+        hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, d_counts,
                     strands, metric, nullptr, loci);
         CU(cudaMemcpyAsync(counts + c.q0 * slots, d_counts, n * slots * 8, cudaMemcpyDeviceToHost, ws->st));
         g_prof.d2h += n * slots * 8;
       }
       CU(cudaStreamSynchronize(ws->st));
+      if (out)  // (the chunk's CSR starts at 0)
+        for (uint64_t i = o; i < o + nv; i++) out->off[i] += base;
     }
   } catch (...) {
     cudaStreamSynchronize(ws->st);
@@ -1648,7 +1582,7 @@ void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint
   hamming_check_index(ix, metric_name(metric));
   const uint64_t per = strands ? 2 : 1;  // result slots per read
   const size_t nr = ix->reps.size();
-  std::vector<HammingSink> sinks(nr);
+  std::vector<HostHits> sinks(nr, HostHits{hit_mismatches != nullptr, {}, {}, {}});
   std::vector<std::pair<uint64_t, uint64_t>> ranges(nr, {0, 0});
   for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
     ranges[ri] = {lo, hi};
@@ -1658,7 +1592,7 @@ void hamming_locate_impl(const awry_index* ix, const uint8_t* qbytes, const uint
   uint64_t total = 0;
   for (size_t ri = 0; ri < nr; ri++) {
     const auto [lo, hi] = ranges[ri];
-    const HammingSink& s = sinks[ri];
+    const HostHits& s = sinks[ri];
     for (uint64_t i = 0; i < per * (hi - lo); i++) hit_off[per * lo + i] = total + s.off[i];
     const uint64_t n = s.hits.size(), fit = capacity > total ? std::min(n, capacity - total) : 0;
     if (fit) {
@@ -1770,8 +1704,7 @@ void hamming_count_device_impl(const awry_index* ix, int replica, const uint8_t*
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
   uint64_t e[2] = {0, 0};
   device_batch_ends(d_qoff, nq, st, e, strands);
-  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, nullptr, strands, metric, nullptr,
-              loci);
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, d_counts, strands, metric, nullptr, loci);
 }
 
 // awry_locate_device_{hamming,edit}[_strands]: the hits of the nq (or 2 nq virtual) queries, in stream-ordered device
@@ -1796,13 +1729,13 @@ void hamming_locate_device_impl(const awry_index* ix, int replica, const uint8_t
   uint64_t e[2] = {0, 0};
   device_batch_ends(d_qoff, nq, st, e, strands);
   DeviceHits out{d_hit_off, d_hits, d_dist, n_hits};
-  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, nullptr, strands, metric, &out, loci);
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, strands, metric, &out, loci);
 }
 
 // ------------------------------------------------------------------ alignment of located hits (awry_align_*)
 
-// One batch of reads on one replica, on stream `st`: the prepass of hamming_run (the reads packed; both strands: the
-// virtual offsets and words), each search query's length (0: refused), then the hits in slices of at most
+// One batch of reads on one replica, on stream `st`: the prepass of hamming_run (pack_search_queries), each search
+// query's length (0: refused), then the hits in slices of at most
 // hamming_slice(): the query of every hit from the hit offsets (hamming_map's scatter and max-scan), and one
 // alignment per hit.  d_hit_off (nv + 1) holds absolute hit indices; hit hit0 + i is d_hits[i] and gets d_out[i].
 // `check_base` >= 0: a refused read fails the call, reported as read check_base + q; < 0: it stays latched in *d_flag.
@@ -1811,32 +1744,20 @@ void align_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint
                const uint64_t* d_hit_off, uint64_t hit0, const awry_hit* d_hits, uint64_t n_hits, awry_alignment* d_out,
                cudaStream_t st) {
   const uint32_t shift = strands ? 1 : 0;
-  const uint64_t nv = nq << shift, nbytes = b_hi - b_lo;
+  const uint64_t nv = nq << shift;
   StreamScratch sc(st);
-  const uint64_t rw_n = packed_words(0, nq, nbytes), w_lo = 4 * (b_lo >> 6);
-  const uint64_t v_lo = b_lo << shift, v_hi = b_hi << shift, vw_n = packed_words(0, nv, nbytes << shift), vw_lo = 4 * (v_lo >> 6);
-  uint64_t* const d_rw = sc.get<uint64_t>(rw_n) - w_lo;
-  const uint64_t *d_vw = d_rw, *d_voff = d_qoff;
-  CU(launch_pack(AWRY_NUCLEOTIDE, d_qbytes, d_qoff, nq, d_rw, b_lo, b_hi, d_flag, st));
-  if (strands) {
-    uint64_t* const voff = sc.get<uint64_t>(nv + 1);
-    uint64_t* const vw = sc.get<uint64_t>(vw_n) - vw_lo;
-    CU(launch_strand_offsets(d_qoff, nq, b_lo, b_hi, voff, st));
-    CU(launch_strand_words(d_rw, d_qoff, nq, b_lo, b_hi, voff, vw, st));
-    d_voff = voff;
-    d_vw = vw;
-  }
+  const SearchQueries sq = pack_search_queries(sc, d_qbytes, d_qoff, nq, b_lo, b_hi, strands, d_flag, st);
   uint32_t* const d_qlen = sc.get<uint32_t>(nv);
   AlignSlice a{};
-  a.qwords = d_vw;
-  a.qw_lo = strands ? vw_lo : w_lo;
-  a.qw_n = strands ? vw_n : rw_n;
-  a.qoff = d_voff;
+  a.qwords = sq.words;
+  a.qw_lo = sq.w_lo;
+  a.qw_n = sq.w_n;
+  a.qoff = sq.off;
   a.qlen = d_qlen;
   a.nq = nv;
   a.hit_end = d_hit_off + nv;
   a.hit_total = hit0 + n_hits;
-  CU(launch_align_reads(d_vw, d_voff, nv, v_lo, v_hi, a.qw_lo, a.qw_n, k, shift, d_qlen, d_flag, st));
+  CU(launch_align_reads(sq.words, sq.off, nv, sq.lo, sq.hi, sq.w_lo, sq.w_n, k, shift, d_qlen, d_flag, st));
   if (check_base >= 0) {
     unsigned long long flag = ~0ull;
     CU(cudaMemcpyAsync(&flag, d_flag, 8, cudaMemcpyDeviceToHost, st));

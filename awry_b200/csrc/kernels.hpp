@@ -190,15 +190,12 @@ cudaError_t launch_hamming_pieces(const uint64_t* d_qoff, uint64_t nq, uint32_t 
 // likewise with the piece offsets of launch_hamming_pieces; a query refused by its prepass (or empty) is skipped.
 cudaError_t launch_hamming_piece_words(const uint64_t* d_qwords, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo,
                                        uint64_t b_hi, uint32_t k, uint64_t* d_pwords, cudaStream_t s);
-// d_qcand[i] = d_hoff[(k+1) i] for i = 0 .. nq (candidate range of each query)
-cudaError_t launch_hamming_query_bounds(const uint64_t* d_hoff, uint32_t k, uint64_t nq, uint64_t* d_qcand, cudaStream_t s);
 // piece of every candidate of the slice [c0, c0 + n) (cub convention: d_temp == nullptr sizes the scratch)
 cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_t c0, uint64_t n, uint32_t* d_map,
                                void* d_temp, size_t& temp_bytes, cudaStream_t s);
-// what the verification kernels do with an accepted candidate: COUNT adds it to counts, LOCATE writes a key per
-// candidate of the slice (slices cut at read boundaries, sorted per slice), PLACE writes the key into its query's
-// range of a CSR computed by a COUNT pass over the same candidates (device-resident locate, DESIGN.md §1e)
-enum VerifyMode { VERIFY_COUNT = 0, VERIFY_LOCATE = 1, VERIFY_PLACE = 2 };
+// what the verification kernels do with an accepted candidate: COUNT adds it to counts, PLACE writes its key into
+// its query's range of a CSR computed by a COUNT pass over the same candidates (locate, DESIGN.md §1e)
+enum VerifyMode { VERIFY_COUNT = 0, VERIFY_PLACE = 1 };
 // one slice of candidates for the verification kernel
 struct HammingSlice {
   const uint64_t* qwords;       // packed reads, biased as for launch_search: read q at word 4 (q + (qoff[q] >> 6))
@@ -214,48 +211,35 @@ struct HammingSlice {
     uint64_t* counts;           // count: (k+1) per read, zeroed by the caller
     const uint64_t* hit_off;    // place: read q's keys go to keys[hit_off[q] .. hit_off[q + 1])
   };
-  uint64_t* keys;               // locate: (s << 2 | d) or ~0 per candidate of the slice; place: the keys of the batch
-  uint64_t* acc;                // locate: accepted candidates per read of the slice, zeroed by the caller;
-                                // place: keys placed so far per read of the batch (the cursor), zeroed by the caller
-  uint64_t q0;                  // locate: first read of the slice (place: 0)
+  uint64_t* keys;               // place: the keys (s << 2 | d) of the batch
+  uint64_t* acc;                // place: keys placed so far per read of the batch (the cursor), zeroed by the caller
 };
 cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                   cudaStream_t s);
-// locate: the n < 2^31 keys of a slice sorted per read (segment i = d_qcand[i] - c0 .. d_qcand[i+1] - c0)
+// the n < 2^31 keys of a part of a CSR sorted per query (segment i = d_off[i] - base .. d_off[i+1] - base)
 cudaError_t sort_hamming_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg,
-                              const uint64_t* d_qcand, uint64_t c0, void* d_temp, size_t& temp_bytes, cudaStream_t s);
+                              const uint64_t* d_off, uint64_t base, void* d_temp, size_t& temp_bytes, cudaStream_t s);
 cudaError_t scan_u64(const uint64_t* d_in, uint64_t* d_out, uint64_t n, void* d_temp, size_t& temp_bytes, cudaStream_t s);
 // device-resident locate: d_sums[q] = the sum of read q's k + 1 counts, q < nq, and d_sums[nq] = 0 (its exclusive scan
 // is the CSR over the reads)
 cudaError_t launch_hamming_row_sums(const uint64_t* d_counts, uint32_t k, uint64_t nq, uint64_t* d_sums, cudaStream_t s);
 // sorted keys (s << 2 | d) -> the text positions s in place, and the distances d to d_dist unless it is null
 cudaError_t launch_hamming_decode(uint64_t* d_keys, uint64_t n, uint8_t* d_dist, cudaStream_t s);
-// accepted sorted keys -> text positions and distances at offset d_qh[q - q0] + rank in the read's segment
-cudaError_t launch_hamming_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
-                                   const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
-                                   uint8_t* d_dist, cudaStream_t s);
 
 // ---- kernels_edit.cu: edit-distance search (<= k substitutions, insertions, deletions) on the Hamming candidates.
-// Every candidate names 2k + 1 starts, so locate keeps 2k + 1 key slots per candidate (slot k + δ: start s0 - δ).
+// Every candidate names 2k + 1 starts (start s0 - δ, δ = -k .. k).
 cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                cudaStream_t s);
-// locate: the n < 2^31 key slots of a slice sorted per read (segment i = slots * (d_qcand[i] - c0) ..)
-cudaError_t sort_edit_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg, const uint64_t* d_qcand,
-                           uint64_t c0, uint32_t slots, void* d_temp, size_t& temp_bytes, cudaStream_t s);
-cudaError_t launch_edit_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
-                                const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
-                                uint8_t* d_dist, cudaStream_t s);
-// loci of n edit-distance hits sorted per query (DESIGN.md §1g); d_off: their CSR (nq + 1, from 0), d_map: the query of
-// every hit (launch_hamming_map over d_off).  A hit is the key (s << 2 | d) at d_pos when d_dist is null, else d_pos /
-// d_dist.  d_counts (nq (k+1), zeroed) not null: each locus adds 1 to d_counts[q (k+1) + d]; otherwise d_keep (n + 1)
-// gets 1 per locus, 0 per other hit and at n.
-cudaError_t launch_edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, const uint64_t* d_off, const uint32_t* d_map,
-                             uint64_t n, uint32_t k, uint64_t* d_keep, uint64_t* d_counts, cudaStream_t s);
+// loci of n edit-distance hits sorted per query (DESIGN.md §1g); d_keys: their keys (s << 2 | d), d_off: their CSR
+// (nq + 1, from 0), d_map: the query of every hit (launch_hamming_map over d_off).  d_counts (nq (k+1), zeroed) not
+// null: each locus adds 1 to d_counts[q (k+1) + d]; otherwise d_keep (n + 1) gets 1 per locus, 0 per other hit and at n.
+cudaError_t launch_edit_loci(const uint64_t* d_keys, const uint64_t* d_off, const uint32_t* d_map, uint64_t n, uint32_t k,
+                             uint64_t* d_keep, uint64_t* d_counts, cudaStream_t s);
 // d_off[q] = d_P[d_off[q]], q = 0 .. nq: the loci's CSR from the exclusive scan d_P of the keep flags
 cudaError_t launch_edit_loci_offsets(const uint64_t* d_P, uint64_t* d_off, uint64_t nq, cudaStream_t s);
-// the loci (d_P[i + 1] > d_P[i]) of the n hits d_pos [/ d_dist] to slot d_P[i] of d_pos_out [/ d_dist_out]
-cudaError_t launch_edit_loci_compact(const uint64_t* d_P, uint64_t n, const uint64_t* d_pos, const uint8_t* d_dist,
-                                     uint64_t* d_pos_out, uint8_t* d_dist_out, cudaStream_t s);
+// the keys of the loci (d_P[i + 1] > d_P[i]) among the n keys d_keys to slot d_P[i] of d_keys_out
+cudaError_t launch_edit_loci_compact(const uint64_t* d_P, uint64_t n, const uint64_t* d_keys, uint64_t* d_keys_out,
+                                     cudaStream_t s);
 
 // ---- kernels_align.cu: the alignment of located Hamming and edit-distance hits (awry_align_*, DESIGN.md §1f)
 // d_qlen[v] = the length L of search query v (read or virtual query, packed in d_qwords as for launch_search), or 0 when

@@ -4,10 +4,6 @@
 // a_{j+1}), every exact occurrence of piece j at text position p is a candidate, s0 = p - a_j.  Only the
 // verification differs: a start whose best alignment keeps piece j intact lies in [s0 - k, s0 + k], so a candidate
 // names 2k + 1 starts, and each gets its distance d(s) from one banded DP (DESIGN.md §1d).
-#include <cub/device/device_segmented_sort.cuh>
-#include <thrust/iterator/counting_iterator.h>
-#include <thrust/iterator/transform_iterator.h>
-
 #include "kernels_common.cuh"
 
 namespace awry {
@@ -29,8 +25,7 @@ __device__ __forceinline__ bool piece_at(const IndexView& ix, const uint32_t* rq
 // in [-k, k] never leaves them.  Row L, diagonal δ is d(s0 - δ).  Cells hold min(distance, k + 1).
 // Start s (d(s) <= k) is reported by its OWNER only: the smallest (j', p') over exact occurrences of piece j' at
 // p' with |p' - a_j' - s| <= k -- such an occurrence exists and is a candidate whose range contains s, so every
-// start comes out once.  Count: counts[q (k+1) + d] += 1.  Locate: keys[(2k+1) i + k + δ] = (s << 2) | d, or ~0,
-// and acc[q - q0] += the candidate's accepted starts.  Place: the candidate takes popc(acc) consecutive slots
+// start comes out once.  Count: counts[q (k+1) + d] += 1.  Place: the candidate takes popc(acc) consecutive slots
 // keys[hit_off[q] + acc[q] ..] (acc[q] += popc) and writes its accepted starts' keys there.
 template <int K, int MODE>
 __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingSlice a) {
@@ -132,13 +127,7 @@ __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingS
         acc &= ~smaller;
       }
     }
-    if (MODE == VERIFY_LOCATE) {
-      uint64_t* const keys = a.keys + uint64_t(2 * K + 1) * i;
-#pragma unroll
-      for (int t = 0; t <= 2 * K; t++)
-        keys[t] = (acc >> t) & 1u ? (uint64_t(s0 - (t - K)) << 2) | dist[t] : ~0ull;
-      if (acc) atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + (q - a.q0), (unsigned long long)__popc(acc));
-    } else if (MODE == VERIFY_PLACE) {
+    if (MODE == VERIFY_PLACE) {
       if (acc) {
         uint64_t at = a.hit_off[q] + atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + q,
                                                (unsigned long long)__popc(acc));
@@ -158,9 +147,7 @@ __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingS
 template <int K>
 static void launch_edit_verify_k(const IndexView& ix, const HammingSlice& a, VerifyMode mode, unsigned grid,
                                  cudaStream_t s) {
-  if (mode == VERIFY_LOCATE)
-    edit_verify_kernel<K, VERIFY_LOCATE><<<grid, 256, 0, s>>>(ix, a);
-  else if (mode == VERIFY_PLACE)
+  if (mode == VERIFY_PLACE)
     edit_verify_kernel<K, VERIFY_PLACE><<<grid, 256, 0, s>>>(ix, a);
   else
     edit_verify_kernel<K, VERIFY_COUNT><<<grid, 256, 0, s>>>(ix, a);
@@ -181,65 +168,20 @@ cudaError_t launch_edit_verify(const IndexView& ix, const HammingSlice& a, uint3
   return cudaGetLastError();
 }
 
-// locate: the key slots of a slice sorted per read, as sort_hamming_keys, with `slots` keys per candidate
-struct SlotBound {
-  const uint64_t* qcand;
-  uint64_t c0, slots;
-  __host__ __device__ long long operator()(uint64_t i) const { return (long long)((qcand[i] - c0) * slots); }
-};
-cudaError_t sort_edit_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg, const uint64_t* d_qcand,
-                           uint64_t c0, uint32_t slots, void* d_temp, size_t& temp_bytes, cudaStream_t s) {
-  if (n >= (1ull << 31)) return cudaErrorInvalidValue;
-  thrust::counting_iterator<uint64_t> idx(0);
-  auto begin = thrust::make_transform_iterator(idx, SlotBound{d_qcand, c0, slots});
-  cudaError_t e = cub::DeviceSegmentedSort::SortKeys(d_temp, temp_bytes, d_keys, d_sorted, (long long)n, (long long)nseg,
-                                                     begin, begin + 1, s);
-  if (d_temp != nullptr) COUNT_LAUNCH();
-  return e;
-}
-
-// sorted key slots -> text positions and distances at the read's CSR slot (hamming_compact_kernel with `slots` keys
-// per candidate: slot i belongs to candidate c0 + i / slots)
-__global__ void edit_compact_kernel(const uint64_t* __restrict__ sorted, const uint32_t* __restrict__ map, uint64_t n,
-                                    uint32_t pieces, uint32_t slots, const uint64_t* __restrict__ qcand, uint64_t c0,
-                                    uint64_t q0, const uint64_t* __restrict__ qh, uint64_t* __restrict__ pos,
-                                    uint8_t* __restrict__ dist) {
-  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
-  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
-    const uint64_t key = sorted[i];
-    if (key == ~0ull) continue;
-    const uint64_t q = map[i / slots] / pieces;
-    const uint64_t o = qh[q - q0] + (i - (qcand[q] - c0) * slots);
-    pos[o] = key >> 2;
-    dist[o] = uint8_t(key & 3);
-  }
-}
-
-cudaError_t launch_edit_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
-                                const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
-                                uint8_t* d_dist, cudaStream_t s) {
-  if (n == 0) return cudaSuccess;
-  const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
-  edit_compact_kernel<<<grid, 256, 0, s>>>(d_sorted, d_map, n, k + 1, 2 * k + 1, d_qcand, c0, q0, d_qh, d_pos, d_dist);
-  COUNT_LAUNCH();
-  return cudaGetLastError();
-}
-
 // ---- loci (awry_*_edit_loci, DESIGN.md §1g): one thread per hit of hits sorted per query (ascending, distinct starts).
 // Hit i of query q = map[i] (range off[q] .. off[q + 1]) is a locus unless (a) a hit within k of it has a smaller
 // distance, or (b) its distance is >= 1 and the start just before it is a hit at the same distance.  Positions are
-// distinct, so the hits within k of i are among its k neighbours on each side.  Hit i: key pos[i] = (s << 2) | d when
-// dist is null, else s = pos[i], d = dist[i].  Count: counts[q (k+1) + d] += 1 per locus.  Otherwise keep[i] = 1 for a
-// locus, else 0, and keep[n] = 0.
-__device__ __forceinline__ void loci_hit(const uint64_t* pos, const uint8_t* dist, uint64_t i, uint64_t& s, uint32_t& d) {
-  const uint64_t x = pos[i];
-  s = dist ? x : x >> 2;
-  d = dist ? dist[i] : uint32_t(x & 3);
+// distinct, so the hits within k of i are among its k neighbours on each side.  Hit i is the key keys[i] = (s << 2) | d.
+// Count: counts[q (k+1) + d] += 1 per locus.  Otherwise keep[i] = 1 for a locus, else 0, and keep[n] = 0.
+__device__ __forceinline__ void loci_hit(const uint64_t* keys, uint64_t i, uint64_t& s, uint32_t& d) {
+  const uint64_t x = keys[i];
+  s = x >> 2;
+  d = uint32_t(x & 3);
 }
 
-__global__ void edit_loci_kernel(const uint64_t* __restrict__ pos, const uint8_t* __restrict__ dist,
-                                 const uint64_t* __restrict__ off, const uint32_t* __restrict__ map, uint64_t n,
-                                 uint32_t k, uint64_t* __restrict__ keep, uint64_t* __restrict__ counts) {
+__global__ void edit_loci_kernel(const uint64_t* __restrict__ keys, const uint64_t* __restrict__ off,
+                                 const uint32_t* __restrict__ map, uint64_t n, uint32_t k, uint64_t* __restrict__ keep,
+                                 uint64_t* __restrict__ counts) {
   const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
   for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
     const uint32_t q = map[i];
@@ -247,16 +189,16 @@ __global__ void edit_loci_kernel(const uint64_t* __restrict__ pos, const uint8_t
     AWRY_CHK(lo <= i && i < hi);
     uint64_t s, t;
     uint32_t d, e;
-    loci_hit(pos, dist, i, s, d);
+    loci_hit(keys, i, s, d);
     bool locus = true;
     for (uint32_t j = 1; j <= k && i - lo >= j && locus; j++) {
-      loci_hit(pos, dist, i - j, t, e);
+      loci_hit(keys, i - j, t, e);
       AWRY_CHK(t < s);
       if (s - t > k) break;
       locus = e > d || (e == d && (d == 0 || t + 1 != s));
     }
     for (uint32_t j = 1; j <= k && i + j < hi && locus; j++) {
-      loci_hit(pos, dist, i + j, t, e);
+      loci_hit(keys, i + j, t, e);
       AWRY_CHK(t > s);
       if (t - s > k) break;
       locus = e >= d;
@@ -270,11 +212,11 @@ __global__ void edit_loci_kernel(const uint64_t* __restrict__ pos, const uint8_t
   }
 }
 
-cudaError_t launch_edit_loci(const uint64_t* d_pos, const uint8_t* d_dist, const uint64_t* d_off, const uint32_t* d_map,
-                             uint64_t n, uint32_t k, uint64_t* d_keep, uint64_t* d_counts, cudaStream_t s) {
+cudaError_t launch_edit_loci(const uint64_t* d_keys, const uint64_t* d_off, const uint32_t* d_map, uint64_t n, uint32_t k,
+                             uint64_t* d_keep, uint64_t* d_counts, cudaStream_t s) {
   if (n == 0) return cudaSuccess;
   const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
-  edit_loci_kernel<<<grid, 256, 0, s>>>(d_pos, d_dist, d_off, d_map, n, k, d_keep, d_counts);
+  edit_loci_kernel<<<grid, 256, 0, s>>>(d_keys, d_off, d_map, n, k, d_keep, d_counts);
   COUNT_LAUNCH();
   return cudaGetLastError();
 }
@@ -292,24 +234,22 @@ cudaError_t launch_edit_loci_offsets(const uint64_t* d_P, uint64_t* d_off, uint6
   return cudaGetLastError();
 }
 
-// hit i is a locus iff P[i + 1] > P[i]; it goes to slot P[i] of pos_out (and dist_out when dist is not null)
-__global__ void edit_loci_compact_kernel(const uint64_t* __restrict__ P, uint64_t n, const uint64_t* __restrict__ pos,
-                                         const uint8_t* __restrict__ dist, uint64_t* __restrict__ pos_out,
-                                         uint8_t* __restrict__ dist_out) {
+// hit i is a locus iff P[i + 1] > P[i]; its key goes to slot P[i] of keys_out
+__global__ void edit_loci_compact_kernel(const uint64_t* __restrict__ P, uint64_t n, const uint64_t* __restrict__ keys,
+                                         uint64_t* __restrict__ keys_out) {
   const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
   for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
     const uint64_t o = P[i];
     if (P[i + 1] == o) continue;
-    pos_out[o] = pos[i];
-    if (dist) dist_out[o] = dist[i];
+    keys_out[o] = keys[i];
   }
 }
 
-cudaError_t launch_edit_loci_compact(const uint64_t* d_P, uint64_t n, const uint64_t* d_pos, const uint8_t* d_dist,
-                                     uint64_t* d_pos_out, uint8_t* d_dist_out, cudaStream_t s) {
+cudaError_t launch_edit_loci_compact(const uint64_t* d_P, uint64_t n, const uint64_t* d_keys, uint64_t* d_keys_out,
+                                     cudaStream_t s) {
   if (n == 0) return cudaSuccess;
   const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
-  edit_loci_compact_kernel<<<grid, 256, 0, s>>>(d_P, n, d_pos, d_dist, d_pos_out, d_dist_out);
+  edit_loci_compact_kernel<<<grid, 256, 0, s>>>(d_P, n, d_keys, d_keys_out);
   COUNT_LAUNCH();
   return cudaGetLastError();
 }

@@ -83,20 +83,6 @@ cudaError_t launch_hamming_piece_words(const uint64_t* d_qwords, const uint64_t*
   return cudaGetLastError();
 }
 
-// qcand[i] = hoff[(k+1) i], i = 0 .. nq: the candidates of query i are [qcand[i], qcand[i+1])
-__global__ void hamming_query_bounds_kernel(const uint64_t* __restrict__ hoff, uint32_t k, uint64_t nq,
-                                            uint64_t* __restrict__ qcand) {
-  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
-  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i <= nq; i += stride) qcand[i] = hoff[(k + 1) * i];
-}
-
-cudaError_t launch_hamming_query_bounds(const uint64_t* d_hoff, uint32_t k, uint64_t nq, uint64_t* d_qcand, cudaStream_t s) {
-  const unsigned grid = unsigned(std::min<uint64_t>((nq + 256) / 256, 148 * 16));
-  hamming_query_bounds_kernel<<<grid, 256, 0, s>>>(d_hoff, k, nq, d_qcand);
-  COUNT_LAUNCH();
-  return cudaGetLastError();
-}
-
 // candidate -> piece map of the slice [c0, c0 + n): piece g is written where its candidates start (and at 0 when
 // they began before the slice), then an inclusive max-scan carries it over the rest.  One thread per piece and one
 // scan, so a piece with 10^4 occurrences costs what 10^4 singletons cost.
@@ -136,9 +122,9 @@ cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_
 // mismatches of each piece against the packed read, and the group adds them up; it stops once the total exceeds k.
 // The window of search-order symbol j is rtext[rb0 + j] with rb0 = bwt_len - s - L (rtext[i] = text[bwt_len - 1 - i],
 // layout.cuh): read and text are two forward streams.  A candidate is accepted iff its distance d <= k and its piece
-// j is the smallest one without a mismatch.  Count: counts[q (k+1) + d] += 1.  Locate: keys[i] = (s << 2) | d, or ~0
-// (rejected), and acc[q - q0] += 1.  Place: (s << 2) | d goes to keys[hit_off[q] + acc[q]++] (one slot of the range
-// the count pass gave q; the order within it is settled by the sort that follows).
+// j is the smallest one without a mismatch.  Count: counts[q (k+1) + d] += 1.  Place: (s << 2) | d goes to
+// keys[hit_off[q] + acc[q]++] (one slot of the range the count pass gave q; the order within it is settled by the
+// sort that follows).
 template <int K, int MODE>
 __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, HammingSlice a) {
   constexpr uint32_t FULL = 0xffffffffu;
@@ -212,10 +198,7 @@ __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, Hammi
     const uint32_t before = ((1u << P) - 1u) & ~((1u << (P - j)) - 1u);
     const bool accept = live && tot <= uint32_t(K) && (hit_pieces & before) == before;
     if (sub == 0 && i < a.n) {
-      if (MODE == VERIFY_LOCATE) {
-        a.keys[i] = accept ? (s << 2) | tot : ~0ull;
-        if (accept) atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + (q - a.q0), 1ull);
-      } else if (MODE == VERIFY_PLACE) {
+      if (MODE == VERIFY_PLACE) {
         if (accept) {
           const uint64_t at = a.hit_off[q] + atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + q, 1ull);
           AWRY_CHK(at < a.hit_off[q + 1]);
@@ -230,9 +213,7 @@ __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, Hammi
 
 template <int K>
 static void launch_verify_k(const IndexView& ix, const HammingSlice& a, VerifyMode mode, unsigned grid, cudaStream_t s) {
-  if (mode == VERIFY_LOCATE)
-    hamming_verify_kernel<K, VERIFY_LOCATE><<<grid, 256, 0, s>>>(ix, a);
-  else if (mode == VERIFY_PLACE)
+  if (mode == VERIFY_PLACE)
     hamming_verify_kernel<K, VERIFY_PLACE><<<grid, 256, 0, s>>>(ix, a);
   else
     hamming_verify_kernel<K, VERIFY_COUNT><<<grid, 256, 0, s>>>(ix, a);
@@ -253,26 +234,26 @@ cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, ui
   return cudaGetLastError();
 }
 
-// locate: keys of the slice sorted per query (rejected keys, ~0, go to the end of their segment).  The segment
-// bounds are the reads' candidate bounds made slice-local (qcand[i] - c0): CUB's segmented sort reads its offsets as
-// int, so the slice holds fewer than 2^31 candidates and its bounds must not be the absolute ones.
-struct SliceBound {
-  const uint64_t* qcand;
-  uint64_t c0;
-  __host__ __device__ long long operator()(uint64_t i) const { return (long long)(qcand[i] - c0); }
+// keys sorted per query.  The segment bounds are the CSR offsets made local to the part sorted (off[i] - base): CUB's
+// segmented sort reads its offsets as int, so a part holds fewer than 2^31 keys and its bounds must not be the
+// absolute ones.
+struct PartBound {
+  const uint64_t* off;
+  uint64_t base;
+  __host__ __device__ long long operator()(uint64_t i) const { return (long long)(off[i] - base); }
 };
 cudaError_t sort_hamming_keys(const uint64_t* d_keys, uint64_t* d_sorted, uint64_t n, uint64_t nseg,
-                              const uint64_t* d_qcand, uint64_t c0, void* d_temp, size_t& temp_bytes, cudaStream_t s) {
+                              const uint64_t* d_off, uint64_t base, void* d_temp, size_t& temp_bytes, cudaStream_t s) {
   if (n >= (1ull << 31)) return cudaErrorInvalidValue;
   thrust::counting_iterator<uint64_t> idx(0);
-  auto begin = thrust::make_transform_iterator(idx, SliceBound{d_qcand, c0});
+  auto begin = thrust::make_transform_iterator(idx, PartBound{d_off, base});
   cudaError_t e = cub::DeviceSegmentedSort::SortKeys(d_temp, temp_bytes, d_keys, d_sorted, (long long)n, (long long)nseg,
                                                      begin, begin + 1, s);
   if (d_temp != nullptr) COUNT_LAUNCH();
   return e;
 }
 
-// exclusive sum of n u64 (the per-query accepted counts -> the slice's CSR offsets)
+// exclusive sum of n u64 (counts or keep flags -> their offsets)
 cudaError_t scan_u64(const uint64_t* d_in, uint64_t* d_out, uint64_t n, void* d_temp, size_t& temp_bytes, cudaStream_t s) {
   cudaError_t e = cub::DeviceScan::ExclusiveSum(d_temp, temp_bytes, d_in, d_out, (long long)n, s);
   if (d_temp != nullptr) COUNT_LAUNCH();
@@ -310,31 +291,6 @@ cudaError_t launch_hamming_decode(uint64_t* d_keys, uint64_t n, uint8_t* d_dist,
   if (n == 0) return cudaSuccess;
   const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
   hamming_decode_kernel<<<grid, 256, 0, s>>>(d_keys, n, d_dist);
-  COUNT_LAUNCH();
-  return cudaGetLastError();
-}
-
-// sorted keys -> text positions and distances at the query's CSR slot: the accepted keys lead their segment
-__global__ void hamming_compact_kernel(const uint64_t* __restrict__ sorted, const uint32_t* __restrict__ map, uint64_t n,
-                                       uint32_t pieces, const uint64_t* __restrict__ qcand, uint64_t c0, uint64_t q0,
-                                       const uint64_t* __restrict__ qh, uint64_t* __restrict__ pos, uint8_t* __restrict__ dist) {
-  const uint64_t stride = gridDim.x * uint64_t(blockDim.x);
-  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
-    const uint64_t key = sorted[i];
-    if (key == ~0ull) continue;
-    const uint64_t q = map[i] / pieces;
-    const uint64_t o = qh[q - q0] + (c0 + i - qcand[q]);
-    pos[o] = key >> 2;
-    dist[o] = uint8_t(key & 3);
-  }
-}
-
-cudaError_t launch_hamming_compact(const uint64_t* d_sorted, const uint32_t* d_map, uint64_t n, uint32_t k,
-                                   const uint64_t* d_qcand, uint64_t c0, uint64_t q0, const uint64_t* d_qh, uint64_t* d_pos,
-                                   uint8_t* d_dist, cudaStream_t s) {
-  if (n == 0) return cudaSuccess;
-  const unsigned grid = unsigned(std::min<uint64_t>((n + 255) / 256, 148 * 16));
-  hamming_compact_kernel<<<grid, 256, 0, s>>>(d_sorted, d_map, n, k + 1, d_qcand, c0, q0, d_qh, d_pos, d_dist);
   COUNT_LAUNCH();
   return cudaGetLastError();
 }

@@ -242,7 +242,10 @@ int awry_locate_batch_packed2(const awry_index *index, const uint8_t *crumbs, co
  *             length L <= k (every window would match) -> AWRY_ERR_INVALID_QUERY; a protein index, or one without
  *             the unsampled suffix array and the text on the device (AWRY_B200_FULL_SA=0, AWRY_B200_TEXT=0,
  *             AWRY_B200_PAIR_INDEX=0, a file that samples every suffix array entry (ratio 1), not enough device
- *             memory, 64-bit row pointers) -> AWRY_ERR_UNSUPPORTED.
+ *             memory, 64-bit row pointers) -> AWRY_ERR_UNSUPPORTED.  Locate works through chunks of queries (at most
+ *             512 k queries and 64 MB, as awry_locate_batch) and, as awry_locate_device_hamming, holds a chunk's hits
+ *             on the device: when they do not fit, or one query has 2^31 hits or more -> AWRY_ERR_NOMEM, naming the
+ *             hit total.
  * Scheme (pigeonhole): the query is cut into k+1 pieces, piece j = bytes [a_j, a_{j+1}), a_j = floor(j L / (k+1));
  * each piece is searched exactly, an occurrence of piece j at text position p names the window s = p - a_j, and the
  * window is verified against the text on the device.  It is kept iff its distance is <= k and j is the smallest piece
