@@ -1228,6 +1228,12 @@ struct DeviceHits {
   uint64_t* n_hits;
 };
 
+// the outputs of the map flow of hamming_run (awry_map_*): one record (and alignment) per read, device pointers
+struct DeviceMap {
+  awry_mapping* out;
+  awry_alignment* aln;  // nullptr: not wanted
+};
+
 // The loci of n edit-distance hits sorted per query (DESIGN.md §1g), no synchronisation.  d_off (nq + 1, from 0) is the
 // hits' CSR and d_keys their keys (s << 2 | d).  Count (d_counts, nq (k+1), zeroed): every locus adds 1 at
 // [q (k+1) + d].  Otherwise d_P (n + 1) becomes the exclusive scan of the keep flags and d_off the CSR of the loci;
@@ -1284,11 +1290,85 @@ SearchQueries pack_search_queries(StreamScratch& sc, const uint8_t* d_qbytes, co
 // slots per candidate, 1 or 2k + 1, that a slice counts.
 // `loci` (edit only, awry_*_edit_loci, DESIGN.md §1g): only the loci of each query's sorted hits are kept.  Both
 // count and locate take the locate's flow (a count into a CSR of its own) and filter the sorted keys.
+// `map` (awry_map_*, DESIGN.md §1h; edit: with `loci`): the locate flow with the place pass bounded per read by its
+// best distance + 1 from the count pass, then map_select; no synchronisation after the bounded hit total.
 enum Metric { METRIC_HAMMING = 0, METRIC_EDIT = 1 };
 const char* metric_name(Metric metric) { return metric == METRIC_EDIT ? "edit-distance" : "Hamming"; }
+
+// The map flow's last steps (DESIGN.md §1h), in scratch of `sc`, no synchronisation.  d_keys holds the n keys (s << 2
+// | d) within the bound, sorted per search query (edit: the loci, whose total hit_off[nv] <= n stays on the device);
+// d_spare holds n + 1 free keys.  The keys are re-keyed with their strand, merged per read by a segmented sort (both
+// strands), and flagged; a scan ranks each read's best starts and one thread per read writes its record and the
+// primary's alignment input.  n = 0: no read has a hit.
+void map_select(Replica& r, StreamScratch& sc, const SearchQueries& sq, const uint32_t* d_qlen, const uint64_t* hit_off,
+                uint64_t nq, uint32_t shift, uint32_t k, Metric metric, const uint8_t* d_best, uint64_t* d_keys,
+                uint64_t* d_spare, uint64_t n, const DeviceMap& m, cudaStream_t st) {
+  uint64_t* const roff = sc.get<uint64_t>(nq + 1);
+  uint32_t* const second = sc.get<uint32_t>(nq);
+  uint64_t* const rank = sc.get<uint64_t>(n + 1);
+  CU(launch_map_read_offsets(hit_off, nq, shift, roff, st));
+  CU(cudaMemsetAsync(second, 0, nq * 4, st));
+  const uint64_t* keys = d_spare;
+  uint32_t* rmap = nullptr;
+  size_t temp = 0;
+  if (n) {
+    rmap = sc.get<uint32_t>(n);
+    CU(launch_hamming_map(roff, nq, 0, n, rmap, nullptr, temp, st));
+    CU(launch_hamming_map(roff, nq, 0, n, rmap, sc.get<uint8_t>(temp), temp, st));
+    CU(launch_map_rekey(d_keys, hit_off, roff, rmap, nq, n, shift, d_spare, st));
+    if (shift) {  // the two strands' sorted ranges of a read merged (one strand: already in order)
+      temp = 0;
+      CU(sort_hamming_keys(d_spare, d_keys, n, nq, roff, 0, nullptr, temp, st));
+      CU(sort_hamming_keys(d_spare, d_keys, n, nq, roff, 0, sc.get<uint8_t>(temp), temp, st));
+      keys = d_keys;
+    }
+  }
+  CU(launch_map_flags(keys, roff, rmap, d_best, nq, n, shift, rank, second, st));
+  temp = 0;
+  CU(scan_u64(rank, rank, n + 1, nullptr, temp, st));
+  CU(scan_u64(rank, rank, n + 1, sc.get<uint8_t>(temp), temp, st));
+  MapReads mr{};
+  mr.qwords = sq.words;
+  mr.qw_lo = sq.w_lo;
+  mr.qw_n = sq.w_n;
+  mr.qoff = sq.off;
+  mr.qlen = d_qlen;
+  mr.keys = keys;
+  mr.roff = roff;
+  mr.rank = rank;
+  mr.best = d_best;
+  mr.second = second;
+  mr.nq = nq;
+  mr.k = k;
+  mr.shift = shift;
+  mr.out = reinterpret_cast<uint64_t*>(m.out);
+  if (m.aln) {
+    mr.aln_map = sc.get<uint32_t>(nq);
+    mr.aln_hits = sc.get<uint64_t>(2 * nq);
+    mr.aln_end = sc.get<uint64_t>(1);
+  }
+  CU(launch_map_reads(r.view, mr, st));
+  if (!m.aln) return;
+  AlignSlice a{};
+  a.qwords = sq.words;
+  a.qw_lo = sq.w_lo;
+  a.qw_n = sq.w_n;
+  a.qoff = sq.off;
+  a.qlen = d_qlen;
+  a.nq = nq << shift;
+  a.map = mr.aln_map;
+  a.hits = mr.aln_hits;
+  a.out = reinterpret_cast<uint32_t*>(m.aln);
+  a.n = nq;
+  a.hit_end = mr.aln_end;
+  a.hit_total = nq;
+  ProfScope p(1, r.device, st);
+  CU(launch_align_hits(r.view, a, k, metric == METRIC_EDIT, r.sm_count, st));
+}
 void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq, uint64_t b_lo, uint64_t b_hi,
                  uint32_t k, unsigned long long* d_flag, long long check_base, cudaStream_t st, uint64_t* d_counts,
-                 bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr, bool loci = false) {
+                 bool strands = false, Metric metric = METRIC_HAMMING, DeviceHits* dev = nullptr, bool loci = false,
+                 const DeviceMap* map = nullptr) {
   const bool edit = metric == METRIC_EDIT;
   const char* const what = metric_name(metric);
   const uint32_t shift = strands ? 1 : 0;  // virtual query -> read
@@ -1303,9 +1383,14 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
   uint64_t* const d_poff = sc.get<uint64_t>(np + 1);
   SearchQueries sq;
   uint64_t* d_pw;
+  uint32_t* d_qlen = nullptr;  // map: every search query's length, 0 when refused (launch_align_reads)
   {
     ProfScope p(2, r.device, st);
     sq = pack_search_queries(sc, d_qbytes, d_qoff, nq, b_lo, b_hi, strands, d_flag, st);
+    if (map) {
+      d_qlen = sc.get<uint32_t>(nv);
+      CU(launch_align_reads(sq.words, sq.off, nv, sq.lo, sq.hi, sq.w_lo, sq.w_n, k, shift, d_qlen, d_flag, st));
+    }
     d_pw = sc.get<uint64_t>(packed_words(0, np, sq.hi - sq.lo)) - 4 * (sq.lo >> 6);
     CU(launch_hamming_pieces(sq.off, nv, k, sq.lo, sq.hi, shift, d_poff, d_flag, st));
     if (!strands) {
@@ -1368,21 +1453,32 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       CU(edit ? launch_edit_verify(r.view, a, k, mode, r.sm_count, st) : launch_hamming_verify(r.view, a, k, mode, r.sm_count, st));
     }
   };
-  if (dev || loci) {  // 3. locate (DESIGN.md §1e), and the loci count (§1g)
+  if (dev || loci || map) {  // 3. locate (DESIGN.md §1e), the loci count (§1g), and the map flow (§1h)
     uint64_t* const hit_off = dev ? dev->hit_off : sc.get<uint64_t>(nv + 1);
-    if (!dev) CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
-    // count pass: the CSR over the queries, and the hit total that sizes the outputs (the second synchronisation)
+    if (d_counts) CU(cudaMemsetAsync(d_counts, 0, nv * P * 8, st));
+    // count pass: the CSR over the queries, and the hit total that sizes the outputs (the second synchronisation).
+    // map: only the hits within each read's bound are counted into the CSR.
     a.counts = sc.get<uint64_t>(nv * P);
     CU(cudaMemsetAsync(a.counts, 0, nv * P * 8, st));
     verify_all(VERIFY_COUNT);
     uint64_t* d_sums = sc.get<uint64_t>(nv + 1);
-    CU(launch_hamming_row_sums(a.counts, k, nv, d_sums, st));
+    uint8_t* const d_best = map ? sc.get<uint8_t>(nv) : nullptr;
+    if (map)
+      CU(launch_map_bound(a.counts, d_qlen, nq, k, shift, d_best, d_sums, st));
+    else
+      CU(launch_hamming_row_sums(a.counts, k, nv, d_sums, st));
     CU(scan_u64(d_sums, hit_off, nv + 1, nullptr, temp, st));
     CU(scan_u64(d_sums, hit_off, nv + 1, sc.get<uint8_t>(temp), temp, st));
     uint64_t n = 0;
     CU(cudaMemcpyAsync(&n, hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    if (n == 0) return;
+    if (map && n >= (1ull << 31))
+      fail(AWRY_ERR_NOMEM, "%llu hits within best + 1 in one batch, more than one sort can order (2^31): split it",
+           (unsigned long long)n);
+    if (n == 0) {
+      if (map) map_select(r, sc, sq, d_qlen, hit_off, nq, shift, k, metric, d_best, nullptr, nullptr, 0, *map, st);
+      return;
+    }
     // CUB's segmented sort reads its offsets as int: more than 2^31 - 1 keys are sorted in parts cut at query
     // boundaries, which needs the offsets on the host (the only case that reads them back)
     std::vector<std::pair<uint64_t, uint64_t>> parts{{0, nv}};  // query ranges
@@ -1414,8 +1510,8 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       if (dev->dist) d_dist = out.get<uint8_t>(m);
     };
     try {
-      if (!loci) outputs(n);
-      d_keys = sc.get<uint64_t>(loci ? n + 1 : n);
+      if (!loci && !map) outputs(n);
+      d_keys = sc.get<uint64_t>(loci || map ? n + 1 : n);
       d_sorted = sc.get<uint64_t>(n);
     } catch (const ApiError& x) {
       if (x.code != AWRY_ERR_NOMEM) throw;
@@ -1425,8 +1521,9 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     a.keys = d_keys;
     a.acc = sc.get<uint64_t>(nv);
     a.hit_off = hit_off;
+    a.best = d_best;
     CU(cudaMemsetAsync(a.acc, 0, nv * 8, st));
-    verify_all(VERIFY_PLACE);
+    verify_all(map ? VERIFY_PLACE_BEST : VERIFY_PLACE);
     // order: a query's positions are distinct, so the sorted keys do not depend on the order the atomics gave
     for (const auto& [q0, q1] : parts) {
       const uint64_t b = off.empty() ? 0 : off[q0], m = off.empty() ? n : off[q1] - off[q0];
@@ -1438,8 +1535,14 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
     if (loci) {
       // the filter over the whole batch at once (its scans take 64-bit sizes); d_keys, free after the sort, takes
       // the scan of the keep flags.  The locus total sizes the outputs: the third synchronisation.
-      edit_loci(d_sorted, hit_off, nv, n, k, d_keys, dev ? nullptr : d_counts, st);
-      if (!dev) return;
+      edit_loci(d_sorted, hit_off, nv, n, k, d_keys, d_counts, st);
+      if (d_counts) return;
+      if (map) {  // (the locus total stays on the device: the hit total sizes the compaction)
+        uint64_t* const d_loci = sc.get<uint64_t>(n);
+        CU(launch_edit_loci_compact(d_keys, n, d_sorted, d_loci, st));
+        map_select(r, sc, sq, d_qlen, hit_off, nq, shift, k, metric, d_best, d_loci, d_keys, n, *map, st);
+        return;
+      }
       uint64_t m = 0;
       CU(cudaMemcpyAsync(&m, hit_off + nv, 8, cudaMemcpyDeviceToHost, st));
       CU(cudaStreamSynchronize(st));
@@ -1455,6 +1558,10 @@ void hamming_run(Replica& r, const uint8_t* d_qbytes, const uint64_t* d_qoff, ui
       CU(launch_edit_loci_compact(d_keys, n, d_sorted, d_loci, st));
       d_sorted = d_loci;
       n = m;
+    }
+    if (map) {
+      map_select(r, sc, sq, d_qlen, hit_off, nq, shift, k, metric, d_best, d_sorted, d_keys, n, *map, st);
+      return;
     }
     CU(launch_hamming_decode(d_sorted, n, d_dist, st));
     CU(launch_map_locations(r.view, d_sorted, n, reinterpret_cast<uint64_t*>(d_hits), st));
@@ -1875,6 +1982,85 @@ void align_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbyte
             n_hits, d_out, st);
 }
 
+// ------------------------------------------------------------------ read mapping (awry_map_*)
+
+void map_check_index(const awry_index* ix, uint32_t strands, uint64_t nq) {
+  need(ix);
+  if (strands) strands_check_index(ix);
+  hamming_check_index(ix, "read mapping");
+  if ((nq << strands) >= (1ull << 32) - 1) fail(AWRY_ERR_INVALID_ARG, "batch too large for one mapping call: split it");
+}
+
+// awry_map_batch: reads [lo, hi) of host buffers on replica ri, in chunks of reads; each chunk's records (and
+// alignments) are copied straight into its slice of out (aln)
+void map_on_replica(const awry_index* ix, size_t ri, const uint8_t* qbytes, const uint64_t* qoff, uint64_t lo, uint64_t hi,
+                    Metric metric, bool strands, uint32_t k, awry_mapping* out, awry_alignment* aln) {
+  if (lo >= hi) return;
+  Replica& r = *ix->reps[ri];
+  DeviceGuard dg(r.device);
+  const uint64_t max_bytes = std::min(chunk_max_bytes(), locate_chunk_bytes());
+  if (qoff[hi] < qoff[lo]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone (queries %llu..%llu)",
+                                (unsigned long long)lo, (unsigned long long)hi);
+  auto chunks = make_chunks(qoff, lo, hi, locate_chunk_q(), max_bytes);
+  validate_chunks(chunks, max_bytes);
+  Workspace* ws = r.acquire();
+  try {
+    for (const Chunk& c : chunks) {
+      const uint64_t n = c.q1 - c.q0, nbytes = c.b1 - c.b0;
+      StreamScratch sc(ws->st);
+      Workspace::grow_dev(ws->d_qbytes, ws->d_qbytes_cap, size_t(nbytes) + 16);
+      Workspace::grow_dev(ws->d_qoff, ws->d_qoff_cap, size_t(n) + 1);
+      if (nbytes) CU(cudaMemcpyAsync(ws->d_qbytes, qbytes + c.b0, nbytes, cudaMemcpyHostToDevice, ws->st));
+      CU(cudaMemcpyAsync(ws->d_qoff, qoff + c.q0, (n + 1) * 8, cudaMemcpyHostToDevice, ws->st));
+      g_prof.h2d += nbytes + (n + 1) * 8;
+      CU(cudaMemsetAsync(ws->d_flag, 0xff, 8, ws->st));
+      const DeviceMap dm{sc.get<awry_mapping>(n), aln ? sc.get<awry_alignment>(n) : nullptr};
+      hamming_run(r, ws->d_qbytes - c.b0, ws->d_qoff, n, c.b0, c.b1, k, ws->d_flag, (long long)c.q0, ws->st, nullptr,
+                  strands, metric, nullptr, metric == METRIC_EDIT, &dm);
+      CU(cudaMemcpyAsync(out + c.q0, dm.out, n * sizeof(awry_mapping), cudaMemcpyDeviceToHost, ws->st));
+      if (aln) CU(cudaMemcpyAsync(aln + c.q0, dm.aln, n * sizeof(awry_alignment), cudaMemcpyDeviceToHost, ws->st));
+      g_prof.d2h += n * (sizeof(awry_mapping) + (aln ? sizeof(awry_alignment) : 0));
+      CU(cudaStreamSynchronize(ws->st));
+    }
+  } catch (...) {
+    cudaStreamSynchronize(ws->st);
+    r.release(ws);
+    throw;
+  }
+  r.release(ws);
+}
+
+void map_batch_impl(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t metric,
+                    uint32_t strands, uint32_t k, awry_mapping* out, awry_alignment* aln) {
+  align_check_args(metric, strands, k);
+  map_check_index(ix, strands, nq);
+  if (nq == 0) return;
+  if (!qbytes || !qoff || !out) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  if (qoff[nq] < qoff[0]) fail(AWRY_ERR_INVALID_ARG, "query offsets are not monotone");
+  for_each_replica_range(ix, qoff, nq, [&](size_t ri, uint64_t lo, uint64_t hi) {
+    map_on_replica(ix, ri, qbytes, qoff, lo, hi, Metric(metric), strands != 0, k, out, aln);
+  });
+}
+
+void map_device_impl(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                     uint32_t metric, uint32_t strands, uint32_t k, awry_mapping* d_out, awry_alignment* d_aln,
+                     void* cuda_stream) {
+  align_check_args(metric, strands, k);
+  if (nq && (!d_qbytes || !d_qoff || !d_out)) fail(AWRY_ERR_INVALID_ARG, "null argument");
+  map_check_index(ix, strands, nq);
+  if (replica < 0 || size_t(replica) >= ix->reps.size()) fail(AWRY_ERR_INVALID_ARG, "replica out of range");
+  if (nq == 0) return;
+  if (strands) strands_check_device_batch(nq);
+  Replica& r = *ix->reps[size_t(replica)];
+  DeviceGuard dg(r.device);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  uint64_t e[2] = {0, 0};
+  device_batch_ends(d_qoff, nq, st, e, strands != 0);
+  const DeviceMap dm{d_out, d_aln};
+  hamming_run(r, d_qbytes, d_qoff, nq, e[0], e[1], k, r.d_async_flag, -1, st, nullptr, strands != 0, Metric(metric),
+              nullptr, metric == METRIC_EDIT, &dm);
+}
+
 // awry_alignment_cigar: run-length encoded op letters; '=' runs fill the query between the ops
 void alignment_cigar_impl(const awry_alignment* a, uint32_t query_len, char* buf, size_t cap, size_t* needed) {
   if (!a || (!buf && cap)) fail(AWRY_ERR_INVALID_ARG, "null argument");
@@ -2168,6 +2354,17 @@ int awry_align_device(const awry_index* ix, int replica, const uint8_t* d_qbytes
 
 int awry_alignment_cigar(const awry_alignment* a, uint32_t query_len, char* buf, size_t cap, size_t* needed) {
   return guarded([&] { alignment_cigar_impl(a, query_len, buf, cap, needed); });
+}
+
+int awry_map_batch(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq, uint32_t metric,
+                   uint32_t strands, uint32_t k, awry_mapping* out, awry_alignment* aln) {
+  return guarded([&] { map_batch_impl(ix, qbytes, qoff, nq, metric, strands, k, out, aln); });
+}
+
+int awry_map_device(const awry_index* ix, int replica, const uint8_t* d_qbytes, const uint64_t* d_qoff, uint64_t nq,
+                    uint32_t metric, uint32_t strands, uint32_t k, awry_mapping* d_out, awry_alignment* d_aln,
+                    void* cuda_stream) {
+  return guarded([&] { map_device_impl(ix, replica, d_qbytes, d_qoff, nq, metric, strands, k, d_out, d_aln, cuda_stream); });
 }
 
 int awry_count_batch_strands(const awry_index* ix, const uint8_t* qbytes, const uint64_t* qoff, uint64_t nq,

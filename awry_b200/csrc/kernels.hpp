@@ -194,8 +194,10 @@ cudaError_t launch_hamming_piece_words(const uint64_t* d_qwords, const uint64_t*
 cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_t c0, uint64_t n, uint32_t* d_map,
                                void* d_temp, size_t& temp_bytes, cudaStream_t s);
 // what the verification kernels do with an accepted candidate: COUNT adds it to counts, PLACE writes its key into
-// its query's range of a CSR computed by a COUNT pass over the same candidates (locate, DESIGN.md §1e)
-enum VerifyMode { VERIFY_COUNT = 0, VERIFY_PLACE = 1 };
+// its query's range of a CSR computed by a COUNT pass over the same candidates (locate, DESIGN.md §1e).  PLACE_BEST
+// (read mapping, DESIGN.md §1h) places only the keys within the bound of HammingSlice::best, into a CSR counted under
+// the same bound.
+enum VerifyMode { VERIFY_COUNT = 0, VERIFY_PLACE = 1, VERIFY_PLACE_BEST = 2 };
 // one slice of candidates for the verification kernel
 struct HammingSlice {
   const uint64_t* qwords;       // packed reads, biased as for launch_search: read q at word 4 (q + (qoff[q] >> 6))
@@ -213,6 +215,8 @@ struct HammingSlice {
   };
   uint64_t* keys;               // place: the keys (s << 2 | d) of the batch
   uint64_t* acc;                // place: keys placed so far per read of the batch (the cursor), zeroed by the caller
+  const uint8_t* best;          // place-best: per query, the best distance of its read (0xff: none, nothing placed);
+                                // a key at distance d is placed iff d <= min(best + 1, k)
 };
 cudaError_t launch_hamming_verify(const IndexView& ix, const HammingSlice& a, uint32_t k, VerifyMode mode, int sm_count,
                                   cudaStream_t s);
@@ -263,6 +267,47 @@ struct AlignSlice {
   uint64_t hit_total;
 };
 cudaError_t launch_align_hits(const IndexView& ix, const AlignSlice& a, uint32_t k, bool edit, int sm_count, cudaStream_t s);
+
+// ---- kernels_map.cu: read mapping, the best locus per read (awry_map_*, DESIGN.md §1h).  Read q stands for the
+// search queries v = q << shift .. (q << shift) + (1 << shift) - 1 (shift 1: both strands, v = 2q + 1 is rc(q)).
+// From the count pass (d_counts, nv (k+1)): d_best[v] = the smallest d with a hit over all of q's queries, for each
+// of them, 0xff when there is none or d_qlen[q << shift] == 0 (refused: nothing of it is placed); d_sums[v] = v's hits
+// at d <= min(best + 1, k), d_sums[nv] = 0 (its exclusive scan is the CSR of the bounded place pass)
+cudaError_t launch_map_bound(const uint64_t* d_counts, const uint32_t* d_qlen, uint64_t nq, uint32_t k, uint32_t shift,
+                             uint8_t* d_best, uint64_t* d_sums, cudaStream_t s);
+// d_roff[q] = d_hit_off[q << shift], q = 0 .. nq: the hits' CSR over the reads
+cudaError_t launch_map_read_offsets(const uint64_t* d_hit_off, uint64_t nq, uint32_t shift, uint64_t* d_roff,
+                                    cudaStream_t s);
+// the hits' keys (s << 2 | d) -> (s << 3) | (d << 1) | strand, strand = whether the hit lies in the range of v = 2q + 1.
+// d_rmap: the read of every hit (launch_hamming_map over d_roff); n bounds the hits, whose total is d_roff[nq]
+cudaError_t launch_map_rekey(const uint64_t* d_keys, const uint64_t* d_hit_off, const uint64_t* d_roff,
+                             const uint32_t* d_rmap, uint64_t nq, uint64_t n, uint32_t shift, uint64_t* d_out,
+                             cudaStream_t s);
+// over the re-keyed hits sorted per read: the first entry of each start represents it (smallest distance, then strand
+// 0).  d_flag[i] (n + 1 entries, 0 past the total) = 1 for a representative at the read's best distance;
+// d_second[q] (zeroed) += 1 for one at best + 1
+cudaError_t launch_map_flags(const uint64_t* d_keys, const uint64_t* d_roff, const uint32_t* d_rmap, const uint8_t* d_best,
+                             uint64_t nq, uint64_t n, uint32_t shift, uint64_t* d_flag, uint32_t* d_second,
+                             cudaStream_t s);
+// one read per thread: its awry_mapping record, and the inputs of launch_align_hits for its primary
+struct MapReads {
+  const uint64_t* qwords;  // packed search queries, biased as for launch_search (the read itself at v = q << shift)
+  uint64_t qw_lo, qw_n;    // the words that exist: [qw_lo, qw_lo + qw_n) (checked build)
+  const uint64_t* qoff;    // their offsets (nv + 1)
+  const uint32_t* qlen;    // launch_align_reads (0: refused)
+  const uint64_t* keys;    // re-keyed hits sorted per read
+  const uint64_t* roff;    // nq + 1
+  const uint64_t* rank;    // exclusive scan of launch_map_flags' flags
+  const uint8_t* best;     // launch_map_bound
+  const uint32_t* second;  // launch_map_flags
+  uint64_t nq;
+  uint32_t k, shift;
+  uint64_t* out;           // 4 u64 per read (awry_mapping)
+  uint32_t* aln_map;       // nullptr, or per read its primary's search query (for launch_align_hits)
+  uint64_t* aln_hits;      // per read its primary (seq_idx, local_pos), ~0 when unmapped
+  uint64_t* aln_end;       // [0] = nq (the AlignSlice hit total)
+};
+cudaError_t launch_map_reads(const IndexView& ix, const MapReads& m, cudaStream_t s);
 
 cudaError_t launch_single_update(const IndexView& ix, uint64_t sp, uint64_t ep, uint32_t dsym,
                                  uint64_t* d_out2, cudaStream_t s);

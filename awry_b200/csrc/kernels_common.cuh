@@ -263,5 +263,26 @@ __device__ __forceinline__ AminoSlice amino_slice(const u32x8& x, uint32_t sub, 
   return r;
 }
 
+// get_seq_location, intended semantics (sequence_index.rs:108-141; SURVEY.md Q4)
+__device__ __forceinline__ void map_location(const IndexView& ix, uint64_t loc, uint64_t* out2) {
+  uint32_t lo = 0;
+  if (ix.n_seqs > 1) {
+    uint32_t hi = ix.n_seqs - 1;
+    while (lo < hi) {
+      uint32_t mid = (lo + hi + 1) >> 1;
+      if (__ldg(ix.seq_starts + mid) <= loc)
+        lo = mid;
+      else
+        hi = mid - 1;
+    }
+  }
+  AWRY_CHK(lo < ix.n_seqs && loc >= __ldg(ix.seq_starts + lo));
+  out2[0] = lo;
+  out2[1] = loc - __ldg(ix.seq_starts + lo);
+}
+
+// VERIFY_PLACE_BEST (read mapping, DESIGN.md §1h): a hit at distance d of a read whose best distance is b (0xff: none)
+// is placed iff d <= min(b + 1, k)
+__device__ __forceinline__ bool within_map_bound(uint32_t d, uint32_t b, uint32_t k) { return b != 0xffu && d <= min(b + 1u, k); }
 
 }  // namespace awry

@@ -26,7 +26,8 @@ __device__ __forceinline__ bool piece_at(const IndexView& ix, const uint32_t* rq
 // Start s (d(s) <= k) is reported by its OWNER only: the smallest (j', p') over exact occurrences of piece j' at
 // p' with |p' - a_j' - s| <= k -- such an occurrence exists and is a candidate whose range contains s, so every
 // start comes out once.  Count: counts[q (k+1) + d] += 1.  Place: the candidate takes popc(acc) consecutive slots
-// keys[hit_off[q] + acc[q] ..] (acc[q] += popc) and writes its accepted starts' keys there.
+// keys[hit_off[q] + acc[q] ..] (acc[q] += popc) and writes its accepted starts' keys there.  Place-best: the same for
+// the accepted starts within the bound of a.best[q].
 template <int K, int MODE>
 __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingSlice a) {
   constexpr int P = K + 1, W = 4 * K + 1, B = 2 * K;  // pieces, band width, diagonal offset of δ = 0
@@ -126,8 +127,14 @@ __global__ void __launch_bounds__(256) edit_verify_kernel(IndexView ix, HammingS
         }
         acc &= ~smaller;
       }
+      if (MODE == VERIFY_PLACE_BEST && acc) {
+        const uint8_t b = a.best[q];
+#pragma unroll
+        for (int t = 0; t <= 2 * K; t++)
+          if (!within_map_bound(dist[t], b, K)) acc &= ~(1u << t);
+      }
     }
-    if (MODE == VERIFY_PLACE) {
+    if (MODE != VERIFY_COUNT) {
       if (acc) {
         uint64_t at = a.hit_off[q] + atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + q,
                                                (unsigned long long)__popc(acc));
@@ -149,6 +156,8 @@ static void launch_edit_verify_k(const IndexView& ix, const HammingSlice& a, Ver
                                  cudaStream_t s) {
   if (mode == VERIFY_PLACE)
     edit_verify_kernel<K, VERIFY_PLACE><<<grid, 256, 0, s>>>(ix, a);
+  else if (mode == VERIFY_PLACE_BEST)
+    edit_verify_kernel<K, VERIFY_PLACE_BEST><<<grid, 256, 0, s>>>(ix, a);
   else
     edit_verify_kernel<K, VERIFY_COUNT><<<grid, 256, 0, s>>>(ix, a);
 }

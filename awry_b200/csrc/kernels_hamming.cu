@@ -124,7 +124,7 @@ cudaError_t launch_hamming_map(const uint64_t* d_hoff, uint64_t npieces, uint64_
 // layout.cuh): read and text are two forward streams.  A candidate is accepted iff its distance d <= k and its piece
 // j is the smallest one without a mismatch.  Count: counts[q (k+1) + d] += 1.  Place: (s << 2) | d goes to
 // keys[hit_off[q] + acc[q]++] (one slot of the range the count pass gave q; the order within it is settled by the
-// sort that follows).
+// sort that follows).  Place-best: the same for the keys within the bound of a.best[q].
 template <int K, int MODE>
 __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, HammingSlice a) {
   constexpr uint32_t FULL = 0xffffffffu;
@@ -198,8 +198,8 @@ __global__ void __launch_bounds__(256) hamming_verify_kernel(IndexView ix, Hammi
     const uint32_t before = ((1u << P) - 1u) & ~((1u << (P - j)) - 1u);
     const bool accept = live && tot <= uint32_t(K) && (hit_pieces & before) == before;
     if (sub == 0 && i < a.n) {
-      if (MODE == VERIFY_PLACE) {
-        if (accept) {
+      if (MODE != VERIFY_COUNT) {
+        if (accept && (MODE == VERIFY_PLACE || within_map_bound(tot, a.best[q], K))) {
           const uint64_t at = a.hit_off[q] + atomicAdd(reinterpret_cast<unsigned long long*>(a.acc) + q, 1ull);
           AWRY_CHK(at < a.hit_off[q + 1]);
           a.keys[at] = (s << 2) | tot;
@@ -215,6 +215,8 @@ template <int K>
 static void launch_verify_k(const IndexView& ix, const HammingSlice& a, VerifyMode mode, unsigned grid, cudaStream_t s) {
   if (mode == VERIFY_PLACE)
     hamming_verify_kernel<K, VERIFY_PLACE><<<grid, 256, 0, s>>>(ix, a);
+  else if (mode == VERIFY_PLACE_BEST)
+    hamming_verify_kernel<K, VERIFY_PLACE_BEST><<<grid, 256, 0, s>>>(ix, a);
   else
     hamming_verify_kernel<K, VERIFY_COUNT><<<grid, 256, 0, s>>>(ix, a);
 }

@@ -34,24 +34,6 @@ cudaError_t scan_hit_offsets(const IndexView& ix, const void* d_sp_cnt, uint64_t
   return e;
 }
 
-// get_seq_location, intended semantics (sequence_index.rs:108-141; SURVEY.md Q4)
-__device__ __forceinline__ void map_location(const IndexView& ix, uint64_t loc, uint64_t* out2) {
-  uint32_t lo = 0;
-  if (ix.n_seqs > 1) {
-    uint32_t hi = ix.n_seqs - 1;
-    while (lo < hi) {
-      uint32_t mid = (lo + hi + 1) >> 1;
-      if (__ldg(ix.seq_starts + mid) <= loc)
-        lo = mid;
-      else
-        hi = mid - 1;
-    }
-  }
-  AWRY_CHK(lo < ix.n_seqs && loc >= __ldg(ix.seq_starts + lo));
-  out2[0] = lo;
-  out2[1] = loc - __ldg(ix.seq_starts + lo);
-}
-
 // Pass 2a: expand the CSR (query -> hit range) into one BWT row per hit, written into the low
 // 32 bits of each output slot (the walk overwrites the slot with the result).  A lane writes the
 // first 8 rows of its query; longer intervals are written by the whole warp, so a query with 10^5

@@ -135,7 +135,8 @@ EXPORTS = ["awry_read_sequence_file", "awry_index_build", "awry_build_index_file
            "awry_locate_batch_edit_strands", "awry_count_device_edit_strands", "awry_locate_device_hamming",
            "awry_locate_device_hamming_strands", "awry_locate_device_edit", "awry_locate_device_edit_strands",
            "awry_align_batch", "awry_align_device", "awry_alignment_cigar", "awry_count_batch_edit_loci",
-           "awry_locate_batch_edit_loci", "awry_count_device_edit_loci", "awry_locate_device_edit_loci"]
+           "awry_locate_batch_edit_loci", "awry_count_device_edit_loci", "awry_locate_device_edit_loci",
+           "awry_map_batch", "awry_map_device"]
 
 
 def native():
@@ -228,6 +229,8 @@ def native():
     L.awry_align_batch.argtypes = [vp, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, vp]
     L.awry_align_device.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, u64, vp, vp]
     L.awry_alignment_cigar.argtypes = [vp, C.c_uint32, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.awry_map_batch.argtypes = [vp, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp]
+    L.awry_map_device.argtypes = [vp, i32, vp, vp, u64, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, vp]
     _LIB = L
     return L
 
@@ -258,6 +261,12 @@ EDIT_OP_DTYPE = np.dtype([("qpos", "<u4"), ("tpos", "<u4"), ("op", "u1"), ("quer
 ALIGNMENT_DTYPE = np.dtype([("text_len", "<u4"), ("distance", "u1"), ("n_ops", "u1"), ("pad", "u1", (2,)),
                             ("ops", EDIT_OP_DTYPE, (3,))])
 assert ALIGNMENT_DTYPE.itemsize == 44
+
+# awry_mapping (include/awry_b200.h): 32 bytes; seq_idx / local_pos are ~0 when the read is unmapped
+MAP_UNMAPPED, MAP_REFUSED = 1, 2
+MAPPING_DTYPE = np.dtype([("seq_idx", "<u8"), ("local_pos", "<u8"), ("n_best", "<u4"), ("n_second", "<u4"),
+                          ("distance", "u1"), ("strand", "u1"), ("mapq", "u1"), ("flags", "u1"), ("pad", "<u4")])
+assert MAPPING_DTYPE.itemsize == 32
 
 
 def cigar(alignment, query_len: int) -> str:
@@ -789,6 +798,30 @@ class FmIndex:
         bytes (ALIGNMENT_DTYPE) on the device.  Returns without waiting; see device_check"""
         _check(native().awry_align_device(self._h, replica, d_qbytes, d_qoff, nq, _METRICS[metric], int(bool(strands)),
                                           int(max_dist), d_hit_off, d_hits, n_hits, d_out, stream))
+
+    # ---- read mapping: the best locus per read (include/awry_b200.h) -------------------------
+    def map_packed(self, qbytes: np.ndarray, qoff: np.ndarray, metric, max_dist: int, strands: bool = True,
+                   align: bool = True):
+        """-> (MAPPING_DTYPE[nq], ALIGNMENT_DTYPE[nq] or None): each read's best locus under metric "hamming" / "edit"
+        within max_dist, over both strands (strands=True) or the read as given: distance, the number of distinct starts
+        at it and one worse, the primary hit (chosen among the best by a hash of the read), its strand, mapping
+        quality, and (align) its alignment"""
+        qbytes = np.ascontiguousarray(qbytes, dtype=np.uint8)
+        qoff = np.ascontiguousarray(qoff, dtype=np.uint64)
+        nq = len(qoff) - 1
+        out = np.zeros(max(1, nq), dtype=MAPPING_DTYPE)
+        aln = np.zeros(max(1, nq), dtype=ALIGNMENT_DTYPE) if align else None
+        _check(native().awry_map_batch(self._h, qbytes.ctypes.data, qoff.ctypes.data, nq, _METRICS[metric],
+                                       int(bool(strands)), int(max_dist), out.ctypes.data,
+                                       aln.ctypes.data if align else None))
+        return out[:nq], (aln[:nq] if align else None)
+
+    def map_device(self, d_qbytes: int, d_qoff: int, nq: int, metric, max_dist: int, d_out: int, d_aln: int = None,
+                   strands: bool = True, stream: int = 0, replica: int = 0):
+        """map_packed on device pointers: d_out = nq x 32 bytes (MAPPING_DTYPE), d_aln = None or nq x 44 bytes
+        (ALIGNMENT_DTYPE), both on the device.  Returns without waiting; see device_check"""
+        _check(native().awry_map_device(self._h, replica, d_qbytes, d_qoff, nq, _METRICS[metric], int(bool(strands)),
+                                        int(max_dist), d_out, d_aln, stream))
 
     # ---- streaming reads-file front-end (FASTQ / FASTA parsed on the device) ---------------
     def count_reads_file(self, path) -> np.ndarray:

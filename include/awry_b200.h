@@ -521,6 +521,74 @@ int awry_align_device(const awry_index *index, int replica, const uint8_t *d_qby
  * record, n_ops > 3, or ops that are out of order or do not fit L. */
 int awry_alignment_cigar(const awry_alignment *a, uint32_t query_len, char *buf, size_t cap, size_t *needed);
 
+/* ------------------------------------------------------------------ read mapping: the best locus per read
+ * The calls above return every hit within k; a read mapper wants one answer per read: its best locus over the searched
+ * strands, whether that locus is unique, how far the runner-up is, and its alignment.  These calls give that record
+ * for one batch, metric AWRY_METRIC_HAMMING or AWRY_METRIC_EDIT, strands 0 or 1, k <= 3.  Virtual queries (v = q, or
+ * v = 2q for q and v = 2q + 1 for rc(q)), text, n and global starts are as in the blocks above.
+ *   H_v       Hamming: exactly the windows awry_locate_batch_hamming[_strands] returns for v; edit: exactly the loci
+ *             awry_locate_batch_edit_loci(strands) returns for v (mapping by start, with its shifted copies, would
+ *             only inflate the counts).  d_v(s) is the distance of start s in H_v.
+ *   per read  q's virtual queries merged by global start s: D(s) = min of d_v(s) over the v with s in H_v; strand(s) =
+ *             the smaller strand attaining it.  A start found on both strands at one distance (a palindromic window)
+ *             counts once, on strand 0.
+ *   best      best = min D(s); B = {s : D(s) = best} in ascending s.  n_best = |B|; n_second = |{s : D(s) = best + 1}|
+ *             if best < k, else 0 (that stratum was not searched).
+ *   primary   B[h mod n_best], with h a hash of the read's own content: c_i = the code of read byte i as exact search
+ *             maps it (A/a 0, C/c 1, G/g 2, T/t/U/u 3, any other byte 4), taken on the read as given, never on rc(q);
+ *             h0 = FNV-1a-64 over the bytes c_0 .. c_{L-1} (basis 0xcbf29ce484222325, prime 0x100000001b3); h =
+ *             fmix64(h0): x ^= x >> 33; x *= 0xff51afd7ed558ccd; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53; x ^= x >> 33.
+ *             So equal loci (the copies of a repeat) share the reads between them, and the choice depends on the read
+ *             alone: the same for every batch split, chunk size, replica, host or device call.  There is no seed.
+ *   mapq      this project's definition, shaped after the approximate mapping quality of backtracking short-read
+ *             mappers with c1 = n_best, c2 = n_second: 0 if the read is unmapped or n_best >= 2; 25 if best = k
+ *             (uniqueness beyond k is unknown); otherwise AWRY_MAPQ_SECOND[min(n_second, 255)]: 37 for n_second = 0,
+ *             else max(0, 23 - g(n_second)) with g(n) = floor(4.343 ln n + 0.5).
+ *   aln       NULL: not made.  Otherwise, for a mapped read, aln[q] is exactly what awry_align_batch(metric, strands, k)
+ *             returns for the single hit `hit` of v = (q << strands) | strand (ops in rc(q) coordinates on strand 1);
+ *             for an unmapped read the "no alignment" record (distance k + 1, n_ops 0, text_len 0).
+ *   refused   an empty read, one with '$' / '#', with L <= k or with offsets outside the batch: the host call fails with
+ *             AWRY_ERR_INVALID_QUERY naming it; the device call latches it for awry_device_check and its record is
+ *             AWRY_MAP_UNMAPPED | AWRY_MAP_REFUSED (whatever the search made of its bytes).
+ *   errors    metric > 1, strands > 1, k > 3, a null pointer or a bad replica -> AWRY_ERR_INVALID_ARG; a protein index
+ *             or one without the unsampled suffix array and the text -> AWRY_ERR_UNSUPPORTED; a batch too large for one
+ *             approximate run -> the Hamming block's error; more than 2^31 hits within best + 1 in one batch ->
+ *             AWRY_ERR_NOMEM (split the batch).
+ *   device    outputs are the caller's (nq entries, sizes known up front): nothing to release.  awry_map_device
+ *             synchronises as the device locates do (the offsets read-back, the candidate total, the hit total within
+ *             the bound) and returns without waiting for its last kernels; results are bit for bit the host call's.
+ * Scheme (DESIGN.md §1h): the count pass of the locate gives each read's best distance; only hits within best + 1 are
+ * placed, sorted, filtered to loci (edit) and merged per read by one segmented sort; one thread per hit marks each
+ * start's first entry, a scan ranks the best ones, and one thread per read writes its record. */
+enum { AWRY_MAP_UNMAPPED = 1, AWRY_MAP_REFUSED = 2 };
+typedef struct awry_mapping {
+  awry_hit hit;      /* primary locus (seq_idx, local_pos); both ~0 when unmapped */
+  uint32_t n_best;   /* distinct starts at `distance` over the searched strands; 0 when unmapped */
+  uint32_t n_second; /* distinct starts at distance + 1; 0 when distance == k or unmapped */
+  uint8_t distance;  /* best; k + 1 when unmapped */
+  uint8_t strand;    /* 0: q, 1: rc(q) */
+  uint8_t mapq;
+  uint8_t flags;     /* AWRY_MAP_UNMAPPED (no locus <= k), AWRY_MAP_REFUSED (also unmapped) */
+  uint32_t pad;      /* 0 */
+} awry_mapping;
+typedef char awry_mapping_is_32_bytes[sizeof(awry_mapping) == 32 ? 1 : -1];
+/* mapq of a unique read with best < k, by min(n_second, 255) */
+#define AWRY_MAPQ_SECOND \
+  {37, 23, 20, 18, 17, 16, 15, 15, 14, 13, 13, 13, 12, 12, 12, 11, 11, 11, 10, 10, 10, 10, 10, 9, 9, 9, 9, 9, 9, 8, 8, 8,  \
+   8, 8, 8, 8, 7, 7, 7, 7, 7, 7, 7, 7, 7, 6, 6, 6, 6, 6, 6, 6, 6, 6, 6, 6, 6, 5, 5, 5, 5, 5, 5, 5,  \
+   5, 5, 5, 5, 5, 5, 5, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 3, 3, 3, 3, 3, 3,  \
+   3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2,  \
+   2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 2, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1,  \
+   1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,  \
+   0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,  \
+   0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0}
+int awry_map_batch(const awry_index *index, const uint8_t *qbytes, const uint64_t *qoff, uint64_t nq, uint32_t metric,
+                   uint32_t strands /* 0 or 1 */, uint32_t k, awry_mapping *out /* nq */,
+                   awry_alignment *aln /* NULL or nq */);
+int awry_map_device(const awry_index *index, int replica, const uint8_t *d_qbytes, const uint64_t *d_qoff, uint64_t nq,
+                    uint32_t metric, uint32_t strands, uint32_t k, awry_mapping *d_out /* nq */,
+                    awry_alignment *d_aln /* NULL or nq */, void *cuda_stream);
+
 /* ------------------------------------------------------------------ streaming reads-file front-end
  * SURVEY.md 8(f) rank 4.  The reference's users parse their reads on the CPU and pass `&str`s to
  * parallel_count / parallel_locate (fm_index.rs:455-487); these entry points take the FASTQ ('@') or

@@ -338,6 +338,22 @@ class FmIndex {
                            hits.data(), out.data()));
     return out;
   }
+  // Read mapping (no counterpart in the reference): each query's best locus within k under `metric`, over both strands
+  // or the query as given, with its uniqueness, mapping quality and (align) its alignment; second is empty unless align
+  std::pair<std::vector<awry_mapping>, std::vector<awry_alignment>> parallel_map(const std::vector<std::string_view>& queries,
+                                                                               uint32_t metric, uint32_t k,
+                                                                               bool strands = true,
+                                                                               bool align = true) const {
+    std::vector<uint8_t> bytes;
+    std::vector<uint64_t> off;
+    pack(queries, bytes, off);
+    std::pair<std::vector<awry_mapping>, std::vector<awry_alignment>> out;
+    out.first.resize(queries.size());
+    if (align) out.second.resize(queries.size());
+    check(awry_map_batch(h_, bytes.data(), off.data(), queries.size(), metric, strands ? 1 : 0, k, out.first.data(),
+                         align ? out.second.data() : nullptr));
+    return out;
+  }
   // the extended CIGAR (=, X, I, D) of one alignment of a query of length query_len, e.g. "47=1X102="
   static std::string cigar(const awry_alignment& a, uint32_t query_len) {
     size_t need = 0;

@@ -47,6 +47,23 @@ pub struct awry_alignment {
     pub ops: [awry_edit_op; 3],
 }
 
+pub const AWRY_MAP_UNMAPPED: u8 = 1;
+pub const AWRY_MAP_REFUSED: u8 = 2;
+
+/// the best locus of one read (include/awry_b200.h: awry_mapping, 32 bytes); hit is (~0, ~0) when unmapped
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default, PartialEq, Eq)]
+pub struct awry_mapping {
+    pub hit: awry_hit,
+    pub n_best: u32,
+    pub n_second: u32,
+    pub distance: u8,
+    pub strand: u8,
+    pub mapq: u8,
+    pub flags: u8,
+    pub pad: u32,
+}
+
 #[repr(C)]
 #[derive(Clone, Copy)]
 pub struct awry_info {
@@ -236,6 +253,11 @@ extern "C" {
                              n_hits: u64, d_out: *mut awry_alignment, cuda_stream: *mut c_void) -> c_int;
     pub fn awry_alignment_cigar(a: *const awry_alignment, query_len: u32, buf: *mut c_char, cap: usize,
                                 needed: *mut usize) -> c_int;
+    pub fn awry_map_batch(index: *const awry_index, qbytes: *const u8, qoff: *const u64, nq: u64, metric: u32,
+                          strands: u32, k: u32, out: *mut awry_mapping, aln: *mut awry_alignment) -> c_int;
+    pub fn awry_map_device(index: *const awry_index, replica: c_int, d_qbytes: *const u8, d_qoff: *const u64, nq: u64,
+                           metric: u32, strands: u32, k: u32, d_out: *mut awry_mapping, d_aln: *mut awry_alignment,
+                           cuda_stream: *mut c_void) -> c_int;
     pub fn awry_set_host_threads(n: c_int) -> c_int;
     pub fn awry_host_threads() -> c_int;
     pub fn awry_profile_enable(on: c_int) -> c_int;
